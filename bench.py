@@ -2,7 +2,7 @@
 """bench.py -- spin·steps/s of the fused Bloch simulation, forward + adjoint backward.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c4|c5|small]
-                    [--dtype f32|f64] [--scaling strong|weak] [--no-graph]
+                    [--dtype f32|f64] [--scaling strong|weak] [--no-graph] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic input (BASELINE.md / SURVEY.md 8d):
 ``M = spins.applypulse(pulse, loc_=..., Δf_=..., b1Map_=...)``; ``loss = ((M - target)**2).sum()``; ``loss.backward()``
@@ -20,6 +20,9 @@ loss and gradients back into pinned memory, all inside one wall-clock timed regi
 ``--impl reference`` times the UNMODIFIED reference (oracle/_ref, staged by oracle/Makefile: its own
 ``SpinCube.applypulse`` + ``backward`` through its own public API) on the host cores, on a bounded sub-cube of the same
 workload; without a staged copy it times the oracle port and says so (``cpu_baseline.kind``).
+
+``--dump-outputs DIR`` writes what the last timed step returned (M, rf.grad, gr.grad, loss) as ``DIR/<name>.npy``.  The
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -30,6 +33,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True        # the tree may be read-only: importing the package from it must not write there
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
@@ -164,6 +168,7 @@ class Problem:
     def __init__(self, workload, scaling, dtype, dev, rank, world):
         from mrphy import mobjs, parallel
         self.parallel = parallel
+        self.keep_M, self.M = False, None     # keep_M: hold on to the magnetisation of the latest step in self.M
         self.N, self.n, self.nT = WORKLOADS[workload]
         N, n, nT = self.N, self.n, self.nT
         self.dtype, self.dev, self.world = dtype, dev, world
@@ -204,6 +209,8 @@ class Problem:
     def local_step(self, sp=None, pulse=None, d=None):
         sp, pulse, d = (self.sp, self.pulse, self.d) if sp is None else (sp, pulse, d)
         M = sp.applypulse(pulse, loc_=d['loc'], Δf_=d['df'], b1Map_=d['b1'])
+        if self.keep_M:
+            self.M = M
         loss = ((M - self.tgt) ** 2).sum()
         loss.backward()
         return loss
@@ -223,13 +230,31 @@ def barrier(world):
     torch.cuda.synchronize()
 
 
-def timed_region(P, steps, flush, use_graph=True):
+DUMP_MAX_SPINS = 1 << 20       # M rows written by --dump-outputs: 12 MB in fp32, 25 MB in fp64
+
+
+def step_outputs(M, pulse, loss):
+    """What one step hands its caller, as host arrays in the working dtype: M (the magnetisation applypulse returns; shape
+    (N, nM, 3), or above DUMP_MAX_SPINS spins the rows of a fixed seeded sample of the flattened (N * nM, 3) spins, in
+    ascending order), rf.grad, gr.grad and the loss."""
+    M = M.detach()
+    if M.shape[0] * M.shape[1] > DUMP_MAX_SPINS:
+        M = M.reshape(-1, 3)
+        idx = torch.randperm(M.shape[0], generator=torch.Generator().manual_seed(0))[:DUMP_MAX_SPINS].sort().values
+        M = M[idx.to(M.device)]
+    return {'M': M.cpu().numpy(), 'rf_grad': pulse.rf.grad.cpu().numpy(), 'gr_grad': pulse.gr.grad.cpu().numpy(),
+            'loss': loss.detach().cpu().numpy()}
+
+
+def timed_region(P, steps, flush, use_graph=True, out=None):
     """-> (ms summed over `steps` steps, our kernel launches, launch mode).  The whole step -- pack, forward, loss,
     adjoint backward, finalize and (N > 1) the in-place all-reduce -- is recorded once into a CUDA graph and replayed;
-    if NCCL refuses the capture the all-reduce stays eager behind the replay; --no-graph times eager launches."""
+    if NCCL refuses the capture the all-reduce stays eager behind the replay; --no-graph times eager launches.
+    `out` (a dict) receives host copies of what the last timed step returned to its caller (see step_outputs)."""
     from mrphy import _cabi
     pulse, world = P.pulse, P.world
     graph, per_step, mode, g_loss = None, None, 'eager', None
+    P.keep_M = out is not None
     if use_graph:
         for with_comm, cmode in (((True, 'global'), (True, 'thread_local'), (False, 'global')) if world > 1 else ((False, 'global'),)):
             try:
@@ -277,6 +302,9 @@ def timed_region(P, steps, flush, use_graph=True):
     barrier(world)
     ms = sum(x.elapsed_time(y) for x, y in evs)
     n_launch = per_step * steps if graph is not None else _cabi.launch_counter - l0
+    if out is not None:
+        out.update(step_outputs(P.M, pulse, loss))
+    P.keep_M, P.M = False, None
     loss = float(loss)
     pulse.rf.grad = pulse.gr.grad = None
     del graph
@@ -488,9 +516,10 @@ def measure(workload, scaling, args, dev, rank, world, flush, full):
         P.pulse.rf.grad = P.pulse.gr.grad = None
         P.step()
     barrier(world)
-    ms_total, launches, mode, loss = timed_region(P, args.steps, flush, not args.no_graph)
+    outputs = {} if full and args.dump_outputs and rank == 0 else None
+    ms_total, launches, mode, loss = timed_region(P, args.steps, flush, not args.no_graph, outputs)
     res = {'ms_total': ms_total, 'launches': launches, 'mode': mode, 'loss': loss, 'nM': P.nM, 'N': P.N, 'nT': P.nT,
-           'policy': _ops.trig_policy() if dtype == torch.float32 else 'fp64'}
+           'policy': _ops.trig_policy() if dtype == torch.float32 else 'fp64', 'outputs': outputs}
     if full:
         pinned = {k: v.pin_memory() for k, v in P.host.items()}
         res['e2e'] = e2e_region(P, args.steps, flush, pinned)
@@ -552,6 +581,10 @@ def run_ours(args):
         sampler.start()
     r = measure(args.workload, scaling, args, dev, rank, world, flush, full=True)
     clocks = sampler.stop() if rank == 0 else None
+    if r['outputs'] is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in r['outputs'].items():
+            np.save(os.path.join(args.dump_outputs, name + '.npy'), a)
     c2 = None
     if args.workload != 'c2' and world == 1 and not args.no_extras:     # the 1-GPU configuration of BASELINE.json, same run
         c2 = measure('c2', 'weak', args, dev, rank, world, flush, full=False)
@@ -742,6 +775,13 @@ if __name__ == '__main__':
     ap.add_argument('--no-graph', action='store_true', help='time eager launches instead of a CUDA graph replay')
     ap.add_argument('--no-extras', action='store_true', help='skip the C2 leg and the CPU / eager reference legs')
     ap.add_argument('--ref-device', default='cpu', choices=['cpu', 'cuda'], help='(reference arm) where the reference runs')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step returned (M, rf_grad, gr_grad, loss; rank 0) as DIR/<name>.npy; '
+                         f'M of more than {DUMP_MAX_SPINS} spins is a fixed seeded sample of them')
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
+    if a.dump_outputs and a.impl != 'ours':
+        ap.error('--dump-outputs applies to --impl ours')
     a.warmup = max(a.warmup, 3) if a.impl == 'ours' else a.warmup
     (run_ours if a.impl == 'ours' else run_reference)(a)

@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define MRPHY_ABI_VERSION 5
+#define MRPHY_ABI_VERSION 6
 
 enum mrphy_dtype { MRPHY_F32 = 0, MRPHY_F64 = 1 };
 
@@ -244,6 +244,24 @@ int mrphy_design_waveform(const mrphy_reparam_args* a, void* cuda_stream);
 int mrphy_blochsim_fused_bwd_design(const mrphy_fused_args* a, int wave_is_packed, const mrphy_reparam_args* d,
                                     void* cuda_stream);
 
+/* Per-spin gradients of the fused backward: what the autograd of rfgr2beff gives upstream for loc, df, b1Map and gamma
+ * (beffective.py:137-167), without the dense field or dL/dBeff.  Each output is the sum over time that
+ * mrphy_rfgr2beff_spin_grads forms from dL/dBeff, with the same meaning and layout:
+ *   gloc (N,nM,3)     = sum_t gr[:,t] * gBz[t]                              (dL/dloc)
+ *   gsz  (N,nM)       = sum_t gBz[t]                                        (dL/ddf = gsz/gamma, dL/dgamma = -gsz*df/gamma^2)
+ *   gb1  (N,nM,2,nC)  = sum_t (rx_c gBx + ry_c gBy,  rx_c gBy - ry_c gBx)    (dL/db1Map; requires a->b1)
+ * contiguous, any of them NULL = not wanted (not all three).  Everything else as mrphy_blochsim_fused_bwd, whose results
+ * (gMi, grf, ggr) are bitwise those of a call without per-spin gradients.  With MRPHY_SKIP_GRF | MRPHY_SKIP_GGR (a fixed
+ * pulse) the backward forms no spin reduction and skips the finalize launch.  No workspace beyond
+ * mrphy_fused_partial_elems().                                                                                        */
+typedef struct mrphy_spin_grad_args {
+  void* gloc;  /* out (N,nM,3) contiguous, or NULL */
+  void* gsz;   /* out (N,nM)   contiguous, or NULL */
+  void* gb1;   /* out (N,nM,2,nC) contiguous, or NULL (requires a->b1) */
+} mrphy_spin_grad_args;
+int mrphy_blochsim_fused_bwd_spin(const mrphy_fused_args* a, int wave_is_packed, const mrphy_spin_grad_args* s,
+                                  void* cuda_stream);
+
 /* Amplitude limits of the design loop (SURVEY 8f-2), replacing utils.rfclamp (utils.py:217-236) and utils.sclamp
  * (utils.py:278-293) and their autograd, one launch each way:
  *   kind 1  rf (N,2,nT,nC):  out = rf * min((rfmax[n,c] - eps) / |rf|, 1),  |rf| over the xy axis
@@ -278,8 +296,8 @@ int mrphy_mask_copy(const mrphy_mask_args* a, void* cuda_stream);
 
 /* sizeof() of the argument structs as this library was compiled, for bindings to check their mirror of the layout:
  * which = 0 mrphy_param, 1 mrphy_fused_args, 2 mrphy_beff_args, 3 mrphy_rfgr2beff_args, 4 mrphy_beff2ab_args,
- * 5 mrphy_beff2uphi_args, 6 mrphy_freeprec_args, 7 mrphy_reparam_args, 8 mrphy_mask_args, 9 mrphy_clamp_args; 0 for any
- * other value. */
+ * 5 mrphy_beff2uphi_args, 6 mrphy_freeprec_args, 7 mrphy_reparam_args, 8 mrphy_mask_args, 9 mrphy_clamp_args,
+ * 10 mrphy_spin_grad_args; 0 for any other value. */
 size_t mrphy_sizeof_args(int which);
 
 /* Number of kernel launches the last forward / backward call on this thread issued. */

@@ -8,6 +8,7 @@
 //   fused_fwd_kernel<T,..>    one spin, or two spins packed in an f2 (FFMA2), per thread; checkpoint every K steps
 //   fused_bwd_kernel<T,..>    time-reversed state reconstruction + adjoint + spin reduction (only the gradient rows
 //                             asked for: ROWS); tiles owned through SM-aware virtual CTA ids (SCHED_*)
+//                             SG: also the per-spin sums over time behind dL/dloc, dL/ddf, dL/db1Map (sg_fold)
 //   grad_finalize_kernel<T>   deterministic sum of the per-CTA partials, reference layout out (grad_finalize.cuh)
 //
 // Data layout in HBM (T = float | double):
@@ -158,6 +159,12 @@ template <typename T> struct KArgs {
   int* sched;          // SM-aware tile ownership of the backward (null: CTA b owns tiles b, b+P, ...), see SCHED_* below
   int n_sm, c_per_sm;
   int* done;           // finished-CTA counters of grad_finalize_design_kernel, one per batch entry (null: no design tail); zeroed here
+};
+// per-spin gradient outputs of the SG backward (mrphy_spin_grad_args; each may be null).  A kernel parameter of its own behind
+// the others, so that the kernels without per-spin gradients keep their parameter offsets.
+template <typename T> struct SgOut {
+  T* gloc; T* gsz; T* gb1;
+  bool any() const { return gloc || gsz || gb1; }
 };
 
 // Scheduling workspace of the backward kernel (ints, zeroed before every launch; lives behind the partial sums).
@@ -493,12 +500,64 @@ __device__ __forceinline__ void warp_tile_reduce_weighted(const unsigned char* f
   }
 }
 
+// Per-spin gradients of the SG backward, in the reference's terms (mrphy_rfgr2beff_spin_grads) with G = dL/dBeff = -g F,
+// g = 2 pi gamma dt:  gloc = sum_t gr(t) G_z,  gsz = sum_t G_z,  gb1_c = sum_t conj(rx_c + i ry_c) (G_x + i G_y).
+// A thread sums F over the steps of one staged chunk in registers, acc = [sum gr F_z (3) | sum F_z | Re_c (NC) | Im_c (NC)],
+// and folds that chunk sum into the outputs at the chunk's end -- a two-level sum over time that adds nothing per step.  The
+// outputs belong to the thread that owns the spin: a plain read-modify-write.  The chunk processed first (time runs
+// backwards) stores; the last one (c == 0) also scales by -g and, single coil, turns the frame sums back to the lab frame
+// (the spin's own frame is the lab frame turned by arg b1: G_lab = e^{i arg b1} G_frame, bloch_math.cuh: make_consts).
+template <typename T, typename V, int NC, int PK>
+__device__ __forceinline__ void sg_fold(const KArgs<T>& a, const SgOut<T>& o, int n, const int (&idx)[PK], const bool (&ok)[PK], bool first,
+                                        bool last, const SpinConst<V, NC>& k, const V (&acc)[4 + 2 * NC]) {
+  constexpr int NA = 4 + 2 * NC;
+#pragma unroll
+  for (int q = 0; q < PK; ++q) {
+    if (!ok[q]) continue;
+    const size_t s = (size_t)n * a.nM + idx[q];
+    T v[NA];
+#pragma unroll
+    for (int w = 0; w < NA; ++w) v[w] = q == 0 ? getq<0>(acc[w]) : getq<1>(acc[w]);
+    T* const pl = o.gloc ? o.gloc + s * 3 : nullptr;
+    T* const pz = o.gsz ? o.gsz + s : nullptr;
+    T* const pb = o.gb1 ? o.gb1 + s * 2 * a.nC : nullptr;
+    if (!first) {
+      if (pl) { v[0] += pl[0]; v[1] += pl[1]; v[2] += pl[2]; }
+      if (pz) v[3] += pz[0];
+      if (pb) {
+#pragma unroll
+        for (int c = 0; c < NC; ++c)
+          if (c < a.nC) { v[4 + c] += pb[c]; v[4 + NC + c] += pb[a.nC + c]; }
+      }
+    }
+    if (last) {
+      const T ng = (T)(-6.283185307179586476925286766559 * ld_param(a.gamma, n, idx[q]) * ld_param(a.dt, n, 0));
+#pragma unroll
+      for (int w = 0; w < NA; ++w) v[w] *= ng;
+      if (NC == 1) {   // frame -> lab: (re + i im) * (fc + i fs)
+        const T fc = q == 0 ? getq<0>(k.fc) : getq<1>(k.fc), fs = q == 0 ? getq<0>(k.fs) : getq<1>(k.fs);
+        const T re = v[4], im = v[5];
+        v[4] = fnma_(fs, im, fc * re);
+        v[5] = fma_(fs, re, fc * im);
+      }
+    }
+    if (pl) { pl[0] = v[0]; pl[1] = v[1]; pl[2] = v[2]; }
+    if (pz) pz[0] = v[3];
+    if (pb) {
+#pragma unroll
+      for (int c = 0; c < NC; ++c)
+        if (c < a.nC) { pb[c] = v[4 + c]; pb[a.nC + c] = v[4 + NC + c]; }
+    }
+  }
+}
+
 // ------------------------------------------------------------------------------------------
 // backward
 // ROWS: which gradients the caller wants -- bit 0 dL/drf (rows [0, 2 NC)), bit 1 dL/dgr (rows [2 NC, W)); the other rows
 // of the spin reduction are neither formed nor reduced (an RF-only design skips 3 of its 5 rows).
-template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, int ROWS = 3>
-__global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : (sizeof(T) == 8 && NC == 1 ? 4 : (sizeof(T) == 4 && NC > 1 ? MRPHY_MC_MINB : 1)))) fused_bwd_kernel(const KArgs<T> a, const int need_gmi) {
+// SG: also the per-spin gradients (sg_fold).  ROWS == 0 (SG only, a fixed pulse): no transposition tile, no partial sums.
+template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, int ROWS = 3, bool SG = false>
+__global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : (sizeof(T) == 8 && NC == 1 ? 4 : (sizeof(T) == 4 && NC > 1 ? MRPHY_MC_MINB : 1)))) fused_bwd_kernel(const KArgs<T> a, const int need_gmi, const SgOut<T> sgo) {
   typedef typename Pack<T, PK>::type V;
   using L = BwdSmem<T, NC, BLKT, PK>;
   constexpr int W = L::W, TR = L::TR, NW = L::NW;
@@ -556,7 +615,8 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : 
     const uint32_t total = it + (uint32_t)my_tiles * (uint32_t)nChunks;   // `it` once this id's last chunk is consumed
     T* part = a.partials + ((size_t)n * a.P + vid) * W * (size_t)nT;
     if (my_tiles == 0) {   // an id without work still owns a partial slot: zero it
-      for (int e = tid; e < W * nT; e += BLKT) part[e] = (T)0;
+      if constexpr (ROWS != 0)
+        for (int e = tid; e < W * nT; e += BLKT) part[e] = (T)0;
     } else if (tid == 0) {
       mbar_arrive_expect_tx(&full[it & 1], chunk_bytes);
       bulk_g2s(wbuf[it & 1], wave_n + (size_t)(nChunks - 1) * WS * TCP, chunk_bytes, &full[it & 1]);
@@ -582,7 +642,7 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : 
     load_vec3_tile<T, V, PK, BLKT>(a.gMo + (int64_t)n * a.gMo_sn, a.gMo_sm, tile, nM, idx, scr, hx, hy, hz);
     to_frame(k, mx, my);   // Mo and dL/dMo enter the spin's transverse frame, dL/dMi leaves it (single coil)
     to_frame(k, hx, hy);
-    if constexpr (WRED) {   // this spin's weights for the reduce phase (the previous tile's last reduce ended with a CTA barrier)
+    if constexpr (WRED && ROWS != 0) {   // this spin's weights for the reduce phase (the previous tile's last reduce ended with a CTA barrier)
       T* wrow = wt + (size_t)lane * L::WP;
 #pragma unroll
       for (int q = 0; q < NC; ++q) { wrow[q] = lane0(k.cbr[q]); wrow[NC + q] = lane0(k.cbi[q]); }
@@ -614,6 +674,11 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : 
       mbar_wait(&full[it & 1], (it >> 1) & 1);
       const T* wb = wbuf[it & 1];
       const int ns = min(K, nT - c * K);
+      V sacc[SG ? 4 + 2 * NC : 1];   // SG: this chunk's per-spin sums (sg_fold)
+      if constexpr (SG) {
+#pragma unroll
+        for (int w = 0; w < 4 + 2 * NC; ++w) sacc[w] = V(0.0f);
+      }
       // one adjoint step; the W per-thread gradient contributions go to row `row` of the warp's tile
       auto one_step = [&](const T (&s)[W], int row) {
         V rx[NC], ry[NC], bx, by, bz, Fx, Fy, Fz;
@@ -621,6 +686,18 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : 
         for (int q = 0; q < NC; ++q) { rx[q] = V(s[q]); ry[q] = V(s[NC + q]); }
         field<V, NC>(k, rx, ry, V(s[2 * NC]), V(s[2 * NC + 1]), V(s[2 * NC + 2]), bx, by, bz);
         step_bwd<V, POL, RELAX, NC>(k, bx, by, bz, mx, my, mz, hx, hy, hz, Fx, Fy, Fz);
+        if constexpr (SG) {
+          sacc[0] = fma_(V(s[2 * NC]), Fz, sacc[0]);
+          sacc[1] = fma_(V(s[2 * NC + 1]), Fz, sacc[1]);
+          sacc[2] = fma_(V(s[2 * NC + 2]), Fz, sacc[2]);
+          sacc[3] = sacc[3] + Fz;
+#pragma unroll
+          for (int q = 0; q < NC; ++q) {
+            sacc[4 + q] = fma_(rx[q], Fx, fma_(ry[q], Fy, sacc[4 + q]));
+            sacc[4 + NC + q] = fma_(rx[q], Fy, fnma_(ry[q], Fx, sacc[4 + NC + q]));
+          }
+        }
+        if constexpr (ROWS == 0) return;
         if constexpr (WRED) {   // multi-coil: only F goes to the tile; the weights are applied in the reduce phase
           T fv[4] = {lane0(Fx), lane0(Fy), lane0(Fz), (T)0};
           float4* dst = reinterpret_cast<float4*>(ft + ((size_t)lane * L::P16 + (size_t)row * L::E16) * 16);
@@ -668,6 +745,7 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : 
             one_step(s, j - j0);
           }
         }
+        if constexpr (ROWS != 0) {
         __syncwarp();
         T(*ctab)[W][TR] = cta + (size_t)(red_par & 1) * NW;   // this tile's half of the double buffer
         if constexpr (WRED) warp_tile_reduce_weighted<T, NC, TR, W0, W1>(ft, wt, lane, ctab[warp]);
@@ -686,8 +764,11 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : 
           }
         }
         ++red_par;
+        }
         j1 = j0;
       }
+      if constexpr (SG) sg_fold<T, V, NC, PK>(a, sgo, n, idx, ok, c == nChunks - 1, c == 0, k, sacc);
+      if constexpr (ROWS == 0) __syncthreads();   // (else the reduce's barrier) everyone is done with wbuf[it&1] before it is refilled
       if (c > 0) {   // resynchronise the reconstructed state with the forward checkpoint
         mx = kx; my = ky; mz = kz;
       }
@@ -1326,10 +1407,10 @@ int launch_fwd_s(KArgs<T> k, const Plan& p, cudaStream_t st) {
   CK(cudaGetLastError());
   return MRPHY_OK;
 }
-template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, int ROWS = 3>
-int launch_bwd_s(KArgs<T> k, const Plan& p, int need_gmi, cudaStream_t st) {
+template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, int ROWS = 3, bool SG = false>
+int launch_bwd_s(KArgs<T> k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg = SgOut<T>{}) {
   constexpr size_t smem = BwdSmem<T, NC, BLKT, PK>::bytes;
-  auto kern = fused_bwd_kernel<T, POL, RELAX, NC, PK, BLKT, ROWS>;
+  auto kern = fused_bwd_kernel<T, POL, RELAX, NC, PK, BLKT, ROWS, SG>;
   CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   // static + dynamic may exceed 48 KB
   int occ = 0;
   CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, BLKT, smem));
@@ -1350,11 +1431,11 @@ int launch_bwd_s(KArgs<T> k, const Plan& p, int need_gmi, cudaStream_t st) {
     CK(cudaMemsetAsync(k.sched, 0, sizeof(int) * (size_t)(SCHED_CLAIM + k.P), st));
   }
   if (getenv("MRPHY_B200_DEBUG"))
-    fprintf(stderr, "[mrphy_b200] fused_bwd<%s,NC=%d,PK=%d,BLK=%d,%s> grid=(%d,%d) tiles=%d occ=%d smem=%zu K=%d\n",
-            sizeof(T) == 4 ? "f32" : "f64", NC, PK, BLKT, POL == TRIG_PRECISE ? "precise" : "fast", k.P, k.N, q.tiles, occ,
-            smem, p.K);
+    fprintf(stderr, "[mrphy_b200] fused_bwd<%s,NC=%d,PK=%d,BLK=%d,%s,ROWS=%d,SG=%d> grid=(%d,%d) tiles=%d occ=%d smem=%zu K=%d\n",
+            sizeof(T) == 4 ? "f32" : "f64", NC, PK, BLKT, POL == TRIG_PRECISE ? "precise" : "fast", ROWS, (int)SG, k.P, k.N,
+            q.tiles, occ, smem, p.K);
   timing_begin(st);
-  kern<<<grid, BLKT, smem, st>>>(k, need_gmi);
+  kern<<<grid, BLKT, smem, st>>>(k, need_gmi, sg);
   timing_end(st);
   ++g_launches;
   CK(cudaGetLastError());
@@ -1415,17 +1496,26 @@ int launch_fwd_tc(const KArgs<float>& k, const Plan& p, cudaStream_t st) {
 #endif
   return launch_fwd_tc_pk<POL, RELAX, NC, 2>(k, p, st);
 }
+// backward with per-spin gradients: the ROWS == 0 kernel when no waveform gradient is wanted, else all rows (the finalize
+// reads only the wanted ones)
 template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT>
-int launch_any(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaStream_t st) {
+int launch_bwd_sg(const KArgs<T>& k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg) {
+  return p.rows == 0 ? launch_bwd_s<T, POL, RELAX, NC, PK, BLKT, 0, true>(k, p, need_gmi, st, sg)
+                     : launch_bwd_s<T, POL, RELAX, NC, PK, BLKT, 3, true>(k, p, need_gmi, st, sg);
+}
+template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT>
+int launch_any(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg) {
+  if (bwd && sg.any()) return launch_bwd_sg<T, POL, RELAX, NC, PK, BLKT>(k, p, need_gmi, st, sg);
   return bwd ? launch_bwd_s<T, POL, RELAX, NC, PK, BLKT>(k, p, need_gmi, st)
              : launch_fwd_s<T, POL, RELAX, NC, PK, BLKT>(k, p, st);
 }
 
 template <typename T, int POL, bool RELAX>
-int dispatch_nc(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaStream_t st) {
+int dispatch_nc(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg) {
   if constexpr (sizeof(T) == 4) {
     if (p.PK == 2) {
       if (!bwd) return launch_fwd_s<T, POL, RELAX, 1, 2, 64>(k, p, st);
+      if (sg.any()) return launch_bwd_sg<T, POL, RELAX, 1, 2, MRPHY_BWD_BLKT>(k, p, need_gmi, st, sg);
       if (p.rows == 1) return launch_bwd_s<T, POL, RELAX, 1, 2, MRPHY_BWD_BLKT, 1>(k, p, need_gmi, st);   // dL/drf only
       if (p.rows == 2) return launch_bwd_s<T, POL, RELAX, 1, 2, MRPHY_BWD_BLKT, 2>(k, p, need_gmi, st);   // dL/dgr only
       return launch_bwd_s<T, POL, RELAX, 1, 2, MRPHY_BWD_BLKT>(k, p, need_gmi, st);
@@ -1439,6 +1529,7 @@ int dispatch_nc(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaSt
     if (p.NC == 2 && env_int("MRPHY_B200_NC2_PACK", 2) == 2) {
       if (!bwd) return launch_fwd_s<T, POL, RELAX, 2, 2, 64>(k, p, st);
       if (env_int("MRPHY_B200_NC2_PACK_BWD", 2) == 2) {
+        if (sg.any()) return launch_bwd_sg<T, POL, RELAX, 2, 2, MRPHY_BWD_BLKT>(k, p, need_gmi, st, sg);
         if (p.rows == 1) return launch_bwd_s<T, POL, RELAX, 2, 2, MRPHY_BWD_BLKT, 1>(k, p, need_gmi, st);
         if (p.rows == 2) return launch_bwd_s<T, POL, RELAX, 2, 2, MRPHY_BWD_BLKT, 2>(k, p, need_gmi, st);
         return launch_bwd_s<T, POL, RELAX, 2, 2, MRPHY_BWD_BLKT>(k, p, need_gmi, st);
@@ -1456,29 +1547,31 @@ int dispatch_nc(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaSt
       if constexpr (sizeof(T) == 4) return fail(MRPHY_ERR_ARG, "internal: fp32 single-coil scalar kernels not built%s");
       else
 #endif
-      return launch_any<T, POL, RELAX, 1, 1, 128>(bwd, k, p, need_gmi, st);
-    case 2: return launch_any<T, POL, RELAX, 2, 1, 128>(bwd, k, p, need_gmi, st);
-    case 4: return launch_any<T, POL, RELAX, 4, 1, 128>(bwd, k, p, need_gmi, st);
-    case 8: return launch_any<T, POL, RELAX, 8, 1, 128>(bwd, k, p, need_gmi, st);
-    case 16: return launch_any<T, POL, RELAX, 16, 1, 128>(bwd, k, p, need_gmi, st);
+      return launch_any<T, POL, RELAX, 1, 1, 128>(bwd, k, p, need_gmi, st, sg);
+    case 2: return launch_any<T, POL, RELAX, 2, 1, 128>(bwd, k, p, need_gmi, st, sg);
+    case 4: return launch_any<T, POL, RELAX, 4, 1, 128>(bwd, k, p, need_gmi, st, sg);
+    case 8: return launch_any<T, POL, RELAX, 8, 1, 128>(bwd, k, p, need_gmi, st, sg);
+    case 16: return launch_any<T, POL, RELAX, 16, 1, 128>(bwd, k, p, need_gmi, st, sg);
   }
   return fail(MRPHY_ERR_ARG, "internal: bad NC%s");
 #endif
 }
 
 template <typename T>
-int dispatch(bool bwd, const mrphy_fused_args* a, const Plan& p, cudaStream_t st, int* done = nullptr) {
+int dispatch(bool bwd, const mrphy_fused_args* a, const Plan& p, cudaStream_t st, int* done = nullptr,
+             const mrphy_spin_grad_args* sg = nullptr) {
   KArgs<T> k = make_kargs<T>(a, p);
   k.done = done;
+  const SgOut<T> so = sg ? SgOut<T>{(T*)sg->gloc, (T*)sg->gsz, (T*)sg->gb1} : SgOut<T>{};
   const bool relax = a->T1.ptr != nullptr;
   const bool precise = (a->flags & MRPHY_TRIG_PRECISE) != 0 && sizeof(T) == 4 && !(bwd && (a->flags & MRPHY_TRIG_FAST_BWD));
   const int need_gmi = (a->flags & MRPHY_NEED_GMI) ? 1 : 0;
   if (precise) {
-    return relax ? dispatch_nc<T, TRIG_PRECISE, true>(bwd, k, p, need_gmi, st)
-                 : dispatch_nc<T, TRIG_PRECISE, false>(bwd, k, p, need_gmi, st);
+    return relax ? dispatch_nc<T, TRIG_PRECISE, true>(bwd, k, p, need_gmi, st, so)
+                 : dispatch_nc<T, TRIG_PRECISE, false>(bwd, k, p, need_gmi, st, so);
   }
-  return relax ? dispatch_nc<T, TRIG_FAST, true>(bwd, k, p, need_gmi, st)
-               : dispatch_nc<T, TRIG_FAST, false>(bwd, k, p, need_gmi, st);
+  return relax ? dispatch_nc<T, TRIG_FAST, true>(bwd, k, p, need_gmi, st, so)
+               : dispatch_nc<T, TRIG_FAST, false>(bwd, k, p, need_gmi, st, so);
 }
 
 template <typename T>
@@ -1510,17 +1603,21 @@ int check_design(const mrphy_fused_args* a, const mrphy_reparam_args* d) {
 }
 
 template <typename T>
-int run_bwd(const mrphy_fused_args* a, int wave_is_packed, const mrphy_reparam_args* d, cudaStream_t st) {
+int run_bwd(const mrphy_fused_args* a, int wave_is_packed, const mrphy_reparam_args* d, cudaStream_t st,
+            const mrphy_spin_grad_args* sg = nullptr) {
   Plan p;
   int rc = make_plan(a, &p, true);
   if (rc) return rc;
   if ((rc = check_common<T>(a, true))) return rc;
   if (d && (rc = check_design(a, d))) return rc;
+  if (sg && !sg->gloc && !sg->gsz && !sg->gb1) return fail(MRPHY_ERR_ARG, "spin gradients: gloc, gsz, gb1 are all null%s");
+  if (sg && sg->gb1 && !a->b1) return fail(MRPHY_ERR_ARG, "spin gradients: gb1 needs b1%s");
   // (after a tensor-core forward `wave` holds that kernel's operand tiles: the backward stages its own layout over them)
   if ((!wave_is_packed || p.tc) && (rc = launch_pack<T>(a, p, st))) return rc;
   // finished-CTA counters of the design tail: behind the scheduling ints, zeroed by the backward kernel itself
   int* const done = d ? reinterpret_cast<int*>((T*)a->partials + (size_t)a->N * p.Pmax * p.W * (size_t)a->nT) + SCHED_CLAIM + p.Pmax : nullptr;
-  if ((rc = dispatch<T>(true, a, p, st, done))) return rc;
+  if ((rc = dispatch<T>(true, a, p, st, done, sg))) return rc;
+  if (sg && p.rows == 0) return MRPHY_OK;   // per-spin gradients only: nothing to finalize
   dim3 grid((a->nT + 31) / 32, p.W, a->N), block(32, 32);
   const int coil_dim = (a->flags & MRPHY_RF_COIL_DIM) ? 1 : 0;
   const int w_lo = (p.rows & 1) ? 0 : 2 * p.NC, w_hi = (p.rows & 2) ? p.W : 2 * p.NC;
@@ -1565,4 +1662,14 @@ extern "C" int mrphy_blochsim_fused_bwd_design(const mrphy_fused_args* a, int wa
   if (!a || !d) return fail(MRPHY_ERR_ARG, "null args%s");
   cudaStream_t st = (cudaStream_t)cuda_stream;
   return a->dtype == MRPHY_F64 ? run_bwd<double>(a, wave_is_packed, d, st) : run_bwd<float>(a, wave_is_packed, d, st);
+}
+
+extern "C" int mrphy_blochsim_fused_bwd_spin(const mrphy_fused_args* a, int wave_is_packed, const mrphy_spin_grad_args* s,
+                                             void* cuda_stream) {
+  g_launches = 0;
+  g_err[0] = 0;
+  if (!a || !s) return fail(MRPHY_ERR_ARG, "null args%s");
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  return a->dtype == MRPHY_F64 ? run_bwd<double>(a, wave_is_packed, nullptr, st, s)
+                               : run_bwd<float>(a, wave_is_packed, nullptr, st, s);
 }

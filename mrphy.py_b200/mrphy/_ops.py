@@ -166,9 +166,10 @@ def _fake_blochsim_fused_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flag
             Mi.new_empty((N * chunks * chunk,)))
 
 
-def _fused_bwd_call(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, design=None):
+def _fused_bwd_call(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, design=None, spin=None):
     """The backward launch sequence; `design` = (rho, theta, rfmax, ts, smax, ddt, rf_kind, gr_kind) adds the adjoint of the
-    re-parametrisation to the gradient epilogue (mrphy_blochsim_fused_bwd_design).  -> (gMi, flat, grho, gtheta, gts)."""
+    re-parametrisation to the gradient epilogue (mrphy_blochsim_fused_bwd_design), `spin` = (want_loc, want_sz, want_b1) the
+    per-spin gradients (mrphy_blochsim_fused_bwd_spin).  -> (gMi, flat, grho, gtheta, gts) | (gMi, flat, gloc, gsz, gb1)."""
     L = _cabi.lib()
     a = _cabi.FusedArgs()
     _fill_common(a, None, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags)
@@ -193,6 +194,17 @@ def _fused_bwd_call(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt,
     a.gMi, a.grf, a.ggr, a.partials = (gMi.data_ptr() if need_gmi else None), (grf.data_ptr() if want_rf else None), \
         (ggr.data_ptr() if want_gr else None), partials.data_ptr()
     grho = gtheta = gts = flat[:0]
+    if spin is not None:
+        want_loc, want_sz, want_b1 = spin
+        e = lambda shape, on: torch.empty(shape if on else (0,), **kw)
+        gloc, gsz, gb1 = e((a.N, a.nM, 3), want_loc), e((a.N, a.nM), want_sz), e((a.N, a.nM, 2, a.nC), want_b1)
+        s = _cabi.SpinGradArgs()
+        s.gloc, s.gsz, s.gb1 = (gloc.data_ptr() if want_loc else None), (gsz.data_ptr() if want_sz else None), \
+            (gb1.data_ptr() if want_b1 else None)
+        with torch.cuda.device(Mo.device):
+            _cabi.check(L.mrphy_blochsim_fused_bwd_spin(a, 1, s, _stream()), 'blochsim_fused_bwd_spin')
+        _cabi.count_launches()
+        return gMi, flat, gloc, gsz, gb1
     if design is None:
         with torch.cuda.device(Mo.device):
             _cabi.check(L.mrphy_blochsim_fused_bwd(a, 1, _stream()), 'blochsim_fused_bwd')
@@ -230,6 +242,24 @@ def _impl_blochsim_fused_bwd_design(gMo: Tensor, Mo: Tensor, ckpt: Tensor, wave:
                            (rho, theta, rfmax, ts, smax, ddt, rf_kind, gr_kind))
 
 
+def _impl_blochsim_fused_bwd_spin(gMo: Tensor, Mo: Tensor, ckpt: Tensor, wave: Tensor, rf: Tensor, gr: Tensor, loc: Tensor,
+                                  df: Optional[Tensor], b1: Optional[Tensor], T1: Optional[Tensor], T2: Optional[Tensor],
+                                  gamma: Tensor, dt: Tensor, K: int, flags: int, want_loc: bool, want_sz: bool, want_b1: bool):
+    """As blochsim_fused_bwd, plus the per-spin sums over time of dL/dBeff (empty where not wanted): gloc (N,nM,3) =
+    sum_t gr*gBz, gsz (N,nM) = sum_t gBz, gb1 (N,nM,2,nC) -- the outputs of rfgr2beff_spin_grads, formed inside the backward
+    kernel without the dense field.  want_b1 needs b1."""
+    return _fused_bwd_call(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags,
+                           spin=(bool(want_loc), bool(want_sz), bool(want_b1)))
+
+
+def _fake_blochsim_fused_bwd_spin(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, want_loc, want_sz,
+                                  want_b1):
+    gMi, flat = _fake_blochsim_fused_bwd(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags)
+    N, nM, nC = loc.shape[0], loc.shape[1], (rf.shape[3] if rf.ndim == 4 else 1)
+    e = lambda shape, on: Mo.new_empty(shape if on else (0,))
+    return gMi, flat, e((N, nM, 3), want_loc), e((N, nM), want_sz), e((N, nM, 2, nC), want_b1)
+
+
 def _fake_blochsim_fused_bwd_design(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, rho, theta, rfmax,
                                     ts, smax, ddt, rf_kind, gr_kind):
     gMi, flat = _fake_blochsim_fused_bwd(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags)
@@ -261,12 +291,29 @@ def _fused_setup(ctx, inputs, output):
     ctx.save_for_backward(Mo, ckpt, wave, rf, gr, loc, gamma, dt, *[x for x in (df, b1, T1, T2) if x is not None])
 
 
+def _param_2d(x: Tensor) -> Tensor:
+    """A per-spin constant viewed the way `_param` reads it: (N|1, nM|1) from that, (N|1,) per batch entry, () or trailing
+    singleton dims."""
+    v = x
+    while v.ndim > 2 and v.shape[-1] == 1:
+        v = v[..., 0]
+    return v.reshape(1, 1) if v.ndim == 0 else (v[:, None] if v.ndim == 1 else v)
+
+
+def _as_param_grad(g: Tensor, x: Tensor) -> Tensor:
+    """A per-spin gradient (N,nM) reduced to the shape and dtype of the op input `x` (see `_param_2d`)."""
+    return g.sum_to_size(_param_2d(x).shape).reshape(x.shape).to(x.dtype)
+
+
 def _fused_backward(ctx, gMo, _gckpt, _gwave):
     Mo, ckpt, wave, rf, gr, loc, gamma, dt, *opt = ctx.saved_tensors
     opt = list(opt)
     df, b1, T1, T2 = (opt.pop(0) if h else None for h in ctx.has)
     need = ctx.needs_input_grad
-    if not any(need[0:3]):
+    # per-spin gradients (inputs loc, df, b1, gamma): γ reaches the loss only through Bz += df/γ, so without df it has none
+    want_loc, want_b1 = bool(need[3]), bool(need[5] and b1 is not None)
+    want_sz = df is not None and bool(need[4] or need[8])
+    if not (any(need[0:3]) or want_loc or want_sz or want_b1):
         return (None,) * 12
     if gMo is None:
         gMo = torch.zeros_like(Mo)
@@ -275,9 +322,22 @@ def _fused_backward(ctx, gMo, _gckpt, _gwave):
     # only the gradients autograd asks for: the rows of the spin reduction of the others are not even formed
     flags = ctx.flags | (_cabi.FLAG_NEED_GMI if need[0] else 0) | (0 if need[1] else _cabi.FLAG_SKIP_GRF) | \
         (0 if need[2] else _cabi.FLAG_SKIP_GGR)
-    gMi, flat = blochsim_fused_bwd(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, ctx.K, flags)
+    if not (want_loc or want_sz or want_b1):
+        gMi, flat = blochsim_fused_bwd(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, ctx.K, flags)
+        grf, ggr = split_wave_grads(flat, rf, flags)
+        return (gMi if need[0] else None, grf, ggr) + (None,) * 9
+    gMi, flat, gloc, gsz, gb1 = blochsim_fused_bwd_spin(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, ctx.K,
+                                                        flags, want_loc, want_sz, want_b1)
     grf, ggr = split_wave_grads(flat, rf, flags)
-    return (gMi if need[0] else None, grf, ggr) + (None,) * 9
+    gdf = ggam = None
+    if want_sz:     # ∂Δf = gsz/γ, ∂γ = -gsz·Δf/γ² (the chain rule of Bz += Δf/γ, beffective.py:142)
+        gam2, df2 = _param_2d(gamma), _param_2d(df)
+        if need[4]:
+            gdf = _as_param_grad(gsz / gam2, df)
+        if need[8]:
+            ggam = _as_param_grad(-gsz * df2 / (gam2 * gam2), gamma)
+    return (gMi if need[0] else None, grf, ggr, gloc if want_loc else None, gdf, gb1 if want_b1 else None,
+            None, None, ggam, None, None, None)
 
 
 
@@ -719,7 +779,7 @@ def _mask_backward(ctx, g):
 # registration: raw torch.library definitions (schema + CUDA impl + fake), which cost ~20 us per call instead of
 # the ~130 us of the `torch.library.custom_op` convenience wrapper -- it matters for test-scale problems
 _LIB = torch.library.Library('mrphy_b200', 'DEF')
-_SCHEMAS = {'blochsim_fused_fwd': '(Tensor Mi, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor, Tensor)', 'blochsim_fused_bwd': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'blochsim_fused_bwd_design': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? ddt, int rf_kind, int gr_kind) -> (Tensor, Tensor, Tensor, Tensor, Tensor)', 'blochsim_beff_fwd': '(Tensor Mi, Tensor Beff, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'blochsim_beff_bwd': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor Beff, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'rfgr2beff': '(Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor gamma) -> Tensor', 'rfgr2beff_bwd': '(Tensor gB, Tensor rf, Tensor gr, Tensor loc, Tensor? b1) -> (Tensor, Tensor)', 'rfgr2beff_spin_grads': '(Tensor gB, Tensor rf, Tensor gr, bool want_loc, bool want_b1) -> (Tensor, Tensor, Tensor)', 'beff2ab': '(Tensor beff, Tensor E1, Tensor E2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor, Tensor)', 'beff2ab_bwd': '(Tensor gA, Tensor gB, Tensor A, Tensor B, Tensor ckpt, Tensor beff, Tensor E1, Tensor E2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'beff2uphi': '(Tensor beff, Tensor g) -> (Tensor, Tensor)', 'beff2uphi_bwd': '(Tensor? gU, Tensor? gPhi, Tensor beff, Tensor g) -> (Tensor, Tensor)', 'freeprec': '(Tensor Mi, Tensor dur, Tensor? T1, Tensor? T2, Tensor? df, bool adjoint) -> Tensor', 'design_waveform': '(Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? dt, int rf_kind, int gr_kind) -> (Tensor, Tensor)', 'design_waveform_bwd': '(Tensor? grf, Tensor? ggr, Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? dt, int rf_kind, int gr_kind) -> (Tensor, Tensor, Tensor)', 'mask_copy': '(Tensor v, Tensor idx, Tensor inv, bool fill_zero) -> Tensor', 'clamp_waveform': '(Tensor x, Tensor lim, float eps, int kind) -> Tensor', 'clamp_waveform_bwd': '(Tensor g, Tensor x, Tensor lim, float eps, int kind) -> Tensor'}
+_SCHEMAS = {'blochsim_fused_fwd': '(Tensor Mi, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor, Tensor)', 'blochsim_fused_bwd': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'blochsim_fused_bwd_design': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? ddt, int rf_kind, int gr_kind) -> (Tensor, Tensor, Tensor, Tensor, Tensor)', 'blochsim_fused_bwd_spin': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, bool want_loc, bool want_sz, bool want_b1) -> (Tensor, Tensor, Tensor, Tensor, Tensor)', 'blochsim_beff_fwd': '(Tensor Mi, Tensor Beff, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'blochsim_beff_bwd': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor Beff, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'rfgr2beff': '(Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor gamma) -> Tensor', 'rfgr2beff_bwd': '(Tensor gB, Tensor rf, Tensor gr, Tensor loc, Tensor? b1) -> (Tensor, Tensor)', 'rfgr2beff_spin_grads': '(Tensor gB, Tensor rf, Tensor gr, bool want_loc, bool want_b1) -> (Tensor, Tensor, Tensor)', 'beff2ab': '(Tensor beff, Tensor E1, Tensor E2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor, Tensor)', 'beff2ab_bwd': '(Tensor gA, Tensor gB, Tensor A, Tensor B, Tensor ckpt, Tensor beff, Tensor E1, Tensor E2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'beff2uphi': '(Tensor beff, Tensor g) -> (Tensor, Tensor)', 'beff2uphi_bwd': '(Tensor? gU, Tensor? gPhi, Tensor beff, Tensor g) -> (Tensor, Tensor)', 'freeprec': '(Tensor Mi, Tensor dur, Tensor? T1, Tensor? T2, Tensor? df, bool adjoint) -> Tensor', 'design_waveform': '(Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? dt, int rf_kind, int gr_kind) -> (Tensor, Tensor)', 'design_waveform_bwd': '(Tensor? grf, Tensor? ggr, Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? dt, int rf_kind, int gr_kind) -> (Tensor, Tensor, Tensor)', 'mask_copy': '(Tensor v, Tensor idx, Tensor inv, bool fill_zero) -> Tensor', 'clamp_waveform': '(Tensor x, Tensor lim, float eps, int kind) -> Tensor', 'clamp_waveform_bwd': '(Tensor g, Tensor x, Tensor lim, float eps, int kind) -> Tensor'}
 
 
 def _register(name, impl, fake):
@@ -732,6 +792,7 @@ def _register(name, impl, fake):
 blochsim_fused_fwd = _register('blochsim_fused_fwd', _impl_blochsim_fused_fwd, _fake_blochsim_fused_fwd)
 blochsim_fused_bwd = _register('blochsim_fused_bwd', _impl_blochsim_fused_bwd, _fake_blochsim_fused_bwd)
 blochsim_fused_bwd_design = _register('blochsim_fused_bwd_design', _impl_blochsim_fused_bwd_design, _fake_blochsim_fused_bwd_design)
+blochsim_fused_bwd_spin = _register('blochsim_fused_bwd_spin', _impl_blochsim_fused_bwd_spin, _fake_blochsim_fused_bwd_spin)
 blochsim_beff_fwd = _register('blochsim_beff_fwd', _impl_blochsim_beff_fwd, _fake_blochsim_beff_fwd)
 blochsim_beff_bwd = _register('blochsim_beff_bwd', _impl_blochsim_beff_bwd, _fake_blochsim_beff_bwd)
 rfgr2beff_cuda = _register('rfgr2beff', _impl_rfgr2beff, _fake_rfgr2beff)
@@ -953,10 +1014,15 @@ def default_flags() -> int:
 def fused_applypulse(M_: Tensor, rf: Tensor, gr: Tensor, loc_: Tensor, *, Δf_: Optional[Tensor] = None,
                      b1Map_: Optional[Tensor] = None, T1_: Optional[Tensor] = None, T2_: Optional[Tensor] = None,
                      γ_: Tensor, dt: Tensor, ckpt: Optional[int] = None, flags: Optional[int] = None) -> Tensor:
-    """Fused waveform -> magnetisation op on compact arrays; differentiable wrt ``M_``, ``rf``, ``gr``.
+    """Fused waveform -> magnetisation op on compact arrays; differentiable wrt ``M_``, ``rf``, ``gr`` and the spins'
+    ``loc_``, ``Δf_``, ``b1Map_``, ``γ_`` (as the reference's autograd through rfgr2beff; γ only through ``Δf_/γ``).
 
     ``M_`` (N,nM,3), ``rf`` (N,2,nT[,nCoils]), ``gr`` (N,3,nT), ``loc_`` (N,nM,3), ``Δf_`` (N,nM),
     ``b1Map_`` (N,nM,2[,nCoils]), ``T1_/T2_/γ_`` broadcastable to (N,nM), ``dt`` () or (N|1,).
+
+    The per-spin gradients are sums over time that the fused backward forms per spin, without the dense field.  When one
+    of those inputs requires grad, a re-parametrised rf / gr (``tag_design``) is differentiated in two stages -- the
+    simulation's backward, then the chain's own adjoint -- as with ``MRPHY_B200_FUSE_DESIGN=0``.
     """
     _require_cuda(M_, rf, gr, loc_, Δf_, b1Map_, T1_, T2_)
     dtype, dev = M_.dtype, M_.device
@@ -998,7 +1064,8 @@ def fused_applypulse(M_: Tensor, rf: Tensor, gr: Tensor, loc_: Tensor, *, Δf_: 
     if ckpt is None and dtype == torch.float32 and b1 is not None and b1.shape[3] >= 3:
         K = min(K, TC_K_MAX)                     # the tensor-core kernels stage 32 steps per chunk
     fl = default_flags() if flags is None else flags
-    if torch.is_grad_enabled() and os.environ.get('MRPHY_B200_FUSE_DESIGN', '1') != '0':
+    spin_grad = any(x is not None and x.requires_grad for x in (loc_, Δf_, b1Map_, γ_))
+    if torch.is_grad_enabled() and not spin_grad and os.environ.get('MRPHY_B200_FUSE_DESIGN', '1') != '0':
         # rf and/or gr straight out of the re-parametrisation chain: differentiate w.r.t. the design variables in the
         # simulation's own gradient epilogue (see _FusedDesignApply)
         r_rf, r_gr = _design_of(rf_in, rf), _design_of(gr_in, gr)

@@ -53,6 +53,13 @@ def _one_of(full, compact, extract):
     return compact if full is None else extract(full)
 
 
+def _explicit_route(pulse, b1Map_, spin_inputs) -> bool:
+    """Gradients w.r.t. spin inputs through the dense field and the explicit-``Beff`` kernels: only for more than 16
+    transmit coils with a ``b1Map``, which the fused kernels do not take (everything else runs fused)."""
+    many_coils = b1Map_ is not None and pulse.rf.ndim == 4 and pulse.rf.shape[3] > 16
+    return many_coils and torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in spin_inputs)
+
+
 
 def _mask_kernel_ok(v: Tensor) -> bool:
     """embed/extract run the one-pass CUDA gather for floating CUDA tensors; anything else (CPU objects, integer or
@@ -391,18 +398,18 @@ class SpinArray(_Obj):
         the result in ``M_`` (with its autograd graph, as upstream); ``doEmbed`` returns `(N,*Nd,xyz)` instead of
         the compact `(N,nM,xyz)`.
 
-        All ``nT`` steps run in one fused CUDA kernel and gradients reach ``pulse.rf``, ``pulse.gr`` and ``M_``.
-        If ``loc``/``Δf``/``b1Map``/``γ`` themselves require grad, the field is materialised (``pulse2beff``) and the
-        explicit-``Beff`` kernels are used, which keeps upstream's autograd behaviour for those inputs.
+        All ``nT`` steps run in one fused CUDA kernel and gradients reach ``pulse.rf``, ``pulse.gr`` and ``M_``, and
+        ``loc``/``Δf``/``b1Map``/``γ`` when they require grad (upstream's autograd through rfgr2beff; the fused backward
+        forms these per-spin sums without materialising the field).  Only more than 16 transmit coils with a ``b1Map``,
+        which the fused kernels do not take, materialise the field (``pulse2beff``) and run the explicit-``Beff``
+        kernels, whose per-spin pass takes at most 16 coils as well.
         """
         assert (loc_ is None) != (loc is None)
         loc_ = loc_ if loc is None else self.extract(loc)
         Δf_ = _one_of(Δf, Δf_, self.extract)
         b1Map_ = _one_of(b1Map, b1Map_, self.extract)
         T1_, T2_ = (self.T1_, self.T2_) if doRelax else (None, None)
-        wants_geometry_grad = torch.is_grad_enabled() and any(
-            t is not None and t.requires_grad for t in (loc_, Δf_, b1Map_, self.γ_))
-        if wants_geometry_grad:
+        if _explicit_route(pulse, b1Map_, (loc_, Δf_, b1Map_, self.γ_)):
             beff_ = self.pulse2beff(pulse, loc_=loc_, Δf_=Δf_, b1Map_=b1Map_)
             M_ = sims.blochsim(self.M_, beff_, T1=T1_, T2=T2_, γ=self.γ_, dt=pulse.dt)
         else:
@@ -452,7 +459,7 @@ class SpinArray(_Obj):
         or float, seconds; free precession like :meth:`freeprec`).  Equivalent to chaining the two methods with
         ``doUpdate=True`` (mobjs.py:394-450, 555-592), but the magnetisation stays a compact device tensor from the first
         kernel to the last -- no embed / extract / attribute coercion per stage, no host synchronisation -- and the result is
-        differentiable w.r.t. every pulse's ``rf`` / ``gr`` and ``M_``.  The chain is CUDA-graph capturable as a whole
+        differentiable w.r.t. every pulse's ``rf`` / ``gr``, ``M_`` and the spin inputs as in :meth:`applypulse`.  The chain is CUDA-graph capturable as a whole
         (``mrphy.graphs.capture``): one replay per sequence.  Arguments and flags as in :meth:`applypulse`.
         """
         assert (loc_ is None) != (loc is None)
@@ -460,13 +467,11 @@ class SpinArray(_Obj):
         Δf_ = _one_of(Δf, Δf_, self.extract)
         b1Map_ = _one_of(b1Map, b1Map_, self.extract)
         T1_, T2_ = (self.T1_, self.T2_) if doRelax else (None, None)
-        geometry_grad = torch.is_grad_enabled() and any(
-            t is not None and t.requires_grad for t in (loc_, Δf_, b1Map_, self.γ_))
         M_ = self.M_
         for ev in events:
             if isinstance(ev, Pulse):
                 p = ev.to(device=self.device, dtype=self.dtype)
-                if geometry_grad:
+                if _explicit_route(p, b1Map_, (loc_, Δf_, b1Map_, self.γ_)):
                     beff_ = p.beff(loc_, γ=self.γ_, Δf=Δf_, b1Map=b1Map_)
                     M_ = sims.blochsim(M_, beff_, T1=T1_, T2=T2_, γ=self.γ_, dt=p.dt)
                 else:

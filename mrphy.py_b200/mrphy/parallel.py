@@ -7,6 +7,10 @@ beffective.py:137-165).  So each rank owns a contiguous range of the COMPACT spi
 all-reduce(sum) of the flat ``[rf.grad ‖ gr.grad ‖ extras]`` buffer (N·nT·(2·nCoils+3) elements, 80 KB
 for nT=4000).  Geometry stays global: the shard is a ``SpinArray`` with explicit ``loc_`` sliced from the
 global cube -- do not rebuild a smaller ``SpinCube`` (``_update_loc_`` centres on ``n//2``).
+
+Per-spin gradients (``loc_``, ``Δf_``, ``b1Map_``, ``γ_`` requiring grad) are local to a shard and need no collective.
+A ``Δf`` or ``γ`` that is ONE tensor broadcast over spins gets, on each rank, only the sum over that rank's spins; this
+module does not all-reduce it -- sum it over ranks yourself if you need the global gradient.
 """
 from typing import Optional, Tuple
 

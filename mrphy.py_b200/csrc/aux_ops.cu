@@ -111,77 +111,30 @@ __global__ void __launch_bounds__(256, sizeof(T) == 8 ? 3 : 4) rfgr2beff_kernel(
 }
 
 // ---- adjoint of rfgr2beff: the sums over spins ------------------------------------------------------
-// Threads run along time (the xyz triplets of 256 consecutive steps of one spin are 3 KB contiguous, so a warp's
-// three strided loads cover whole lines); a block owns 256 steps x one range of spins and keeps its W = 2*NC+3
-// running sums in registers; the spins' constants (b1, loc) are staged through shared memory 32 spins at a time.
-// Block partials go to partials[N][S][W][nT]; grad_finalize_kernel sums the S slices in fixed order.
-template <typename T, int NC>
-__global__ void __launch_bounds__(256) rfgr2beff_bwd_kernel(const mrphy_rfgr2beff_args a, const int per_split) {
-  constexpr int W = 2 * NC + 3, CH = 32;
-  __shared__ T cst[CH][W];
-  const int n = blockIdx.z, split = blockIdx.y, S = gridDim.y, tid = threadIdx.x;
-  const int t = blockIdx.x * 256 + tid;
-  const bool valid = t < a.nT;
-  const int i0 = split * per_split, i1 = min(a.nM, i0 + per_split);
-  T arx[NC], ary[NC], ag[3] = {0, 0, 0};
-#pragma unroll
-  for (int c = 0; c < NC; ++c) arx[c] = ary[c] = (T)0;
-  const T* G = (const T*)a.gBeff + ((size_t)n * a.nM * a.nT + (valid ? t : 0)) * 3;
-  for (int c0 = i0; c0 < i1; c0 += CH) {
-    const int cnt = min(CH, i1 - c0);
-    __syncthreads();
-    for (int e = tid; e < cnt * W; e += 256) {
-      const int s = e / W, w = e - s * W, i = c0 + s;
-      T v;
-      if (w < 2 * NC) {     // Re / Im of b1 for coil w % NC; without a b1Map the (summed) coil sees b1 = 1
-        const int c = w % NC;
-        v = a.b1 ? (c < a.nC ? ((const T*)a.b1)[(int64_t)n * a.b1_sn + (int64_t)i * a.b1_sm + (w / NC) * a.nC + c] : (T)0)
-                 : (w < NC ? (T)1 : (T)0);
-      } else {
-        v = ((const T*)a.loc)[(int64_t)n * a.loc_sn + (int64_t)i * a.loc_sm + (w - 2 * NC)];
-      }
-      cst[s][w] = v;
-    }
-    __syncthreads();
-    if (!valid) continue;
-#pragma unroll 4
-    for (int s = 0; s < cnt; ++s) {
-      const T* g = G + (size_t)(c0 + s) * a.nT * 3;
-      const T gx = g[0], gy = g[1], gz = g[2];
-#pragma unroll
-      for (int c = 0; c < NC; ++c) {
-        const T br = cst[s][c], bi = cst[s][NC + c];
-        arx[c] = fma_(br, gx, fma_(bi, gy, arx[c]));     // adjoint of Bx = br rx - bi ry, By = br ry + bi rx
-        ary[c] = fma_(br, gy, fnma_(bi, gx, ary[c]));
-      }
-#pragma unroll
-      for (int q = 0; q < 3; ++q) ag[q] = fma_(cst[s][2 * NC + q], gz, ag[q]);
-    }
-  }
-  if (!valid) return;
-  T* P = (T*)a.partials + (((size_t)n * S + split) * W) * (size_t)a.nT + t;
-#pragma unroll
-  for (int c = 0; c < NC; ++c) { P[(size_t)c * a.nT] = arx[c]; P[(size_t)(NC + c) * a.nT] = ary[c]; }
-#pragma unroll
-  for (int q = 0; q < 3; ++q) P[(size_t)(2 * NC + q) * a.nT] = ag[q];
-}
-
-// Same reduction with the rows staged by the TMA engine: one 1-D bulk copy (cp.async.bulk, 3 KB = 256 steps x xyz)
-// per spin, G spins per stage, two stages on mbarriers -- 24 KB in flight per block, no registers or L1 sectors spent
-// on the strided xyz pattern; threads then read their own triplet from shared memory (stride 3: conflict-free).
-// Needs 16-byte aligned rows: nT % 4 == 0 (the launcher falls back to the kernel above otherwise).
-template <typename T> struct RBTma {
-  static constexpr int G = 32 / (int)sizeof(T);                       // spins per stage: 8 (fp32), 4 (fp64)
+// Threads run along time: a block owns 256 steps x one range of spins and keeps its W = 2*NC+3 running sums in
+// registers; the spins' constants (b1, loc) are staged through shared memory one group of G spins at a time, two
+// stages on one barrier per group.  ALIGNED (nT % 4 == 0 and a 16-byte aligned gBeff: every row is) stages the rows
+// too, by the TMA engine: one 1-D bulk copy (cp.async.bulk, 3 KB = 256 steps x xyz) per spin, G spins per stage on
+// mbarriers -- 24 KB in flight per block, no registers or L1 sectors spent on the strided xyz pattern; threads then
+// read their own triplet from shared memory (stride 3: conflict-free).  Otherwise each thread reads its own triplet
+// from global memory (the xyz triplets of 256 consecutive steps of one spin are 3 KB contiguous, so a warp's three
+// strided loads cover whole lines).  Block partials go to partials[N][S][W][nT]; grad_finalize_kernel sums the S
+// slices in fixed order.
+template <typename T, bool ALIGNED> struct RBCfg {
+  static constexpr int G = ALIGNED ? 32 / (int)sizeof(T) : 32;        // spins per stage: 8 (fp32), 4 (fp64); 32 unstaged
   static constexpr int TBK = 256;
-  static constexpr size_t buf_bytes = (size_t)2 * G * 3 * TBK * sizeof(T);   // 48 KB
+  static constexpr size_t buf_bytes = ALIGNED ? (size_t)2 * G * 3 * TBK * sizeof(T) : 0;   // 48 KB of rows
+  __host__ __device__ static constexpr size_t cst_bytes(int W) { return ((sizeof(T) * 2 * G * W + 15) / 16) * 16; }
+  __host__ __device__ static constexpr size_t smem(int W) { return buf_bytes + cst_bytes(W) + 16; }   // rows, constants, 2 mbarriers
 };
-template <typename T, int NC>
-__global__ void __launch_bounds__(256) rfgr2beff_bwd_tma_kernel(const mrphy_rfgr2beff_args a, const int per_split) {
-  constexpr int W = 2 * NC + 3, G = RBTma<T>::G, TBK = RBTma<T>::TBK;
+template <typename T, int NC, bool ALIGNED>
+__global__ void __launch_bounds__(256) rfgr2beff_bwd_kernel(const mrphy_rfgr2beff_args a, const int per_split) {
+  using C = RBCfg<T, ALIGNED>;
+  constexpr int W = 2 * NC + 3, G = C::G, TBK = C::TBK;
   extern __shared__ __align__(128) unsigned char rb_smem[];
   T(*buf)[G][3 * TBK] = reinterpret_cast<T(*)[G][3 * TBK]>(rb_smem);
-  T(*cst)[G][W] = reinterpret_cast<T(*)[G][W]>(rb_smem + RBTma<T>::buf_bytes);
-  uint64_t* full = reinterpret_cast<uint64_t*>(rb_smem + RBTma<T>::buf_bytes + ((sizeof(T) * 2 * G * W + 15) / 16) * 16);
+  T(*cst)[G][W] = reinterpret_cast<T(*)[G][W]>(rb_smem + C::buf_bytes);
+  uint64_t* full = reinterpret_cast<uint64_t*>(rb_smem + C::buf_bytes + C::cst_bytes(W));
   const int n = blockIdx.z, split = blockIdx.y, S = gridDim.y, tid = threadIdx.x;
   const int t0 = blockIdx.x * TBK, len = min(TBK, a.nT - t0);
   const uint32_t row_bytes = (uint32_t)(len * 3 * sizeof(T));
@@ -189,7 +142,7 @@ __global__ void __launch_bounds__(256) rfgr2beff_bwd_tma_kernel(const mrphy_rfgr
   const int i0 = split * per_split, i1 = min(a.nM, i0 + per_split);
   const int ngroups = (i1 - i0 + G - 1) / G;
   const T* Gb = (const T*)a.gBeff + ((size_t)n * a.nM * a.nT + t0) * 3;
-  if (tid == 0) {
+  if (ALIGNED && tid == 0) {
     mbar_init(&full[0], 1);
     mbar_init(&full[1], 1);
     fence_barrier_init();
@@ -197,7 +150,7 @@ __global__ void __launch_bounds__(256) rfgr2beff_bwd_tma_kernel(const mrphy_rfgr
   __syncthreads();
   auto issue = [&](int g, int s) {
     const int c0 = i0 + g * G, cnt = min(G, i1 - c0);
-    if (tid == 0) {
+    if (ALIGNED && tid == 0) {
       mbar_arrive_expect_tx(&full[s], row_bytes * cnt);
       for (int q = 0; q < cnt; ++q) bulk_g2s(buf[s][q], Gb + (size_t)(c0 + q) * a.nT * 3, row_bytes, &full[s]);
     }
@@ -222,11 +175,12 @@ __global__ void __launch_bounds__(256) rfgr2beff_bwd_tma_kernel(const mrphy_rfgr
   for (int g = 0; g < ngroups; ++g) {
     const int s = g & 1, cnt = min(G, i1 - (i0 + g * G));
     if (g + 1 < ngroups) issue(g + 1, s ^ 1);   // that stage was drained in iteration g-1 (barrier below)
-    mbar_wait(&full[s], (g >> 1) & 1);
+    if (ALIGNED) mbar_wait(&full[s], (g >> 1) & 1);
     if (valid) {
 #pragma unroll 4
       for (int q = 0; q < cnt; ++q) {
-        const T gx = buf[s][q][3 * tid], gy = buf[s][q][3 * tid + 1], gz = buf[s][q][3 * tid + 2];
+        const T* gp = ALIGNED ? &buf[s][q][3 * tid] : Gb + (size_t)(i0 + g * G + q) * a.nT * 3 + 3 * tid;
+        const T gx = gp[0], gy = gp[1], gz = gp[2];
 #pragma unroll
         for (int c = 0; c < NC; ++c) {
           const T br = cst[s][q][c], bi = cst[s][q][NC + c];
@@ -573,20 +527,13 @@ int rb_plan(const mrphy_rfgr2beff_args* a, RBPlan* p) {
 
 template <typename T, int NC>
 int launch_rb(const mrphy_rfgr2beff_args* a, const RBPlan& p, cudaStream_t st) {
-  dim3 grid(p.tblocks, p.S, a->N);
-  const bool tma = a->nT % 4 == 0 && ((uintptr_t)a->gBeff & 15) == 0 && !getenv("MRPHY_B200_RB_NOTMA");
-  if (tma) {
-    constexpr size_t smem = RBTma<T>::buf_bytes + ((sizeof(T) * 2 * RBTma<T>::G * (2 * NC + 3) + 15) / 16) * 16 + 16;
-    auto kern = rfgr2beff_bwd_tma_kernel<T, NC>;
-    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    timing_begin(st);
-    kern<<<grid, 256, smem, st>>>(*a, p.per_split);
-    timing_end(st);
-  } else {
-    timing_begin(st);
-    rfgr2beff_bwd_kernel<T, NC><<<grid, 256, 0, st>>>(*a, p.per_split);
-    timing_end(st);
-  }
+  const bool al = a->nT % 4 == 0 && ((uintptr_t)a->gBeff & 15) == 0;
+  auto kern = al ? rfgr2beff_bwd_kernel<T, NC, true> : rfgr2beff_bwd_kernel<T, NC, false>;
+  const size_t smem = al ? RBCfg<T, true>::smem(p.W) : RBCfg<T, false>::smem(p.W);
+  CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  timing_begin(st);
+  kern<<<dim3(p.tblocks, p.S, a->N), 256, smem, st>>>(*a, p.per_split);
+  timing_end(st);
   ++launch_count();
   CK(cudaGetLastError());
   dim3 fgrid((a->nT + 31) / 32, p.W, a->N), fblock(32, 32);

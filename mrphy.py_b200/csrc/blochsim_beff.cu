@@ -1,14 +1,15 @@
 // Explicit-field Bloch simulation for sm_100a: the API-faithful replacement of sims.BlochSim
 // (sims.py:24-269) for callers that pass a dense Beff (N,nM,nT,3).  HBM-bound: 12 B/spin.step
-// read forward; 12 B read + 12 B written backward (fp32).  Each warp owns 32 spins and moves
-// [32 spins] x [TB steps x 3] tiles between HBM and shared memory with 128-byte coalesced row
-// accesses; one thread then walks its own row (odd pitch => conflict-free).  The backward pass
-// overwrites the tile in place with dL/dBeff and streams it back out the same way.  States are
-// not stored: time-reversed reconstruction + checkpoints every K steps, as in the fused path.
+// read forward; 12 B read + 12 B written backward (fp32).  Each warp owns 32 spins and streams
+// [32 spins] x [192-byte] tiles of their Beff rows through a ring in shared memory with cp.async;
+// one thread then walks its own row.  The backward pass overwrites the tile in place with
+// dL/dBeff and streams it back out the same way.  States are not stored: time-reversed
+// reconstruction + checkpoints every K steps, as in the fused path.
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdlib.h>
 #include <string.h>
+
+#include <type_traits>
 
 #include "../../include/mrphy_b200.h"
 #include "abi_common.cuh"
@@ -18,12 +19,6 @@ namespace mrphy {
 
 constexpr int EBLK = 128;
 constexpr int EWARP = EBLK / 32;
-
-template <typename T> struct ECfg {
-  static constexpr int TB = 128 / (int)sizeof(T);   // steps per tile: 32 (fp32), 16 (fp64)
-  static constexpr int PITCH = 3 * TB + 1;
-  static constexpr size_t smem = (size_t)EWARP * 32 * PITCH * sizeof(T);
-};
 
 template <typename T> struct EArgs {
   int N, nM, nT, K, nCk;
@@ -43,188 +38,87 @@ __device__ __forceinline__ void load_consts(const EArgs<T>& a, int n, int i, Spi
   g = (T)(6.283185307179586476925286766559 * gam * dt);   // sims.py:62
 }
 
-// warp-cooperative tile copy HBM -> smem: row r holds steps [t0, t0+len) of spin (i0 + r)
-template <typename T>
-__device__ __forceinline__ void tile_load(const T* __restrict__ B, int64_t B_sm, int i0, int nM, int t0, int len,
-                                          T* tile, int lane) {
-  constexpr int PITCH = ECfg<T>::PITCH;
-  const int cols = 3 * len;
-#pragma unroll 4
-  for (int r = 0; r < 32; ++r) {
-    const int i = min(i0 + r, nM - 1);
-    const T* src = B + (int64_t)i * B_sm + (int64_t)t0 * 3;
-    for (int c = lane; c < cols; c += 32) tile[r * PITCH + c] = src[c];
-  }
-}
-template <typename T>
-__device__ __forceinline__ void tile_store(T* __restrict__ G, int64_t G_sm, int i0, int nM, int t0, int len,
-                                           const T* tile, int lane) {
-  constexpr int PITCH = ECfg<T>::PITCH;
-  const int cols = 3 * len;
-#pragma unroll 4
-  for (int r = 0; r < 32; ++r) {
-    const int i = i0 + r;
-    if (i >= nM) break;
-    T* dst = G + (int64_t)i * G_sm + (int64_t)t0 * 3;
-    for (int c = lane; c < cols; c += 32) dst[c] = tile[r * PITCH + c];
-  }
-}
-
-template <typename T, int POL, bool RELAX>
-__global__ void __launch_bounds__(EBLK) beff_fwd_kernel(const EArgs<T> a) {
-  constexpr int TB = ECfg<T>::TB, PITCH = ECfg<T>::PITCH;
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, n = blockIdx.y;
-  T* tile = reinterpret_cast<T*>(smem_raw) + (size_t)warp * 32 * PITCH;
-  const int nM = a.nM, nT = a.nT, K = a.K;
-  const int i0 = (blockIdx.x * EWARP + warp) * 32;
-  if (i0 >= nM) return;
-  const bool ok = i0 + lane < nM;
-  const int i = ok ? i0 + lane : nM - 1;
-  SpinConst<T, 1> k;
-  T g;
-  load_consts<T, RELAX>(a, n, i, k, g);
-  const T* mp = a.Mi + (int64_t)n * a.Mi_sn + (int64_t)i * a.Mi_sm;
-  T mx = mp[0], my = mp[1], mz = mp[2];
-  const T* Bn = a.B + (int64_t)n * a.B_sn;
-  const T* row = tile + lane * PITCH;
-  for (int t0 = 0; t0 < nT; t0 += TB) {
-    const int len = min(TB, nT - t0);
-    tile_load<T>(Bn, a.B_sm, i0, nM, t0, len, tile, lane);
-    __syncwarp();
-    for (int j = 0; j < len; ++j) {
-      step_fwd<T, POL, RELAX>(g * row[3 * j], g * row[3 * j + 1], g * row[3 * j + 2], k.e1, k.e2, mx, my, mz);
-      const int t1 = t0 + j + 1;
-      if (t1 % K == 0 && t1 < nT && ok) {
-        T* cp = a.ckpt + ((size_t)n * a.nCk + (t1 / K - 1)) * 3 * (size_t)nM;
-        cp[i] = mx; cp[(size_t)nM + i] = my; cp[2 * (size_t)nM + i] = mz;
-      }
-    }
-    __syncwarp();
-  }
-  if (ok) {
-    T* op = a.Mo + ((size_t)n * nM + i) * 3;
-    op[0] = mx; op[1] = my; op[2] = mz;
-  }
-}
-
-template <typename T, int POL, bool RELAX>
-__global__ void __launch_bounds__(EBLK) beff_bwd_kernel(const EArgs<T> a, const int need_gmi, const int need_gb) {
-  constexpr int TB = ECfg<T>::TB, PITCH = ECfg<T>::PITCH;
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, n = blockIdx.y;
-  T* tile = reinterpret_cast<T*>(smem_raw) + (size_t)warp * 32 * PITCH;
-  const int nM = a.nM, nT = a.nT, K = a.K;
-  const int i0 = (blockIdx.x * EWARP + warp) * 32;
-  if (i0 >= nM) return;
-  const bool ok = i0 + lane < nM;
-  const int i = ok ? i0 + lane : nM - 1;
-  SpinConst<T, 1> k;
-  T g;
-  load_consts<T, RELAX>(a, n, i, k, g);
-  const T* mp = a.Mo + ((size_t)n * nM + i) * 3;
-  T mx = mp[0], my = mp[1], mz = mp[2];
-  const T* gp = a.gMo + (int64_t)n * a.gMo_sn + (int64_t)i * a.gMo_sm;
-  T hx = gp[0], hy = gp[1], hz = gp[2];
-  const T* Bn = a.B + (int64_t)n * a.B_sn;
-  T* Gn = a.gB + (size_t)n * nM * (size_t)nT * 3;
-  T* row = tile + lane * PITCH;
-  const T ng = -g;
-  for (int t0 = ((nT - 1) / TB) * TB; t0 >= 0; t0 -= TB) {
-    const int len = min(TB, nT - t0);
-    tile_load<T>(Bn, a.B_sm, i0, nM, t0, len, tile, lane);
-    __syncwarp();
-    for (int j = len - 1; j >= 0; --j) {
-      T Fx, Fy, Fz;
-      step_bwd<T, POL, RELAX, 1>(k, g * row[3 * j], g * row[3 * j + 1], g * row[3 * j + 2], mx, my, mz, hx, hy, hz,
-                                 Fx, Fy, Fz);
-      row[3 * j] = ng * Fx;       // dL/dBeff = -2*pi*gamma*dt * F   (sims.py:194, 234-259)
-      row[3 * j + 1] = ng * Fy;
-      row[3 * j + 2] = ng * Fz;
-      const int t = t0 + j;
-      if (t % K == 0 && t > 0) {   // resynchronise with the forward checkpoint (state after t steps)
-        const T* cp = a.ckpt + ((size_t)n * a.nCk + (t / K - 1)) * 3 * (size_t)nM;
-        mx = cp[i]; my = cp[(size_t)nM + i]; mz = cp[2 * (size_t)nM + i];
-      }
-    }
-    __syncwarp();
-    if (need_gb) tile_store<T>(Gn, (int64_t)nT * 3, i0, nM, t0, len, tile, lane);
-    __syncwarp();
-  }
-  if (need_gmi && ok) {
-    T* op = a.gMi + ((size_t)n * nM + i) * 3;
-    op[0] = hx; op[1] = hy; op[2] = hz;
-  }
-}
-
 // ------------------------------------------------------------------------------------------
-// v2 tile pipeline (used when every Beff row is 16-byte aligned: nT*3*sizeof(T) % 16 == 0).
-// A tile row is 192 data bytes (16 fp32 steps / 8 fp64 steps) + 16 bytes pad = 208-byte pitch, so that
-//  * the warp fills it with 16-byte cp.async (LDGSTS.128) straight from HBM, double-buffered: tile k+1 is in
-//    flight while tile k is consumed, no registers staged;
+// Tile pipeline.  A tile row is 192 data bytes (16 fp32 steps / 8 fp64 steps) + 16 bytes pad = 208-byte pitch, so that
+//  * the warp fills it with cp.async straight from HBM, double-buffered: tile k+1 is in flight while tile k is consumed,
+//    no registers staged;
 //  * each thread reads its own row with LDS.128 without bank conflicts (20*r mod 32 hits 8 distinct quads);
-//  * the backward overwrites the row in place with dL/dBeff and the warp streams it out with 16-byte stores.
-#ifndef MRPHY_BEFF_ROWB
-#define MRPHY_BEFF_ROWB 192
-#endif
-#ifndef MRPHY_BEFF_NST
-#define MRPHY_BEFF_NST 2
-#endif
-constexpr int NST = MRPHY_BEFF_NST;   // tiles in the per-warp ring (NST - 1 in flight while one is consumed)
-constexpr int ROWB = MRPHY_BEFF_ROWB, PITCHB = ROWB + 16, CHUNKS = ROWB / 16;   // 12 chunks of 16 B per row (pitch 13 x 16 B: odd)
+//  * the backward overwrites the row in place with dL/dBeff and the warp streams it out with coalesced stores.
+// ALIGNED (every Beff row starts on 16 bytes: rows_aligned16) moves 16-byte chunks (LDGSTS.128, 128-bit stores); other
+// rows move element by element into the same layout, which needs only the element alignment every tensor has.
+constexpr int NST = 2;     // tiles in the per-warp ring (NST - 1 in flight while one is consumed)
+constexpr int ROWB = 192, PITCHB = ROWB + 16;   // pitch 13 x 16 B: odd
 
-__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gmem_src)
-               : "memory");
+template <int E>           // one copy of E bytes: 16 with .cg (L2 only), 4 or 8 with .ca (the only form for < 16 B)
+__device__ __forceinline__ void cp_async(void* smem_dst, const void* gmem_src) {
+  if constexpr (E == 16)
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gmem_src)
+                 : "memory");
+  else
+    asm volatile("cp.async.ca.shared.global [%0], [%1], %2;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gmem_src),
+                 "n"(E) : "memory");
 }
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
+// unit of the warp-cooperative tile copies: a 16-byte chunk on aligned rows, one element otherwise
+template <typename T, bool ALIGNED> struct TileCopy {
+  using V = std::conditional_t<ALIGNED, float4, T>;
+  static constexpr int LG = ALIGNED ? 4 : (sizeof(T) == 8 ? 3 : 2), E = 1 << LG;   // bytes per copy: 16, 8 or 4
+  static constexpr int CHUNKS = ROWB / E;                                           // copies per full row
+  static_assert(sizeof(V) == E, "copy unit");
+};
+
 // warp-cooperative async copy of rows [i0, i0+32) x bytes [t0*3*sizeof(T), +nbytes) into `tile`
-template <typename T, int ROWS = 32>
+template <typename T, bool ALIGNED, int ROWS = 32>
 __device__ __forceinline__ void tile_load_async(const T* __restrict__ B, int64_t B_sm, int i0, int nM, int t0, int nbytes,
                                                 unsigned char* tile, int lane) {
-  const int nch = nbytes >> 4;             // chunks per row in this tile (<= 12)
+  using C = TileCopy<T, ALIGNED>;
+  constexpr int E = C::E, CHUNKS = C::CHUNKS;
+  const int nch = nbytes >> C::LG;         // chunks per row in this tile
   const unsigned char* base = reinterpret_cast<const unsigned char*>(B + (int64_t)t0 * 3);
   const int64_t rowb = B_sm * (int64_t)sizeof(T);
-  if (nch == CHUNKS) {                     // full tile: compile-time divisor, 12 copies per lane (per 32 rows)
+  // full tile of 16-byte chunks: compile-time divisor, 12 copies per lane (per 32 rows).  Element copies always take the
+  // loop below: unrolled, their 24 or 48 copies per lane would hold as many addresses in registers.
+  if (ALIGNED && nch == CHUNKS) {
 #pragma unroll
     for (int k = 0; k < CHUNKS * ROWS / 32; ++k) {
       const int q = k * 32 + lane, r = q / CHUNKS, c = q - r * CHUNKS;
-      cp_async16(tile + r * PITCHB + c * 16, base + (int64_t)min(i0 + r, nM - 1) * rowb + c * 16);
+      cp_async<E>(tile + r * PITCHB + c * E, base + (int64_t)min(i0 + r, nM - 1) * rowb + c * E);
     }
     return;
   }
   for (int q = lane; q < ROWS * nch; q += 32) {
     const int r = q / nch, c = q - r * nch;
-    cp_async16(tile + r * PITCHB + c * 16, base + (int64_t)min(i0 + r, nM - 1) * rowb + c * 16);
+    cp_async<E>(tile + r * PITCHB + c * E, base + (int64_t)min(i0 + r, nM - 1) * rowb + c * E);
   }
 }
-template <typename T, int ROWS = 32>
-__device__ __forceinline__ void tile_store16(T* __restrict__ G, int64_t G_sm, int i0, int nM, int t0, int nbytes,
-                                             const unsigned char* tile, int lane) {
-  const int nch = nbytes >> 4;
+template <typename T, bool ALIGNED, int ROWS = 32>
+__device__ __forceinline__ void tile_store(T* __restrict__ G, int64_t G_sm, int i0, int nM, int t0, int nbytes,
+                                           const unsigned char* tile, int lane) {
+  using C = TileCopy<T, ALIGNED>;
+  using V = typename C::V;
+  constexpr int E = C::E, CHUNKS = C::CHUNKS;
+  const int nch = nbytes >> C::LG;
   unsigned char* base = reinterpret_cast<unsigned char*>(G + (int64_t)t0 * 3);
   const int64_t rowb = G_sm * (int64_t)sizeof(T);
-  if (nch == CHUNKS) {
+  if (ALIGNED && nch == CHUNKS) {
 #pragma unroll
     for (int k = 0; k < CHUNKS * ROWS / 32; ++k) {
       const int q = k * 32 + lane, r = q / CHUNKS, c = q - r * CHUNKS;
       if (i0 + r < nM)
-        *reinterpret_cast<float4*>(base + (int64_t)(i0 + r) * rowb + c * 16) =
-            *reinterpret_cast<const float4*>(tile + r * PITCHB + c * 16);
+        *reinterpret_cast<V*>(base + (int64_t)(i0 + r) * rowb + c * E) = *reinterpret_cast<const V*>(tile + r * PITCHB + c * E);
     }
     return;
   }
   for (int q = lane; q < ROWS * nch; q += 32) {
     const int r = q / nch, c = q - r * nch;
     if (i0 + r < nM)
-      *reinterpret_cast<float4*>(base + (int64_t)(i0 + r) * rowb + c * 16) =
-          *reinterpret_cast<const float4*>(tile + r * PITCHB + c * 16);
+      *reinterpret_cast<V*>(base + (int64_t)(i0 + r) * rowb + c * E) = *reinterpret_cast<const V*>(tile + r * PITCHB + c * E);
   }
 }
 
-template <typename T, int POL, bool RELAX, bool BWD>
+template <typename T, int POL, bool RELAX, bool BWD, bool ALIGNED>
 __global__ void __launch_bounds__(EBLK) beff_v2_kernel(const EArgs<T> a, const int need_gmi, const int need_gb) {
   constexpr int TB = ROWB / (3 * (int)sizeof(T));      // steps per tile: 16 (fp32), 8 (fp64)
   constexpr int PITCH = PITCHB / (int)sizeof(T);       // row pitch in elements
@@ -273,13 +167,13 @@ __global__ void __launch_bounds__(EBLK) beff_v2_kernel(const EArgs<T> a, const i
   // empty one past the end), so "all but the newest NST - 1 groups" is always "tile q has landed"
 #pragma unroll
   for (int p = 0; p < NST - 1; ++p) {
-    if (p < ntiles) tile_load_async<T>(Bn, a.B_sm, i0, nM, tile_t0(p), tile_len(p) * 3 * (int)sizeof(T), buf0 + p * 32 * PITCHB, lane);
+    if (p < ntiles) tile_load_async<T, ALIGNED>(Bn, a.B_sm, i0, nM, tile_t0(p), tile_len(p) * 3 * (int)sizeof(T), buf0 + p * 32 * PITCHB, lane);
     cp_async_commit();
   }
   for (int q = 0; q < ntiles; ++q) {
     unsigned char* cur = buf0 + (q % NST) * 32 * PITCHB;
     if (q + NST - 1 < ntiles)
-      tile_load_async<T>(Bn, a.B_sm, i0, nM, tile_t0(q + NST - 1), tile_len(q + NST - 1) * 3 * (int)sizeof(T),
+      tile_load_async<T, ALIGNED>(Bn, a.B_sm, i0, nM, tile_t0(q + NST - 1), tile_len(q + NST - 1) * 3 * (int)sizeof(T),
                          buf0 + ((q + NST - 1) % NST) * 32 * PITCHB, lane);
     cp_async_commit();
     cp_async_wait<NST - 1>();
@@ -289,13 +183,18 @@ __global__ void __launch_bounds__(EBLK) beff_v2_kernel(const EArgs<T> a, const i
     // 48 bytes = GS steps per group, moved with three conflict-free 128-bit accesses
     constexpr int GS = 16 / (int)sizeof(T);            // 4 (fp32) or 2 (fp64) steps
     constexpr int GV = 3 * GS;                         // values per group
+    // Aligned rows hold a multiple of GS steps.  Otherwise the last group of the last tile in time can hold gl < GS steps
+    // (it is the first group the backward processes): it runs its gl steps on the per-step path and leaves the rest of v,
+    // stale data inside the row, untouched.  No zero padding: a zero-field step is not the identity under relaxation.
+    auto group_len = [&](int j0) { return ALIGNED ? GS : min(GS, len - j0); };
     if (!BWD) {
       for (int j0 = 0; j0 < len; j0 += GS) {
+        const int gl = group_len(j0);
         T v[GV];
         float4* v4 = reinterpret_cast<float4*>(v);
         const float4* src = reinterpret_cast<const float4*>(row + 3 * j0);
         v4[0] = src[0]; v4[1] = src[1]; v4[2] = src[2];
-        if (until > GS) {
+        if (until > GS && gl == GS) {
 #pragma unroll
           for (int u = 0; u < GS; ++u)
             step_fwd<T, POL, RELAX>(g * v[3 * u], g * v[3 * u + 1], g * v[3 * u + 2], k.e1, k.e2, mx, my, mz);
@@ -303,6 +202,7 @@ __global__ void __launch_bounds__(EBLK) beff_v2_kernel(const EArgs<T> a, const i
         } else {
 #pragma unroll
           for (int u = 0; u < GS; ++u) {
+            if (u >= gl) break;
             step_fwd<T, POL, RELAX>(g * v[3 * u], g * v[3 * u + 1], g * v[3 * u + 2], k.e1, k.e2, mx, my, mz);
             if (--until == 0) {
               if (t0 + j0 + u + 1 < nT && ok) {
@@ -315,12 +215,13 @@ __global__ void __launch_bounds__(EBLK) beff_v2_kernel(const EArgs<T> a, const i
         }
       }
     } else {
-      for (int j0 = len - GS; j0 >= 0; j0 -= GS) {
+      for (int j0 = ALIGNED ? len - GS : (len - 1) / GS * GS; j0 >= 0; j0 -= GS) {
+        const int gl = group_len(j0);
         T v[GV];
         float4* v4 = reinterpret_cast<float4*>(v);
         float4* src = reinterpret_cast<float4*>(row + 3 * j0);
         v4[0] = src[0]; v4[1] = src[1]; v4[2] = src[2];
-        if (until > GS) {
+        if (until > GS && gl == GS) {
 #pragma unroll
           for (int u = GS - 1; u >= 0; --u) {
             T Fx, Fy, Fz;
@@ -334,6 +235,7 @@ __global__ void __launch_bounds__(EBLK) beff_v2_kernel(const EArgs<T> a, const i
         } else {
 #pragma unroll
           for (int u = GS - 1; u >= 0; --u) {
+            if (u >= gl) continue;
             T Fx, Fy, Fz;
             step_bwd<T, POL, RELAX, 1>(k, g * v[3 * u], g * v[3 * u + 1], g * v[3 * u + 2], mx, my, mz, hx, hy, hz,
                                        Fx, Fy, Fz);
@@ -352,7 +254,7 @@ __global__ void __launch_bounds__(EBLK) beff_v2_kernel(const EArgs<T> a, const i
         src[0] = v4[0]; src[1] = v4[1]; src[2] = v4[2];
       }
       __syncwarp();
-      if (need_gb) tile_store16<T>(Gn, (int64_t)nT * 3, i0, nM, t0, len * 3 * (int)sizeof(T), cur, lane);
+      if (need_gb) tile_store<T, ALIGNED>(Gn, (int64_t)nT * 3, i0, nM, t0, len * 3 * (int)sizeof(T), cur, lane);
     }
     __syncwarp();   // the buffer is refilled two iterations later, after every lane has left it
   }
@@ -410,42 +312,16 @@ bool rows_aligned16(const mrphy_beff_args* a) {
 
 template <typename T, int POL, bool RELAX>
 int launch_e(bool bwd, const mrphy_beff_args* a, cudaStream_t st) {
-  const EArgs<T> e = make_eargs<T>(a);
+  const bool al = rows_aligned16<T>(a);
+  auto kern = bwd ? (al ? beff_v2_kernel<T, POL, RELAX, true, true> : beff_v2_kernel<T, POL, RELAX, true, false>)
+                  : (al ? beff_v2_kernel<T, POL, RELAX, false, true> : beff_v2_kernel<T, POL, RELAX, false, false>);
+  constexpr size_t smem = (size_t)EWARP * NST * 32 * PITCHB;
+  const int gmi = bwd && (a->flags & MRPHY_NEED_GMI) ? 1 : 0, gb = bwd && (a->flags & MRPHY_NEED_GBEFF) ? 1 : 0;
   dim3 grid((a->nM + EBLK - 1) / EBLK, a->N);
-  if (rows_aligned16<T>(a) && !getenv("MRPHY_B200_BEFF_V1")) {   // cp.async double-buffered tiles
-    constexpr size_t smem2 = (size_t)EWARP * NST * 32 * PITCHB;
-    const int gmi = (a->flags & MRPHY_NEED_GMI) ? 1 : 0, gb = (a->flags & MRPHY_NEED_GBEFF) ? 1 : 0;
-    if (bwd) {
-      auto kern = beff_v2_kernel<T, POL, RELAX, true>;
-      CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
-      timing_begin(st);
-      kern<<<grid, EBLK, smem2, st>>>(e, gmi, gb);
-      timing_end(st);
-    } else {
-      auto kern = beff_v2_kernel<T, POL, RELAX, false>;
-      CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
-      timing_begin(st);
-      kern<<<grid, EBLK, smem2, st>>>(e, 0, 0);
-      timing_end(st);
-    }
-    ++launch_count();
-    CK(cudaGetLastError());
-    return MRPHY_OK;
-  }
-  constexpr size_t smem = ECfg<T>::smem;
-  if (bwd) {
-    auto kern = beff_bwd_kernel<T, POL, RELAX>;
-    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    timing_begin(st);
-    kern<<<grid, EBLK, smem, st>>>(e, (a->flags & MRPHY_NEED_GMI) ? 1 : 0, (a->flags & MRPHY_NEED_GBEFF) ? 1 : 0);
-    timing_end(st);
-  } else {
-    auto kern = beff_fwd_kernel<T, POL, RELAX>;
-    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    timing_begin(st);
-    kern<<<grid, EBLK, smem, st>>>(e);
-    timing_end(st);
-  }
+  CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  timing_begin(st);
+  kern<<<grid, EBLK, smem, st>>>(make_eargs<T>(a), gmi, gb);
+  timing_end(st);
   ++launch_count();
   CK(cudaGetLastError());
   return MRPHY_OK;

@@ -6,6 +6,7 @@ fp32-vs-fp64 distance on the same inputs where that is larger (SURVEY App. B: no
 this recurrence, the reference's included, gets below ~2e-5 at nT~1000 with multi-radian steps);
 rf/gr gradients <= 1e-4 relative in fp32, <= 1e-9 relative in fp64.
 """
+import itertools
 import os
 
 import numpy as np
@@ -375,25 +376,48 @@ def test_explicit_beff_vs_oracle_and_fused(dev):
         assert rel(rf.grad, ref['grf']) < tolG and rel(gr.grad, ref['ggr']) < tolG
 
 
-@pytest.mark.parametrize('nM,nT', [(200, 152), (64, 16), (1, 4), (333, 1000)])
-def test_explicit_beff_aligned_rows_fp32(dev, nM, nT):
-    """fp32 explicit-field kernels on 16-byte-aligned rows (the cp.async tile pipeline): ragged spin counts (odd, < 32, not
-    a multiple of the CTA), partial last tiles, checkpoints that fall inside tiles; values and both gradients against the
-    fp64 oracle within the fp32 rule."""
+@pytest.mark.parametrize('dtype,nM,nT,case', [
+    # 16-byte-aligned rows (nT % 4 == 0 in fp32, even in fp64): 16-byte copies
+    (f32, 200, 152, ''), (f32, 64, 16, ''), (f32, 1, 4, ''), (f32, 333, 1000, ''), (f64, 77, 152, ''), (f64, 1, 2, ''),
+    # other rows: element copies, and a last tile that ends in a partial group of steps
+    (f32, 200, 151, ''), (f32, 45, 17, ''), (f32, 33, 3, ''), (f32, 1, 1, ''), (f64, 77, 151, ''), (f64, 5, 9, ''),
+    (f64, 1, 1, ''),
+    (f32, 100, 152, 'offset'),                    # aligned nT, but the data pointer is one element into a buffer
+    (f32, 70, 151, 'ckpt3'), (f64, 70, 151, 'ckpt3'),   # checkpoints every 3 steps: some inside the partial group
+    (f32, 50, 151, 'M0only'),                     # no dL/dBeff is stored
+])
+def test_explicit_beff_tile_pipeline(dev, monkeypatch, dtype, nM, nT, case):
+    """Explicit-field kernels on both row alignments: ragged spin counts (odd, < 32, not a multiple of the CTA), partial
+    last tiles and groups, checkpoints that fall inside tiles and groups; values and both gradients against the fp64
+    oracle (fp64: 1e-12 / 1e-9; fp32: the fp32 rule)."""
     from oracle import bloch_oracle as orc
     from mrphy import sims
-    p = _random_problem(100 + nM, 2, nM, nT, 1, has_b1=True, relax=True, dtype=f32)
-    beff = orc.rfgr2beff(p['rf'], p['gr'], p['loc'], df=p['df'], b1=p['b1'], gamma=p['gam']).to(f32)
+    if case == 'ckpt3':
+        monkeypatch.setenv('MRPHY_B200_CKPT', '3')
+    p = _random_problem(100 + nM, 2, nM, nT, 1, has_b1=True, relax=True, dtype=dtype)
+    beff = orc.rfgr2beff(p['rf'], p['gr'], p['loc'], df=p['df'], b1=p['b1'], gamma=p['gam']).to(dtype)
     Mo64, gM64, gB64 = orc.blochsim_adj(p['M0'], beff, p['w'], T1=p['T1'], T2=p['T2'], gamma=p['gam'], dt=p['dt'])
-    Mo32, _, _ = orc.blochsim_adj(p['M0'].to(f32), beff, p['w'].to(f32), T1=p['T1'].to(f32), T2=p['T2'].to(f32),
-                                  gamma=p['gam'].to(f32), dt=p['dt'].to(f32), dtype=f32)
-    M0 = p['M0'].to(dev, f32).requires_grad_(True)
-    B = beff.to(dev).requires_grad_(True)
-    assert (B.stride(1) * 4) % 16 == 0
-    Mo = sims.blochsim(M0, B, T1=p['T1'].to(dev, f32), T2=p['T2'].to(dev, f32), γ=p['gam'].to(dev), dt=p['dt'].to(dev))
-    (Mo * p['w'].to(dev, f32)).sum().backward()
-    assert mx(Mo, Mo64) < _fp32_bound(Mo32, Mo64)
-    assert rel(B.grad, gB64) < RTOL_G32 and rel(M0.grad, gM64) < RTOL_G32
+    if dtype == f32:
+        Mo32, _, _ = orc.blochsim_adj(p['M0'].to(f32), beff, p['w'].to(f32), T1=p['T1'].to(f32), T2=p['T2'].to(f32),
+                                      gamma=p['gam'].to(f32), dt=p['dt'].to(f32), dtype=f32)
+        tolM, tolG = _fp32_bound(Mo32, Mo64), RTOL_G32
+    else:
+        tolM, tolG = ATOL64, RTOL_G64
+    M0 = p['M0'].to(dev, dtype).requires_grad_(True)
+    off = 1 if case == 'offset' else 0
+    B = torch.empty(beff.numel() + off, dtype=dtype, device=dev)[off:].view(beff.shape)
+    B.copy_(beff)
+    B.requires_grad_(case != 'M0only')
+    es = B.element_size()
+    aligned = B.data_ptr() % 16 == 0 and (B.stride(1) * es) % 16 == 0 and (B.stride(0) * es) % 16 == 0
+    assert aligned == ((nT * 3 * es) % 16 == 0 and off == 0)     # the case runs the instantiation it was written for
+    Mo = sims.blochsim(M0, B, T1=p['T1'].to(dev, dtype), T2=p['T2'].to(dev, dtype), γ=p['gam'].to(dev), dt=p['dt'].to(dev))
+    (Mo * p['w'].to(dev, dtype)).sum().backward()
+    assert mx(Mo, Mo64) < tolM and rel(M0.grad, gM64) < tolG
+    if case == 'M0only':
+        assert B.grad is None
+    else:
+        assert rel(B.grad, gB64) < tolG
 
 
 def test_defaults_fp64_constants_with_fp32_state(dev):
@@ -553,8 +577,10 @@ def test_rfgr2beff_kernel_and_its_chain_rule(dev):
     from mrphy import beffective
     gen = torch.Generator().manual_seed(4)
     U = lambda *s: (torch.rand(s, generator=gen, dtype=f64) * 2 - 1)
-    for Nd, nC, has_b1 in (((7,), 2, True), ((3, 2, 2), 0, False), ((5,), 3, False), ((6,), 0, True)):
-        N, nT = 2, 9
+    # nT = 9 reads dL/dBeff rows straight from global memory; nT = 260 (two 256-step blocks) stages them by TMA
+    for (Nd, nC, has_b1), nT in itertools.product((((7,), 2, True), ((3, 2, 2), 0, False), ((5,), 3, False), ((6,), 0, True)),
+                                                  (9, 260)):
+        N = 2
         rf = U(N, 2, nT, nC) if nC else U(N, 2, nT)
         ins = dict(rf=rf, gr=U(N, 3, nT), loc=U(N, *Nd, 3) * 5, df=U(N, *Nd) * 100,
                    b1=(U(N, *Nd, 2, nC) if nC else U(N, *Nd, 2)) if has_b1 else None, gam=4257.6 * (1 + 0.1 * U(N, *Nd)))

@@ -262,6 +262,21 @@ typedef struct mrphy_spin_grad_args {
 int mrphy_blochsim_fused_bwd_spin(const mrphy_fused_args* a, int wave_is_packed, const mrphy_spin_grad_args* s,
                                   void* cuda_stream);
 
+/* The magnetisation during the pulse: the fused forward also writes the state after every `every` steps,
+ *   Mt[n][r][xyz][i] = M of spin i after (r+1)*every steps, r = 0 .. nR-1, nR = nT / every   (lab frame, like Mo)
+ * -- what mrphy_blochsim_fused_fwd returns as Mo for the pulse cut to its first (r+1)*every samples.  The backward takes
+ * dL/dMt in the same layout on top of dL/dMo.  Mo, ckpt and, in the backward, gMi, grf, ggr and the per-spin gradients
+ * (s, or NULL for none) mean what they mean for mrphy_blochsim_fused_fwd / _bwd / _bwd_spin; a->gMo is required (zeros
+ * when the loss ignores Mo).  Up to 16 transmit coils, like every fused entry.  No workspace beyond the existing ones. */
+typedef struct mrphy_record_args {
+  int32_t every, nR;     /* 1 <= every <= nT, nR == nT / every                              */
+  void* Mt;              /* fwd: out [N][nR][3][nM] contiguous, lab frame                    */
+  const void* gMt;       /* bwd: in, dL/dMt in the same layout                               */
+} mrphy_record_args;
+int mrphy_blochsim_fused_fwd_rec(const mrphy_fused_args* a, const mrphy_record_args* r, void* cuda_stream);
+int mrphy_blochsim_fused_bwd_rec(const mrphy_fused_args* a, int wave_is_packed, const mrphy_record_args* r,
+                                 const mrphy_spin_grad_args* s /* NULL: no per-spin gradients */, void* cuda_stream);
+
 /* Amplitude limits of the design loop (SURVEY 8f-2), replacing utils.rfclamp (utils.py:217-236) and utils.sclamp
  * (utils.py:278-293) and their autograd, one launch each way:
  *   kind 1  rf (N,2,nT,nC):  out = rf * min((rfmax[n,c] - eps) / |rf|, 1),  |rf| over the xy axis
@@ -297,7 +312,7 @@ int mrphy_mask_copy(const mrphy_mask_args* a, void* cuda_stream);
 /* sizeof() of the argument structs as this library was compiled, for bindings to check their mirror of the layout:
  * which = 0 mrphy_param, 1 mrphy_fused_args, 2 mrphy_beff_args, 3 mrphy_rfgr2beff_args, 4 mrphy_beff2ab_args,
  * 5 mrphy_beff2uphi_args, 6 mrphy_freeprec_args, 7 mrphy_reparam_args, 8 mrphy_mask_args, 9 mrphy_clamp_args,
- * 10 mrphy_spin_grad_args; 0 for any other value. */
+ * 10 mrphy_spin_grad_args, 11 mrphy_record_args; 0 for any other value. */
 size_t mrphy_sizeof_args(int which);
 
 /* Number of kernel launches the last forward / backward call on this thread issued. */

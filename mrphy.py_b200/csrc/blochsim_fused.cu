@@ -6,15 +6,19 @@
 // Kernels in this file
 //   pack_waveform_kernel      rf (N,2,nT[,nC]), gr (N,3,nT) -> wave[N][chunk][W][TCP]  (W = 2*NC+3)
 //   fused_fwd_kernel<T,..>    one spin, or two spins packed in an f2 (FFMA2), per thread; checkpoint every K steps
+//                             REC: also the state every `every` steps (Mt, rec_store)
 //   fused_bwd_kernel<T,..>    time-reversed state reconstruction + adjoint + spin reduction (only the gradient rows
 //                             asked for: ROWS); tiles owned through SM-aware virtual CTA ids (SCHED_*)
 //                             SG: also the per-spin sums over time behind dL/dloc, dL/ddf, dL/db1Map (sg_fold)
+//                             REC: dL/dMt joins the adjoint at the recorded steps (rec_load)
+//   fused_fwd_tc_kernel<..>   fp32, >= 4 coils: the transmit field on the tensor cores (below); REC as fused_fwd_kernel
 //   grad_finalize_kernel<T>   deterministic sum of the per-CTA partials, reference layout out (grad_finalize.cuh)
 //
 // Data layout in HBM (T = float | double):
 //   wave      [N][nChunks][W][TCP]   one chunk = K steps (TCP = K rounded up to 4): a chunk is
 //                                    ONE contiguous 16-byte-aligned block -> one 1-D TMA bulk copy
 //   ckpt      [N][nChunks-1][3][nM]  state after (c+1)*K steps, SoA so warps store 128-B lines
+//   Mt, gMt   [N][nR][3][nM]         REC: state after (r+1)*every steps (lab frame) and its gradient, SoA likewise
 //   partials  [N][P][W][nT]          gradient partial sums, one slot per (virtual) CTA id, P ids per batch entry;
 //                                    behind them 264 + P ints of scheduling state of the backward (SCHED_*)
 #include <cuda_runtime.h>
@@ -166,6 +170,13 @@ template <typename T> struct SgOut {
   T* gloc; T* gsz; T* gb1;
   bool any() const { return gloc || gsz || gb1; }
 };
+// recorded magnetisation of the REC kernels (mrphy_record_args): the forward writes Mt, the backward reads dL/dMt, both
+// [N][nR][3][nM] (SoA like the checkpoints), entry r = the state after (r+1)*every steps in the lab frame.  A kernel
+// parameter of its own behind the others, like SgOut.
+template <typename T> struct RecOut {
+  T* Mt; const T* gMt;
+  int every, nR;
+};
 
 // Scheduling workspace of the backward kernel (ints, zeroed before every launch; lives behind the partial sums).
 // The hardware spreads the P = c * n_sm co-resident CTAs breadth-first over the SMs, but not in blockIdx order (measured,
@@ -268,6 +279,40 @@ __device__ __forceinline__ void load_vec3_tile(const T* base, int64_t stride, in
   }
 }
 
+// REC forward: state r (lab frame) of PK spins -> Mt[n][r][xyz][spin], streaming stores as the checkpoints; padding
+// lanes store nothing
+template <typename T, typename V, int PK>
+__device__ __forceinline__ void rec_store(const RecOut<T>& o, int nM, int n, int r, const int (&idx)[PK], const bool (&ok)[PK],
+                                          V x, V y, V z) {
+  T* p = o.Mt + ((size_t)n * o.nR + r) * 3 * (size_t)nM;
+  if (ok[0]) {
+    __stcs(p + idx[0], getq<0>(x));
+    __stcs(p + (size_t)nM + idx[0], getq<0>(y));
+    __stcs(p + 2 * (size_t)nM + idx[0], getq<0>(z));
+  }
+  if (PK == 2 && ok[PK - 1]) {
+    __stcs(p + idx[PK - 1], getq<1>(x));
+    __stcs(p + (size_t)nM + idx[PK - 1], getq<1>(y));
+    __stcs(p + 2 * (size_t)nM + idx[PK - 1], getq<1>(z));
+  }
+}
+// REC backward: dL/dMt[r] of PK spins, turned into the spin frame; zero in padding lanes (their idx is a real spin)
+template <typename T, typename V, int NC, int PK>
+__device__ __forceinline__ void rec_load(const RecOut<T>& o, int nM, int n, int r, const int (&idx)[PK], const bool (&ok)[PK],
+                                         const SpinConst<V, NC>& k, V& x, V& y, V& z) {
+  const T* p = o.gMt + ((size_t)n * o.nR + r) * 3 * (size_t)nM;
+  T v[PK][3];
+#pragma unroll
+  for (int q = 0; q < PK; ++q) {
+#pragma unroll
+    for (int e = 0; e < 3; ++e) v[q][e] = ok[q] ? __ldcs(p + e * (size_t)nM + idx[q]) : (T)0;
+  }
+  x = mkv(v[0][0], v[PK - 1][0], (V*)nullptr);
+  y = mkv(v[0][1], v[PK - 1][1], (V*)nullptr);
+  z = mkv(v[0][2], v[PK - 1][2], (V*)nullptr);
+  to_frame(k, x, y);
+}
+
 // ------------------------------------------------------------------------------------------
 // pack: one thread per element of wave[N][nChunks][W][TCP]
 template <typename T>
@@ -303,8 +348,9 @@ __global__ void pack_waveform_kernel(const T* __restrict__ rf, int64_t rf_sn, in
 
 // ------------------------------------------------------------------------------------------
 // forward.  PK spins per thread (PK == 2: packed f2 arithmetic), BLKT threads per CTA.
-template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT>
-__global__ void __launch_bounds__(BLKT, (PK == 2 ? (NC == 1 ? 14 : MRPHY_NC2_MINB) : 1)) fused_fwd_kernel(const KArgs<T> a) {
+// REC: also the state after every `rec.every` steps (rec_store), tracked by a countdown (no per-step division).
+template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, bool REC = false>
+__global__ void __launch_bounds__(BLKT, (PK == 2 ? (NC == 1 ? 14 : MRPHY_NC2_MINB) : 1)) fused_fwd_kernel(const KArgs<T> a, const RecOut<T> rec) {
   typedef typename Pack<T, PK>::type V;
   constexpr int W = 2 * NC + 3;
   constexpr int WS = WaveLayout<T, W>::WS;
@@ -347,6 +393,7 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? (NC == 1 ? 14 : MRPHY_NC2_MIN
     }
     load_vec3_tile<T, V, PK, BLKT>(a.Mi + (int64_t)n * a.Mi_sn, a.Mi_sm, tile, nM, idx, scr, mx, my, mz);
     to_frame(k, mx, my);   // single coil: the spin's own transverse frame (bloch_math.cuh: make_consts); checkpoints stay in it
+    int rc = rec.every, rr = 0;   // REC: steps to the next recorded state, its index
     for (int c = 0; c < nChunks; ++c, ++it) {
       if (tid == 0 && it + 1 < total) {   // prefetch the next chunk (possibly chunk 0 of the next tile)
         const int cn = (c + 1 == nChunks) ? 0 : c + 1;
@@ -363,6 +410,14 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? (NC == 1 ? 14 : MRPHY_NC2_MIN
         for (int q = 0; q < NC; ++q) { rx[q] = V(s[q]); ry[q] = V(s[NC + q]); }
         field<V, NC>(k, rx, ry, V(s[2 * NC]), V(s[2 * NC + 1]), V(s[2 * NC + 2]), bx, by, bz);
         step_fwd<V, POL, RELAX>(bx, by, bz, k.e1, k.e2, mx, my, mz);
+        if constexpr (REC) {
+          if (--rc == 0) {   // recorded states leave the spin frame (a copy: the state stays in it)
+            V x = mx, y = my;
+            from_frame(k, x, y);
+            rec_store<T, V, PK>(rec, nM, n, rr++, idx, ok, x, y, mz);
+            rc = rec.every;
+          }
+        }
       };
       int j = 0;
       // 4 steps per iteration with 128-bit broadcast loads, while the staged samples fit ~40 registers
@@ -556,8 +611,10 @@ __device__ __forceinline__ void sg_fold(const KArgs<T>& a, const SgOut<T>& o, in
 // ROWS: which gradients the caller wants -- bit 0 dL/drf (rows [0, 2 NC)), bit 1 dL/dgr (rows [2 NC, W)); the other rows
 // of the spin reduction are neither formed nor reduced (an RF-only design skips 3 of its 5 rows).
 // SG: also the per-spin gradients (sg_fold).  ROWS == 0 (SG only, a fixed pulse): no transposition tile, no partial sums.
-template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, int ROWS = 3, bool SG = false>
-__global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : (sizeof(T) == 8 && NC == 1 ? 4 : (sizeof(T) == 4 && NC > 1 ? MRPHY_MC_MINB : 1)))) fused_bwd_kernel(const KArgs<T> a, const int need_gmi, const SgOut<T> sgo) {
+// REC: the loss also depends on the recorded states: dL/dMt[r] joins the adjoint before the adjoint of the step that
+// produced state r, so that everything downstream (F, the spin reduction, sg_fold, dL/dMi) sees the total dL/dm.
+template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, int ROWS = 3, bool SG = false, bool REC = false>
+__global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : (sizeof(T) == 8 && NC == 1 ? 4 : (sizeof(T) == 4 && NC > 1 ? MRPHY_MC_MINB : 1)))) fused_bwd_kernel(const KArgs<T> a, const int need_gmi, const SgOut<T> sgo, const RecOut<T> rec) {
   typedef typename Pack<T, PK>::type V;
   using L = BwdSmem<T, NC, BLKT, PK>;
   constexpr int W = L::W, TR = L::TR, NW = L::NW;
@@ -656,6 +713,14 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : 
       const V zm = mkv(z0, z1, (V*)nullptr);
       hx = hx * zm; hy = hy * zm; hz = hz * zm;
     }
+    // REC: steps (backwards from the end) before the last recorded state, its index, and its dL/dMt loaded one record ahead
+    int rc = 0, rr = 0;
+    V gx, gy, gz;
+    if constexpr (REC) {
+      rc = nT - rec.nR * rec.every;
+      rr = rec.nR - 1;
+      rec_load<T, V, NC, PK>(rec, nM, n, rr, idx, ok, k, gx, gy, gz);
+    }
     for (int c = nChunks - 1; c >= 0; --c, ++it) {
       if (tid == 0 && it + 1 < total) {
         const int cn = (c == 0) ? nChunks - 1 : c - 1;
@@ -681,6 +746,14 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : 
       }
       // one adjoint step; the W per-thread gradient contributions go to row `row` of the warp's tile
       auto one_step = [&](const T (&s)[W], int row) {
+        if constexpr (REC) {
+          if (rc == 0) {   // this step produced recorded state rr: h += dL/dMt[rr], then fetch the next one back in time
+            hx = hx + gx; hy = hy + gy; hz = hz + gz;
+            if (--rr >= 0) rec_load<T, V, NC, PK>(rec, nM, n, rr, idx, ok, k, gx, gy, gz);
+            rc = rec.every;
+          }
+          --rc;
+        }
         V rx[NC], ry[NC], bx, by, bz, Fx, Fy, Fz;
 #pragma unroll
         for (int q = 0; q < NC; ++q) { rx[q] = V(s[q]); ry[q] = V(s[NC + q]); }
@@ -977,8 +1050,9 @@ __device__ __forceinline__ void tc_issue(const float* sa, const float* wb, int r
     tc_issue<NC, PK>(sa, wbuf[(it + 1) % NST], rows, tmem + ((it + 1) % NBUF) * C::BUF_COLS, &mma_bar[(it + 1) % NBUF]);    \
   }
 
-template <int POL, bool RELAX, int NC, int PK>
-__global__ void __launch_bounds__(128, (NC <= 8 ? 4 : (PK == 1 ? 3 : 2))) fused_fwd_tc_kernel(const KArgs<float> a) {
+// REC as in fused_fwd_kernel (this kernel has no spin frame: the state is in the lab frame throughout)
+template <int POL, bool RELAX, int NC, int PK, bool REC = false>
+__global__ void __launch_bounds__(128, (NC <= 8 ? 4 : (PK == 1 ? 3 : 2))) fused_fwd_tc_kernel(const KArgs<float> a, const RecOut<float> rec) {
   using L = TcLayout<NC>;
   using C = TcCfg<NC, PK>;
   typedef float T;
@@ -1045,6 +1119,7 @@ __global__ void __launch_bounds__(128, (NC <= 8 ? 4 : (PK == 1 ? 3 : 2))) fused_
     tc::fence_before_sync();
     __syncthreads();
     const V glx = k.glx, gly = k.gly, glz = k.glz, gbz0 = k.gbz0, e1 = k.e1, e2 = k.e2;
+    int rc = rec.every, rr = 0;   // REC: steps to the next recorded state, its index
     for (int c = 0; c < nChunks; ++c, ++it) {
       TC_CHUNK_BEGIN(FWD_CHUNK_OF, c == 0, c + 1 < nChunks)
       const float* gw = wbuf[it % NST] + (size_t)2 * L::KC * rows * 4;   // gr rows [3][TCP]
@@ -1064,6 +1139,12 @@ __global__ void __launch_bounds__(128, (NC <= 8 ? 4 : (PK == 1 ? 3 : 2))) fused_
             const V bz = fma_(glx, V(g[0][u]), fma_(gly, V(g[1][u]), fma_(glz, V(g[2][u]), gbz0)));
             const V bx = mkv(b[0][2 * u], b[PK - 1][2 * u], (V*)nullptr), by = mkv(b[0][2 * u + 1], b[PK - 1][2 * u + 1], (V*)nullptr);
             step_fwd<V, POL, RELAX>(bx, by, bz, e1, e2, mx, my, mz);
+            if constexpr (REC) {
+              if (--rc == 0) {
+                rec_store<T, V, PK>(rec, nM, n, rr++, idx, ok, mx, my, mz);
+                rc = rec.every;
+              }
+            }
           }
         }
       };
@@ -1393,24 +1474,29 @@ int launch_pack(const mrphy_fused_args* a, const Plan& p, cudaStream_t st, bool 
 // P (CTAs per batch entry) actually launched by the last backward kernel; the finalize kernel needs it
 thread_local int g_last_P = 0;
 
-template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT>
-int launch_fwd_s(KArgs<T> k, const Plan& p, cudaStream_t st) {
-  auto kern = fused_fwd_kernel<T, POL, RELAX, NC, PK, BLKT>;
+template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, bool REC = false>
+int launch_fwd_s(KArgs<T> k, const Plan& p, cudaStream_t st, const RecOut<T>& rec = RecOut<T>{}) {
+  auto kern = fused_fwd_kernel<T, POL, RELAX, NC, PK, BLKT, REC>;
   int occ = 0;
   CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, BLKT, 0));
   k.P = pick_ctas(p, k.N, occ, false, BLKT / 32);
   dim3 grid(k.P, k.N);
+  if (REC && getenv("MRPHY_B200_DEBUG"))
+    fprintf(stderr, "[mrphy_b200] fused_fwd<%s,NC=%d,PK=%d,BLK=%d,%s,REC=1> grid=(%d,%d) tiles=%d occ=%d K=%d every=%d\n",
+            sizeof(T) == 4 ? "f32" : "f64", NC, PK, BLKT, POL == TRIG_PRECISE ? "precise" : "fast", k.P, k.N, p.tiles, occ, p.K,
+            rec.every);
   timing_begin(st);
-  kern<<<grid, BLKT, 0, st>>>(k);
+  kern<<<grid, BLKT, 0, st>>>(k, rec);
   timing_end(st);
   ++g_launches;
   CK(cudaGetLastError());
   return MRPHY_OK;
 }
-template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, int ROWS = 3, bool SG = false>
-int launch_bwd_s(KArgs<T> k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg = SgOut<T>{}) {
+template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, int ROWS = 3, bool SG = false, bool REC = false>
+int launch_bwd_s(KArgs<T> k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg = SgOut<T>{},
+                 const RecOut<T>& rec = RecOut<T>{}) {
   constexpr size_t smem = BwdSmem<T, NC, BLKT, PK>::bytes;
-  auto kern = fused_bwd_kernel<T, POL, RELAX, NC, PK, BLKT, ROWS, SG>;
+  auto kern = fused_bwd_kernel<T, POL, RELAX, NC, PK, BLKT, ROWS, SG, REC>;
   CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   // static + dynamic may exceed 48 KB
   int occ = 0;
   CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, BLKT, smem));
@@ -1431,11 +1517,11 @@ int launch_bwd_s(KArgs<T> k, const Plan& p, int need_gmi, cudaStream_t st, const
     CK(cudaMemsetAsync(k.sched, 0, sizeof(int) * (size_t)(SCHED_CLAIM + k.P), st));
   }
   if (getenv("MRPHY_B200_DEBUG"))
-    fprintf(stderr, "[mrphy_b200] fused_bwd<%s,NC=%d,PK=%d,BLK=%d,%s,ROWS=%d,SG=%d> grid=(%d,%d) tiles=%d occ=%d smem=%zu K=%d\n",
-            sizeof(T) == 4 ? "f32" : "f64", NC, PK, BLKT, POL == TRIG_PRECISE ? "precise" : "fast", ROWS, (int)SG, k.P, k.N,
-            q.tiles, occ, smem, p.K);
+    fprintf(stderr, "[mrphy_b200] fused_bwd<%s,NC=%d,PK=%d,BLK=%d,%s,ROWS=%d,SG=%d%s> grid=(%d,%d) tiles=%d occ=%d smem=%zu K=%d\n",
+            sizeof(T) == 4 ? "f32" : "f64", NC, PK, BLKT, POL == TRIG_PRECISE ? "precise" : "fast", ROWS, (int)SG,
+            REC ? ",REC=1" : "", k.P, k.N, q.tiles, occ, smem, p.K);
   timing_begin(st);
-  kern<<<grid, BLKT, smem, st>>>(k, need_gmi, sg);
+  kern<<<grid, BLKT, smem, st>>>(k, need_gmi, sg, rec);
   timing_end(st);
   ++g_launches;
   CK(cudaGetLastError());
@@ -1464,11 +1550,11 @@ int tc_occupancy(Kern kern, size_t dyn_smem, int tmem_cols) {
 }
 
 // tensor-core multi-coil kernels (fp32): at most 4 CTAs per SM, each owns 128 of the 512 TMEM columns
-template <int POL, bool RELAX, int NC, int PK>
-int launch_fwd_tc_pk(KArgs<float> k, const Plan& p, cudaStream_t st) {
+template <int POL, bool RELAX, int NC, int PK, bool REC = false>
+int launch_fwd_tc_pk(KArgs<float> k, const Plan& p, cudaStream_t st, const RecOut<float>& rec) {
   using C = TcCfg<NC, PK>;
   constexpr size_t smem = C::bytes;
-  auto kern = fused_fwd_tc_kernel<POL, RELAX, NC, PK>;
+  auto kern = fused_fwd_tc_kernel<POL, RELAX, NC, PK, REC>;
   CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   k.TCP = p.tc_TCP;
   k.chunk_elems = p.tc_chunk_elems;
@@ -1479,46 +1565,50 @@ int launch_fwd_tc_pk(KArgs<float> k, const Plan& p, cudaStream_t st) {
   if (k.P > tiles) k.P = tiles;
   dim3 grid(k.P, k.N);
   if (getenv("MRPHY_B200_DEBUG"))
-    fprintf(stderr, "[mrphy_b200] fused_fwd_tc<NC=%d,PK=%d> grid=(%d,%d) tiles=%d occ=%d smem=%zu K=%d\n", NC, PK, k.P, k.N, tiles, occ, smem, p.K);
+    fprintf(stderr, "[mrphy_b200] fused_fwd_tc<NC=%d,PK=%d%s> grid=(%d,%d) tiles=%d occ=%d smem=%zu K=%d\n", NC, PK,
+            REC ? ",REC=1" : "", k.P, k.N, tiles, occ, smem, p.K);
   timing_begin(st);
-  kern<<<grid, 128, smem, st>>>(k);
+  kern<<<grid, 128, smem, st>>>(k, rec);
   timing_end(st);
   ++g_launches;
   CK(cudaGetLastError());
   return MRPHY_OK;
 }
-template <int POL, bool RELAX, int NC>
-int launch_fwd_tc(const KArgs<float>& k, const Plan& p, cudaStream_t st) {
+template <int POL, bool RELAX, int NC, bool REC = false>
+int launch_fwd_tc(const KArgs<float>& k, const Plan& p, cudaStream_t st, const RecOut<float>& rec) {
   // two spin tiles per CTA (packed f2 step): measured 3 % (4, 8 coils) to 17 % (16 coils) faster than one tile with two TMEM
   // buffers; a build with -DMRPHY_TC_SCALAR also carries the one-tile kernels (MRPHY_B200_TC_PACK=1) for measurements
 #ifdef MRPHY_TC_SCALAR
-  if (env_int("MRPHY_B200_TC_PACK", 2) == 1) return launch_fwd_tc_pk<POL, RELAX, NC, 1>(k, p, st);
+  if (env_int("MRPHY_B200_TC_PACK", 2) == 1) return launch_fwd_tc_pk<POL, RELAX, NC, 1, REC>(k, p, st, rec);
 #endif
-  return launch_fwd_tc_pk<POL, RELAX, NC, 2>(k, p, st);
+  return launch_fwd_tc_pk<POL, RELAX, NC, 2, REC>(k, p, st, rec);
 }
 // backward with per-spin gradients: the ROWS == 0 kernel when no waveform gradient is wanted, else all rows (the finalize
 // reads only the wanted ones)
-template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT>
-int launch_bwd_sg(const KArgs<T>& k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg) {
-  return p.rows == 0 ? launch_bwd_s<T, POL, RELAX, NC, PK, BLKT, 0, true>(k, p, need_gmi, st, sg)
-                     : launch_bwd_s<T, POL, RELAX, NC, PK, BLKT, 3, true>(k, p, need_gmi, st, sg);
+template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, bool REC = false>
+int launch_bwd_sg(const KArgs<T>& k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg, const RecOut<T>& rec) {
+  return p.rows == 0 ? launch_bwd_s<T, POL, RELAX, NC, PK, BLKT, 0, true, REC>(k, p, need_gmi, st, sg, rec)
+                     : launch_bwd_s<T, POL, RELAX, NC, PK, BLKT, 3, true, REC>(k, p, need_gmi, st, sg, rec);
 }
-template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT>
-int launch_any(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg) {
-  if (bwd && sg.any()) return launch_bwd_sg<T, POL, RELAX, NC, PK, BLKT>(k, p, need_gmi, st, sg);
-  return bwd ? launch_bwd_s<T, POL, RELAX, NC, PK, BLKT>(k, p, need_gmi, st)
-             : launch_fwd_s<T, POL, RELAX, NC, PK, BLKT>(k, p, st);
+template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, bool REC = false>
+int launch_any(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg,
+               const RecOut<T>& rec) {
+  if (bwd && sg.any()) return launch_bwd_sg<T, POL, RELAX, NC, PK, BLKT, REC>(k, p, need_gmi, st, sg, rec);
+  return bwd ? launch_bwd_s<T, POL, RELAX, NC, PK, BLKT, 3, false, REC>(k, p, need_gmi, st, sg, rec)
+             : launch_fwd_s<T, POL, RELAX, NC, PK, BLKT, REC>(k, p, st, rec);
 }
 
-template <typename T, int POL, bool RELAX>
-int dispatch_nc(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg) {
+// REC: the recording kernels (RecOut set), instantiated only here
+template <typename T, int POL, bool RELAX, bool REC = false>
+int dispatch_nc(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg,
+                const RecOut<T>& rec = RecOut<T>{}) {
   if constexpr (sizeof(T) == 4) {
     if (p.PK == 2) {
-      if (!bwd) return launch_fwd_s<T, POL, RELAX, 1, 2, 64>(k, p, st);
-      if (sg.any()) return launch_bwd_sg<T, POL, RELAX, 1, 2, MRPHY_BWD_BLKT>(k, p, need_gmi, st, sg);
-      if (p.rows == 1) return launch_bwd_s<T, POL, RELAX, 1, 2, MRPHY_BWD_BLKT, 1>(k, p, need_gmi, st);   // dL/drf only
-      if (p.rows == 2) return launch_bwd_s<T, POL, RELAX, 1, 2, MRPHY_BWD_BLKT, 2>(k, p, need_gmi, st);   // dL/dgr only
-      return launch_bwd_s<T, POL, RELAX, 1, 2, MRPHY_BWD_BLKT>(k, p, need_gmi, st);
+      if (!bwd) return launch_fwd_s<T, POL, RELAX, 1, 2, 64, REC>(k, p, st, rec);
+      if (sg.any()) return launch_bwd_sg<T, POL, RELAX, 1, 2, MRPHY_BWD_BLKT, REC>(k, p, need_gmi, st, sg, rec);
+      if (p.rows == 1) return launch_bwd_s<T, POL, RELAX, 1, 2, MRPHY_BWD_BLKT, 1, false, REC>(k, p, need_gmi, st, sg, rec);   // dL/drf only
+      if (p.rows == 2) return launch_bwd_s<T, POL, RELAX, 1, 2, MRPHY_BWD_BLKT, 2, false, REC>(k, p, need_gmi, st, sg, rec);   // dL/dgr only
+      return launch_bwd_s<T, POL, RELAX, 1, 2, MRPHY_BWD_BLKT, 3, false, REC>(k, p, need_gmi, st, sg, rec);
     }
   }
 #ifdef MRPHY_ONLY_PK2   /* tuning builds (profiles/operand_model.py): compile the default fp32 kernels only */
@@ -1527,18 +1617,18 @@ int dispatch_nc(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaSt
   if constexpr (sizeof(T) == 4) {
     // forward with 2 coils: two spins per thread (FFMA2) like the single-coil kernel; same tiles of 128 spins, same staging
     if (p.NC == 2 && env_int("MRPHY_B200_NC2_PACK", 2) == 2) {
-      if (!bwd) return launch_fwd_s<T, POL, RELAX, 2, 2, 64>(k, p, st);
+      if (!bwd) return launch_fwd_s<T, POL, RELAX, 2, 2, 64, REC>(k, p, st, rec);
       if (env_int("MRPHY_B200_NC2_PACK_BWD", 2) == 2) {
-        if (sg.any()) return launch_bwd_sg<T, POL, RELAX, 2, 2, MRPHY_BWD_BLKT>(k, p, need_gmi, st, sg);
-        if (p.rows == 1) return launch_bwd_s<T, POL, RELAX, 2, 2, MRPHY_BWD_BLKT, 1>(k, p, need_gmi, st);
-        if (p.rows == 2) return launch_bwd_s<T, POL, RELAX, 2, 2, MRPHY_BWD_BLKT, 2>(k, p, need_gmi, st);
-        return launch_bwd_s<T, POL, RELAX, 2, 2, MRPHY_BWD_BLKT>(k, p, need_gmi, st);
+        if (sg.any()) return launch_bwd_sg<T, POL, RELAX, 2, 2, MRPHY_BWD_BLKT, REC>(k, p, need_gmi, st, sg, rec);
+        if (p.rows == 1) return launch_bwd_s<T, POL, RELAX, 2, 2, MRPHY_BWD_BLKT, 1, false, REC>(k, p, need_gmi, st, sg, rec);
+        if (p.rows == 2) return launch_bwd_s<T, POL, RELAX, 2, 2, MRPHY_BWD_BLKT, 2, false, REC>(k, p, need_gmi, st, sg, rec);
+        return launch_bwd_s<T, POL, RELAX, 2, 2, MRPHY_BWD_BLKT, 3, false, REC>(k, p, need_gmi, st, sg, rec);
       }
     }
     if (p.tc && !bwd) {   // forward with >= 4 coils: transmit field on the tensor cores
-      if (p.NC == 4) return launch_fwd_tc<POL, RELAX, 4>(k, p, st);
-      if (p.NC == 8) return launch_fwd_tc<POL, RELAX, 8>(k, p, st);
-      return launch_fwd_tc<POL, RELAX, 16>(k, p, st);
+      if (p.NC == 4) return launch_fwd_tc<POL, RELAX, 4, REC>(k, p, st, rec);
+      if (p.NC == 8) return launch_fwd_tc<POL, RELAX, 8, REC>(k, p, st, rec);
+      return launch_fwd_tc<POL, RELAX, 16, REC>(k, p, st, rec);
     }
   }
   switch (p.NC) {
@@ -1547,25 +1637,41 @@ int dispatch_nc(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaSt
       if constexpr (sizeof(T) == 4) return fail(MRPHY_ERR_ARG, "internal: fp32 single-coil scalar kernels not built%s");
       else
 #endif
-      return launch_any<T, POL, RELAX, 1, 1, 128>(bwd, k, p, need_gmi, st, sg);
-    case 2: return launch_any<T, POL, RELAX, 2, 1, 128>(bwd, k, p, need_gmi, st, sg);
-    case 4: return launch_any<T, POL, RELAX, 4, 1, 128>(bwd, k, p, need_gmi, st, sg);
-    case 8: return launch_any<T, POL, RELAX, 8, 1, 128>(bwd, k, p, need_gmi, st, sg);
-    case 16: return launch_any<T, POL, RELAX, 16, 1, 128>(bwd, k, p, need_gmi, st, sg);
+      return launch_any<T, POL, RELAX, 1, 1, 128, REC>(bwd, k, p, need_gmi, st, sg, rec);
+    case 2: return launch_any<T, POL, RELAX, 2, 1, 128, REC>(bwd, k, p, need_gmi, st, sg, rec);
+    case 4: return launch_any<T, POL, RELAX, 4, 1, 128, REC>(bwd, k, p, need_gmi, st, sg, rec);
+    case 8: return launch_any<T, POL, RELAX, 8, 1, 128, REC>(bwd, k, p, need_gmi, st, sg, rec);
+    case 16: return launch_any<T, POL, RELAX, 16, 1, 128, REC>(bwd, k, p, need_gmi, st, sg, rec);
   }
   return fail(MRPHY_ERR_ARG, "internal: bad NC%s");
 #endif
 }
 
+// the recording kernels: fp64 has one trigonometry (TRIG_FAST names it), so only fp32 instantiates both
+template <typename T>
+int dispatch_rec(bool bwd, const KArgs<T>& k, const Plan& p, bool relax, bool precise, int need_gmi, cudaStream_t st,
+                 const SgOut<T>& so, const RecOut<T>& ro) {
+  if constexpr (sizeof(T) == 4) {
+    if (precise)
+      return relax ? dispatch_nc<T, TRIG_PRECISE, true, true>(bwd, k, p, need_gmi, st, so, ro)
+                   : dispatch_nc<T, TRIG_PRECISE, false, true>(bwd, k, p, need_gmi, st, so, ro);
+  }
+  return relax ? dispatch_nc<T, TRIG_FAST, true, true>(bwd, k, p, need_gmi, st, so, ro)
+               : dispatch_nc<T, TRIG_FAST, false, true>(bwd, k, p, need_gmi, st, so, ro);
+}
+
 template <typename T>
 int dispatch(bool bwd, const mrphy_fused_args* a, const Plan& p, cudaStream_t st, int* done = nullptr,
-             const mrphy_spin_grad_args* sg = nullptr) {
+             const mrphy_spin_grad_args* sg = nullptr, const mrphy_record_args* rec = nullptr) {
   KArgs<T> k = make_kargs<T>(a, p);
   k.done = done;
   const SgOut<T> so = sg ? SgOut<T>{(T*)sg->gloc, (T*)sg->gsz, (T*)sg->gb1} : SgOut<T>{};
   const bool relax = a->T1.ptr != nullptr;
   const bool precise = (a->flags & MRPHY_TRIG_PRECISE) != 0 && sizeof(T) == 4 && !(bwd && (a->flags & MRPHY_TRIG_FAST_BWD));
   const int need_gmi = (a->flags & MRPHY_NEED_GMI) ? 1 : 0;
+  if (rec)
+    return dispatch_rec<T>(bwd, k, p, relax, precise, need_gmi, st, so,
+                           RecOut<T>{(T*)rec->Mt, (const T*)rec->gMt, rec->every, rec->nR});
   if (precise) {
     return relax ? dispatch_nc<T, TRIG_PRECISE, true>(bwd, k, p, need_gmi, st, so)
                  : dispatch_nc<T, TRIG_PRECISE, false>(bwd, k, p, need_gmi, st, so);
@@ -1574,14 +1680,23 @@ int dispatch(bool bwd, const mrphy_fused_args* a, const Plan& p, cudaStream_t st
                : dispatch_nc<T, TRIG_FAST, false>(bwd, k, p, need_gmi, st, so);
 }
 
+// the record stride and its buffer (Mt for the forward, gMt for the backward)
+int check_record(const mrphy_fused_args* a, const mrphy_record_args* r, bool bwd) {
+  if (r->every < 1 || r->every > a->nT || r->nR != a->nT / r->every)
+    return fail(MRPHY_ERR_ARG, "record: need 1 <= every <= nT and nR == nT / every%s");
+  if (bwd ? !r->gMt : !r->Mt) return fail(MRPHY_ERR_ARG, bwd ? "record: gMt is null%s" : "record: Mt is null%s");
+  return MRPHY_OK;
+}
+
 template <typename T>
-int run_fwd(const mrphy_fused_args* a, cudaStream_t st) {
+int run_fwd(const mrphy_fused_args* a, cudaStream_t st, const mrphy_record_args* rec = nullptr) {
   Plan p;
   int rc = make_plan(a, &p, true);
   if (rc) return rc;
   if ((rc = check_common<T>(a, false))) return rc;
+  if (rec && (rc = check_record(a, rec, false))) return rc;
   if ((rc = launch_pack<T>(a, p, st, p.tc != 0))) return rc;
-  return dispatch<T>(false, a, p, st);
+  return dispatch<T>(false, a, p, st, nullptr, nullptr, rec);
 }
 
 // the re-parametrisation the design tail can take: adjoint of an rf half and/or a gradient half that ends in a gradient
@@ -1604,19 +1719,20 @@ int check_design(const mrphy_fused_args* a, const mrphy_reparam_args* d) {
 
 template <typename T>
 int run_bwd(const mrphy_fused_args* a, int wave_is_packed, const mrphy_reparam_args* d, cudaStream_t st,
-            const mrphy_spin_grad_args* sg = nullptr) {
+            const mrphy_spin_grad_args* sg = nullptr, const mrphy_record_args* rec = nullptr) {
   Plan p;
   int rc = make_plan(a, &p, true);
   if (rc) return rc;
   if ((rc = check_common<T>(a, true))) return rc;
   if (d && (rc = check_design(a, d))) return rc;
+  if (rec && (rc = check_record(a, rec, true))) return rc;
   if (sg && !sg->gloc && !sg->gsz && !sg->gb1) return fail(MRPHY_ERR_ARG, "spin gradients: gloc, gsz, gb1 are all null%s");
   if (sg && sg->gb1 && !a->b1) return fail(MRPHY_ERR_ARG, "spin gradients: gb1 needs b1%s");
   // (after a tensor-core forward `wave` holds that kernel's operand tiles: the backward stages its own layout over them)
   if ((!wave_is_packed || p.tc) && (rc = launch_pack<T>(a, p, st))) return rc;
   // finished-CTA counters of the design tail: behind the scheduling ints, zeroed by the backward kernel itself
   int* const done = d ? reinterpret_cast<int*>((T*)a->partials + (size_t)a->N * p.Pmax * p.W * (size_t)a->nT) + SCHED_CLAIM + p.Pmax : nullptr;
-  if ((rc = dispatch<T>(true, a, p, st, done, sg))) return rc;
+  if ((rc = dispatch<T>(true, a, p, st, done, sg, rec))) return rc;
   if (sg && p.rows == 0) return MRPHY_OK;   // per-spin gradients only: nothing to finalize
   dim3 grid((a->nT + 31) / 32, p.W, a->N), block(32, 32);
   const int coil_dim = (a->flags & MRPHY_RF_COIL_DIM) ? 1 : 0;
@@ -1672,4 +1788,22 @@ extern "C" int mrphy_blochsim_fused_bwd_spin(const mrphy_fused_args* a, int wave
   cudaStream_t st = (cudaStream_t)cuda_stream;
   return a->dtype == MRPHY_F64 ? run_bwd<double>(a, wave_is_packed, nullptr, st, s)
                                : run_bwd<float>(a, wave_is_packed, nullptr, st, s);
+}
+
+extern "C" int mrphy_blochsim_fused_fwd_rec(const mrphy_fused_args* a, const mrphy_record_args* r, void* cuda_stream) {
+  g_launches = 0;
+  g_err[0] = 0;
+  if (!a || !r) return fail(MRPHY_ERR_ARG, "null args%s");
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  return a->dtype == MRPHY_F64 ? run_fwd<double>(a, st, r) : run_fwd<float>(a, st, r);
+}
+
+extern "C" int mrphy_blochsim_fused_bwd_rec(const mrphy_fused_args* a, int wave_is_packed, const mrphy_record_args* r,
+                                            const mrphy_spin_grad_args* s, void* cuda_stream) {
+  g_launches = 0;
+  g_err[0] = 0;
+  if (!a || !r) return fail(MRPHY_ERR_ARG, "null args%s");
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  return a->dtype == MRPHY_F64 ? run_bwd<double>(a, wave_is_packed, nullptr, st, s, r)
+                               : run_bwd<float>(a, wave_is_packed, nullptr, st, s, r);
 }

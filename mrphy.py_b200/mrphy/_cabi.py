@@ -122,6 +122,10 @@ class SpinGradArgs(ctypes.Structure):
     _fields_ = [('gloc', c_vp), ('gsz', c_vp), ('gb1', c_vp)]
 
 
+class RecordArgs(ctypes.Structure):
+    _fields_ = [('every', c_i32), ('nR', c_i32), ('Mt', c_vp), ('gMt', c_vp)]
+
+
 EXPORTS = {   # name -> (restype, argtypes); tests check every symbol include/mrphy_b200.h declares
     'mrphy_abi_version': (ctypes.c_int, []),
     'mrphy_last_error': (ctypes.c_char_p, []),
@@ -137,6 +141,9 @@ EXPORTS = {   # name -> (restype, argtypes); tests check every symbol include/mr
     'mrphy_blochsim_fused_bwd': (ctypes.c_int, [ctypes.POINTER(FusedArgs), ctypes.c_int, c_vp]),
     'mrphy_blochsim_fused_bwd_design': (ctypes.c_int, [ctypes.POINTER(FusedArgs), ctypes.c_int, ctypes.POINTER(ReparamArgs), c_vp]),
     'mrphy_blochsim_fused_bwd_spin': (ctypes.c_int, [ctypes.POINTER(FusedArgs), ctypes.c_int, ctypes.POINTER(SpinGradArgs), c_vp]),
+    'mrphy_blochsim_fused_fwd_rec': (ctypes.c_int, [ctypes.POINTER(FusedArgs), ctypes.POINTER(RecordArgs), c_vp]),
+    'mrphy_blochsim_fused_bwd_rec': (ctypes.c_int, [ctypes.POINTER(FusedArgs), ctypes.c_int, ctypes.POINTER(RecordArgs),
+                                                    ctypes.POINTER(SpinGradArgs), c_vp]),
     'mrphy_beff_ckpt_elems': (ctypes.c_size_t, [ctypes.POINTER(BeffArgs)]),
     'mrphy_blochsim_beff_fwd': (ctypes.c_int, [ctypes.POINTER(BeffArgs), c_vp]),
     'mrphy_blochsim_beff_bwd': (ctypes.c_int, [ctypes.POINTER(BeffArgs), c_vp]),
@@ -178,7 +185,7 @@ def lib():
                     raise RuntimeError(f'mrphy (B200): ABI version mismatch: library {L.mrphy_abi_version()} '
                                        f'!= binding {ABI_VERSION}; rebuild with mrphy.py_b200/build.py')
                 mirrors = (Param, FusedArgs, BeffArgs, RfGr2BeffArgs, Beff2abArgs, Beff2uphiArgs, FreePrecArgs, ReparamArgs,
-                           MaskArgs, ClampArgs, SpinGradArgs)
+                           MaskArgs, ClampArgs, SpinGradArgs, RecordArgs)
                 for which, cls in enumerate(mirrors):
                     if L.mrphy_sizeof_args(which) != ctypes.sizeof(cls):
                         raise RuntimeError(f'mrphy (B200): layout of {cls.__name__} ({ctypes.sizeof(cls)} B) differs from '

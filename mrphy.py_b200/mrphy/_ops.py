@@ -5,6 +5,7 @@ with ``beffective.rfgr2beff`` (beffective.py:107-168) followed by ``sims.BlochSi
 ``.backward`` (sims.py:31-269) and the autograd of ``rfgr2beff``.  ``fused_applypulse`` is the
 Python-level entry used by ``mobjs.SpinArray.applypulse`` (mobjs.py:394-450).
 """
+import numbers
 import os
 import weakref
 from typing import Optional, Tuple
@@ -166,10 +167,12 @@ def _fake_blochsim_fused_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flag
             Mi.new_empty((N * chunks * chunk,)))
 
 
-def _fused_bwd_call(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, design=None, spin=None):
+def _fused_bwd_call(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, design=None, spin=None, rec=None):
     """The backward launch sequence; `design` = (rho, theta, rfmax, ts, smax, ddt, rf_kind, gr_kind) adds the adjoint of the
     re-parametrisation to the gradient epilogue (mrphy_blochsim_fused_bwd_design), `spin` = (want_loc, want_sz, want_b1) the
-    per-spin gradients (mrphy_blochsim_fused_bwd_spin).  -> (gMi, flat, grho, gtheta, gts) | (gMi, flat, gloc, gsz, gb1)."""
+    per-spin gradients (mrphy_blochsim_fused_bwd_spin), `rec` = (every, gMt) the gradient of the recorded states
+    (mrphy_blochsim_fused_bwd_rec, with or without `spin`).
+    -> (gMi, flat, grho, gtheta, gts) | (gMi, flat, gloc, gsz, gb1)."""
     L = _cabi.lib()
     a = _cabi.FusedArgs()
     _fill_common(a, None, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags)
@@ -194,15 +197,23 @@ def _fused_bwd_call(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt,
     a.gMi, a.grf, a.ggr, a.partials = (gMi.data_ptr() if need_gmi else None), (grf.data_ptr() if want_rf else None), \
         (ggr.data_ptr() if want_gr else None), partials.data_ptr()
     grho = gtheta = gts = flat[:0]
-    if spin is not None:
-        want_loc, want_sz, want_b1 = spin
+    if spin is not None or rec is not None:
+        want_loc, want_sz, want_b1 = spin if spin is not None else (False, False, False)
         e = lambda shape, on: torch.empty(shape if on else (0,), **kw)
         gloc, gsz, gb1 = e((a.N, a.nM, 3), want_loc), e((a.N, a.nM), want_sz), e((a.N, a.nM, 2, a.nC), want_b1)
-        s = _cabi.SpinGradArgs()
-        s.gloc, s.gsz, s.gb1 = (gloc.data_ptr() if want_loc else None), (gsz.data_ptr() if want_sz else None), \
-            (gb1.data_ptr() if want_b1 else None)
+        s = None
+        if want_loc or want_sz or want_b1:
+            s = _cabi.SpinGradArgs()
+            s.gloc, s.gsz, s.gb1 = (gloc.data_ptr() if want_loc else None), (gsz.data_ptr() if want_sz else None), \
+                (gb1.data_ptr() if want_b1 else None)
         with torch.cuda.device(Mo.device):
-            _cabi.check(L.mrphy_blochsim_fused_bwd_spin(a, 1, s, _stream()), 'blochsim_fused_bwd_spin')
+            if rec is None:
+                _cabi.check(L.mrphy_blochsim_fused_bwd_spin(a, 1, s, _stream()), 'blochsim_fused_bwd_spin')
+            else:
+                every, gMt = rec
+                r = _cabi.RecordArgs()
+                r.every, r.nR, r.gMt = every, a.nT // every, gMt.data_ptr()
+                _cabi.check(L.mrphy_blochsim_fused_bwd_rec(a, 1, r, s, _stream()), 'blochsim_fused_bwd_rec')
         _cabi.count_launches()
         return gMi, flat, gloc, gsz, gb1
     if design is None:
@@ -250,6 +261,49 @@ def _impl_blochsim_fused_bwd_spin(gMo: Tensor, Mo: Tensor, ckpt: Tensor, wave: T
     kernel without the dense field.  want_b1 needs b1."""
     return _fused_bwd_call(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags,
                            spin=(bool(want_loc), bool(want_sz), bool(want_b1)))
+
+
+def _impl_blochsim_fused_fwd_rec(Mi: Tensor, rf: Tensor, gr: Tensor, loc: Tensor, df: Optional[Tensor], b1: Optional[Tensor],
+                                 T1: Optional[Tensor], T2: Optional[Tensor], gamma: Tensor, dt: Tensor, K: int, flags: int,
+                                 every: int) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """As blochsim_fused_fwd, plus Mt (N, nR, 3, nM), nR = nT // every: the state after (r+1)*every steps, lab frame.
+    -> (Mo, Mt, ckpt, wave)."""
+    L = _cabi.lib()
+    a = _cabi.FusedArgs()
+    _fill_common(a, Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags)
+    kw = {'dtype': Mi.dtype, 'device': Mi.device}
+    Mo = torch.empty((a.N, a.nM, 3), **kw)
+    Mt = torch.empty((a.N, a.nT // every, 3, a.nM), **kw)
+    ckpt = torch.empty(L.mrphy_fused_ckpt_elems(a), **kw)
+    wave = torch.empty(L.mrphy_fused_wave_elems(a), **kw)
+    a.Mo, a.ckpt, a.wave = Mo.data_ptr(), ckpt.data_ptr(), wave.data_ptr()
+    r = _cabi.RecordArgs()
+    r.every, r.nR, r.Mt = every, a.nT // every, Mt.data_ptr()
+    with torch.cuda.device(Mi.device):
+        _cabi.check(L.mrphy_blochsim_fused_fwd_rec(a, r, _stream()), 'blochsim_fused_fwd_rec')
+    _cabi.count_launches()
+    return Mo, Mt, ckpt, wave
+
+
+def _fake_blochsim_fused_fwd_rec(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every):
+    Mo, ckpt, wave = _fake_blochsim_fused_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags)
+    return Mo, Mi.new_empty((loc.shape[0], rf.shape[2] // every, 3, loc.shape[1])), ckpt, wave
+
+
+def _impl_blochsim_fused_bwd_rec(gMo: Tensor, gMt: Tensor, Mo: Tensor, ckpt: Tensor, wave: Tensor, rf: Tensor, gr: Tensor,
+                                 loc: Tensor, df: Optional[Tensor], b1: Optional[Tensor], T1: Optional[Tensor],
+                                 T2: Optional[Tensor], gamma: Tensor, dt: Tensor, K: int, flags: int, every: int,
+                                 want_loc: bool, want_sz: bool, want_b1: bool):
+    """As blochsim_fused_bwd_spin, with dL/dMt (N, nR, 3, nM) contiguous -- the gradient of blochsim_fused_fwd_rec's Mt --
+    on top of dL/dMo; no per-spin gradient wanted is fine."""
+    return _fused_bwd_call(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags,
+                           spin=(bool(want_loc), bool(want_sz), bool(want_b1)), rec=(every, gMt))
+
+
+def _fake_blochsim_fused_bwd_rec(gMo, gMt, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every, want_loc,
+                                 want_sz, want_b1):
+    return _fake_blochsim_fused_bwd_spin(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, want_loc,
+                                         want_sz, want_b1)
 
 
 def _fake_blochsim_fused_bwd_spin(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, want_loc, want_sz,
@@ -305,7 +359,7 @@ def _as_param_grad(g: Tensor, x: Tensor) -> Tensor:
     return g.sum_to_size(_param_2d(x).shape).reshape(x.shape).to(x.dtype)
 
 
-def _fused_backward(ctx, gMo, _gckpt, _gwave):
+def _fused_backward(ctx, gMo, _gckpt, _gwave, gMt=None):
     Mo, ckpt, wave, rf, gr, loc, gamma, dt, *opt = ctx.saved_tensors
     opt = list(opt)
     df, b1, T1, T2 = (opt.pop(0) if h else None for h in ctx.has)
@@ -322,12 +376,20 @@ def _fused_backward(ctx, gMo, _gckpt, _gwave):
     # only the gradients autograd asks for: the rows of the spin reduction of the others are not even formed
     flags = ctx.flags | (_cabi.FLAG_NEED_GMI if need[0] else 0) | (0 if need[1] else _cabi.FLAG_SKIP_GRF) | \
         (0 if need[2] else _cabi.FLAG_SKIP_GGR)
-    if not (want_loc or want_sz or want_b1):
+    if gMt is not None:
+        # dL/dMt in the kernel's layout (N, nR, 3, nM) and dtype: a loss formed elementwise from the permuted view the caller
+        # got hands its gradient back in that layout already; anything else costs this one copy
+        if gMt.dtype != Mo.dtype or not gMt.is_contiguous():
+            gMt = torch.empty(gMt.shape, dtype=Mo.dtype, device=Mo.device).copy_(gMt)
+        gMi, flat, gloc, gsz, gb1 = blochsim_fused_bwd_rec(gMo, gMt, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt,
+                                                           ctx.K, flags, ctx.every, want_loc, want_sz, want_b1)
+    elif not (want_loc or want_sz or want_b1):
         gMi, flat = blochsim_fused_bwd(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, ctx.K, flags)
         grf, ggr = split_wave_grads(flat, rf, flags)
         return (gMi if need[0] else None, grf, ggr) + (None,) * 9
-    gMi, flat, gloc, gsz, gb1 = blochsim_fused_bwd_spin(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, ctx.K,
-                                                        flags, want_loc, want_sz, want_b1)
+    else:
+        gMi, flat, gloc, gsz, gb1 = blochsim_fused_bwd_spin(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt,
+                                                            ctx.K, flags, want_loc, want_sz, want_b1)
     grf, ggr = split_wave_grads(flat, rf, flags)
     gdf = ggam = None
     if want_sz:     # ∂Δf = gsz/γ, ∂γ = -gsz·Δf/γ² (the chain rule of Bz += Δf/γ, beffective.py:142)
@@ -340,6 +402,17 @@ def _fused_backward(ctx, gMo, _gckpt, _gwave):
             None, None, ggam, None, None, None)
 
 
+def _fused_rec_setup(ctx, inputs, output):
+    Mo, _Mt, ckpt, wave = output
+    _fused_setup(ctx, inputs[:12], (Mo, ckpt, wave))
+    ctx.every = inputs[12]
+    ctx.set_materialize_grads(False)      # a loss that ignores Mt (or M) hands None for it, not a tensor of zeros
+
+
+def _fused_rec_backward(ctx, gMo, gMt, _gckpt, _gwave):
+    """With no gradient on Mt this is the backward of blochsim_fused_fwd (same entry, same bits); else the REC backward,
+    with dL/dMo = 0 when the loss ignores M."""
+    return _fused_backward(ctx, gMo, None, None, gMt) + (None,)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -779,7 +852,7 @@ def _mask_backward(ctx, g):
 # registration: raw torch.library definitions (schema + CUDA impl + fake), which cost ~20 us per call instead of
 # the ~130 us of the `torch.library.custom_op` convenience wrapper -- it matters for test-scale problems
 _LIB = torch.library.Library('mrphy_b200', 'DEF')
-_SCHEMAS = {'blochsim_fused_fwd': '(Tensor Mi, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor, Tensor)', 'blochsim_fused_bwd': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'blochsim_fused_bwd_design': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? ddt, int rf_kind, int gr_kind) -> (Tensor, Tensor, Tensor, Tensor, Tensor)', 'blochsim_fused_bwd_spin': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, bool want_loc, bool want_sz, bool want_b1) -> (Tensor, Tensor, Tensor, Tensor, Tensor)', 'blochsim_beff_fwd': '(Tensor Mi, Tensor Beff, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'blochsim_beff_bwd': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor Beff, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'rfgr2beff': '(Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor gamma) -> Tensor', 'rfgr2beff_bwd': '(Tensor gB, Tensor rf, Tensor gr, Tensor loc, Tensor? b1) -> (Tensor, Tensor)', 'rfgr2beff_spin_grads': '(Tensor gB, Tensor rf, Tensor gr, bool want_loc, bool want_b1) -> (Tensor, Tensor, Tensor)', 'beff2ab': '(Tensor beff, Tensor E1, Tensor E2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor, Tensor)', 'beff2ab_bwd': '(Tensor gA, Tensor gB, Tensor A, Tensor B, Tensor ckpt, Tensor beff, Tensor E1, Tensor E2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'beff2uphi': '(Tensor beff, Tensor g) -> (Tensor, Tensor)', 'beff2uphi_bwd': '(Tensor? gU, Tensor? gPhi, Tensor beff, Tensor g) -> (Tensor, Tensor)', 'freeprec': '(Tensor Mi, Tensor dur, Tensor? T1, Tensor? T2, Tensor? df, bool adjoint) -> Tensor', 'design_waveform': '(Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? dt, int rf_kind, int gr_kind) -> (Tensor, Tensor)', 'design_waveform_bwd': '(Tensor? grf, Tensor? ggr, Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? dt, int rf_kind, int gr_kind) -> (Tensor, Tensor, Tensor)', 'mask_copy': '(Tensor v, Tensor idx, Tensor inv, bool fill_zero) -> Tensor', 'clamp_waveform': '(Tensor x, Tensor lim, float eps, int kind) -> Tensor', 'clamp_waveform_bwd': '(Tensor g, Tensor x, Tensor lim, float eps, int kind) -> Tensor'}
+_SCHEMAS = {'blochsim_fused_fwd': '(Tensor Mi, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor, Tensor)', 'blochsim_fused_bwd': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'blochsim_fused_bwd_design': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? ddt, int rf_kind, int gr_kind) -> (Tensor, Tensor, Tensor, Tensor, Tensor)', 'blochsim_fused_bwd_spin': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, bool want_loc, bool want_sz, bool want_b1) -> (Tensor, Tensor, Tensor, Tensor, Tensor)', 'blochsim_fused_fwd_rec': '(Tensor Mi, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, int every) -> (Tensor, Tensor, Tensor, Tensor)', 'blochsim_fused_bwd_rec': '(Tensor gMo, Tensor gMt, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, int every, bool want_loc, bool want_sz, bool want_b1) -> (Tensor, Tensor, Tensor, Tensor, Tensor)', 'blochsim_beff_fwd': '(Tensor Mi, Tensor Beff, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'blochsim_beff_bwd': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor Beff, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'rfgr2beff': '(Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor gamma) -> Tensor', 'rfgr2beff_bwd': '(Tensor gB, Tensor rf, Tensor gr, Tensor loc, Tensor? b1) -> (Tensor, Tensor)', 'rfgr2beff_spin_grads': '(Tensor gB, Tensor rf, Tensor gr, bool want_loc, bool want_b1) -> (Tensor, Tensor, Tensor)', 'beff2ab': '(Tensor beff, Tensor E1, Tensor E2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor, Tensor)', 'beff2ab_bwd': '(Tensor gA, Tensor gB, Tensor A, Tensor B, Tensor ckpt, Tensor beff, Tensor E1, Tensor E2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'beff2uphi': '(Tensor beff, Tensor g) -> (Tensor, Tensor)', 'beff2uphi_bwd': '(Tensor? gU, Tensor? gPhi, Tensor beff, Tensor g) -> (Tensor, Tensor)', 'freeprec': '(Tensor Mi, Tensor dur, Tensor? T1, Tensor? T2, Tensor? df, bool adjoint) -> Tensor', 'design_waveform': '(Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? dt, int rf_kind, int gr_kind) -> (Tensor, Tensor)', 'design_waveform_bwd': '(Tensor? grf, Tensor? ggr, Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? dt, int rf_kind, int gr_kind) -> (Tensor, Tensor, Tensor)', 'mask_copy': '(Tensor v, Tensor idx, Tensor inv, bool fill_zero) -> Tensor', 'clamp_waveform': '(Tensor x, Tensor lim, float eps, int kind) -> Tensor', 'clamp_waveform_bwd': '(Tensor g, Tensor x, Tensor lim, float eps, int kind) -> Tensor'}
 
 
 def _register(name, impl, fake):
@@ -793,6 +866,8 @@ blochsim_fused_fwd = _register('blochsim_fused_fwd', _impl_blochsim_fused_fwd, _
 blochsim_fused_bwd = _register('blochsim_fused_bwd', _impl_blochsim_fused_bwd, _fake_blochsim_fused_bwd)
 blochsim_fused_bwd_design = _register('blochsim_fused_bwd_design', _impl_blochsim_fused_bwd_design, _fake_blochsim_fused_bwd_design)
 blochsim_fused_bwd_spin = _register('blochsim_fused_bwd_spin', _impl_blochsim_fused_bwd_spin, _fake_blochsim_fused_bwd_spin)
+blochsim_fused_fwd_rec = _register('blochsim_fused_fwd_rec', _impl_blochsim_fused_fwd_rec, _fake_blochsim_fused_fwd_rec)
+blochsim_fused_bwd_rec = _register('blochsim_fused_bwd_rec', _impl_blochsim_fused_bwd_rec, _fake_blochsim_fused_bwd_rec)
 blochsim_beff_fwd = _register('blochsim_beff_fwd', _impl_blochsim_beff_fwd, _fake_blochsim_beff_fwd)
 blochsim_beff_bwd = _register('blochsim_beff_bwd', _impl_blochsim_beff_bwd, _fake_blochsim_beff_bwd)
 rfgr2beff_cuda = _register('rfgr2beff', _impl_rfgr2beff, _fake_rfgr2beff)
@@ -809,6 +884,8 @@ mask_copy_cuda = _register('mask_copy', _impl_mask_copy, _fake_mask_copy)
 clamp_waveform_cuda = _register('clamp_waveform', _impl_clamp_waveform, lambda x, lim, eps, kind: x.new_empty(x.shape))
 clamp_waveform_bwd_cuda = _register('clamp_waveform_bwd', _impl_clamp_waveform_bwd, lambda g, x, lim, eps, kind: x.new_empty(x.shape))
 torch.library.register_autograd('mrphy_b200::blochsim_fused_fwd', _fused_backward, setup_context=_fused_setup, lib=_LIB)
+torch.library.register_autograd('mrphy_b200::blochsim_fused_fwd_rec', _fused_rec_backward, setup_context=_fused_rec_setup,
+                                lib=_LIB)
 torch.library.register_autograd('mrphy_b200::design_waveform', _design_backward, setup_context=_design_setup, lib=_LIB)
 torch.library.register_autograd('mrphy_b200::mask_copy', _mask_backward, setup_context=_mask_setup, lib=_LIB)
 torch.library.register_autograd('mrphy_b200::clamp_waveform', _clamp_backward, setup_context=_clamp_setup, lib=_LIB)
@@ -1013,7 +1090,8 @@ def default_flags() -> int:
 
 def fused_applypulse(M_: Tensor, rf: Tensor, gr: Tensor, loc_: Tensor, *, Δf_: Optional[Tensor] = None,
                      b1Map_: Optional[Tensor] = None, T1_: Optional[Tensor] = None, T2_: Optional[Tensor] = None,
-                     γ_: Tensor, dt: Tensor, ckpt: Optional[int] = None, flags: Optional[int] = None) -> Tensor:
+                     γ_: Tensor, dt: Tensor, ckpt: Optional[int] = None, flags: Optional[int] = None,
+                     record: Optional[int] = None):
     """Fused waveform -> magnetisation op on compact arrays; differentiable wrt ``M_``, ``rf``, ``gr`` and the spins'
     ``loc_``, ``Δf_``, ``b1Map_``, ``γ_`` (as the reference's autograd through rfgr2beff; γ only through ``Δf_/γ``).
 
@@ -1023,7 +1101,15 @@ def fused_applypulse(M_: Tensor, rf: Tensor, gr: Tensor, loc_: Tensor, *, Δf_: 
     The per-spin gradients are sums over time that the fused backward forms per spin, without the dense field.  When one
     of those inputs requires grad, a re-parametrised rf / gr (``tag_design``) is differentiated in two stages -- the
     simulation's backward, then the chain's own adjoint -- as with ``MRPHY_B200_FUSE_DESIGN=0``.
+
+    ``record = s`` (an integer, 1 <= s <= nT) also returns the magnetisation during the pulse: ``(M, Mt)`` instead of ``M``,
+    ``Mt`` (N,nM,nR,3) with nR = nT // s and ``Mt[:, :, r]`` the state after (r+1)·s steps in the lab frame -- what ``M``
+    is for the pulse cut to its first (r+1)·s samples (the last entry is ``M`` when s divides nT).  ``Mt`` is a permuted
+    view of the kernel's (N,nR,xyz,nM) output and is not contiguous.  Losses on ``Mt``, on ``M`` or on both are
+    differentiable like ``M`` alone; a re-parametrised waveform is then differentiated in two stages, as above.
     """
+    if record is not None:
+        record = _check_record(record, rf, b1Map_)
     _require_cuda(M_, rf, gr, loc_, Δf_, b1Map_, T1_, T2_)
     dtype, dev = M_.dtype, M_.device
     if dtype not in _F:
@@ -1035,9 +1121,11 @@ def fused_applypulse(M_: Tensor, rf: Tensor, gr: Tensor, loc_: Tensor, *, Δf_: 
         mv = lambda x: None if x is None else (on_device(x, dev) if x.dtype in _F else on_device(x, dev, dtype))
         K = int(ckpt) if ckpt is not None else pick_ckpt_interval(mv(dt), mv(T1_), mv(T2_))
         up = lambda x: None if x is None else x.to(torch.float64)
-        Mo = fused_applypulse(up(M_), up(rf), up(gr), up(loc_), Δf_=up(Δf_), b1Map_=up(b1Map_), T1_=up(T1_), T2_=up(T2_),
-                              γ_=γ_, dt=dt, ckpt=K)
-        return Mo.to(torch.float32)
+        out = fused_applypulse(up(M_), up(rf), up(gr), up(loc_), Δf_=up(Δf_), b1Map_=up(b1Map_), T1_=up(T1_), T2_=up(T2_),
+                               γ_=γ_, dt=dt, ckpt=K, record=record)
+        if record is not None:
+            return out[0].to(torch.float32), out[1].to(torch.float32)
+        return out.to(torch.float32)
     assert (T1_ is None) == (T2_ is None)      # both or neither (sims.py:68)
     N, nM = loc_.shape[0], loc_.shape[1]
     assert M_.shape == (N, nM, 3) and loc_.shape == (N, nM, 3)
@@ -1065,7 +1153,7 @@ def fused_applypulse(M_: Tensor, rf: Tensor, gr: Tensor, loc_: Tensor, *, Δf_: 
         K = min(K, TC_K_MAX)                     # the tensor-core kernels stage 32 steps per chunk
     fl = default_flags() if flags is None else flags
     spin_grad = any(x is not None and x.requires_grad for x in (loc_, Δf_, b1Map_, γ_))
-    if torch.is_grad_enabled() and not spin_grad and os.environ.get('MRPHY_B200_FUSE_DESIGN', '1') != '0':
+    if torch.is_grad_enabled() and not spin_grad and record is None and os.environ.get('MRPHY_B200_FUSE_DESIGN', '1') != '0':
         # rf and/or gr straight out of the re-parametrisation chain: differentiate w.r.t. the design variables in the
         # simulation's own gradient epilogue (see _FusedDesignApply)
         r_rf, r_gr = _design_of(rf_in, rf), _design_of(gr_in, gr)
@@ -1075,5 +1163,21 @@ def fused_applypulse(M_: Tensor, rf: Tensor, gr: Tensor, loc_: Tensor, *, Δf_: 
             return _FusedDesignApply.apply(Mi, rf.detach() if r_rf is not None else rf, gr.detach() if r_gr is not None else gr,
                                            rho, theta, ts, loc, df, b1, T1, T2, gam, dtt, rfmax, smax, ddt, K, fl,
                                            r_rf.kind if r_rf is not None else 0, r_gr.kind if r_gr is not None else 0)
+    if record is not None:
+        Mo, Mt, _, _ = blochsim_fused_fwd_rec(Mi, rf, gr, loc, df, b1, T1, T2, gam, dtt, K, fl, record)
+        return Mo, Mt.permute(0, 3, 1, 2)
     Mo, _, _ = blochsim_fused_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gam, dtt, K, fl)
     return Mo
+
+
+def _check_record(record, rf: Tensor, b1Map_: Optional[Tensor]) -> int:
+    """The record stride `fused_applypulse` takes, or ValueError (before anything runs)."""
+    if isinstance(record, bool) or not isinstance(record, numbers.Integral):
+        raise ValueError(f'mrphy (B200): record must be an integer number of steps, got {record!r}')
+    nT = rf.shape[2]
+    if not 1 <= record <= nT:
+        raise ValueError(f'mrphy (B200): record={record} is outside [1, nT = {nT}]')
+    if b1Map_ is not None and rf.ndim == 4 and rf.shape[3] > 16:
+        raise ValueError(f'mrphy (B200): record needs the fused kernels, which take at most 16 transmit coils with a b1Map '
+                         f'(got {rf.shape[3]}); the explicit-Beff route does not record')
+    return int(record)

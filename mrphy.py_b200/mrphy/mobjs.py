@@ -390,7 +390,8 @@ class SpinArray(_Obj):
         doEmbed: bool = False,
         doRelax: bool = True,
         doUpdate: bool = False,
-    ) -> Tensor:
+        record: Optional[int] = None,
+    ):
         r"""Simulate ``pulse`` on these spins and return the magnetisation.
 
         ``loc`` ⊻ ``loc_`` `(N,*Nd ⊻ nM,xyz)` [cm] is required; ``Δf`` ⊻ ``Δf_`` `(N,*Nd ⊻ nM)` [Hz] and ``b1Map`` ⊻
@@ -403,12 +404,25 @@ class SpinArray(_Obj):
         forms these per-spin sums without materialising the field).  Only more than 16 transmit coils with a ``b1Map``,
         which the fused kernels do not take, materialise the field (``pulse2beff``) and run the explicit-``Beff``
         kernels, whose per-spin pass takes at most 16 coils as well.
+
+        ``record = s`` (an integer, 1 <= s <= nT) also returns the magnetisation during the pulse: ``(M, Mt)``, ``Mt``
+        `(N,nM,nR,xyz)` (`(N,*Nd,nR,xyz)` with ``doEmbed``), nR = nT // s, ``Mt[..., r, :]`` the state after (r+1)·s
+        steps -- ``M`` of the pulse cut to its first (r+1)·s samples.  Compact ``Mt`` is a non-contiguous view.
+        ``doUpdate`` stores ``M`` only.  Gradients flow through both.  Refused (ValueError) beyond 16 transmit coils
+        with a ``b1Map``: the explicit-``Beff`` route does not record.
         """
         assert (loc_ is None) != (loc is None)
         loc_ = loc_ if loc is None else self.extract(loc)
         Δf_ = _one_of(Δf, Δf_, self.extract)
         b1Map_ = _one_of(b1Map, b1Map_, self.extract)
         T1_, T2_ = (self.T1_, self.T2_) if doRelax else (None, None)
+        if record is not None:
+            p = pulse.to(device=self.device, dtype=self.dtype)
+            M_, Mt_ = _ops.fused_applypulse(self.M_, p.rf, p.gr, loc_, Δf_=Δf_, b1Map_=b1Map_, T1_=T1_, T2_=T2_,
+                                            γ_=self.γ_, dt=p.dt, record=record)
+            if doUpdate:
+                self.M_ = M_
+            return (self.embed(M_), self.embed(Mt_)) if doEmbed else (M_, Mt_)
         if _explicit_route(pulse, b1Map_, (loc_, Δf_, b1Map_, self.γ_)):
             beff_ = self.pulse2beff(pulse, loc_=loc_, Δf_=Δf_, b1Map_=b1Map_)
             M_ = sims.blochsim(self.M_, beff_, T1=T1_, T2=T2_, γ=self.γ_, dt=pulse.dt)
@@ -614,11 +628,12 @@ class SpinCube(SpinArray):
         doEmbed: bool = False,
         doRelax: bool = True,
         doUpdate: bool = False,
-    ) -> Tensor:
+        record: Optional[int] = None,
+    ):
         r"""As :meth:`SpinArray.applypulse` with the cube's ``loc_`` and ``Δf_``; only ``b1Map`` ⊻ ``b1Map_`` is given."""
         b1Map_ = _one_of(b1Map, b1Map_, self.extract)
         return self.spinarray.applypulse(pulse, loc_=self.loc_, Δf_=self.Δf_, b1Map_=b1Map_, doEmbed=doEmbed,
-                                         doRelax=doRelax, doUpdate=doUpdate)
+                                         doRelax=doRelax, doUpdate=doUpdate, record=record)
 
     def applysequence(self, events, *, b1Map: OptT = None, b1Map_: OptT = None, doEmbed: bool = False, doRelax: bool = True,
                       doUpdate: bool = False) -> Tensor:

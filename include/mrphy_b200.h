@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define MRPHY_ABI_VERSION 6
+#define MRPHY_ABI_VERSION 7
 
 enum mrphy_dtype { MRPHY_F32 = 0, MRPHY_F64 = 1 };
 
@@ -93,6 +93,15 @@ typedef struct mrphy_fused_args {
   void* grf;       /* out (N,2,nT[,nC]) contiguous                                             */
   void* ggr;       /* out (N,3,nT) contiguous                                                  */
   void* partials;  /* scratch, mrphy_fused_partial_elems() elements of T                       */
+
+  /* options, off when zero / NULL (see the entry points below) */
+  int32_t every, nR;   /* record: 1 <= every <= nT, nR == nT / every                                 */
+  void* Mt;            /* record, fwd: out [N][nR][3][nM] contiguous                                 */
+  const void* gMt;     /* record, bwd: in, dL/dMt in the same layout                                 */
+  void* gloc;          /* per-spin gradients, bwd: out (N,nM,3) contiguous, or NULL                  */
+  void* gsz;           /* per-spin gradients, bwd: out (N,nM) contiguous, or NULL                    */
+  void* gb1;           /* per-spin gradients, bwd: out (N,nM,2,nC) contiguous, or NULL (needs b1)    */
+  const struct mrphy_reparam_args* design;   /* design tail, bwd: the re-parametrisation, or NULL  */
 } mrphy_fused_args;
 
 int mrphy_abi_version(void);
@@ -106,11 +115,40 @@ size_t mrphy_fused_ckpt_elems(const mrphy_fused_args* a);
 size_t mrphy_fused_wave_elems(const mrphy_fused_args* a);
 size_t mrphy_fused_partial_elems(const mrphy_fused_args* a);
 
-/* Forward: writes Mo and ckpt.  Launches: pack_waveform, blochsim_fused_fwd.                    */
+/* Forward: writes Mo and ckpt.  Launches: pack_waveform, blochsim_fused_fwd.
+ *
+ * Record (a->every != 0): the magnetisation during the pulse.  The forward also writes the state after every `every` steps,
+ *   Mt[n][r][xyz][i] = M of spin i after (r+1)*every steps, r = 0 .. nR-1, nR = nT / every   (lab frame, like Mo)
+ * -- what the forward returns as Mo for the pulse cut to its first (r+1)*every samples.  Needs a->Mt.  Up to 16 transmit
+ * coils, like every fused call.  No workspace beyond the existing ones.                                               */
 int mrphy_blochsim_fused_fwd(const mrphy_fused_args* a, void* cuda_stream);
 /* Backward: reads Mo, ckpt, gMo; writes grf, ggr (and gMi).  Launches: pack_waveform (unless
  * `wave` still holds the packed waveform of the matching forward: pass wave_is_packed != 0),
- * blochsim_fused_bwd, grad_reduce_finalize.                                                     */
+ * blochsim_fused_bwd, grad_reduce_finalize.  Three options, each off when its fields are zero / NULL:
+ *
+ * Record (a->every != 0): the backward of a recording forward with the same every / nR.  It takes dL/dMt (a->gMt, in
+ * the layout of Mt) on top of dL/dMo; a->gMo is required (zeros when the loss ignores Mo).
+ *
+ * Per-spin gradients (any of a->gloc, a->gsz, a->gb1 non-NULL): what the autograd of rfgr2beff gives upstream for loc,
+ * df, b1Map and gamma (beffective.py:137-167), without the dense field or dL/dBeff.  Each output is the sum over time
+ * that mrphy_rfgr2beff_spin_grads forms from dL/dBeff, with the same meaning and layout:
+ *   gloc (N,nM,3)     = sum_t gr[:,t] * gBz[t]                              (dL/dloc)
+ *   gsz  (N,nM)       = sum_t gBz[t]                                        (dL/ddf = gsz/gamma, dL/dgamma = -gsz*df/gamma^2)
+ *   gb1  (N,nM,2,nC)  = sum_t (rx_c gBx + ry_c gBy,  rx_c gBy - ry_c gBx)    (dL/db1Map; requires a->b1)
+ * contiguous, any of them NULL = not wanted.  gMi, grf and ggr are bitwise those of a call without per-spin gradients.
+ * With MRPHY_SKIP_GRF | MRPHY_SKIP_GGR (a fixed pulse) the backward forms no spin reduction and skips the finalize
+ * launch.  Combines with record.
+ *
+ * Design tail (a->design non-NULL): the adjoint of the re-parametrisation fused into the gradient epilogue (SURVEY 8f-2):
+ * what autograd does upstream in two stages -- BlochSim.backward (sims.py:187-269) -> dL/drf, dL/dgr, then the backward
+ * of utils.t-rho-theta2rf / l-rho-theta2rf / ts2s / s2g (utils.py:114-131, 239-256, 293-330) -> dL/drho, dL/dtheta,
+ * dL/dts.  `design` describes the chain that produced a->rf and/or a->gr: adjoint != 0, dtype / N / nT as in `a`,
+ * nC = trailing coil dimension of rf; rf_kind 0..2 and gr_kind 0..2 as in mrphy_design_waveform (0: that waveform is
+ * not re-parametrised); design->grf / ->ggr are ignored -- the tail reads a->grf / a->ggr, which are written as usual.
+ * Same launches: the last CTA of the epilogue to finish for a batch entry evaluates that entry's adjoint and writes
+ * design->grho, ->gtheta, ->gts.  Combines with neither record nor per-spin gradients (MRPHY_ERR_ARG).
+ *
+ * No option needs workspace beyond mrphy_fused_partial_elems().                                                      */
 int mrphy_blochsim_fused_bwd(const mrphy_fused_args* a, int wave_is_packed, void* cuda_stream);
 
 /* Arguments of the explicit-field path: the API-faithful replacement of sims.BlochSim
@@ -233,50 +271,6 @@ typedef struct mrphy_reparam_args {
 } mrphy_reparam_args;
 int mrphy_design_waveform(const mrphy_reparam_args* a, void* cuda_stream);
 
-/* mrphy_blochsim_fused_bwd with the adjoint of the re-parametrisation fused into its gradient epilogue (SURVEY 8f-2): what
- * autograd does upstream in two stages -- BlochSim.backward (sims.py:187-269) -> dL/drf, dL/dgr, then the backward of
- * utils.t-rho-theta2rf / l-rho-theta2rf / ts2s / s2g (utils.py:114-131, 239-256, 293-330) -> dL/drho, dL/dtheta, dL/dts.
- * `d` describes the chain that produced a->rf and/or a->gr: adjoint != 0, dtype / N / nT as in `a`, nC = trailing coil
- * dimension of rf; rf_kind 0..2 and gr_kind 0..2 as in mrphy_design_waveform (0: that waveform is not re-parametrised);
- * d->grf / d->ggr are ignored -- the tail reads a->grf / a->ggr, which are written as usual.  Same launches as
- * mrphy_blochsim_fused_bwd: the last CTA of the epilogue to finish for a batch entry evaluates that entry's adjoint and
- * writes d->grho, d->gtheta, d->gts.  a->partials as sized by mrphy_fused_partial_elems().                          */
-int mrphy_blochsim_fused_bwd_design(const mrphy_fused_args* a, int wave_is_packed, const mrphy_reparam_args* d,
-                                    void* cuda_stream);
-
-/* Per-spin gradients of the fused backward: what the autograd of rfgr2beff gives upstream for loc, df, b1Map and gamma
- * (beffective.py:137-167), without the dense field or dL/dBeff.  Each output is the sum over time that
- * mrphy_rfgr2beff_spin_grads forms from dL/dBeff, with the same meaning and layout:
- *   gloc (N,nM,3)     = sum_t gr[:,t] * gBz[t]                              (dL/dloc)
- *   gsz  (N,nM)       = sum_t gBz[t]                                        (dL/ddf = gsz/gamma, dL/dgamma = -gsz*df/gamma^2)
- *   gb1  (N,nM,2,nC)  = sum_t (rx_c gBx + ry_c gBy,  rx_c gBy - ry_c gBx)    (dL/db1Map; requires a->b1)
- * contiguous, any of them NULL = not wanted (not all three).  Everything else as mrphy_blochsim_fused_bwd, whose results
- * (gMi, grf, ggr) are bitwise those of a call without per-spin gradients.  With MRPHY_SKIP_GRF | MRPHY_SKIP_GGR (a fixed
- * pulse) the backward forms no spin reduction and skips the finalize launch.  No workspace beyond
- * mrphy_fused_partial_elems().                                                                                        */
-typedef struct mrphy_spin_grad_args {
-  void* gloc;  /* out (N,nM,3) contiguous, or NULL */
-  void* gsz;   /* out (N,nM)   contiguous, or NULL */
-  void* gb1;   /* out (N,nM,2,nC) contiguous, or NULL (requires a->b1) */
-} mrphy_spin_grad_args;
-int mrphy_blochsim_fused_bwd_spin(const mrphy_fused_args* a, int wave_is_packed, const mrphy_spin_grad_args* s,
-                                  void* cuda_stream);
-
-/* The magnetisation during the pulse: the fused forward also writes the state after every `every` steps,
- *   Mt[n][r][xyz][i] = M of spin i after (r+1)*every steps, r = 0 .. nR-1, nR = nT / every   (lab frame, like Mo)
- * -- what mrphy_blochsim_fused_fwd returns as Mo for the pulse cut to its first (r+1)*every samples.  The backward takes
- * dL/dMt in the same layout on top of dL/dMo.  Mo, ckpt and, in the backward, gMi, grf, ggr and the per-spin gradients
- * (s, or NULL for none) mean what they mean for mrphy_blochsim_fused_fwd / _bwd / _bwd_spin; a->gMo is required (zeros
- * when the loss ignores Mo).  Up to 16 transmit coils, like every fused entry.  No workspace beyond the existing ones. */
-typedef struct mrphy_record_args {
-  int32_t every, nR;     /* 1 <= every <= nT, nR == nT / every                              */
-  void* Mt;              /* fwd: out [N][nR][3][nM] contiguous, lab frame                    */
-  const void* gMt;       /* bwd: in, dL/dMt in the same layout                               */
-} mrphy_record_args;
-int mrphy_blochsim_fused_fwd_rec(const mrphy_fused_args* a, const mrphy_record_args* r, void* cuda_stream);
-int mrphy_blochsim_fused_bwd_rec(const mrphy_fused_args* a, int wave_is_packed, const mrphy_record_args* r,
-                                 const mrphy_spin_grad_args* s /* NULL: no per-spin gradients */, void* cuda_stream);
-
 /* Amplitude limits of the design loop (SURVEY 8f-2), replacing utils.rfclamp (utils.py:217-236) and utils.sclamp
  * (utils.py:278-293) and their autograd, one launch each way:
  *   kind 1  rf (N,2,nT,nC):  out = rf * min((rfmax[n,c] - eps) / |rf|, 1),  |rf| over the xy axis
@@ -311,8 +305,8 @@ int mrphy_mask_copy(const mrphy_mask_args* a, void* cuda_stream);
 
 /* sizeof() of the argument structs as this library was compiled, for bindings to check their mirror of the layout:
  * which = 0 mrphy_param, 1 mrphy_fused_args, 2 mrphy_beff_args, 3 mrphy_rfgr2beff_args, 4 mrphy_beff2ab_args,
- * 5 mrphy_beff2uphi_args, 6 mrphy_freeprec_args, 7 mrphy_reparam_args, 8 mrphy_mask_args, 9 mrphy_clamp_args,
- * 10 mrphy_spin_grad_args, 11 mrphy_record_args; 0 for any other value. */
+ * 5 mrphy_beff2uphi_args, 6 mrphy_freeprec_args, 7 mrphy_reparam_args, 8 mrphy_mask_args, 9 mrphy_clamp_args;
+ * 0 for any other value. */
 size_t mrphy_sizeof_args(int which);
 
 /* Number of kernel launches the last forward / backward call on this thread issued. */

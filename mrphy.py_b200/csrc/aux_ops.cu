@@ -467,8 +467,6 @@ extern "C" size_t mrphy_sizeof_args(int which) {
     case 7: return sizeof(mrphy_reparam_args);
     case 8: return sizeof(mrphy_mask_args);
     case 9: return sizeof(mrphy_clamp_args);
-    case 10: return sizeof(mrphy_spin_grad_args);
-    case 11: return sizeof(mrphy_record_args);
   }
   return 0;
 }

@@ -164,13 +164,13 @@ template <typename T> struct KArgs {
   int n_sm, c_per_sm;
   int* done;           // finished-CTA counters of grad_finalize_design_kernel, one per batch entry (null: no design tail); zeroed here
 };
-// per-spin gradient outputs of the SG backward (mrphy_spin_grad_args; each may be null).  A kernel parameter of its own behind
+// per-spin gradient outputs of the SG backward (gloc, gsz, gb1 of mrphy_fused_args; each may be null).  A kernel parameter of its own behind
 // the others, so that the kernels without per-spin gradients keep their parameter offsets.
 template <typename T> struct SgOut {
   T* gloc; T* gsz; T* gb1;
   bool any() const { return gloc || gsz || gb1; }
 };
-// recorded magnetisation of the REC kernels (mrphy_record_args): the forward writes Mt, the backward reads dL/dMt, both
+// recorded magnetisation of the REC kernels (every, nR, Mt, gMt of mrphy_fused_args): the forward writes Mt, the backward reads dL/dMt, both
 // [N][nR][3][nM] (SoA like the checkpoints), entry r = the state after (r+1)*every steps in the lab frame.  A kernel
 // parameter of its own behind the others, like SgOut.
 template <typename T> struct RecOut {
@@ -1474,8 +1474,8 @@ int launch_pack(const mrphy_fused_args* a, const Plan& p, cudaStream_t st, bool 
 // P (CTAs per batch entry) actually launched by the last backward kernel; the finalize kernel needs it
 thread_local int g_last_P = 0;
 
-template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, bool REC = false>
-int launch_fwd_s(KArgs<T> k, const Plan& p, cudaStream_t st, const RecOut<T>& rec = RecOut<T>{}) {
+template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, bool REC>
+int launch_fwd_s(KArgs<T> k, const Plan& p, cudaStream_t st, const RecOut<T>& rec) {
   auto kern = fused_fwd_kernel<T, POL, RELAX, NC, PK, BLKT, REC>;
   int occ = 0;
   CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, BLKT, 0));
@@ -1492,9 +1492,8 @@ int launch_fwd_s(KArgs<T> k, const Plan& p, cudaStream_t st, const RecOut<T>& re
   CK(cudaGetLastError());
   return MRPHY_OK;
 }
-template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, int ROWS = 3, bool SG = false, bool REC = false>
-int launch_bwd_s(KArgs<T> k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg = SgOut<T>{},
-                 const RecOut<T>& rec = RecOut<T>{}) {
+template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, int ROWS, bool SG, bool REC>
+int launch_bwd_s(KArgs<T> k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg, const RecOut<T>& rec) {
   constexpr size_t smem = BwdSmem<T, NC, BLKT, PK>::bytes;
   auto kern = fused_bwd_kernel<T, POL, RELAX, NC, PK, BLKT, ROWS, SG, REC>;
   CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   // static + dynamic may exceed 48 KB
@@ -1550,7 +1549,7 @@ int tc_occupancy(Kern kern, size_t dyn_smem, int tmem_cols) {
 }
 
 // tensor-core multi-coil kernels (fp32): at most 4 CTAs per SM, each owns 128 of the 512 TMEM columns
-template <int POL, bool RELAX, int NC, int PK, bool REC = false>
+template <int POL, bool RELAX, int NC, int PK, bool REC>
 int launch_fwd_tc_pk(KArgs<float> k, const Plan& p, cudaStream_t st, const RecOut<float>& rec) {
   using C = TcCfg<NC, PK>;
   constexpr size_t smem = C::bytes;
@@ -1574,7 +1573,7 @@ int launch_fwd_tc_pk(KArgs<float> k, const Plan& p, cudaStream_t st, const RecOu
   CK(cudaGetLastError());
   return MRPHY_OK;
 }
-template <int POL, bool RELAX, int NC, bool REC = false>
+template <int POL, bool RELAX, int NC, bool REC>
 int launch_fwd_tc(const KArgs<float>& k, const Plan& p, cudaStream_t st, const RecOut<float>& rec) {
   // two spin tiles per CTA (packed f2 step): measured 3 % (4, 8 coils) to 17 % (16 coils) faster than one tile with two TMEM
   // buffers; a build with -DMRPHY_TC_SCALAR also carries the one-tile kernels (MRPHY_B200_TC_PACK=1) for measurements
@@ -1583,48 +1582,36 @@ int launch_fwd_tc(const KArgs<float>& k, const Plan& p, cudaStream_t st, const R
 #endif
   return launch_fwd_tc_pk<POL, RELAX, NC, 2, REC>(k, p, st, rec);
 }
-// backward with per-spin gradients: the ROWS == 0 kernel when no waveform gradient is wanted, else all rows (the finalize
-// reads only the wanted ones)
-template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, bool REC = false>
-int launch_bwd_sg(const KArgs<T>& k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg, const RecOut<T>& rec) {
-  return p.rows == 0 ? launch_bwd_s<T, POL, RELAX, NC, PK, BLKT, 0, true, REC>(k, p, need_gmi, st, sg, rec)
-                     : launch_bwd_s<T, POL, RELAX, NC, PK, BLKT, 3, true, REC>(k, p, need_gmi, st, sg, rec);
-}
-template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, bool REC = false>
-int launch_any(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg,
-               const RecOut<T>& rec) {
-  if (bwd && sg.any()) return launch_bwd_sg<T, POL, RELAX, NC, PK, BLKT, REC>(k, p, need_gmi, st, sg, rec);
-  return bwd ? launch_bwd_s<T, POL, RELAX, NC, PK, BLKT, 3, false, REC>(k, p, need_gmi, st, sg, rec)
-             : launch_fwd_s<T, POL, RELAX, NC, PK, BLKT, REC>(k, p, st, rec);
+// One launch of the kernels with spins in registers: the forward, or the backward with its ROWS / SG.  With per-spin gradients
+// the backward takes the ROWS == 0 kernel when no waveform gradient is wanted, else all rows (the finalize reads only the
+// wanted ones); without, the spin-packed kernels also come with dL/drf-only and dL/dgr-only rows.
+template <typename T, int POL, bool RELAX, int NC, int PK, bool REC>
+int launch(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg, const RecOut<T>& rec) {
+  if (!bwd) return launch_fwd_s<T, POL, RELAX, NC, PK, PK == 2 ? 64 : 128, REC>(k, p, st, rec);
+  constexpr int B = PK == 2 ? MRPHY_BWD_BLKT : 128;
+  if (sg.any())
+    return p.rows == 0 ? launch_bwd_s<T, POL, RELAX, NC, PK, B, 0, true, REC>(k, p, need_gmi, st, sg, rec)
+                       : launch_bwd_s<T, POL, RELAX, NC, PK, B, 3, true, REC>(k, p, need_gmi, st, sg, rec);
+  if constexpr (PK == 2) {
+    if (p.rows == 1) return launch_bwd_s<T, POL, RELAX, NC, PK, B, 1, false, REC>(k, p, need_gmi, st, sg, rec);   // dL/drf only
+    if (p.rows == 2) return launch_bwd_s<T, POL, RELAX, NC, PK, B, 2, false, REC>(k, p, need_gmi, st, sg, rec);   // dL/dgr only
+  }
+  return launch_bwd_s<T, POL, RELAX, NC, PK, B, 3, false, REC>(k, p, need_gmi, st, sg, rec);
 }
 
-// REC: the recording kernels (RecOut set), instantiated only here
-template <typename T, int POL, bool RELAX, bool REC = false>
+template <typename T, int POL, bool RELAX, bool REC>
 int dispatch_nc(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg,
-                const RecOut<T>& rec = RecOut<T>{}) {
+                const RecOut<T>& rec) {
   if constexpr (sizeof(T) == 4) {
-    if (p.PK == 2) {
-      if (!bwd) return launch_fwd_s<T, POL, RELAX, 1, 2, 64, REC>(k, p, st, rec);
-      if (sg.any()) return launch_bwd_sg<T, POL, RELAX, 1, 2, MRPHY_BWD_BLKT, REC>(k, p, need_gmi, st, sg, rec);
-      if (p.rows == 1) return launch_bwd_s<T, POL, RELAX, 1, 2, MRPHY_BWD_BLKT, 1, false, REC>(k, p, need_gmi, st, sg, rec);   // dL/drf only
-      if (p.rows == 2) return launch_bwd_s<T, POL, RELAX, 1, 2, MRPHY_BWD_BLKT, 2, false, REC>(k, p, need_gmi, st, sg, rec);   // dL/dgr only
-      return launch_bwd_s<T, POL, RELAX, 1, 2, MRPHY_BWD_BLKT, 3, false, REC>(k, p, need_gmi, st, sg, rec);
-    }
+    if (p.PK == 2) return launch<T, POL, RELAX, 1, 2, REC>(bwd, k, p, need_gmi, st, sg, rec);
   }
 #ifdef MRPHY_ONLY_PK2   /* tuning builds (profiles/operand_model.py): compile the default fp32 kernels only */
   return fail(MRPHY_ERR_ARG, "built with MRPHY_ONLY_PK2%s");
 #else
   if constexpr (sizeof(T) == 4) {
-    // forward with 2 coils: two spins per thread (FFMA2) like the single-coil kernel; same tiles of 128 spins, same staging
-    if (p.NC == 2 && env_int("MRPHY_B200_NC2_PACK", 2) == 2) {
-      if (!bwd) return launch_fwd_s<T, POL, RELAX, 2, 2, 64, REC>(k, p, st, rec);
-      if (env_int("MRPHY_B200_NC2_PACK_BWD", 2) == 2) {
-        if (sg.any()) return launch_bwd_sg<T, POL, RELAX, 2, 2, MRPHY_BWD_BLKT, REC>(k, p, need_gmi, st, sg, rec);
-        if (p.rows == 1) return launch_bwd_s<T, POL, RELAX, 2, 2, MRPHY_BWD_BLKT, 1, false, REC>(k, p, need_gmi, st, sg, rec);
-        if (p.rows == 2) return launch_bwd_s<T, POL, RELAX, 2, 2, MRPHY_BWD_BLKT, 2, false, REC>(k, p, need_gmi, st, sg, rec);
-        return launch_bwd_s<T, POL, RELAX, 2, 2, MRPHY_BWD_BLKT, 3, false, REC>(k, p, need_gmi, st, sg, rec);
-      }
-    }
+    // 2 coils: two spins per thread (FFMA2) like the single-coil kernels; same tiles of 128 spins, same staging
+    if (p.NC == 2 && env_int("MRPHY_B200_NC2_PACK", 2) == 2 && (!bwd || env_int("MRPHY_B200_NC2_PACK_BWD", 2) == 2))
+      return launch<T, POL, RELAX, 2, 2, REC>(bwd, k, p, need_gmi, st, sg, rec);
     if (p.tc && !bwd) {   // forward with >= 4 coils: transmit field on the tensor cores
       if (p.NC == 4) return launch_fwd_tc<POL, RELAX, 4, REC>(k, p, st, rec);
       if (p.NC == 8) return launch_fwd_tc<POL, RELAX, 8, REC>(k, p, st, rec);
@@ -1637,66 +1624,63 @@ int dispatch_nc(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaSt
       if constexpr (sizeof(T) == 4) return fail(MRPHY_ERR_ARG, "internal: fp32 single-coil scalar kernels not built%s");
       else
 #endif
-      return launch_any<T, POL, RELAX, 1, 1, 128, REC>(bwd, k, p, need_gmi, st, sg, rec);
-    case 2: return launch_any<T, POL, RELAX, 2, 1, 128, REC>(bwd, k, p, need_gmi, st, sg, rec);
-    case 4: return launch_any<T, POL, RELAX, 4, 1, 128, REC>(bwd, k, p, need_gmi, st, sg, rec);
-    case 8: return launch_any<T, POL, RELAX, 8, 1, 128, REC>(bwd, k, p, need_gmi, st, sg, rec);
-    case 16: return launch_any<T, POL, RELAX, 16, 1, 128, REC>(bwd, k, p, need_gmi, st, sg, rec);
+      return launch<T, POL, RELAX, 1, 1, REC>(bwd, k, p, need_gmi, st, sg, rec);
+    case 2: return launch<T, POL, RELAX, 2, 1, REC>(bwd, k, p, need_gmi, st, sg, rec);
+    case 4: return launch<T, POL, RELAX, 4, 1, REC>(bwd, k, p, need_gmi, st, sg, rec);
+    case 8: return launch<T, POL, RELAX, 8, 1, REC>(bwd, k, p, need_gmi, st, sg, rec);
+    case 16: return launch<T, POL, RELAX, 16, 1, REC>(bwd, k, p, need_gmi, st, sg, rec);
   }
   return fail(MRPHY_ERR_ARG, "internal: bad NC%s");
 #endif
 }
 
-// the recording kernels: fp64 has one trigonometry (TRIG_FAST names it), so only fp32 instantiates both
-template <typename T>
-int dispatch_rec(bool bwd, const KArgs<T>& k, const Plan& p, bool relax, bool precise, int need_gmi, cudaStream_t st,
-                 const SgOut<T>& so, const RecOut<T>& ro) {
-  if constexpr (sizeof(T) == 4) {
-    if (precise)
-      return relax ? dispatch_nc<T, TRIG_PRECISE, true, true>(bwd, k, p, need_gmi, st, so, ro)
-                   : dispatch_nc<T, TRIG_PRECISE, false, true>(bwd, k, p, need_gmi, st, so, ro);
-  }
-  return relax ? dispatch_nc<T, TRIG_FAST, true, true>(bwd, k, p, need_gmi, st, so, ro)
-               : dispatch_nc<T, TRIG_FAST, false, true>(bwd, k, p, need_gmi, st, so, ro);
+template <typename T, int POL>
+int dispatch_pol(bool bwd, const KArgs<T>& k, const Plan& p, bool relax, bool rec, int need_gmi, cudaStream_t st,
+                 const SgOut<T>& sg, const RecOut<T>& ro) {
+  if (rec)
+    return relax ? dispatch_nc<T, POL, true, true>(bwd, k, p, need_gmi, st, sg, ro)
+                 : dispatch_nc<T, POL, false, true>(bwd, k, p, need_gmi, st, sg, ro);
+  return relax ? dispatch_nc<T, POL, true, false>(bwd, k, p, need_gmi, st, sg, ro)
+               : dispatch_nc<T, POL, false, false>(bwd, k, p, need_gmi, st, sg, ro);
 }
 
+// the record option is on when any of its fields is set (check_record then wants all of them consistent)
+bool recording(const mrphy_fused_args* a) { return a->every || a->nR || a->Mt || a->gMt; }
+
 template <typename T>
-int dispatch(bool bwd, const mrphy_fused_args* a, const Plan& p, cudaStream_t st, int* done = nullptr,
-             const mrphy_spin_grad_args* sg = nullptr, const mrphy_record_args* rec = nullptr) {
+int dispatch(bool bwd, const mrphy_fused_args* a, const Plan& p, cudaStream_t st, int* done) {
   KArgs<T> k = make_kargs<T>(a, p);
   k.done = done;
-  const SgOut<T> so = sg ? SgOut<T>{(T*)sg->gloc, (T*)sg->gsz, (T*)sg->gb1} : SgOut<T>{};
+  const SgOut<T> sg{(T*)a->gloc, (T*)a->gsz, (T*)a->gb1};
+  const bool rec = recording(a);
+  const RecOut<T> ro = rec ? RecOut<T>{(T*)a->Mt, (const T*)a->gMt, a->every, a->nR} : RecOut<T>{};
   const bool relax = a->T1.ptr != nullptr;
-  const bool precise = (a->flags & MRPHY_TRIG_PRECISE) != 0 && sizeof(T) == 4 && !(bwd && (a->flags & MRPHY_TRIG_FAST_BWD));
   const int need_gmi = (a->flags & MRPHY_NEED_GMI) ? 1 : 0;
-  if (rec)
-    return dispatch_rec<T>(bwd, k, p, relax, precise, need_gmi, st, so,
-                           RecOut<T>{(T*)rec->Mt, (const T*)rec->gMt, rec->every, rec->nR});
-  if (precise) {
-    return relax ? dispatch_nc<T, TRIG_PRECISE, true>(bwd, k, p, need_gmi, st, so)
-                 : dispatch_nc<T, TRIG_PRECISE, false>(bwd, k, p, need_gmi, st, so);
+  // fp64 has one trigonometry (TRIG_FAST names it), so only fp32 instantiates both
+  if constexpr (sizeof(T) == 4) {
+    if ((a->flags & MRPHY_TRIG_PRECISE) && !(bwd && (a->flags & MRPHY_TRIG_FAST_BWD)))
+      return dispatch_pol<T, TRIG_PRECISE>(bwd, k, p, relax, rec, need_gmi, st, sg, ro);
   }
-  return relax ? dispatch_nc<T, TRIG_FAST, true>(bwd, k, p, need_gmi, st, so)
-               : dispatch_nc<T, TRIG_FAST, false>(bwd, k, p, need_gmi, st, so);
+  return dispatch_pol<T, TRIG_FAST>(bwd, k, p, relax, rec, need_gmi, st, sg, ro);
 }
 
 // the record stride and its buffer (Mt for the forward, gMt for the backward)
-int check_record(const mrphy_fused_args* a, const mrphy_record_args* r, bool bwd) {
-  if (r->every < 1 || r->every > a->nT || r->nR != a->nT / r->every)
+int check_record(const mrphy_fused_args* a, bool bwd) {
+  if (a->every < 1 || a->every > a->nT || a->nR != a->nT / a->every)
     return fail(MRPHY_ERR_ARG, "record: need 1 <= every <= nT and nR == nT / every%s");
-  if (bwd ? !r->gMt : !r->Mt) return fail(MRPHY_ERR_ARG, bwd ? "record: gMt is null%s" : "record: Mt is null%s");
+  if (bwd ? !a->gMt : !a->Mt) return fail(MRPHY_ERR_ARG, bwd ? "record: gMt is null%s" : "record: Mt is null%s");
   return MRPHY_OK;
 }
 
 template <typename T>
-int run_fwd(const mrphy_fused_args* a, cudaStream_t st, const mrphy_record_args* rec = nullptr) {
+int run_fwd(const mrphy_fused_args* a, cudaStream_t st) {
   Plan p;
   int rc = make_plan(a, &p, true);
   if (rc) return rc;
   if ((rc = check_common<T>(a, false))) return rc;
-  if (rec && (rc = check_record(a, rec, false))) return rc;
+  if (recording(a) && (rc = check_record(a, false))) return rc;
   if ((rc = launch_pack<T>(a, p, st, p.tc != 0))) return rc;
-  return dispatch<T>(false, a, p, st, nullptr, nullptr, rec);
+  return dispatch<T>(false, a, p, st, nullptr);
 }
 
 // the re-parametrisation the design tail can take: adjoint of an rf half and/or a gradient half that ends in a gradient
@@ -1718,21 +1702,22 @@ int check_design(const mrphy_fused_args* a, const mrphy_reparam_args* d) {
 }
 
 template <typename T>
-int run_bwd(const mrphy_fused_args* a, int wave_is_packed, const mrphy_reparam_args* d, cudaStream_t st,
-            const mrphy_spin_grad_args* sg = nullptr, const mrphy_record_args* rec = nullptr) {
+int run_bwd(const mrphy_fused_args* a, int wave_is_packed, cudaStream_t st) {
   Plan p;
   int rc = make_plan(a, &p, true);
   if (rc) return rc;
   if ((rc = check_common<T>(a, true))) return rc;
+  const mrphy_reparam_args* d = a->design;
+  const bool rec = recording(a), sg = a->gloc || a->gsz || a->gb1;
+  if (d && (rec || sg)) return fail(MRPHY_ERR_ARG, "design: does not combine with record or per-spin gradients%s");
   if (d && (rc = check_design(a, d))) return rc;
-  if (rec && (rc = check_record(a, rec, true))) return rc;
-  if (sg && !sg->gloc && !sg->gsz && !sg->gb1) return fail(MRPHY_ERR_ARG, "spin gradients: gloc, gsz, gb1 are all null%s");
-  if (sg && sg->gb1 && !a->b1) return fail(MRPHY_ERR_ARG, "spin gradients: gb1 needs b1%s");
+  if (rec && (rc = check_record(a, true))) return rc;
+  if (a->gb1 && !a->b1) return fail(MRPHY_ERR_ARG, "spin gradients: gb1 needs b1%s");
   // (after a tensor-core forward `wave` holds that kernel's operand tiles: the backward stages its own layout over them)
   if ((!wave_is_packed || p.tc) && (rc = launch_pack<T>(a, p, st))) return rc;
   // finished-CTA counters of the design tail: behind the scheduling ints, zeroed by the backward kernel itself
   int* const done = d ? reinterpret_cast<int*>((T*)a->partials + (size_t)a->N * p.Pmax * p.W * (size_t)a->nT) + SCHED_CLAIM + p.Pmax : nullptr;
-  if ((rc = dispatch<T>(true, a, p, st, done, sg, rec))) return rc;
+  if ((rc = dispatch<T>(true, a, p, st, done))) return rc;
   if (sg && p.rows == 0) return MRPHY_OK;   // per-spin gradients only: nothing to finalize
   dim3 grid((a->nT + 31) / 32, p.W, a->N), block(32, 32);
   const int coil_dim = (a->flags & MRPHY_RF_COIL_DIM) ? 1 : 0;
@@ -1768,42 +1753,5 @@ extern "C" int mrphy_blochsim_fused_bwd(const mrphy_fused_args* a, int wave_is_p
   g_err[0] = 0;
   if (!a) return fail(MRPHY_ERR_ARG, "null args%s");
   cudaStream_t st = (cudaStream_t)cuda_stream;
-  return a->dtype == MRPHY_F64 ? run_bwd<double>(a, wave_is_packed, nullptr, st) : run_bwd<float>(a, wave_is_packed, nullptr, st);
-}
-
-extern "C" int mrphy_blochsim_fused_bwd_design(const mrphy_fused_args* a, int wave_is_packed, const mrphy_reparam_args* d,
-                                               void* cuda_stream) {
-  g_launches = 0;
-  g_err[0] = 0;
-  if (!a || !d) return fail(MRPHY_ERR_ARG, "null args%s");
-  cudaStream_t st = (cudaStream_t)cuda_stream;
-  return a->dtype == MRPHY_F64 ? run_bwd<double>(a, wave_is_packed, d, st) : run_bwd<float>(a, wave_is_packed, d, st);
-}
-
-extern "C" int mrphy_blochsim_fused_bwd_spin(const mrphy_fused_args* a, int wave_is_packed, const mrphy_spin_grad_args* s,
-                                             void* cuda_stream) {
-  g_launches = 0;
-  g_err[0] = 0;
-  if (!a || !s) return fail(MRPHY_ERR_ARG, "null args%s");
-  cudaStream_t st = (cudaStream_t)cuda_stream;
-  return a->dtype == MRPHY_F64 ? run_bwd<double>(a, wave_is_packed, nullptr, st, s)
-                               : run_bwd<float>(a, wave_is_packed, nullptr, st, s);
-}
-
-extern "C" int mrphy_blochsim_fused_fwd_rec(const mrphy_fused_args* a, const mrphy_record_args* r, void* cuda_stream) {
-  g_launches = 0;
-  g_err[0] = 0;
-  if (!a || !r) return fail(MRPHY_ERR_ARG, "null args%s");
-  cudaStream_t st = (cudaStream_t)cuda_stream;
-  return a->dtype == MRPHY_F64 ? run_fwd<double>(a, st, r) : run_fwd<float>(a, st, r);
-}
-
-extern "C" int mrphy_blochsim_fused_bwd_rec(const mrphy_fused_args* a, int wave_is_packed, const mrphy_record_args* r,
-                                            const mrphy_spin_grad_args* s, void* cuda_stream) {
-  g_launches = 0;
-  g_err[0] = 0;
-  if (!a || !r) return fail(MRPHY_ERR_ARG, "null args%s");
-  cudaStream_t st = (cudaStream_t)cuda_stream;
-  return a->dtype == MRPHY_F64 ? run_bwd<double>(a, wave_is_packed, nullptr, st, s, r)
-                               : run_bwd<float>(a, wave_is_packed, nullptr, st, s, r);
+  return a->dtype == MRPHY_F64 ? run_bwd<double>(a, wave_is_packed, st) : run_bwd<float>(a, wave_is_packed, st);
 }

@@ -14,7 +14,7 @@ LIB_PATH = os.environ.get('MRPHY_B200_LIB') or os.path.join(os.path.dirname(_HER
 MRPHY_F32, MRPHY_F64 = 0, 1
 FLAG_TRIG_PRECISE, FLAG_NEED_GMI, FLAG_RF_COIL_DIM, FLAG_NEED_GBEFF, FLAG_TRIG_FAST_BWD = 1, 2, 4, 8, 16
 FLAG_SKIP_GRF, FLAG_SKIP_GGR, FLAG_ZERO_GRAD_TAIL = 32, 64, 128
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 c_i32, c_i64, c_vp = ctypes.c_int32, ctypes.c_int64, ctypes.c_void_p
 
@@ -36,6 +36,9 @@ class FusedArgs(ctypes.Structure):
         ('Mo', c_vp), ('ckpt', c_vp), ('wave', c_vp),
         ('gMo', c_vp), ('gMo_sn', c_i64), ('gMo_sm', c_i64),
         ('gMi', c_vp), ('grf', c_vp), ('ggr', c_vp), ('partials', c_vp),
+        ('every', c_i32), ('nR', c_i32), ('Mt', c_vp), ('gMt', c_vp),
+        ('gloc', c_vp), ('gsz', c_vp), ('gb1', c_vp),
+        ('design', c_vp),
     ]
 
 
@@ -118,14 +121,6 @@ class ClampArgs(ctypes.Structure):
     ]
 
 
-class SpinGradArgs(ctypes.Structure):
-    _fields_ = [('gloc', c_vp), ('gsz', c_vp), ('gb1', c_vp)]
-
-
-class RecordArgs(ctypes.Structure):
-    _fields_ = [('every', c_i32), ('nR', c_i32), ('Mt', c_vp), ('gMt', c_vp)]
-
-
 EXPORTS = {   # name -> (restype, argtypes); tests check every symbol include/mrphy_b200.h declares
     'mrphy_abi_version': (ctypes.c_int, []),
     'mrphy_last_error': (ctypes.c_char_p, []),
@@ -139,11 +134,6 @@ EXPORTS = {   # name -> (restype, argtypes); tests check every symbol include/mr
     'mrphy_fused_partial_elems': (ctypes.c_size_t, [ctypes.POINTER(FusedArgs)]),
     'mrphy_blochsim_fused_fwd': (ctypes.c_int, [ctypes.POINTER(FusedArgs), c_vp]),
     'mrphy_blochsim_fused_bwd': (ctypes.c_int, [ctypes.POINTER(FusedArgs), ctypes.c_int, c_vp]),
-    'mrphy_blochsim_fused_bwd_design': (ctypes.c_int, [ctypes.POINTER(FusedArgs), ctypes.c_int, ctypes.POINTER(ReparamArgs), c_vp]),
-    'mrphy_blochsim_fused_bwd_spin': (ctypes.c_int, [ctypes.POINTER(FusedArgs), ctypes.c_int, ctypes.POINTER(SpinGradArgs), c_vp]),
-    'mrphy_blochsim_fused_fwd_rec': (ctypes.c_int, [ctypes.POINTER(FusedArgs), ctypes.POINTER(RecordArgs), c_vp]),
-    'mrphy_blochsim_fused_bwd_rec': (ctypes.c_int, [ctypes.POINTER(FusedArgs), ctypes.c_int, ctypes.POINTER(RecordArgs),
-                                                    ctypes.POINTER(SpinGradArgs), c_vp]),
     'mrphy_beff_ckpt_elems': (ctypes.c_size_t, [ctypes.POINTER(BeffArgs)]),
     'mrphy_blochsim_beff_fwd': (ctypes.c_int, [ctypes.POINTER(BeffArgs), c_vp]),
     'mrphy_blochsim_beff_bwd': (ctypes.c_int, [ctypes.POINTER(BeffArgs), c_vp]),
@@ -185,7 +175,7 @@ def lib():
                     raise RuntimeError(f'mrphy (B200): ABI version mismatch: library {L.mrphy_abi_version()} '
                                        f'!= binding {ABI_VERSION}; rebuild with mrphy.py_b200/build.py')
                 mirrors = (Param, FusedArgs, BeffArgs, RfGr2BeffArgs, Beff2abArgs, Beff2uphiArgs, FreePrecArgs, ReparamArgs,
-                           MaskArgs, ClampArgs, SpinGradArgs, RecordArgs)
+                           MaskArgs, ClampArgs)
                 for which, cls in enumerate(mirrors):
                     if L.mrphy_sizeof_args(which) != ctypes.sizeof(cls):
                         raise RuntimeError(f'mrphy (B200): layout of {cls.__name__} ({ctypes.sizeof(cls)} B) differs from '

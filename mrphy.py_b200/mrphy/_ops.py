@@ -5,6 +5,7 @@ with ``beffective.rfgr2beff`` (beffective.py:107-168) followed by ``sims.BlochSi
 ``.backward`` (sims.py:31-269) and the autograd of ``rfgr2beff``.  ``fused_applypulse`` is the
 Python-level entry used by ``mobjs.SpinArray.applypulse`` (mobjs.py:394-450).
 """
+import ctypes
 import numbers
 import os
 import weakref
@@ -136,24 +137,28 @@ def _stream():
 
 
 def _impl_blochsim_fused_fwd(Mi: Tensor, rf: Tensor, gr: Tensor, loc: Tensor, df: Optional[Tensor], b1: Optional[Tensor],
-                       T1: Optional[Tensor], T2: Optional[Tensor], gamma: Tensor, dt: Tensor, K: int,
-                       flags: int) -> Tuple[Tensor, Tensor, Tensor]:
-    """-> (Mo (N,nM,3), ckpt, wave): final magnetisation, K-step checkpoints, packed waveform."""
+                       T1: Optional[Tensor], T2: Optional[Tensor], gamma: Tensor, dt: Tensor, K: int, flags: int,
+                       every: int) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """-> (Mo (N,nM,3), Mt, ckpt, wave): final magnetisation, recorded states, K-step checkpoints, packed waveform.
+    every > 0 records Mt (N, nR, 3, nM), nR = nT // every: the state after (r+1)*every steps, lab frame; else Mt is (0,)."""
     L = _cabi.lib()
     a = _cabi.FusedArgs()
     _fill_common(a, Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags)
     kw = {'dtype': Mi.dtype, 'device': Mi.device}
     Mo = torch.empty((a.N, a.nM, 3), **kw)
+    Mt = torch.empty((a.N, a.nT // every, 3, a.nM) if every else (0,), **kw)
     ckpt = torch.empty(L.mrphy_fused_ckpt_elems(a), **kw)
     wave = torch.empty(L.mrphy_fused_wave_elems(a), **kw)
     a.Mo, a.ckpt, a.wave = Mo.data_ptr(), ckpt.data_ptr(), wave.data_ptr()
+    if every:
+        a.every, a.nR, a.Mt = every, a.nT // every, Mt.data_ptr()
     with torch.cuda.device(Mi.device):
         _cabi.check(L.mrphy_blochsim_fused_fwd(a, _stream()), 'blochsim_fused_fwd')
     _cabi.count_launches()
-    return Mo, ckpt, wave
+    return Mo, Mt, ckpt, wave
 
 
-def _fake_blochsim_fused_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags):
+def _fake_blochsim_fused_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every):
     N, nM, nT = loc.shape[0], loc.shape[1], rf.shape[2]
     chunks = (nT + K - 1) // K
     nc = 1 if b1 is None else (rf.shape[3] if rf.ndim == 4 else 1)
@@ -163,16 +168,26 @@ def _fake_blochsim_fused_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flag
     chunk = WS * ((K + 3) // 4 * 4)
     if Mi.element_size() == 4 and NC >= 4 and K <= TC_K_MAX and os.environ.get('MRPHY_B200_TC', '1')[:1] != '0':
         chunk = max(chunk, ((K + 7) // 8 * 8) * (16 * (NC // 2) + 3))   # csrc: TcLayout (tensor-core operand tiles + gr rows)
-    return (Mi.new_empty((N, nM, 3)), Mi.new_empty((max(N * (chunks - 1) * 3 * nM, 1),)),
-            Mi.new_empty((N * chunks * chunk,)))
+    return (Mi.new_empty((N, nM, 3)), Mi.new_empty((N, nT // every, 3, nM) if every else (0,)),
+            Mi.new_empty((max(N * (chunks - 1) * 3 * nM, 1),)), Mi.new_empty((N * chunks * chunk,)))
 
 
-def _fused_bwd_call(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, design=None, spin=None, rec=None):
-    """The backward launch sequence; `design` = (rho, theta, rfmax, ts, smax, ddt, rf_kind, gr_kind) adds the adjoint of the
-    re-parametrisation to the gradient epilogue (mrphy_blochsim_fused_bwd_design), `spin` = (want_loc, want_sz, want_b1) the
-    per-spin gradients (mrphy_blochsim_fused_bwd_spin), `rec` = (every, gMt) the gradient of the recorded states
-    (mrphy_blochsim_fused_bwd_rec, with or without `spin`).
-    -> (gMi, flat, grho, gtheta, gts) | (gMi, flat, gloc, gsz, gb1)."""
+def _impl_blochsim_fused_bwd(gMo: Tensor, gMt: Optional[Tensor], Mo: Tensor, ckpt: Tensor, wave: Tensor, rf: Tensor,
+                             gr: Tensor, loc: Tensor, df: Optional[Tensor], b1: Optional[Tensor], T1: Optional[Tensor],
+                             T2: Optional[Tensor], gamma: Tensor, dt: Tensor, K: int, flags: int, every: int, want_loc: bool,
+                             want_sz: bool, want_b1: bool, rho: Optional[Tensor], theta: Optional[Tensor],
+                             rfmax: Optional[Tensor], ts: Optional[Tensor], smax: Optional[Tensor], ddt: Optional[Tensor],
+                             rf_kind: int, gr_kind: int):
+    """-> (gMi (N,nM,3) or empty, flat, gloc, gsz, gb1, grho, gtheta, gts); every output not asked for is (0,).
+    flat = [dL/drf like rf (absent with FLAG_SKIP_GRF) | dL/dgr (N,3,nT) (absent with FLAG_SKIP_GGR) | GRAD_TAIL spare
+    elements, zero]; `split_wave_grads` cuts the views.  Options:
+    - every > 0: the backward of a recording forward; gMt = dL/dMt (N, nR, 3, nM) contiguous on top of dL/dMo.
+    - want_loc / want_sz / want_b1: the per-spin sums over time of dL/dBeff, formed inside the backward kernel without the
+      dense field: gloc (N,nM,3) = sum_t gr*gBz, gsz (N,nM) = sum_t gBz, gb1 (N,nM,2,nC) -- the outputs of
+      rfgr2beff_spin_grads.  want_b1 needs b1.
+    - rf_kind / gr_kind > 0: (dL/drho, dL/dtheta, dL/dts) of the re-parametrisation (rho, theta, rfmax) -> rf,
+      (ts, smax, ddt) -> gr, evaluated in the tail of the gradient epilogue: no launch of its own.  Combines with neither
+      of the others."""
     L = _cabi.lib()
     a = _cabi.FusedArgs()
     _fill_common(a, None, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags)
@@ -196,31 +211,16 @@ def _fused_bwd_call(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt,
     a.gMo, a.gMo_sn, a.gMo_sm = gMo.data_ptr(), _bstride(gMo, 0), _bstride(gMo, 1)
     a.gMi, a.grf, a.ggr, a.partials = (gMi.data_ptr() if need_gmi else None), (grf.data_ptr() if want_rf else None), \
         (ggr.data_ptr() if want_gr else None), partials.data_ptr()
-    grho = gtheta = gts = flat[:0]
-    if spin is not None or rec is not None:
-        want_loc, want_sz, want_b1 = spin if spin is not None else (False, False, False)
+    gloc = gsz = gb1 = grho = gtheta = gts = flat[:0]
+    if every:
+        a.every, a.nR, a.gMt = every, a.nT // every, gMt.data_ptr()
+    if want_loc or want_sz or want_b1:
         e = lambda shape, on: torch.empty(shape if on else (0,), **kw)
         gloc, gsz, gb1 = e((a.N, a.nM, 3), want_loc), e((a.N, a.nM), want_sz), e((a.N, a.nM, 2, a.nC), want_b1)
-        s = None
-        if want_loc or want_sz or want_b1:
-            s = _cabi.SpinGradArgs()
-            s.gloc, s.gsz, s.gb1 = (gloc.data_ptr() if want_loc else None), (gsz.data_ptr() if want_sz else None), \
-                (gb1.data_ptr() if want_b1 else None)
-        with torch.cuda.device(Mo.device):
-            if rec is None:
-                _cabi.check(L.mrphy_blochsim_fused_bwd_spin(a, 1, s, _stream()), 'blochsim_fused_bwd_spin')
-            else:
-                every, gMt = rec
-                r = _cabi.RecordArgs()
-                r.every, r.nR, r.gMt = every, a.nT // every, gMt.data_ptr()
-                _cabi.check(L.mrphy_blochsim_fused_bwd_rec(a, 1, r, s, _stream()), 'blochsim_fused_bwd_rec')
-        _cabi.count_launches()
-        return gMi, flat, gloc, gsz, gb1
-    if design is None:
-        with torch.cuda.device(Mo.device):
-            _cabi.check(L.mrphy_blochsim_fused_bwd(a, 1, _stream()), 'blochsim_fused_bwd')
-    else:
-        rho, theta, rfmax, ts, smax, ddt, rf_kind, gr_kind = design
+        a.gloc, a.gsz, a.gb1 = (gloc.data_ptr() if want_loc else None), (gsz.data_ptr() if want_sz else None), \
+            (gb1.data_ptr() if want_b1 else None)
+    d = None                                  # the ReparamArgs a.design points to: alive until the call returns
+    if rf_kind or gr_kind:
         d, _ = _reparam_args(rho, theta, rfmax, ts, smax, ddt, rf_kind, gr_kind, True)
         if rf_kind:
             grho, gtheta = torch.empty(rho.shape, **kw), torch.empty(theta.shape, **kw)
@@ -228,102 +228,21 @@ def _fused_bwd_call(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt,
         if gr_kind:
             gts = torch.empty(ts.shape, **kw)
             d.gts = gts.data_ptr()
-        with torch.cuda.device(Mo.device):
-            _cabi.check(L.mrphy_blochsim_fused_bwd_design(a, 1, d, _stream()), 'blochsim_fused_bwd_design')
+        a.design = ctypes.addressof(d)
+    with torch.cuda.device(Mo.device):
+        _cabi.check(L.mrphy_blochsim_fused_bwd(a, 1, _stream()), 'blochsim_fused_bwd')
     _cabi.count_launches()
-    return gMi, flat, grho, gtheta, gts
+    return gMi, flat, gloc, gsz, gb1, grho, gtheta, gts
 
 
-def _impl_blochsim_fused_bwd(gMo: Tensor, Mo: Tensor, ckpt: Tensor, wave: Tensor, rf: Tensor, gr: Tensor, loc: Tensor,
-                       df: Optional[Tensor], b1: Optional[Tensor], T1: Optional[Tensor], T2: Optional[Tensor],
-                       gamma: Tensor, dt: Tensor, K: int, flags: int) -> Tuple[Tensor, Tensor]:
-    """-> (gMi (N,nM,3) or empty, flat): flat = [dL/drf like rf (absent with FLAG_SKIP_GRF) | dL/dgr (N,3,nT) (absent with
-    FLAG_SKIP_GGR) | GRAD_TAIL spare elements, zero]; `split_wave_grads` cuts the views."""
-    return _fused_bwd_call(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags)[:2]
-
-
-def _impl_blochsim_fused_bwd_design(gMo: Tensor, Mo: Tensor, ckpt: Tensor, wave: Tensor, rf: Tensor, gr: Tensor, loc: Tensor,
-                                    df: Optional[Tensor], b1: Optional[Tensor], T1: Optional[Tensor], T2: Optional[Tensor],
-                                    gamma: Tensor, dt: Tensor, K: int, flags: int, rho: Optional[Tensor],
-                                    theta: Optional[Tensor], rfmax: Optional[Tensor], ts: Optional[Tensor],
-                                    smax: Optional[Tensor], ddt: Optional[Tensor], rf_kind: int, gr_kind: int):
-    """As blochsim_fused_bwd, plus (dL/drho, dL/dtheta, dL/dts) of the re-parametrisation that produced rf / gr (empty for an
-    absent half), evaluated in the tail of the gradient epilogue: no launch of its own."""
-    return _fused_bwd_call(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags,
-                           (rho, theta, rfmax, ts, smax, ddt, rf_kind, gr_kind))
-
-
-def _impl_blochsim_fused_bwd_spin(gMo: Tensor, Mo: Tensor, ckpt: Tensor, wave: Tensor, rf: Tensor, gr: Tensor, loc: Tensor,
-                                  df: Optional[Tensor], b1: Optional[Tensor], T1: Optional[Tensor], T2: Optional[Tensor],
-                                  gamma: Tensor, dt: Tensor, K: int, flags: int, want_loc: bool, want_sz: bool, want_b1: bool):
-    """As blochsim_fused_bwd, plus the per-spin sums over time of dL/dBeff (empty where not wanted): gloc (N,nM,3) =
-    sum_t gr*gBz, gsz (N,nM) = sum_t gBz, gb1 (N,nM,2,nC) -- the outputs of rfgr2beff_spin_grads, formed inside the backward
-    kernel without the dense field.  want_b1 needs b1."""
-    return _fused_bwd_call(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags,
-                           spin=(bool(want_loc), bool(want_sz), bool(want_b1)))
-
-
-def _impl_blochsim_fused_fwd_rec(Mi: Tensor, rf: Tensor, gr: Tensor, loc: Tensor, df: Optional[Tensor], b1: Optional[Tensor],
-                                 T1: Optional[Tensor], T2: Optional[Tensor], gamma: Tensor, dt: Tensor, K: int, flags: int,
-                                 every: int) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
-    """As blochsim_fused_fwd, plus Mt (N, nR, 3, nM), nR = nT // every: the state after (r+1)*every steps, lab frame.
-    -> (Mo, Mt, ckpt, wave)."""
-    L = _cabi.lib()
-    a = _cabi.FusedArgs()
-    _fill_common(a, Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags)
-    kw = {'dtype': Mi.dtype, 'device': Mi.device}
-    Mo = torch.empty((a.N, a.nM, 3), **kw)
-    Mt = torch.empty((a.N, a.nT // every, 3, a.nM), **kw)
-    ckpt = torch.empty(L.mrphy_fused_ckpt_elems(a), **kw)
-    wave = torch.empty(L.mrphy_fused_wave_elems(a), **kw)
-    a.Mo, a.ckpt, a.wave = Mo.data_ptr(), ckpt.data_ptr(), wave.data_ptr()
-    r = _cabi.RecordArgs()
-    r.every, r.nR, r.Mt = every, a.nT // every, Mt.data_ptr()
-    with torch.cuda.device(Mi.device):
-        _cabi.check(L.mrphy_blochsim_fused_fwd_rec(a, r, _stream()), 'blochsim_fused_fwd_rec')
-    _cabi.count_launches()
-    return Mo, Mt, ckpt, wave
-
-
-def _fake_blochsim_fused_fwd_rec(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every):
-    Mo, ckpt, wave = _fake_blochsim_fused_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags)
-    return Mo, Mi.new_empty((loc.shape[0], rf.shape[2] // every, 3, loc.shape[1])), ckpt, wave
-
-
-def _impl_blochsim_fused_bwd_rec(gMo: Tensor, gMt: Tensor, Mo: Tensor, ckpt: Tensor, wave: Tensor, rf: Tensor, gr: Tensor,
-                                 loc: Tensor, df: Optional[Tensor], b1: Optional[Tensor], T1: Optional[Tensor],
-                                 T2: Optional[Tensor], gamma: Tensor, dt: Tensor, K: int, flags: int, every: int,
-                                 want_loc: bool, want_sz: bool, want_b1: bool):
-    """As blochsim_fused_bwd_spin, with dL/dMt (N, nR, 3, nM) contiguous -- the gradient of blochsim_fused_fwd_rec's Mt --
-    on top of dL/dMo; no per-spin gradient wanted is fine."""
-    return _fused_bwd_call(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags,
-                           spin=(bool(want_loc), bool(want_sz), bool(want_b1)), rec=(every, gMt))
-
-
-def _fake_blochsim_fused_bwd_rec(gMo, gMt, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every, want_loc,
-                                 want_sz, want_b1):
-    return _fake_blochsim_fused_bwd_spin(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, want_loc,
-                                         want_sz, want_b1)
-
-
-def _fake_blochsim_fused_bwd_spin(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, want_loc, want_sz,
-                                  want_b1):
-    gMi, flat = _fake_blochsim_fused_bwd(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags)
+def _fake_blochsim_fused_bwd(gMo, gMt, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every, want_loc,
+                             want_sz, want_b1, rho, theta, rfmax, ts, smax, ddt, rf_kind, gr_kind):
+    n = (0 if flags & _cabi.FLAG_SKIP_GRF else rf.numel()) + (0 if flags & _cabi.FLAG_SKIP_GGR else rf.shape[0] * 3 * rf.shape[2])
     N, nM, nC = loc.shape[0], loc.shape[1], (rf.shape[3] if rf.ndim == 4 else 1)
     e = lambda shape, on: Mo.new_empty(shape if on else (0,))
-    return gMi, flat, e((N, nM, 3), want_loc), e((N, nM), want_sz), e((N, nM, 2, nC), want_b1)
-
-
-def _fake_blochsim_fused_bwd_design(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, rho, theta, rfmax,
-                                    ts, smax, ddt, rf_kind, gr_kind):
-    gMi, flat = _fake_blochsim_fused_bwd(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags)
-    e = lambda like, on: Mo.new_empty(like.shape if on else (0,))
-    return gMi, flat, e(rho, rf_kind), e(theta, rf_kind), e(ts, gr_kind)
-
-
-def _fake_blochsim_fused_bwd(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags):
-    n = (0 if flags & _cabi.FLAG_SKIP_GRF else rf.numel()) + (0 if flags & _cabi.FLAG_SKIP_GGR else rf.shape[0] * 3 * rf.shape[2])
-    return Mo.new_empty(Mo.shape if flags & _cabi.FLAG_NEED_GMI else (0,)), Mo.new_empty((n + GRAD_TAIL,))
+    return (e(Mo.shape, flags & _cabi.FLAG_NEED_GMI), Mo.new_empty((n + GRAD_TAIL,)), e((N, nM, 3), want_loc),
+            e((N, nM), want_sz), e((N, nM, 2, nC), want_b1), e(rho.shape if rf_kind else (), rf_kind),
+            e(theta.shape if rf_kind else (), rf_kind), e(ts.shape if gr_kind else (), gr_kind))
 
 
 GRAD_TAIL = 4      # spare elements behind the waveform gradients (16-byte granule); [0] is where `parallel` puts the loss
@@ -337,12 +256,29 @@ def split_wave_grads(flat: Tensor, rf: Tensor, flags: int):
     return (flat[:n_rf].view(rf.shape) if n_rf else None), (flat[n_rf:n_rf + n_gr].view(N, 3, nT) if n_gr else None)
 
 
+def _fused_grads(ctx, want, gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, gMt=None, every=0,
+                 spin=(False, False, False), design=(None,) * 6 + (0, 0)):
+    """The fused backward of a forward run with ctx.K, ctx.flags.  want = (dL/dMi, dL/drf, dL/dgr) wanted: the rows of the
+    spin reduction of the others are not even formed.  -> (gMi or None, grf, ggr, gloc, gsz, gb1, grho, gtheta, gts)."""
+    if gMo is None:
+        gMo = torch.zeros_like(Mo)
+    if gMo.stride(-1) != 1 or gMo.dtype != Mo.dtype:
+        gMo = gMo.to(Mo.dtype).contiguous()
+    flags = ctx.flags | (_cabi.FLAG_NEED_GMI if want[0] else 0) | (0 if want[1] else _cabi.FLAG_SKIP_GRF) | \
+        (0 if want[2] else _cabi.FLAG_SKIP_GGR)
+    gMi, flat, *rest = blochsim_fused_bwd(gMo, gMt, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, ctx.K, flags,
+                                          every, *spin, *design)
+    return (gMi if want[0] else None, *split_wave_grads(flat, rf, flags), *rest)
+
+
 def _fused_setup(ctx, inputs, output):
-    Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags = inputs
-    Mo, ckpt, wave = output
-    ctx.K, ctx.flags = K, flags
+    Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every = inputs
+    Mo, _Mt, ckpt, wave = output
+    ctx.K, ctx.flags, ctx.every = K, flags, every
     ctx.has = [x is not None for x in (df, b1, T1, T2)]
     ctx.save_for_backward(Mo, ckpt, wave, rf, gr, loc, gamma, dt, *[x for x in (df, b1, T1, T2) if x is not None])
+    if every:
+        ctx.set_materialize_grads(False)      # a loss that ignores Mt (or M) hands None for it, not a tensor of zeros
 
 
 def _param_2d(x: Tensor) -> Tensor:
@@ -359,7 +295,9 @@ def _as_param_grad(g: Tensor, x: Tensor) -> Tensor:
     return g.sum_to_size(_param_2d(x).shape).reshape(x.shape).to(x.dtype)
 
 
-def _fused_backward(ctx, gMo, _gckpt, _gwave, gMt=None):
+def _fused_backward(ctx, gMo, gMt, _gckpt, _gwave):
+    """With no gradient on Mt (or no record) the backward without record (same kernels, same bits); else the REC backward,
+    with dL/dMo = 0 when the loss ignores M."""
     Mo, ckpt, wave, rf, gr, loc, gamma, dt, *opt = ctx.saved_tensors
     opt = list(opt)
     df, b1, T1, T2 = (opt.pop(0) if h else None for h in ctx.has)
@@ -368,29 +306,14 @@ def _fused_backward(ctx, gMo, _gckpt, _gwave, gMt=None):
     want_loc, want_b1 = bool(need[3]), bool(need[5] and b1 is not None)
     want_sz = df is not None and bool(need[4] or need[8])
     if not (any(need[0:3]) or want_loc or want_sz or want_b1):
-        return (None,) * 12
-    if gMo is None:
-        gMo = torch.zeros_like(Mo)
-    if gMo.stride(-1) != 1 or gMo.dtype != Mo.dtype:
-        gMo = gMo.to(Mo.dtype).contiguous()
-    # only the gradients autograd asks for: the rows of the spin reduction of the others are not even formed
-    flags = ctx.flags | (_cabi.FLAG_NEED_GMI if need[0] else 0) | (0 if need[1] else _cabi.FLAG_SKIP_GRF) | \
-        (0 if need[2] else _cabi.FLAG_SKIP_GGR)
-    if gMt is not None:
+        return (None,) * 13
+    every = ctx.every if gMt is not None else 0
+    if every and (gMt.dtype != Mo.dtype or not gMt.is_contiguous()):
         # dL/dMt in the kernel's layout (N, nR, 3, nM) and dtype: a loss formed elementwise from the permuted view the caller
         # got hands its gradient back in that layout already; anything else costs this one copy
-        if gMt.dtype != Mo.dtype or not gMt.is_contiguous():
-            gMt = torch.empty(gMt.shape, dtype=Mo.dtype, device=Mo.device).copy_(gMt)
-        gMi, flat, gloc, gsz, gb1 = blochsim_fused_bwd_rec(gMo, gMt, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt,
-                                                           ctx.K, flags, ctx.every, want_loc, want_sz, want_b1)
-    elif not (want_loc or want_sz or want_b1):
-        gMi, flat = blochsim_fused_bwd(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, ctx.K, flags)
-        grf, ggr = split_wave_grads(flat, rf, flags)
-        return (gMi if need[0] else None, grf, ggr) + (None,) * 9
-    else:
-        gMi, flat, gloc, gsz, gb1 = blochsim_fused_bwd_spin(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt,
-                                                            ctx.K, flags, want_loc, want_sz, want_b1)
-    grf, ggr = split_wave_grads(flat, rf, flags)
+        gMt = torch.empty(gMt.shape, dtype=Mo.dtype, device=Mo.device).copy_(gMt)
+    gMi, grf, ggr, gloc, gsz, gb1, *_ = _fused_grads(ctx, need[0:3], gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma,
+                                                     dt, gMt if every else None, every, (want_loc, want_sz, want_b1))
     gdf = ggam = None
     if want_sz:     # ∂Δf = gsz/γ, ∂γ = -gsz·Δf/γ² (the chain rule of Bz += Δf/γ, beffective.py:142)
         gam2, df2 = _param_2d(gamma), _param_2d(df)
@@ -398,21 +321,8 @@ def _fused_backward(ctx, gMo, _gckpt, _gwave, gMt=None):
             gdf = _as_param_grad(gsz / gam2, df)
         if need[8]:
             ggam = _as_param_grad(-gsz * df2 / (gam2 * gam2), gamma)
-    return (gMi if need[0] else None, grf, ggr, gloc if want_loc else None, gdf, gb1 if want_b1 else None,
-            None, None, ggam, None, None, None)
-
-
-def _fused_rec_setup(ctx, inputs, output):
-    Mo, _Mt, ckpt, wave = output
-    _fused_setup(ctx, inputs[:12], (Mo, ckpt, wave))
-    ctx.every = inputs[12]
-    ctx.set_materialize_grads(False)      # a loss that ignores Mt (or M) hands None for it, not a tensor of zeros
-
-
-def _fused_rec_backward(ctx, gMo, gMt, _gckpt, _gwave):
-    """With no gradient on Mt this is the backward of blochsim_fused_fwd (same entry, same bits); else the REC backward,
-    with dL/dMo = 0 when the loss ignores M."""
-    return _fused_backward(ctx, gMo, None, None, gMt) + (None,)
+    return (gMi, grf, ggr, gloc if want_loc else None, gdf, gb1 if want_b1 else None, None, None, ggam, None, None, None,
+            None)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -852,7 +762,7 @@ def _mask_backward(ctx, g):
 # registration: raw torch.library definitions (schema + CUDA impl + fake), which cost ~20 us per call instead of
 # the ~130 us of the `torch.library.custom_op` convenience wrapper -- it matters for test-scale problems
 _LIB = torch.library.Library('mrphy_b200', 'DEF')
-_SCHEMAS = {'blochsim_fused_fwd': '(Tensor Mi, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor, Tensor)', 'blochsim_fused_bwd': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'blochsim_fused_bwd_design': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? ddt, int rf_kind, int gr_kind) -> (Tensor, Tensor, Tensor, Tensor, Tensor)', 'blochsim_fused_bwd_spin': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, bool want_loc, bool want_sz, bool want_b1) -> (Tensor, Tensor, Tensor, Tensor, Tensor)', 'blochsim_fused_fwd_rec': '(Tensor Mi, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, int every) -> (Tensor, Tensor, Tensor, Tensor)', 'blochsim_fused_bwd_rec': '(Tensor gMo, Tensor gMt, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, int every, bool want_loc, bool want_sz, bool want_b1) -> (Tensor, Tensor, Tensor, Tensor, Tensor)', 'blochsim_beff_fwd': '(Tensor Mi, Tensor Beff, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'blochsim_beff_bwd': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor Beff, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'rfgr2beff': '(Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor gamma) -> Tensor', 'rfgr2beff_bwd': '(Tensor gB, Tensor rf, Tensor gr, Tensor loc, Tensor? b1) -> (Tensor, Tensor)', 'rfgr2beff_spin_grads': '(Tensor gB, Tensor rf, Tensor gr, bool want_loc, bool want_b1) -> (Tensor, Tensor, Tensor)', 'beff2ab': '(Tensor beff, Tensor E1, Tensor E2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor, Tensor)', 'beff2ab_bwd': '(Tensor gA, Tensor gB, Tensor A, Tensor B, Tensor ckpt, Tensor beff, Tensor E1, Tensor E2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'beff2uphi': '(Tensor beff, Tensor g) -> (Tensor, Tensor)', 'beff2uphi_bwd': '(Tensor? gU, Tensor? gPhi, Tensor beff, Tensor g) -> (Tensor, Tensor)', 'freeprec': '(Tensor Mi, Tensor dur, Tensor? T1, Tensor? T2, Tensor? df, bool adjoint) -> Tensor', 'design_waveform': '(Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? dt, int rf_kind, int gr_kind) -> (Tensor, Tensor)', 'design_waveform_bwd': '(Tensor? grf, Tensor? ggr, Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? dt, int rf_kind, int gr_kind) -> (Tensor, Tensor, Tensor)', 'mask_copy': '(Tensor v, Tensor idx, Tensor inv, bool fill_zero) -> Tensor', 'clamp_waveform': '(Tensor x, Tensor lim, float eps, int kind) -> Tensor', 'clamp_waveform_bwd': '(Tensor g, Tensor x, Tensor lim, float eps, int kind) -> Tensor'}
+_SCHEMAS = {'blochsim_fused_fwd': '(Tensor Mi, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, int every) -> (Tensor, Tensor, Tensor, Tensor)', 'blochsim_fused_bwd': '(Tensor gMo, Tensor? gMt, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, int every, bool want_loc, bool want_sz, bool want_b1, Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? ddt, int rf_kind, int gr_kind) -> (Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor)', 'blochsim_beff_fwd': '(Tensor Mi, Tensor Beff, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'blochsim_beff_bwd': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor Beff, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'rfgr2beff': '(Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor gamma) -> Tensor', 'rfgr2beff_bwd': '(Tensor gB, Tensor rf, Tensor gr, Tensor loc, Tensor? b1) -> (Tensor, Tensor)', 'rfgr2beff_spin_grads': '(Tensor gB, Tensor rf, Tensor gr, bool want_loc, bool want_b1) -> (Tensor, Tensor, Tensor)', 'beff2ab': '(Tensor beff, Tensor E1, Tensor E2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor, Tensor)', 'beff2ab_bwd': '(Tensor gA, Tensor gB, Tensor A, Tensor B, Tensor ckpt, Tensor beff, Tensor E1, Tensor E2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'beff2uphi': '(Tensor beff, Tensor g) -> (Tensor, Tensor)', 'beff2uphi_bwd': '(Tensor? gU, Tensor? gPhi, Tensor beff, Tensor g) -> (Tensor, Tensor)', 'freeprec': '(Tensor Mi, Tensor dur, Tensor? T1, Tensor? T2, Tensor? df, bool adjoint) -> Tensor', 'design_waveform': '(Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? dt, int rf_kind, int gr_kind) -> (Tensor, Tensor)', 'design_waveform_bwd': '(Tensor? grf, Tensor? ggr, Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? dt, int rf_kind, int gr_kind) -> (Tensor, Tensor, Tensor)', 'mask_copy': '(Tensor v, Tensor idx, Tensor inv, bool fill_zero) -> Tensor', 'clamp_waveform': '(Tensor x, Tensor lim, float eps, int kind) -> Tensor', 'clamp_waveform_bwd': '(Tensor g, Tensor x, Tensor lim, float eps, int kind) -> Tensor'}
 
 
 def _register(name, impl, fake):
@@ -864,10 +774,6 @@ def _register(name, impl, fake):
 
 blochsim_fused_fwd = _register('blochsim_fused_fwd', _impl_blochsim_fused_fwd, _fake_blochsim_fused_fwd)
 blochsim_fused_bwd = _register('blochsim_fused_bwd', _impl_blochsim_fused_bwd, _fake_blochsim_fused_bwd)
-blochsim_fused_bwd_design = _register('blochsim_fused_bwd_design', _impl_blochsim_fused_bwd_design, _fake_blochsim_fused_bwd_design)
-blochsim_fused_bwd_spin = _register('blochsim_fused_bwd_spin', _impl_blochsim_fused_bwd_spin, _fake_blochsim_fused_bwd_spin)
-blochsim_fused_fwd_rec = _register('blochsim_fused_fwd_rec', _impl_blochsim_fused_fwd_rec, _fake_blochsim_fused_fwd_rec)
-blochsim_fused_bwd_rec = _register('blochsim_fused_bwd_rec', _impl_blochsim_fused_bwd_rec, _fake_blochsim_fused_bwd_rec)
 blochsim_beff_fwd = _register('blochsim_beff_fwd', _impl_blochsim_beff_fwd, _fake_blochsim_beff_fwd)
 blochsim_beff_bwd = _register('blochsim_beff_bwd', _impl_blochsim_beff_bwd, _fake_blochsim_beff_bwd)
 rfgr2beff_cuda = _register('rfgr2beff', _impl_rfgr2beff, _fake_rfgr2beff)
@@ -884,8 +790,6 @@ mask_copy_cuda = _register('mask_copy', _impl_mask_copy, _fake_mask_copy)
 clamp_waveform_cuda = _register('clamp_waveform', _impl_clamp_waveform, lambda x, lim, eps, kind: x.new_empty(x.shape))
 clamp_waveform_bwd_cuda = _register('clamp_waveform_bwd', _impl_clamp_waveform_bwd, lambda g, x, lim, eps, kind: x.new_empty(x.shape))
 torch.library.register_autograd('mrphy_b200::blochsim_fused_fwd', _fused_backward, setup_context=_fused_setup, lib=_LIB)
-torch.library.register_autograd('mrphy_b200::blochsim_fused_fwd_rec', _fused_rec_backward, setup_context=_fused_rec_setup,
-                                lib=_LIB)
 torch.library.register_autograd('mrphy_b200::design_waveform', _design_backward, setup_context=_design_setup, lib=_LIB)
 torch.library.register_autograd('mrphy_b200::mask_copy', _mask_backward, setup_context=_mask_setup, lib=_LIB)
 torch.library.register_autograd('mrphy_b200::clamp_waveform', _clamp_backward, setup_context=_clamp_setup, lib=_LIB)
@@ -931,11 +835,11 @@ def _design_of(x: Tensor, used: Tensor) -> Optional[_DesignRecord]:
 
 class _FusedDesignApply(torch.autograd.Function):
     """Mo(Mi, rf | (rho, theta), gr | ts): forward = the fused simulation on the waveforms the chain already produced;
-    backward = mrphy_blochsim_fused_bwd_design."""
+    backward = the fused backward with the design tail."""
 
     @staticmethod
     def forward(ctx, Mi, rf, gr, rho, theta, ts, loc, df, b1, T1, T2, gamma, dt, rfmax, smax, ddt, K, flags, rf_kind, gr_kind):
-        Mo, ckpt, wave = blochsim_fused_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags)
+        Mo, _, ckpt, wave = blochsim_fused_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, 0)
         opt = (df, b1, T1, T2, rho, theta, rfmax, ts, smax, ddt)
         ctx.has = [x is not None for x in opt]
         ctx.K, ctx.flags, ctx.kinds = K, flags, (rf_kind, gr_kind)
@@ -952,20 +856,11 @@ class _FusedDesignApply(torch.autograd.Function):
         gk = ctx.kinds[1] if need[5] else 0
         if not (need[0] or need[1] or need[2] or rk or gk):
             return (None,) * 20
-        if gMo.stride(-1) != 1 or gMo.dtype != Mo.dtype:
-            gMo = gMo.to(Mo.dtype).contiguous()
-        flags = ctx.flags | (_cabi.FLAG_NEED_GMI if need[0] else 0) | (0 if (need[1] or rk) else _cabi.FLAG_SKIP_GRF) | \
-            (0 if (need[2] or gk) else _cabi.FLAG_SKIP_GGR)
-        if rk or gk:
-            gMi, flat, grho, gtheta, gts = blochsim_fused_bwd_design(
-                gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, ctx.K, flags, rho if rk else None,
-                theta if rk else None, rfmax if rk else None, ts if gk else None, smax if gk else None, ddt if gk else None,
-                rk, gk)
-        else:
-            gMi, flat = blochsim_fused_bwd(gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, ctx.K, flags)
-            grho = gtheta = gts = None
-        grf, ggr = split_wave_grads(flat, rf, flags)
-        return (gMi if need[0] else None, grf if need[1] else None, ggr if need[2] else None,
+        design = (rho if rk else None, theta if rk else None, rfmax if rk else None, ts if gk else None,
+                  smax if gk else None, ddt if gk else None, rk, gk)
+        gMi, grf, ggr, *_, grho, gtheta, gts = _fused_grads(ctx, (need[0], need[1] or rk, need[2] or gk), gMo, Mo, ckpt,
+                                                            wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, design=design)
+        return (gMi, grf if need[1] else None, ggr if need[2] else None,
                 grho if (rk and need[3]) else None, gtheta if (rk and need[4]) else None, gts if gk else None) + (None,) * 14
 
 
@@ -1163,11 +1058,8 @@ def fused_applypulse(M_: Tensor, rf: Tensor, gr: Tensor, loc_: Tensor, *, Δf_: 
             return _FusedDesignApply.apply(Mi, rf.detach() if r_rf is not None else rf, gr.detach() if r_gr is not None else gr,
                                            rho, theta, ts, loc, df, b1, T1, T2, gam, dtt, rfmax, smax, ddt, K, fl,
                                            r_rf.kind if r_rf is not None else 0, r_gr.kind if r_gr is not None else 0)
-    if record is not None:
-        Mo, Mt, _, _ = blochsim_fused_fwd_rec(Mi, rf, gr, loc, df, b1, T1, T2, gam, dtt, K, fl, record)
-        return Mo, Mt.permute(0, 3, 1, 2)
-    Mo, _, _ = blochsim_fused_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gam, dtt, K, fl)
-    return Mo
+    Mo, Mt, _, _ = blochsim_fused_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gam, dtt, K, fl, record or 0)
+    return Mo if record is None else (Mo, Mt.permute(0, 3, 1, 2))
 
 
 def _check_record(record, rf: Tensor, b1Map_: Optional[Tensor]) -> int:

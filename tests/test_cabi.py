@@ -35,12 +35,13 @@ def test_header_symbols_exported(cabi):
     assert set(names) == set(cabi.EXPORTS), 'python binding and header disagree'
 
 
-def test_abi_version_and_struct_layout(cabi):
+def test_abi_version_and_arg_struct_sizes(cabi):
     L = cabi.lib()
     assert L.mrphy_abi_version() == cabi.ABI_VERSION
     # struct sizes must match the C definition (all 8-byte aligned fields)
     assert ctypes.sizeof(cabi.Param) == 32
-    assert ctypes.sizeof(cabi.FusedArgs) == 8 * 4 + 8 * 3 + 8 * 5 + 8 * 4 + 8 * 3 + 8 * 3 + 32 * 5 + 8 * 3 + 8 * 3 + 8 * 4
+    assert ctypes.sizeof(cabi.FusedArgs) == 8 * 4 + 8 * 3 + 8 * 5 + 8 * 4 + 8 * 3 + 8 * 3 + 32 * 5 + 8 * 3 + 8 * 3 + 8 * 4 + \
+        4 * 2 + 8 * 2 + 8 * 3 + 8                    # options: record, per-spin gradients, design tail
     assert ctypes.sizeof(cabi.BeffArgs) == 6 * 4 + 8 * 3 + 8 * 4 + 32 * 4 + 8 * 2 + 8 * 3 + 8 * 2
     # ... and the C side agrees with every ctypes mirror (the loader checks the same and refuses a mismatch)
     for which, cls in enumerate((cabi.Param, cabi.FusedArgs, cabi.BeffArgs, cabi.RfGr2BeffArgs, cabi.Beff2abArgs,
@@ -65,7 +66,7 @@ def test_sizing_entry_points(cabi):
 
 @pytest.mark.parametrize('nC,K,nT', [(1, 64, 1000), (2, 16, 50), (3, 7, 33), (8, 64, 64), (16, 48, 100),
                                       (8, 32, 100), (4, 16, 50), (16, 24, 70), (5, 1, 9)])   # K <= 32, >= 3 coils: tensor-core operand tiles
-def test_fake_shapes_match_sizing_calls(cabi, nC, K, nT):
+def test_fused_fwd_fake_matches_sizing_calls(cabi, nC, K, nT):
     """The torch.library fake (shape-only) implementation must allocate what the C sizing entry points ask for."""
     import torch
     from mrphy import _ops
@@ -77,8 +78,8 @@ def test_fake_shapes_match_sizing_calls(cabi, nC, K, nT):
     m = dict(device='meta')
     rf = torch.empty(N, 2, nT, nC, **m) if nC > 1 else torch.empty(N, 2, nT, **m)
     b1 = torch.empty(N, nM, 2, nC, **m)
-    Mo, ckpt, wave = _ops._fake_blochsim_fused_fwd(torch.empty(N, nM, 3, **m), rf, torch.empty(N, 3, nT, **m),
-                                                   torch.empty(N, nM, 3, **m), None, b1, None, None, None, None, K, 0)
+    Mo, _, ckpt, wave = _ops._fake_blochsim_fused_fwd(torch.empty(N, nM, 3, **m), rf, torch.empty(N, 3, nT, **m),
+                                                      torch.empty(N, nM, 3, **m), None, b1, None, None, None, None, K, 0, 0)
     assert tuple(Mo.shape) == (N, nM, 3)
     assert ckpt.numel() == max(L.mrphy_fused_ckpt_elems(a), 1)
     assert wave.numel() == L.mrphy_fused_wave_elems(a)

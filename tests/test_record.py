@@ -431,54 +431,83 @@ def test_scale_memory(dev):
 
 
 # ---------------------------------------------------------------------------------------------------------- host only
-def test_record_args_mirror_matches_library():
+def test_record_fields_mirror_matches_library():
     from mrphy import _cabi
     L = _cabi.lib()
-    assert L.mrphy_sizeof_args(11) == ctypes.sizeof(_cabi.RecordArgs) == 8 + 2 * ctypes.sizeof(ctypes.c_void_p)
-    assert L.mrphy_abi_version() == _cabi.ABI_VERSION == 6
-    assert {'mrphy_blochsim_fused_fwd_rec', 'mrphy_blochsim_fused_bwd_rec'} <= set(_cabi.EXPORTS)
+    F = _cabi.FusedArgs
+    assert L.mrphy_sizeof_args(1) == ctypes.sizeof(F)
+    assert (F.every.offset, F.nR.offset) == (F.partials.offset + ctypes.sizeof(ctypes.c_void_p), F.partials.offset + 12)
+    assert F.Mt.offset == F.nR.offset + 4 and F.gMt.offset == F.Mt.offset + ctypes.sizeof(ctypes.c_void_p)
+    assert L.mrphy_abi_version() == _cabi.ABI_VERSION == 7
+    assert {'mrphy_blochsim_fused_fwd', 'mrphy_blochsim_fused_bwd'} <= set(_cabi.EXPORTS)
 
 
-def test_record_entry_points_refuse_bad_args():
-    """Inconsistent every / nR and null buffers come back as MRPHY_ERR_ARG before anything is launched."""
+def _refusable_args():
+    """FusedArgs whose checks all pass up to the options; the pointers are never dereferenced: the checks come first."""
     from mrphy import _cabi
-    L = _cabi.lib()
     a = _cabi.FusedArgs()
     a.dtype, a.N, a.nM, a.nT, a.nC, a.K = _cabi.MRPHY_F32, 1, 4, 10, 1, 8
     for p in ('Mi', 'rf', 'gr', 'loc', 'Mo', 'ckpt', 'wave', 'gMo', 'partials', 'grf', 'ggr'):
-        setattr(a, p, 256)                        # never dereferenced: the checks come first
+        setattr(a, p, 256)
     a.gamma.ptr = a.dt.ptr = 256
+    return a
+
+
+def test_fused_entry_points_refuse_bad_record_fields():
+    """Inconsistent every / nR and null buffers come back as MRPHY_ERR_ARG before anything is launched."""
+    from mrphy import _cabi
+    L = _cabi.lib()
     for every, nR, mt, gmt, bwd, msg in ((0, 0, 256, 256, False, 'every'), (11, 0, 256, 256, False, 'every'),
                                          (3, 4, 256, 256, False, 'nR'), (3, 3, None, 256, False, 'Mt is null'),
                                          (3, 3, 256, None, True, 'gMt is null'), (2, 4, 256, 256, True, 'nR')):
-        r = _cabi.RecordArgs()
-        r.every, r.nR, r.Mt, r.gMt = every, nR, mt, gmt
-        rc = L.mrphy_blochsim_fused_bwd_rec(a, 1, r, None, None) if bwd else L.mrphy_blochsim_fused_fwd_rec(a, r, None)
+        a = _refusable_args()
+        a.every, a.nR, a.Mt, a.gMt = every, nR, mt, gmt
+        rc = L.mrphy_blochsim_fused_bwd(a, 1, None) if bwd else L.mrphy_blochsim_fused_fwd(a, None)
         assert rc == -1, (every, nR, rc)
         assert L.mrphy_last_launch_count() == 0
         err = L.mrphy_last_error().decode()
         assert 'record' in err and (msg in err or 'nR == nT / every' in err), err
 
 
+@pytest.mark.parametrize('other', ['record', 'gloc', 'gsz', 'gb1'])
+def test_design_tail_refuses_record_and_spin_grads(other):
+    """The design tail combines with neither record nor per-spin gradients: MRPHY_ERR_ARG, nothing launched."""
+    from mrphy import _cabi
+    L = _cabi.lib()
+    a = _refusable_args()
+    d = _cabi.ReparamArgs()
+    d.dtype, d.adjoint, d.N, d.nT, d.nC, d.rf_kind = a.dtype, 1, a.N, a.nT, 1, 1
+    d.rho = d.theta = d.rfmax = d.grho = d.gtheta = 256      # a design tail that passes its own checks
+    a.design = ctypes.addressof(d)
+    if other == 'record':
+        a.every, a.nR, a.gMt = 5, 2, 256
+    else:
+        setattr(a, other, 256)
+    assert L.mrphy_blochsim_fused_bwd(a, 1, None) == -1
+    assert L.mrphy_last_launch_count() == 0
+    assert 'design' in L.mrphy_last_error().decode()
+
+
 @pytest.mark.parametrize('nC', [0, 1, 8])
-def test_fakes_allocate_implementation_shapes(nC):
+def test_record_fakes_allocate_implementation_shapes(nC):
     from mrphy import _cabi, _ops
     N, nM, nT, every = 2, 37, 50, 7
     e = lambda *s: torch.empty(s, device='meta')
     rf = e(N, 2, nT, nC) if nC else e(N, 2, nT)
     b1 = e(N, nM, 2, nC) if nC else None
     args = (e(N, nM, 3), rf, e(N, 3, nT), e(N, nM, 3), e(N, nM), b1, None, None, e(1, 1), e(1), 16, 0)
-    Mo, Mt, ckpt, wave = _ops._fake_blochsim_fused_fwd_rec(*args, every)
-    ref = _ops._fake_blochsim_fused_fwd(*args)
-    assert Mo.shape == (N, nM, 3) and Mt.shape == (N, nT // every, 3, nM)
-    assert ckpt.shape == ref[1].shape and wave.shape == ref[2].shape and Mt.dtype == Mo.dtype
+    Mo, Mt, ckpt, wave = _ops._fake_blochsim_fused_fwd(*args, every)
+    ref = _ops._fake_blochsim_fused_fwd(*args, 0)
+    assert Mo.shape == (N, nM, 3) and Mt.shape == (N, nT // every, 3, nM) and ref[1].shape == (0,)
+    assert ckpt.shape == ref[2].shape and wave.shape == ref[3].shape and Mt.dtype == Mo.dtype
     want = (True, True, nC > 0)
-    out = _ops._fake_blochsim_fused_bwd_rec(Mo, Mt, Mo, ckpt, wave, rf, e(N, 3, nT), e(N, nM, 3), e(N, nM), b1, None, None,
-                                            e(1, 1), e(1), 16, _cabi.FLAG_NEED_GMI, every, *want)
-    gMi, flat, gloc, gsz, gb1 = out
+    out = _ops._fake_blochsim_fused_bwd(Mo, Mt, Mo, ckpt, wave, rf, e(N, 3, nT), e(N, nM, 3), e(N, nM), b1, None, None,
+                                        e(1, 1), e(1), 16, _cabi.FLAG_NEED_GMI, every, *want, *(None,) * 6, 0, 0)
+    gMi, flat, gloc, gsz, gb1, *design = out
     assert gMi.shape == (N, nM, 3) and flat.shape == (rf.numel() + N * 3 * nT + _ops.GRAD_TAIL,)
     assert gloc.shape == (N, nM, 3) and gsz.shape == (N, nM)
     assert gb1.shape == ((N, nM, 2, nC) if nC else (0,))
+    assert all(g.shape == (0,) for g in design)
 
 
 @pytest.mark.parametrize('record,match', [(0, 'outside'), (31, 'outside'), (-2, 'outside'), (2.5, 'integer'),

@@ -778,23 +778,26 @@ def test_spin_grads_shard_spins(dev, dtype):
 
 
 # ---- no GPU needed ----------------------------------------------------------------------------------------------------
-def test_spin_grad_args_mirror_matches_library():
+def test_spin_grad_fields_mirror_matches_library():
     from mrphy import _cabi
     L = _cabi.lib()
-    assert L.mrphy_sizeof_args(10) == ctypes.sizeof(_cabi.SpinGradArgs) == 3 * ctypes.sizeof(ctypes.c_void_p)
-    assert L.mrphy_abi_version() == _cabi.ABI_VERSION == 6
-    assert 'mrphy_blochsim_fused_bwd_spin' in _cabi.EXPORTS
+    F, P = _cabi.FusedArgs, ctypes.sizeof(ctypes.c_void_p)
+    assert L.mrphy_sizeof_args(1) == ctypes.sizeof(F)
+    assert (F.gloc.offset, F.gsz.offset, F.gb1.offset) == (F.gMt.offset + P, F.gMt.offset + 2 * P, F.gMt.offset + 3 * P)
+    assert L.mrphy_abi_version() == _cabi.ABI_VERSION == 7
+    assert 'mrphy_blochsim_fused_bwd' in _cabi.EXPORTS
 
 
 @pytest.mark.parametrize('nC,want', [(1, (True, True, True)), (8, (False, True, True)), (0, (True, False, False))])
-def test_fake_allocates_implementation_shapes(nC, want):
+def test_spin_grad_fake_allocates_implementation_shapes(nC, want):
     from mrphy import _cabi, _ops
     N, nM, nT = 2, 37, 50
     e = lambda *s: torch.empty(s, device='meta')
     rf = e(N, 2, nT, nC) if nC else e(N, 2, nT)
-    out = _ops._fake_blochsim_fused_bwd_spin(e(N, nM, 3), e(N, nM, 3), e(10), e(10), rf, e(N, 3, nT), e(N, nM, 3), e(N, nM),
-                                            e(N, nM, 2, max(nC, 1)), None, None, e(1, 1), e(1), 16, _cabi.FLAG_NEED_GMI, *want)
-    gMi, flat, gloc, gsz, gb1 = out
+    out = _ops._fake_blochsim_fused_bwd(e(N, nM, 3), None, e(N, nM, 3), e(10), e(10), rf, e(N, 3, nT), e(N, nM, 3),
+                                        e(N, nM), e(N, nM, 2, max(nC, 1)), None, None, e(1, 1), e(1), 16,
+                                        _cabi.FLAG_NEED_GMI, 0, *want, *(None,) * 6, 0, 0)
+    gMi, flat, gloc, gsz, gb1 = out[:5]
     assert gMi.shape == (N, nM, 3)
     assert flat.shape == (rf.numel() + N * 3 * nT + _ops.GRAD_TAIL,)
     assert gloc.shape == ((N, nM, 3) if want[0] else (0,))

@@ -151,6 +151,30 @@ int mrphy_blochsim_fused_fwd(const mrphy_fused_args* a, void* cuda_stream);
  * No option needs workspace beyond mrphy_fused_partial_elems().                                                      */
 int mrphy_blochsim_fused_bwd(const mrphy_fused_args* a, int wave_is_packed, void* cuda_stream);
 
+/* Readout: the receive signal of the magnetisation every `a->every` steps, summed over the spins inside the forward kernel,
+ *   S[n][xy][r][k] (Sx + i Sy) = sum_i (cx + i cy)[n][i][k] * (Mx + i My)[n][i] after (r+1)*every steps,  r < nR = nT / every
+ * (lab frame, the state record would return; no conjugation, no scale).  rx == NULL: c = 1.  a->every / a->nR give the stride
+ * as for record; the readout excludes record (a->Mt, a->gMt) and the design tail.  S is bitwise reproducible: each CTA of the
+ * forward sums its tiles into its own slot of `work`, and a finalize kernel sums the slots in a fixed order.             */
+typedef struct mrphy_readout_args {
+  int32_t nRx;                            /* receive coils, 1..16                                                  */
+  int32_t _pad;
+  const void* rx; int64_t rx_sn, rx_sm;   /* (N,nM,2,nRx) receive map, inner (2,nRx) contiguous, or NULL (c = 1)    */
+  void* S;                                /* fwd: out (N,2,nR,nRx) contiguous                                      */
+  const void* gS;                         /* bwd: in, dL/dS like S                                                 */
+  void* grx;                              /* bwd: out dL/drx (N,nM,2,nRx) contiguous, or NULL:
+                                             dL/dcx = sum_r (gSx Mx + gSy My),  dL/dcy = sum_r (gSy Mx - gSx My)         */
+  void* work;                             /* fwd: scratch, mrphy_fused_readout_elems() elements of T                */
+} mrphy_readout_args;
+size_t mrphy_fused_readout_elems(const mrphy_fused_args* a, const mrphy_readout_args* r);
+/* The fused pair with a readout; r == NULL is exactly mrphy_blochsim_fused_fwd / _bwd.  Forward launches: pack_waveform,
+ * blochsim_fused_fwd, readout_finalize.  The backward takes dL/dS (r->gS) on top of dL/dMo (a->gMo, zeros when the loss
+ * ignores M) and combines with per-spin gradients.  MRPHY_ERR_ARG before any launch for: a->Mt / a->gMt set, a->design set,
+ * nRx outside 1..16, a null S / work (fwd) or gS (bwd), every / nR inconsistent.                                          */
+int mrphy_blochsim_fused_readout_fwd(const mrphy_fused_args* a, const mrphy_readout_args* r, void* cuda_stream);
+int mrphy_blochsim_fused_readout_bwd(const mrphy_fused_args* a, const mrphy_readout_args* r, int wave_is_packed,
+                                     void* cuda_stream);
+
 /* Arguments of the explicit-field path: the API-faithful replacement of sims.BlochSim
  * (sims.py:24-269) for callers that hand in a dense Beff (N,nM,nT,3), e.g. tests/test_sims.py:88
  * upstream.  Backward returns dL/dMi and the dense dL/dBeff like the reference.                  */
@@ -305,8 +329,8 @@ int mrphy_mask_copy(const mrphy_mask_args* a, void* cuda_stream);
 
 /* sizeof() of the argument structs as this library was compiled, for bindings to check their mirror of the layout:
  * which = 0 mrphy_param, 1 mrphy_fused_args, 2 mrphy_beff_args, 3 mrphy_rfgr2beff_args, 4 mrphy_beff2ab_args,
- * 5 mrphy_beff2uphi_args, 6 mrphy_freeprec_args, 7 mrphy_reparam_args, 8 mrphy_mask_args, 9 mrphy_clamp_args;
- * 0 for any other value. */
+ * 5 mrphy_beff2uphi_args, 6 mrphy_freeprec_args, 7 mrphy_reparam_args, 8 mrphy_mask_args, 9 mrphy_clamp_args,
+ * 10 mrphy_readout_args; 0 for any other value. */
 size_t mrphy_sizeof_args(int which);
 
 /* Number of kernel launches the last forward / backward call on this thread issued. */

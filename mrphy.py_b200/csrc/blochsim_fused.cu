@@ -7,18 +7,23 @@
 //   pack_waveform_kernel      rf (N,2,nT[,nC]), gr (N,3,nT) -> wave[N][chunk][W][TCP]  (W = 2*NC+3)
 //   fused_fwd_kernel<T,..>    one spin, or two spins packed in an f2 (FFMA2), per thread; checkpoint every K steps
 //                             REC: also the state every `every` steps (Mt, rec_store)
+//                             RD (POL & POL_RD): instead the receive signal of those states summed over the CTA's spins
+//                             (ro_accum, ro_flush) into a per-CTA slot
 //   fused_bwd_kernel<T,..>    time-reversed state reconstruction + adjoint + spin reduction (only the gradient rows
 //                             asked for: ROWS); tiles owned through SM-aware virtual CTA ids (SCHED_*)
 //                             SG: also the per-spin sums over time behind dL/dloc, dL/ddf, dL/db1Map (sg_fold)
 //                             REC: dL/dMt joins the adjoint at the recorded steps (rec_load)
+//                             RD: the adjoint of the signal joins there instead (ro_adjoint), and dL/drx per spin
 //   fused_fwd_tc_kernel<..>   fp32, >= 4 coils: the transmit field on the tensor cores (below); REC as fused_fwd_kernel
 //   grad_finalize_kernel<T>   deterministic sum of the per-CTA partials, reference layout out (grad_finalize.cuh)
+//   readout_finalize_kernel<T> RD: deterministic sum of the per-CTA signal slots -> S
 //
 // Data layout in HBM (T = float | double):
 //   wave      [N][nChunks][W][TCP]   one chunk = K steps (TCP = K rounded up to 4): a chunk is
 //                                    ONE contiguous 16-byte-aligned block -> one 1-D TMA bulk copy
 //   ckpt      [N][nChunks-1][3][nM]  state after (c+1)*K steps, SoA so warps store 128-B lines
 //   Mt, gMt   [N][nR][3][nM]         REC: state after (r+1)*every steps (lab frame) and its gradient, SoA likewise
+//   S, gS     [N][2][nR][nRx]        RD: the signal and its gradient; slots of the forward [N][P][nR][2 nRx]
 //   partials  [N][P][W][nT]          gradient partial sums, one slot per (virtual) CTA id, P ids per batch entry;
 //                                    behind them 264 + P ints of scheduling state of the backward (SCHED_*)
 #include <cuda_runtime.h>
@@ -170,13 +175,42 @@ template <typename T> struct SgOut {
   T* gloc; T* gsz; T* gb1;
   bool any() const { return gloc || gsz || gb1; }
 };
+// readout of the RD kernels (mrphy_readout_args): the signal S[n][xy][r][k] = sum_i (cx + i cy)[n][i][k] (Mx + i My)[n][i] of
+// the state after (r+1)*every steps (lab frame).  The forward sums its tiles into its own slot of `part` [N][P][nR][2 nRx]
+// (P = gridDim.x; x values, then y values; readout_finalize_kernel sums the slots in a fixed order); the backward adds the
+// adjoint of S to the adjoint state at the recorded steps (ro_adjoint) and, with grx, forms dL/drx per spin.
+template <typename T> struct RoOut {
+  const T* rx; int64_t rx_sn, rx_sm;   // (N,nM,2,nRx), inner (2,nRx) contiguous, or null: c = 1
+  int nRx, every, nR;
+  int rt;                              // fwd: records per flush, RO_COLS / (2 nRx)
+  T* part;                             // fwd: per-CTA partial sums
+  const T* gS;                         // bwd: dL/dS (N,2,nR,nRx) contiguous
+  T* grx;                              // bwd: dL/drx (N,nM,2,nRx) contiguous, or null
+};
 // recorded magnetisation of the REC kernels (every, nR, Mt, gMt of mrphy_fused_args): the forward writes Mt, the backward reads dL/dMt, both
 // [N][nR][3][nM] (SoA like the checkpoints), entry r = the state after (r+1)*every steps in the lab frame.  A kernel
-// parameter of its own behind the others, like SgOut.
+// parameter of its own behind the others, like SgOut.  The readout of the RD kernels rides behind it (`ro`): appended to
+// the last kernel parameter, it moves no parameter of the kernels without readout.
 template <typename T> struct RecOut {
   T* Mt; const T* gMt;
   int every, nR;
+  RoOut<T> ro;
 };
+// The readout kernels are the instantiations of fused_fwd_kernel, fused_fwd_tc_kernel and fused_bwd_kernel whose policy
+// parameter carries POL_RD (the policy itself is POL & ~POL_RD).  A flag on an existing parameter rather than a parameter of
+// its own keeps the names and the code of every kernel without readout as they are.
+constexpr int POL_RD = 16;
+// Dynamic shared memory of the readout, behind what the kernel already uses (runtime-sized by nRx; V = Pack<T, PK>::type):
+//   forward   w V[2 nRx][BLKT]  |  tiles T[NW][32 columns][32 lanes]  |  ctab T[2][NW][32]
+//   backward  w V[2 nRx][BLKT]  |  acc V[2 nRx][BLKT] (dL/drx sums)   |  gs T[records per chunk][2 nRx] (dL/dS of the chunk)
+// A column of a forward tile is one (record, x|y, coil) value of the 32 lanes of the warp: 32 / (2 nRx) records per flush.
+constexpr int RO_COLS = 32;
+inline size_t ro_fwd_smem(int nRx, int BLKT, int vsz, int tsz) {
+  return (size_t)2 * nRx * BLKT * vsz + (size_t)(BLKT / 32) * RO_COLS * 32 * tsz + (size_t)2 * (BLKT / 32) * 32 * tsz;
+}
+inline size_t ro_bwd_smem(int nRx, int BLKT, int vsz, int tsz, int nrc) {
+  return (size_t)4 * nRx * BLKT * vsz + (size_t)nrc * 2 * nRx * tsz;
+}
 
 // Scheduling workspace of the backward kernel (ints, zeroed before every launch; lives behind the partial sums).
 // The hardware spreads the P = c * n_sm co-resident CTAs breadth-first over the SMs, but not in blockIdx order (measured,
@@ -313,6 +347,107 @@ __device__ __forceinline__ void rec_load(const RecOut<T>& o, int nM, int n, int 
   to_frame(k, x, y);
 }
 
+// RD: the receive weights of this thread's PK spins, w[c] + i w[nRx + c] = c_k e^{i arg b1} (the state is kept in the spin's own
+// frame, single coil: folding the turn into the weight once per spin spares turning the state at every record; elsewhere
+// fc = 1, fs = 0).  Zero in padding lanes.  Each thread reads back only its own entries: no barrier.
+template <typename T, typename V, int NC, int PK, int BLKT>
+__device__ __forceinline__ void ro_weights(const RoOut<T>& ro, int n, const int (&idx)[PK], const bool (&ok)[PK],
+                                           const SpinConst<V, NC>& k, V* w) {
+  const int nRx = ro.nRx;
+  for (int c = 0; c < nRx; ++c) {
+    T wr[PK], wi[PK];
+#pragma unroll
+    for (int q = 0; q < PK; ++q) {
+      T cr = ok[q] ? (T)1 : (T)0, ci = (T)0;
+      if (ro.rx && ok[q]) {
+        const T* p = ro.rx + (int64_t)n * ro.rx_sn + (int64_t)idx[q] * ro.rx_sm;
+        cr = p[c];
+        ci = p[nRx + c];
+      }
+      const T fc = q == 0 ? getq<0>(k.fc) : getq<1>(k.fc), fs = q == 0 ? getq<0>(k.fs) : getq<1>(k.fs);
+      wr[q] = fnma_(fs, ci, fc * cr);
+      wi[q] = fma_(fs, cr, fc * ci);
+    }
+    w[c * BLKT + threadIdx.x] = mkv(wr[0], wr[PK - 1], (V*)nullptr);
+    w[(nRx + c) * BLKT + threadIdx.x] = mkv(wi[0], wi[PK - 1], (V*)nullptr);
+  }
+}
+// RD forward, at a recorded state: this thread's weighted (Sx, Sy) per receive coil (its PK spins added first) into the columns
+// slot * 2 nRx + (c | nRx + c) of its warp's tile
+template <typename T, typename V, int BLKT>
+__device__ __forceinline__ void ro_accum(const RoOut<T>& ro, const V* w, T* tile, int slot, V mx, V my) {
+  const int nRx = ro.nRx, lane = threadIdx.x & 31;
+  T* col = tile + (size_t)slot * 2 * nRx * 32 + lane;
+  for (int c = 0; c < nRx; ++c) {
+    const V wr = w[c * BLKT + threadIdx.x], wi = w[(nRx + c) * BLKT + threadIdx.x];
+    col[c * 32] = hsum(fnma_(wi, my, wr * mx));
+    col[(nRx + c) * 32] = hsum(fma_(wi, mx, wr * my));
+  }
+}
+// RD forward: the CTA sums the nb buffered records r0 .. r0 + nb - 1 of its tiles into its slot, in the manner of
+// warp_tile_reduce: lane l of each warp adds up column l (rotated start: conflict-free), the warps meet in a fixed order
+// through the double-buffered ctab, and thread j owns value j of the slot -- stores on the CTA's first tile, adds on later
+// ones.  One writer per value, no atomics: bitwise reproducible.  Every thread of the CTA must call it (one barrier).
+// nb = the buffered records (bits 0-15) | the parity of ctab (bit 16); it leaves with no records and the other parity.
+template <typename T, int BLKT>
+__device__ __forceinline__ void ro_flush(const RoOut<T>& ro, const T* tiles, T* ctab, int n, int rr, int& nb, bool first) {
+  constexpr int NW = BLKT / 32;
+  const int cnt = nb & 0xffff, par = nb >> 16, r0 = rr - cnt;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, ncol = cnt * 2 * ro.nRx;
+  __syncwarp();
+  const T* t = tiles + (size_t)warp * RO_COLS * 32 + (size_t)lane * 32;
+  T sum = (T)0;
+  if (lane < ncol) {
+#pragma unroll 8
+    for (int q = 0; q < 32; ++q) sum += t[(q + lane) & 31];
+  }
+  T* cb = ctab + (size_t)par * NW * 32;
+  cb[warp * 32 + lane] = sum;
+  __syncthreads();
+  if (tid < ncol) {
+    T s = cb[tid];
+#pragma unroll
+    for (int q = 1; q < NW; ++q) s += cb[q * 32 + tid];
+    T* dst = ro.part + (((size_t)n * gridDim.x + blockIdx.x) * ro.nR + r0) * 2 * ro.nRx + tid;
+    *dst = first ? s : *dst + s;
+  }
+  nb = (par ^ 1) << 16;
+}
+// RD backward, at the step that produced record r: h += the adjoint of S[r] (gs = dL/dS[n, :, r, :], staged), and with grx the
+// per-spin sums acc += conj(m) dL/dS[r] (in the spin frame; ro_grx_store turns them to the lab frame)
+template <typename T, typename V, int BLKT>
+__device__ __forceinline__ void ro_adjoint(const RoOut<T>& ro, const V* w, V* acc, const T* gs, V mx, V my, V& hx, V& hy) {
+  const int nRx = ro.nRx, tid = threadIdx.x;
+  for (int c = 0; c < nRx; ++c) {
+    const V gx = V(gs[c]), gy = V(gs[nRx + c]);
+    const V wr = w[c * BLKT + tid], wi = w[(nRx + c) * BLKT + tid];
+    hx = fma_(wr, gx, fma_(wi, gy, hx));
+    hy = fma_(wr, gy, fnma_(wi, gx, hy));
+    if (ro.grx) {
+      acc[c * BLKT + tid] = fma_(mx, gx, fma_(my, gy, acc[c * BLKT + tid]));
+      acc[(nRx + c) * BLKT + tid] = fma_(mx, gy, fnma_(my, gx, acc[(nRx + c) * BLKT + tid]));
+    }
+  }
+}
+// RD backward, end of a tile: dL/drx = e^{-i arg b1} acc of the thread's spins (dL/dc = sum_r conj(m_lab) dL/dS[r])
+template <typename T, typename V, int NC, int PK, int BLKT>
+__device__ __forceinline__ void ro_grx_store(const RoOut<T>& ro, int n, int nM, const int (&idx)[PK], const bool (&ok)[PK],
+                                             const SpinConst<V, NC>& k, const V* acc) {
+  const int nRx = ro.nRx;
+#pragma unroll
+  for (int q = 0; q < PK; ++q) {
+    if (!ok[q]) continue;
+    const T fc = q == 0 ? getq<0>(k.fc) : getq<1>(k.fc), fs = q == 0 ? getq<0>(k.fs) : getq<1>(k.fs);
+    T* o = ro.grx + ((size_t)n * nM + idx[q]) * 2 * nRx;
+    for (int c = 0; c < nRx; ++c) {
+      const V ax = acc[c * BLKT + threadIdx.x], ay = acc[(nRx + c) * BLKT + threadIdx.x];
+      const T x = q == 0 ? getq<0>(ax) : getq<1>(ax), y = q == 0 ? getq<0>(ay) : getq<1>(ay);
+      o[c] = fma_(fs, y, fc * x);
+      o[nRx + c] = fnma_(fs, x, fc * y);
+    }
+  }
+}
+
 // ------------------------------------------------------------------------------------------
 // pack: one thread per element of wave[N][nChunks][W][TCP]
 template <typename T>
@@ -349,14 +484,22 @@ __global__ void pack_waveform_kernel(const T* __restrict__ rf, int64_t rf_sn, in
 // ------------------------------------------------------------------------------------------
 // forward.  PK spins per thread (PK == 2: packed f2 arithmetic), BLKT threads per CTA.
 // REC: also the state after every `rec.every` steps (rec_store), tracked by a countdown (no per-step division).
+// RD (POL & POL_RD): instead the signal of the state after every `ro.every` steps, on the same countdown (ro_accum / ro_flush).
 template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, bool REC = false>
 __global__ void __launch_bounds__(BLKT, (PK == 2 ? (NC == 1 ? 14 : MRPHY_NC2_MINB) : 1)) fused_fwd_kernel(const KArgs<T> a, const RecOut<T> rec) {
+  constexpr bool RD = (POL & POL_RD) != 0;
+  const RoOut<T>& ro = rec.ro;
   typedef typename Pack<T, PK>::type V;
   constexpr int W = 2 * NC + 3;
   constexpr int WS = WaveLayout<T, W>::WS;
   __shared__ __align__(128) T wbuf[2][WS * ChunkMax<T, NC>::v];
   __shared__ __align__(16) T scr[3 * BLKT * PK];
   __shared__ __align__(8) uint64_t full[2];
+  extern __shared__ __align__(16) unsigned char ro_smem[];   // RD (see RoOut); addresses formed where used: no live registers
+#define RO_W reinterpret_cast<V*>(ro_smem)
+#define RO_TILES reinterpret_cast<T*>(ro_smem + (size_t)2 * ro.nRx * BLKT * sizeof(V))
+#define RO_CTAB (RO_TILES + (BLKT / 32) * RO_COLS * 32)
+  int nb = 0;   // RD: records buffered since the last flush | ctab parity (ro_flush)
   const int tid = threadIdx.x, n = blockIdx.y;
   const int TCP = a.TCP, K = a.K, nT = a.nT, nChunks = a.nChunks, nM = a.nM;
   const uint32_t chunk_bytes = (uint32_t)(WS * TCP * sizeof(T));
@@ -393,7 +536,8 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? (NC == 1 ? 14 : MRPHY_NC2_MIN
     }
     load_vec3_tile<T, V, PK, BLKT>(a.Mi + (int64_t)n * a.Mi_sn, a.Mi_sm, tile, nM, idx, scr, mx, my, mz);
     to_frame(k, mx, my);   // single coil: the spin's own transverse frame (bloch_math.cuh: make_consts); checkpoints stay in it
-    int rc = rec.every, rr = 0;   // REC: steps to the next recorded state, its index
+    int rc = RD ? ro.every : rec.every, rr = 0;   // REC, RD: steps to the next recorded state, its index
+    if constexpr (RD) ro_weights<T, V, NC, PK, BLKT>(ro, n, idx, ok, k, RO_W);
     for (int c = 0; c < nChunks; ++c, ++it) {
       if (tid == 0 && it + 1 < total) {   // prefetch the next chunk (possibly chunk 0 of the next tile)
         const int cn = (c + 1 == nChunks) ? 0 : c + 1;
@@ -409,13 +553,21 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? (NC == 1 ? 14 : MRPHY_NC2_MIN
 #pragma unroll
         for (int q = 0; q < NC; ++q) { rx[q] = V(s[q]); ry[q] = V(s[NC + q]); }
         field<V, NC>(k, rx, ry, V(s[2 * NC]), V(s[2 * NC + 1]), V(s[2 * NC + 2]), bx, by, bz);
-        step_fwd<V, POL, RELAX>(bx, by, bz, k.e1, k.e2, mx, my, mz);
+        step_fwd<V, POL & ~POL_RD, RELAX>(bx, by, bz, k.e1, k.e2, mx, my, mz);
         if constexpr (REC) {
           if (--rc == 0) {   // recorded states leave the spin frame (a copy: the state stays in it)
             V x = mx, y = my;
             from_frame(k, x, y);
             rec_store<T, V, PK>(rec, nM, n, rr++, idx, ok, x, y, mz);
             rc = rec.every;
+          }
+        }
+        if constexpr (RD) {
+          if (--rc == 0) {   // (CTA-uniform: every thread steps the same count)
+            ro_accum<T, V, BLKT>(ro, RO_W, RO_TILES + (size_t)(tid >> 5) * RO_COLS * 32, nb & 0xffff, mx, my);
+            ++rr;
+            if ((++nb & 0xffff) == ro.rt || rr == ro.nR) ro_flush<T, BLKT>(ro, RO_TILES, RO_CTAB, n, rr, nb, tile == (int)blockIdx.x);
+            rc = ro.every;
           }
         }
       };
@@ -457,6 +609,9 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? (NC == 1 ? 14 : MRPHY_NC2_MIN
       __syncthreads();   // everyone is done with wbuf[it&1] before it is refilled
     }
     from_frame(k, mx, my);
+#undef RO_W
+#undef RO_TILES
+#undef RO_CTAB
     if (ok[0]) {
       T* op = a.Mo + ((size_t)n * nM + idx[0]) * 3;
       op[0] = getq<0>(mx); op[1] = getq<0>(my); op[2] = getq<0>(mz);
@@ -465,6 +620,25 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? (NC == 1 ? 14 : MRPHY_NC2_MIN
       T* op = a.Mo + ((size_t)n * nM + idx[PK - 1]) * 3;
       op[0] = getq<1>(mx); op[1] = getq<1>(my); op[2] = getq<1>(mz);
     }
+  }
+}
+
+// S[n][xy][r][k] = sum over the P slots of part[n][p][r][xy * nRx + k] in slot order (bitwise reproducible).  Block (32, 8):
+// 32 consecutive values of a batch entry's slot, the 8 rows take every 8th slot, then meet in a fixed order.
+template <typename T>
+__global__ void readout_finalize_kernel(const T* __restrict__ part, int P, int nR, int nRx, T* __restrict__ S) {
+  __shared__ T red[8][32];
+  const int n = blockIdx.y, cols = nR * 2 * nRx, col = blockIdx.x * 32 + threadIdx.x;
+  T s = (T)0;
+  if (col < cols)
+    for (int p = threadIdx.y; p < P; p += 8) s += part[((size_t)n * P + p) * cols + col];
+  red[threadIdx.y][threadIdx.x] = s;
+  __syncthreads();
+  if (threadIdx.y == 0 && col < cols) {
+#pragma unroll
+    for (int q = 1; q < 8; ++q) s += red[q][threadIdx.x];
+    const int r = col / (2 * nRx), j = col % (2 * nRx), xy = j / nRx, kk = j % nRx;
+    S[(((size_t)n * 2 + xy) * nR + r) * nRx + kk] = s;
   }
 }
 
@@ -613,8 +787,12 @@ __device__ __forceinline__ void sg_fold(const KArgs<T>& a, const SgOut<T>& o, in
 // SG: also the per-spin gradients (sg_fold).  ROWS == 0 (SG only, a fixed pulse): no transposition tile, no partial sums.
 // REC: the loss also depends on the recorded states: dL/dMt[r] joins the adjoint before the adjoint of the step that
 // produced state r, so that everything downstream (F, the spin reduction, sg_fold, dL/dMi) sees the total dL/dm.
+// RD (POL & POL_RD): the adjoint of the readout joins instead, at the same steps (ro_adjoint), and with ro.grx the kernel
+// also forms dL/drx.
 template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, int ROWS = 3, bool SG = false, bool REC = false>
 __global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : (sizeof(T) == 8 && NC == 1 ? 4 : (sizeof(T) == 4 && NC > 1 ? MRPHY_MC_MINB : 1)))) fused_bwd_kernel(const KArgs<T> a, const int need_gmi, const SgOut<T> sgo, const RecOut<T> rec) {
+  constexpr bool RD = (POL & POL_RD) != 0;
+  const RoOut<T>& ro = rec.ro;
   typedef typename Pack<T, PK>::type V;
   using L = BwdSmem<T, NC, BLKT, PK>;
   constexpr int W = L::W, TR = L::TR, NW = L::NW;
@@ -629,6 +807,10 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : 
   T* const wt = reinterpret_cast<T*>(smem_raw + L::red + (size_t)NW * 32 * L::P16 * 16) + (size_t)(threadIdx.x >> 5) * 32 * L::WP;
   T(*cta)[W][TR] = reinterpret_cast<T(*)[W][TR]>(smem_raw + L::cta);          // per-warp tile sums
   uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + L::bar);
+  // RD (see RoOut): the weights, the dL/drx sums and the staged dL/dS behind the kernel's own shared memory
+#define RO_W reinterpret_cast<V*>(smem_raw + L::bytes)
+#define RO_ACC (RO_W + (size_t)2 * ro.nRx * BLKT)
+#define RO_GS reinterpret_cast<T*>(RO_ACC + (size_t)2 * ro.nRx * BLKT)
   __shared__ __align__(16) T scr[3 * BLKT * PK];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, n = blockIdx.y;
   const int TCP = a.TCP, K = a.K, nT = a.nT, nChunks = a.nChunks, nM = a.nM;
@@ -721,7 +903,25 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : 
       rr = rec.nR - 1;
       rec_load<T, V, NC, PK>(rec, nM, n, rr, idx, ok, k, gx, gy, gz);
     }
+    if constexpr (RD) {
+      rc = nT - ro.nR * ro.every;
+      rr = ro.nR - 1;
+      ro_weights<T, V, NC, PK, BLKT>(ro, n, idx, ok, k, RO_W);
+      if (ro.grx)
+        for (int c = 0; c < 2 * ro.nRx; ++c) RO_ACC[c * BLKT + tid] = V(0.0f);
+    }
     for (int c = nChunks - 1; c >= 0; --c, ++it) {
+      [[maybe_unused]] int ro_lo;   // RD: the first record this chunk produced; dL/dS of its records staged in RO_GS
+      if constexpr (RD) {
+        const int t0 = c * K, t1 = t0 + min(K, nT - c * K);   // records r with (r+1) * every - 1 in [t0, t1)
+        ro_lo = (t0 + ro.every) / ro.every - 1;
+        const int hi = min(ro.nR, t1 / ro.every), cols = 2 * ro.nRx;
+        for (int e = tid; e < (hi - ro_lo) * cols; e += BLKT) {
+          const int j = e / cols, v = e % cols;
+          RO_GS[e] = ro.gS[(((size_t)n * 2 + v / ro.nRx) * ro.nR + ro_lo + j) * ro.nRx + v % ro.nRx];
+        }
+        __syncthreads();   // (the previous chunk's last reads of RO_GS precede its last barrier)
+      }
       if (tid == 0 && it + 1 < total) {
         const int cn = (c == 0) ? nChunks - 1 : c - 1;
         const uint32_t sn = (it + 1) & 1;
@@ -754,11 +954,19 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : 
           }
           --rc;
         }
+        if constexpr (RD) {
+          if (rc == 0) {   // this step produced record rr: h += the adjoint of S[rr]
+            ro_adjoint<T, V, BLKT>(ro, RO_W, RO_ACC, RO_GS + (size_t)(rr - ro_lo) * 2 * ro.nRx, mx, my, hx, hy);
+            --rr;
+            rc = ro.every;
+          }
+          --rc;
+        }
         V rx[NC], ry[NC], bx, by, bz, Fx, Fy, Fz;
 #pragma unroll
         for (int q = 0; q < NC; ++q) { rx[q] = V(s[q]); ry[q] = V(s[NC + q]); }
         field<V, NC>(k, rx, ry, V(s[2 * NC]), V(s[2 * NC + 1]), V(s[2 * NC + 2]), bx, by, bz);
-        step_bwd<V, POL, RELAX, NC>(k, bx, by, bz, mx, my, mz, hx, hy, hz, Fx, Fy, Fz);
+        step_bwd<V, POL & ~POL_RD, RELAX, NC>(k, bx, by, bz, mx, my, mz, hx, hy, hz, Fx, Fy, Fz);
         if constexpr (SG) {
           sacc[0] = fma_(V(s[2 * NC]), Fz, sacc[0]);
           sacc[1] = fma_(V(s[2 * NC + 1]), Fz, sacc[1]);
@@ -857,6 +1065,9 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : 
         op[0] = getq<1>(hx); op[1] = getq<1>(hy); op[2] = getq<1>(hz);
       }
     }
+    if constexpr (RD) {
+      if (ro.grx) ro_grx_store<T, V, NC, PK, BLKT>(ro, n, nM, idx, ok, k, RO_ACC);
+    }
   }
    }   // vid >= 0
    if (!a.sched) break;
@@ -882,6 +1093,9 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : 
    if (vid < 0) break;
   }
 #undef NCTA
+#undef RO_W
+#undef RO_ACC
+#undef RO_GS
 #ifdef MRPHY_CTA_TRACE
   if (tid == 0 && blockIdx.x < 8192 && n == 0) g_cta_trace[blockIdx.x][2] = gtime();
 #endif
@@ -1050,9 +1264,12 @@ __device__ __forceinline__ void tc_issue(const float* sa, const float* wb, int r
     tc_issue<NC, PK>(sa, wbuf[(it + 1) % NST], rows, tmem + ((it + 1) % NBUF) * C::BUF_COLS, &mma_bar[(it + 1) % NBUF]);    \
   }
 
-// REC as in fused_fwd_kernel (this kernel has no spin frame: the state is in the lab frame throughout)
+// REC, RD as in fused_fwd_kernel (this kernel has no spin frame: the state is in the lab frame throughout); the readout's
+// shared memory follows C::bytes.
 template <int POL, bool RELAX, int NC, int PK, bool REC = false>
 __global__ void __launch_bounds__(128, (NC <= 8 ? 4 : (PK == 1 ? 3 : 2))) fused_fwd_tc_kernel(const KArgs<float> a, const RecOut<float> rec) {
+  constexpr bool RD = (POL & POL_RD) != 0;
+  const RoOut<float>& ro = rec.ro;
   using L = TcLayout<NC>;
   using C = TcCfg<NC, PK>;
   typedef float T;
@@ -1065,6 +1282,11 @@ __global__ void __launch_bounds__(128, (NC <= 8 ? 4 : (PK == 1 ? 3 : 2))) fused_
   uint64_t* const full = reinterpret_cast<uint64_t*>(smem_raw + C::bars);
   uint64_t* const mma_bar = full + NST;
   uint32_t* const tmem_slot = reinterpret_cast<uint32_t*>(full + NST + 2);
+  // RD (see RoOut), behind C::bytes; addresses formed where used
+#define RO_W reinterpret_cast<V*>(smem_raw + C::bytes)
+#define RO_TILES reinterpret_cast<float*>(smem_raw + C::bytes + (size_t)2 * ro.nRx * BLKT * sizeof(V))
+#define RO_CTAB (RO_TILES + (BLKT / 32) * RO_COLS * 32)
+  int nb = 0;   // RD: records buffered since the last flush | ctab parity (ro_flush)
   const int tid = threadIdx.x, warp = tid >> 5, n = blockIdx.y;
   const int TCP = a.TCP, K = a.K, nT = a.nT, nChunks = a.nChunks, nM = a.nM, rows = 2 * TCP;
   const uint32_t chunk_bytes = (uint32_t)(a.chunk_elems * sizeof(float));
@@ -1119,7 +1341,8 @@ __global__ void __launch_bounds__(128, (NC <= 8 ? 4 : (PK == 1 ? 3 : 2))) fused_
     tc::fence_before_sync();
     __syncthreads();
     const V glx = k.glx, gly = k.gly, glz = k.glz, gbz0 = k.gbz0, e1 = k.e1, e2 = k.e2;
-    int rc = rec.every, rr = 0;   // REC: steps to the next recorded state, its index
+    int rc = RD ? ro.every : rec.every, rr = 0;   // REC, RD: steps to the next recorded state, its index
+    if constexpr (RD) ro_weights<T, V, 1, PK, BLKT>(ro, n, idx, ok, k, RO_W);
     for (int c = 0; c < nChunks; ++c, ++it) {
       TC_CHUNK_BEGIN(FWD_CHUNK_OF, c == 0, c + 1 < nChunks)
       const float* gw = wbuf[it % NST] + (size_t)2 * L::KC * rows * 4;   // gr rows [3][TCP]
@@ -1138,11 +1361,19 @@ __global__ void __launch_bounds__(128, (NC <= 8 ? 4 : (PK == 1 ? 3 : 2))) fused_
           if (j0 + u < ns) {
             const V bz = fma_(glx, V(g[0][u]), fma_(gly, V(g[1][u]), fma_(glz, V(g[2][u]), gbz0)));
             const V bx = mkv(b[0][2 * u], b[PK - 1][2 * u], (V*)nullptr), by = mkv(b[0][2 * u + 1], b[PK - 1][2 * u + 1], (V*)nullptr);
-            step_fwd<V, POL, RELAX>(bx, by, bz, e1, e2, mx, my, mz);
+            step_fwd<V, POL & ~POL_RD, RELAX>(bx, by, bz, e1, e2, mx, my, mz);
             if constexpr (REC) {
               if (--rc == 0) {
                 rec_store<T, V, PK>(rec, nM, n, rr++, idx, ok, mx, my, mz);
                 rc = rec.every;
+              }
+            }
+            if constexpr (RD) {
+              if (--rc == 0) {
+                ro_accum<T, V, BLKT>(ro, RO_W, RO_TILES + (size_t)warp * RO_COLS * 32, nb & 0xffff, mx, my);
+                ++rr;
+                if ((++nb & 0xffff) == ro.rt || rr == ro.nR) ro_flush<T, BLKT>(ro, RO_TILES, RO_CTAB, n, rr, nb, tile == (int)blockIdx.x);
+                rc = ro.every;
               }
             }
           }
@@ -1200,6 +1431,9 @@ __global__ void __launch_bounds__(128, (NC <= 8 ? 4 : (PK == 1 ? 3 : 2))) fused_
     }
   }
 #undef FWD_CHUNK_OF
+#undef RO_W
+#undef RO_TILES
+#undef RO_CTAB
   __syncthreads();
   if (warp == 0) tc::tmem_free<C::TMEM_COLS>(tmem);
 }
@@ -1407,6 +1641,13 @@ extern "C" size_t mrphy_fused_partial_elems(const mrphy_fused_args* a) {
   return (size_t)a->N * p.Pmax * p.W * (size_t)a->nT + (size_t)(SCHED_CLAIM + p.Pmax) + (size_t)a->N;
 }
 
+extern "C" size_t mrphy_fused_readout_elems(const mrphy_fused_args* a, const mrphy_readout_args* r) {
+  Plan p;
+  if (make_plan(a, &p, true) != MRPHY_OK) return 0;
+  if (!r || r->nRx < 1 || r->nRx > 16 || a->nR < 1) return 0;
+  return (size_t)a->N * p.Pmax * (size_t)a->nR * 2 * r->nRx;
+}
+
 namespace {
 
 template <typename T>
@@ -1473,29 +1714,47 @@ int launch_pack(const mrphy_fused_args* a, const Plan& p, cudaStream_t st, bool 
 
 // P (CTAs per batch entry) actually launched by the last backward kernel; the finalize kernel needs it
 thread_local int g_last_P = 0;
+// ... by the last forward kernel: the readout's finalize sums that many slots
+thread_local int g_last_fwd_P = 0;
+// records a staged chunk of K steps can produce (the backward's dL/dS staging)
+inline int ro_chunk_records(int K, int every) { return (K + every - 1) / every; }
 
-template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, bool REC>
+// OPT selects the option of the kernels: 0 none, 1 record (REC), 2 readout (RD, the *_ro_ kernels)
+template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, int OPT>
 int launch_fwd_s(KArgs<T> k, const Plan& p, cudaStream_t st, const RecOut<T>& rec) {
-  auto kern = fused_fwd_kernel<T, POL, RELAX, NC, PK, BLKT, REC>;
+  constexpr bool REC = OPT == 1;
+  const size_t smem = OPT == 2 ? ro_fwd_smem(rec.ro.nRx, BLKT, (int)sizeof(typename Pack<T, PK>::type), (int)sizeof(T)) : 0;
+  auto kern = [] {
+    if constexpr (OPT == 2) return fused_fwd_kernel<T, POL | POL_RD, RELAX, NC, PK, BLKT, false>;
+    else return fused_fwd_kernel<T, POL, RELAX, NC, PK, BLKT, REC>;
+  }();
+  if (smem) CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int occ = 0;
-  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, BLKT, 0));
+  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, BLKT, smem));
   k.P = pick_ctas(p, k.N, occ, false, BLKT / 32);
+  g_last_fwd_P = k.P;
   dim3 grid(k.P, k.N);
-  if (REC && getenv("MRPHY_B200_DEBUG"))
-    fprintf(stderr, "[mrphy_b200] fused_fwd<%s,NC=%d,PK=%d,BLK=%d,%s,REC=1> grid=(%d,%d) tiles=%d occ=%d K=%d every=%d\n",
-            sizeof(T) == 4 ? "f32" : "f64", NC, PK, BLKT, POL == TRIG_PRECISE ? "precise" : "fast", k.P, k.N, p.tiles, occ, p.K,
-            rec.every);
+  if (OPT && getenv("MRPHY_B200_DEBUG"))
+    fprintf(stderr, "[mrphy_b200] fused_fwd<%s,NC=%d,PK=%d,BLK=%d,%s,%s=1> grid=(%d,%d) tiles=%d occ=%d K=%d every=%d\n",
+            sizeof(T) == 4 ? "f32" : "f64", NC, PK, BLKT, POL == TRIG_PRECISE ? "precise" : "fast", REC ? "REC" : "RD", k.P, k.N,
+            p.tiles, occ, p.K, REC ? rec.every : rec.ro.every);
   timing_begin(st);
-  kern<<<grid, BLKT, 0, st>>>(k, rec);
+  kern<<<grid, BLKT, smem, st>>>(k, rec);
   timing_end(st);
   ++g_launches;
   CK(cudaGetLastError());
   return MRPHY_OK;
 }
-template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, int ROWS, bool SG, bool REC>
+template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, int ROWS, bool SG, int OPT>
 int launch_bwd_s(KArgs<T> k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg, const RecOut<T>& rec) {
-  constexpr size_t smem = BwdSmem<T, NC, BLKT, PK>::bytes;
-  auto kern = fused_bwd_kernel<T, POL, RELAX, NC, PK, BLKT, ROWS, SG, REC>;
+  constexpr bool REC = OPT == 1;
+  const size_t smem = BwdSmem<T, NC, BLKT, PK>::bytes +
+                      (OPT == 2 ? ro_bwd_smem(rec.ro.nRx, BLKT, (int)sizeof(typename Pack<T, PK>::type), (int)sizeof(T),
+                                              ro_chunk_records(p.K, rec.ro.every)) : 0);
+  auto kern = [] {
+    if constexpr (OPT == 2) return fused_bwd_kernel<T, POL | POL_RD, RELAX, NC, PK, BLKT, ROWS, SG, false>;
+    else return fused_bwd_kernel<T, POL, RELAX, NC, PK, BLKT, ROWS, SG, REC>;
+  }();
   CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   // static + dynamic may exceed 48 KB
   int occ = 0;
   CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, BLKT, smem));
@@ -1518,7 +1777,7 @@ int launch_bwd_s(KArgs<T> k, const Plan& p, int need_gmi, cudaStream_t st, const
   if (getenv("MRPHY_B200_DEBUG"))
     fprintf(stderr, "[mrphy_b200] fused_bwd<%s,NC=%d,PK=%d,BLK=%d,%s,ROWS=%d,SG=%d%s> grid=(%d,%d) tiles=%d occ=%d smem=%zu K=%d\n",
             sizeof(T) == 4 ? "f32" : "f64", NC, PK, BLKT, POL == TRIG_PRECISE ? "precise" : "fast", ROWS, (int)SG,
-            REC ? ",REC=1" : "", k.P, k.N, q.tiles, occ, smem, p.K);
+            REC ? ",REC=1" : (OPT == 2 ? ",RD=1" : ""), k.P, k.N, q.tiles, occ, smem, p.K);
   timing_begin(st);
   kern<<<grid, BLKT, smem, st>>>(k, need_gmi, sg, rec);
   timing_end(st);
@@ -1549,11 +1808,15 @@ int tc_occupancy(Kern kern, size_t dyn_smem, int tmem_cols) {
 }
 
 // tensor-core multi-coil kernels (fp32): at most 4 CTAs per SM, each owns 128 of the 512 TMEM columns
-template <int POL, bool RELAX, int NC, int PK, bool REC>
+template <int POL, bool RELAX, int NC, int PK, int OPT>
 int launch_fwd_tc_pk(KArgs<float> k, const Plan& p, cudaStream_t st, const RecOut<float>& rec) {
   using C = TcCfg<NC, PK>;
-  constexpr size_t smem = C::bytes;
-  auto kern = fused_fwd_tc_kernel<POL, RELAX, NC, PK, REC>;
+  constexpr bool REC = OPT == 1;
+  const size_t smem = C::bytes + (OPT == 2 ? ro_fwd_smem(rec.ro.nRx, 128, (int)sizeof(typename Pack<float, PK>::type), 4) : 0);
+  auto kern = [] {
+    if constexpr (OPT == 2) return fused_fwd_tc_kernel<POL | POL_RD, RELAX, NC, PK, false>;
+    else return fused_fwd_tc_kernel<POL, RELAX, NC, PK, REC>;
+  }();
   CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   k.TCP = p.tc_TCP;
   k.chunk_elems = p.tc_chunk_elems;
@@ -1562,10 +1825,12 @@ int launch_fwd_tc_pk(KArgs<float> k, const Plan& p, cudaStream_t st, const RecOu
   k.P = (int)((int64_t)sm_count_cached() * occ / k.N);   // every resident slot (pick_ctas trades slots for even passes)
   if (k.P < 1) k.P = 1;
   if (k.P > tiles) k.P = tiles;
+  if (OPT == 2 && k.P > p.Pmax) k.P = p.Pmax;   // one readout slot per CTA: mrphy_fused_readout_elems sized Pmax of them
+  g_last_fwd_P = k.P;
   dim3 grid(k.P, k.N);
   if (getenv("MRPHY_B200_DEBUG"))
     fprintf(stderr, "[mrphy_b200] fused_fwd_tc<NC=%d,PK=%d%s> grid=(%d,%d) tiles=%d occ=%d smem=%zu K=%d\n", NC, PK,
-            REC ? ",REC=1" : "", k.P, k.N, tiles, occ, smem, p.K);
+            REC ? ",REC=1" : (OPT == 2 ? ",RD=1" : ""), k.P, k.N, tiles, occ, smem, p.K);
   timing_begin(st);
   kern<<<grid, 128, smem, st>>>(k, rec);
   timing_end(st);
@@ -1573,37 +1838,37 @@ int launch_fwd_tc_pk(KArgs<float> k, const Plan& p, cudaStream_t st, const RecOu
   CK(cudaGetLastError());
   return MRPHY_OK;
 }
-template <int POL, bool RELAX, int NC, bool REC>
+template <int POL, bool RELAX, int NC, int OPT>
 int launch_fwd_tc(const KArgs<float>& k, const Plan& p, cudaStream_t st, const RecOut<float>& rec) {
   // two spin tiles per CTA (packed f2 step): measured 3 % (4, 8 coils) to 17 % (16 coils) faster than one tile with two TMEM
   // buffers; a build with -DMRPHY_TC_SCALAR also carries the one-tile kernels (MRPHY_B200_TC_PACK=1) for measurements
 #ifdef MRPHY_TC_SCALAR
-  if (env_int("MRPHY_B200_TC_PACK", 2) == 1) return launch_fwd_tc_pk<POL, RELAX, NC, 1, REC>(k, p, st, rec);
+  if (env_int("MRPHY_B200_TC_PACK", 2) == 1) return launch_fwd_tc_pk<POL, RELAX, NC, 1, OPT>(k, p, st, rec);
 #endif
-  return launch_fwd_tc_pk<POL, RELAX, NC, 2, REC>(k, p, st, rec);
+  return launch_fwd_tc_pk<POL, RELAX, NC, 2, OPT>(k, p, st, rec);
 }
 // One launch of the kernels with spins in registers: the forward, or the backward with its ROWS / SG.  With per-spin gradients
 // the backward takes the ROWS == 0 kernel when no waveform gradient is wanted, else all rows (the finalize reads only the
 // wanted ones); without, the spin-packed kernels also come with dL/drf-only and dL/dgr-only rows.
-template <typename T, int POL, bool RELAX, int NC, int PK, bool REC>
+template <typename T, int POL, bool RELAX, int NC, int PK, int OPT>
 int launch(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg, const RecOut<T>& rec) {
-  if (!bwd) return launch_fwd_s<T, POL, RELAX, NC, PK, PK == 2 ? 64 : 128, REC>(k, p, st, rec);
+  if (!bwd) return launch_fwd_s<T, POL, RELAX, NC, PK, PK == 2 ? 64 : 128, OPT>(k, p, st, rec);
   constexpr int B = PK == 2 ? MRPHY_BWD_BLKT : 128;
   if (sg.any())
-    return p.rows == 0 ? launch_bwd_s<T, POL, RELAX, NC, PK, B, 0, true, REC>(k, p, need_gmi, st, sg, rec)
-                       : launch_bwd_s<T, POL, RELAX, NC, PK, B, 3, true, REC>(k, p, need_gmi, st, sg, rec);
+    return p.rows == 0 ? launch_bwd_s<T, POL, RELAX, NC, PK, B, 0, true, OPT>(k, p, need_gmi, st, sg, rec)
+                       : launch_bwd_s<T, POL, RELAX, NC, PK, B, 3, true, OPT>(k, p, need_gmi, st, sg, rec);
   if constexpr (PK == 2) {
-    if (p.rows == 1) return launch_bwd_s<T, POL, RELAX, NC, PK, B, 1, false, REC>(k, p, need_gmi, st, sg, rec);   // dL/drf only
-    if (p.rows == 2) return launch_bwd_s<T, POL, RELAX, NC, PK, B, 2, false, REC>(k, p, need_gmi, st, sg, rec);   // dL/dgr only
+    if (p.rows == 1) return launch_bwd_s<T, POL, RELAX, NC, PK, B, 1, false, OPT>(k, p, need_gmi, st, sg, rec);   // dL/drf only
+    if (p.rows == 2) return launch_bwd_s<T, POL, RELAX, NC, PK, B, 2, false, OPT>(k, p, need_gmi, st, sg, rec);   // dL/dgr only
   }
-  return launch_bwd_s<T, POL, RELAX, NC, PK, B, 3, false, REC>(k, p, need_gmi, st, sg, rec);
+  return launch_bwd_s<T, POL, RELAX, NC, PK, B, 3, false, OPT>(k, p, need_gmi, st, sg, rec);
 }
 
-template <typename T, int POL, bool RELAX, bool REC>
+template <typename T, int POL, bool RELAX, int OPT>
 int dispatch_nc(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg,
                 const RecOut<T>& rec) {
   if constexpr (sizeof(T) == 4) {
-    if (p.PK == 2) return launch<T, POL, RELAX, 1, 2, REC>(bwd, k, p, need_gmi, st, sg, rec);
+    if (p.PK == 2) return launch<T, POL, RELAX, 1, 2, OPT>(bwd, k, p, need_gmi, st, sg, rec);
   }
 #ifdef MRPHY_ONLY_PK2   /* tuning builds (profiles/operand_model.py): compile the default fp32 kernels only */
   return fail(MRPHY_ERR_ARG, "built with MRPHY_ONLY_PK2%s");
@@ -1611,11 +1876,11 @@ int dispatch_nc(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaSt
   if constexpr (sizeof(T) == 4) {
     // 2 coils: two spins per thread (FFMA2) like the single-coil kernels; same tiles of 128 spins, same staging
     if (p.NC == 2 && env_int("MRPHY_B200_NC2_PACK", 2) == 2 && (!bwd || env_int("MRPHY_B200_NC2_PACK_BWD", 2) == 2))
-      return launch<T, POL, RELAX, 2, 2, REC>(bwd, k, p, need_gmi, st, sg, rec);
+      return launch<T, POL, RELAX, 2, 2, OPT>(bwd, k, p, need_gmi, st, sg, rec);
     if (p.tc && !bwd) {   // forward with >= 4 coils: transmit field on the tensor cores
-      if (p.NC == 4) return launch_fwd_tc<POL, RELAX, 4, REC>(k, p, st, rec);
-      if (p.NC == 8) return launch_fwd_tc<POL, RELAX, 8, REC>(k, p, st, rec);
-      return launch_fwd_tc<POL, RELAX, 16, REC>(k, p, st, rec);
+      if (p.NC == 4) return launch_fwd_tc<POL, RELAX, 4, OPT>(k, p, st, rec);
+      if (p.NC == 8) return launch_fwd_tc<POL, RELAX, 8, OPT>(k, p, st, rec);
+      return launch_fwd_tc<POL, RELAX, 16, OPT>(k, p, st, rec);
     }
   }
   switch (p.NC) {
@@ -1624,44 +1889,52 @@ int dispatch_nc(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaSt
       if constexpr (sizeof(T) == 4) return fail(MRPHY_ERR_ARG, "internal: fp32 single-coil scalar kernels not built%s");
       else
 #endif
-      return launch<T, POL, RELAX, 1, 1, REC>(bwd, k, p, need_gmi, st, sg, rec);
-    case 2: return launch<T, POL, RELAX, 2, 1, REC>(bwd, k, p, need_gmi, st, sg, rec);
-    case 4: return launch<T, POL, RELAX, 4, 1, REC>(bwd, k, p, need_gmi, st, sg, rec);
-    case 8: return launch<T, POL, RELAX, 8, 1, REC>(bwd, k, p, need_gmi, st, sg, rec);
-    case 16: return launch<T, POL, RELAX, 16, 1, REC>(bwd, k, p, need_gmi, st, sg, rec);
+      return launch<T, POL, RELAX, 1, 1, OPT>(bwd, k, p, need_gmi, st, sg, rec);
+    case 2: return launch<T, POL, RELAX, 2, 1, OPT>(bwd, k, p, need_gmi, st, sg, rec);
+    case 4: return launch<T, POL, RELAX, 4, 1, OPT>(bwd, k, p, need_gmi, st, sg, rec);
+    case 8: return launch<T, POL, RELAX, 8, 1, OPT>(bwd, k, p, need_gmi, st, sg, rec);
+    case 16: return launch<T, POL, RELAX, 16, 1, OPT>(bwd, k, p, need_gmi, st, sg, rec);
   }
   return fail(MRPHY_ERR_ARG, "internal: bad NC%s");
 #endif
 }
 
 template <typename T, int POL>
-int dispatch_pol(bool bwd, const KArgs<T>& k, const Plan& p, bool relax, bool rec, int need_gmi, cudaStream_t st,
-                 const SgOut<T>& sg, const RecOut<T>& ro) {
-  if (rec)
-    return relax ? dispatch_nc<T, POL, true, true>(bwd, k, p, need_gmi, st, sg, ro)
-                 : dispatch_nc<T, POL, false, true>(bwd, k, p, need_gmi, st, sg, ro);
-  return relax ? dispatch_nc<T, POL, true, false>(bwd, k, p, need_gmi, st, sg, ro)
-               : dispatch_nc<T, POL, false, false>(bwd, k, p, need_gmi, st, sg, ro);
+int dispatch_pol(bool bwd, const KArgs<T>& k, const Plan& p, bool relax, int opt, int need_gmi, cudaStream_t st,
+                 const SgOut<T>& sg, const RecOut<T>& rec) {
+  if (opt == 2)
+    return relax ? dispatch_nc<T, POL, true, 2>(bwd, k, p, need_gmi, st, sg, rec)
+                 : dispatch_nc<T, POL, false, 2>(bwd, k, p, need_gmi, st, sg, rec);
+  if (opt == 1)
+    return relax ? dispatch_nc<T, POL, true, 1>(bwd, k, p, need_gmi, st, sg, rec)
+                 : dispatch_nc<T, POL, false, 1>(bwd, k, p, need_gmi, st, sg, rec);
+  return relax ? dispatch_nc<T, POL, true, 0>(bwd, k, p, need_gmi, st, sg, rec)
+               : dispatch_nc<T, POL, false, 0>(bwd, k, p, need_gmi, st, sg, rec);
 }
 
 // the record option is on when any of its fields is set (check_record then wants all of them consistent)
 bool recording(const mrphy_fused_args* a) { return a->every || a->nR || a->Mt || a->gMt; }
 
+// r: the readout, or null
 template <typename T>
-int dispatch(bool bwd, const mrphy_fused_args* a, const Plan& p, cudaStream_t st, int* done) {
+int dispatch(bool bwd, const mrphy_fused_args* a, const mrphy_readout_args* r, const Plan& p, cudaStream_t st, int* done) {
   KArgs<T> k = make_kargs<T>(a, p);
   k.done = done;
   const SgOut<T> sg{(T*)a->gloc, (T*)a->gsz, (T*)a->gb1};
-  const bool rec = recording(a);
-  const RecOut<T> ro = rec ? RecOut<T>{(T*)a->Mt, (const T*)a->gMt, a->every, a->nR} : RecOut<T>{};
+  const int opt = r ? 2 : recording(a) ? 1 : 0;
+  RecOut<T> rec{};
+  if (opt == 1) rec = RecOut<T>{(T*)a->Mt, (const T*)a->gMt, a->every, a->nR, RoOut<T>{}};
+  if (opt == 2)
+    rec.ro = RoOut<T>{(const T*)r->rx, r->rx_sn, r->rx_sm, r->nRx, a->every, a->nR, RO_COLS / (2 * r->nRx), (T*)r->work,
+                      (const T*)r->gS, (T*)r->grx};
   const bool relax = a->T1.ptr != nullptr;
   const int need_gmi = (a->flags & MRPHY_NEED_GMI) ? 1 : 0;
   // fp64 has one trigonometry (TRIG_FAST names it), so only fp32 instantiates both
   if constexpr (sizeof(T) == 4) {
     if ((a->flags & MRPHY_TRIG_PRECISE) && !(bwd && (a->flags & MRPHY_TRIG_FAST_BWD)))
-      return dispatch_pol<T, TRIG_PRECISE>(bwd, k, p, relax, rec, need_gmi, st, sg, ro);
+      return dispatch_pol<T, TRIG_PRECISE>(bwd, k, p, relax, opt, need_gmi, st, sg, rec);
   }
-  return dispatch_pol<T, TRIG_FAST>(bwd, k, p, relax, rec, need_gmi, st, sg, ro);
+  return dispatch_pol<T, TRIG_FAST>(bwd, k, p, relax, opt, need_gmi, st, sg, rec);
 }
 
 // the record stride and its buffer (Mt for the forward, gMt for the backward)
@@ -1672,15 +1945,33 @@ int check_record(const mrphy_fused_args* a, bool bwd) {
   return MRPHY_OK;
 }
 
+// the readout: its stride (a->every, a->nR), coils and buffers; exclusive with record and the design tail
+int check_readout(const mrphy_fused_args* a, const mrphy_readout_args* r, bool bwd) {
+  if (a->Mt || a->gMt) return fail(MRPHY_ERR_ARG, "readout: does not combine with record (Mt / gMt)%s");
+  if (a->design) return fail(MRPHY_ERR_ARG, "readout: does not combine with the design tail%s");
+  if (a->every < 1 || a->every > a->nT || a->nR != a->nT / a->every)
+    return fail(MRPHY_ERR_ARG, "readout: need 1 <= every <= nT and nR == nT / every%s");
+  if (r->nRx < 1 || r->nRx > 16) return fail(MRPHY_ERR_ARG, "readout: need 1 <= nRx <= 16 receive coils%s");
+  if (bwd ? !r->gS : (!r->S || !r->work)) return fail(MRPHY_ERR_ARG, bwd ? "readout: gS is null%s" : "readout: S or work is null%s");
+  return MRPHY_OK;
+}
+
 template <typename T>
-int run_fwd(const mrphy_fused_args* a, cudaStream_t st) {
+int run_fwd(const mrphy_fused_args* a, const mrphy_readout_args* r, cudaStream_t st) {
   Plan p;
   int rc = make_plan(a, &p, true);
   if (rc) return rc;
   if ((rc = check_common<T>(a, false))) return rc;
-  if (recording(a) && (rc = check_record(a, false))) return rc;
+  if (r && (rc = check_readout(a, r, false))) return rc;
+  if (!r && recording(a) && (rc = check_record(a, false))) return rc;
   if ((rc = launch_pack<T>(a, p, st, p.tc != 0))) return rc;
-  return dispatch<T>(false, a, p, st, nullptr);
+  if ((rc = dispatch<T>(false, a, r, p, st, nullptr))) return rc;
+  if (!r) return MRPHY_OK;
+  dim3 grid((a->nR * 2 * r->nRx + 31) / 32, a->N), block(32, 8);
+  readout_finalize_kernel<T><<<grid, block, 0, st>>>((const T*)r->work, g_last_fwd_P, a->nR, r->nRx, (T*)r->S);
+  ++g_launches;
+  CK(cudaGetLastError());
+  return MRPHY_OK;
 }
 
 // the re-parametrisation the design tail can take: adjoint of an rf half and/or a gradient half that ends in a gradient
@@ -1702,13 +1993,14 @@ int check_design(const mrphy_fused_args* a, const mrphy_reparam_args* d) {
 }
 
 template <typename T>
-int run_bwd(const mrphy_fused_args* a, int wave_is_packed, cudaStream_t st) {
+int run_bwd(const mrphy_fused_args* a, const mrphy_readout_args* r, int wave_is_packed, cudaStream_t st) {
   Plan p;
   int rc = make_plan(a, &p, true);
   if (rc) return rc;
   if ((rc = check_common<T>(a, true))) return rc;
+  if (r && (rc = check_readout(a, r, true))) return rc;
   const mrphy_reparam_args* d = a->design;
-  const bool rec = recording(a), sg = a->gloc || a->gsz || a->gb1;
+  const bool rec = !r && recording(a), sg = a->gloc || a->gsz || a->gb1;
   if (d && (rec || sg)) return fail(MRPHY_ERR_ARG, "design: does not combine with record or per-spin gradients%s");
   if (d && (rc = check_design(a, d))) return rc;
   if (rec && (rc = check_record(a, true))) return rc;
@@ -1717,7 +2009,7 @@ int run_bwd(const mrphy_fused_args* a, int wave_is_packed, cudaStream_t st) {
   if ((!wave_is_packed || p.tc) && (rc = launch_pack<T>(a, p, st))) return rc;
   // finished-CTA counters of the design tail: behind the scheduling ints, zeroed by the backward kernel itself
   int* const done = d ? reinterpret_cast<int*>((T*)a->partials + (size_t)a->N * p.Pmax * p.W * (size_t)a->nT) + SCHED_CLAIM + p.Pmax : nullptr;
-  if ((rc = dispatch<T>(true, a, p, st, done))) return rc;
+  if ((rc = dispatch<T>(true, a, r, p, st, done))) return rc;
   if (sg && p.rows == 0) return MRPHY_OK;   // per-spin gradients only: nothing to finalize
   dim3 grid((a->nT + 31) / 32, p.W, a->N), block(32, 32);
   const int coil_dim = (a->flags & MRPHY_RF_COIL_DIM) ? 1 : 0;
@@ -1741,17 +2033,26 @@ int run_bwd(const mrphy_fused_args* a, int wave_is_packed, cudaStream_t st) {
 }  // namespace
 
 extern "C" int mrphy_blochsim_fused_fwd(const mrphy_fused_args* a, void* cuda_stream) {
-  g_launches = 0;
-  g_err[0] = 0;
-  if (!a) return fail(MRPHY_ERR_ARG, "null args%s");
-  cudaStream_t st = (cudaStream_t)cuda_stream;
-  return a->dtype == MRPHY_F64 ? run_fwd<double>(a, st) : run_fwd<float>(a, st);
+  return mrphy_blochsim_fused_readout_fwd(a, nullptr, cuda_stream);
 }
 
 extern "C" int mrphy_blochsim_fused_bwd(const mrphy_fused_args* a, int wave_is_packed, void* cuda_stream) {
+  return mrphy_blochsim_fused_readout_bwd(a, nullptr, wave_is_packed, cuda_stream);
+}
+
+extern "C" int mrphy_blochsim_fused_readout_fwd(const mrphy_fused_args* a, const mrphy_readout_args* r, void* cuda_stream) {
   g_launches = 0;
   g_err[0] = 0;
   if (!a) return fail(MRPHY_ERR_ARG, "null args%s");
   cudaStream_t st = (cudaStream_t)cuda_stream;
-  return a->dtype == MRPHY_F64 ? run_bwd<double>(a, wave_is_packed, st) : run_bwd<float>(a, wave_is_packed, st);
+  return a->dtype == MRPHY_F64 ? run_fwd<double>(a, r, st) : run_fwd<float>(a, r, st);
+}
+
+extern "C" int mrphy_blochsim_fused_readout_bwd(const mrphy_fused_args* a, const mrphy_readout_args* r, int wave_is_packed,
+                                                void* cuda_stream) {
+  g_launches = 0;
+  g_err[0] = 0;
+  if (!a) return fail(MRPHY_ERR_ARG, "null args%s");
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  return a->dtype == MRPHY_F64 ? run_bwd<double>(a, r, wave_is_packed, st) : run_bwd<float>(a, r, wave_is_packed, st);
 }

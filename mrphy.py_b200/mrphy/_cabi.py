@@ -121,6 +121,14 @@ class ClampArgs(ctypes.Structure):
     ]
 
 
+class ReadoutArgs(ctypes.Structure):
+    _fields_ = [
+        ('nRx', c_i32), ('_pad', c_i32),
+        ('rx', c_vp), ('rx_sn', c_i64), ('rx_sm', c_i64),
+        ('S', c_vp), ('gS', c_vp), ('grx', c_vp), ('work', c_vp),
+    ]
+
+
 EXPORTS = {   # name -> (restype, argtypes); tests check every symbol include/mrphy_b200.h declares
     'mrphy_abi_version': (ctypes.c_int, []),
     'mrphy_last_error': (ctypes.c_char_p, []),
@@ -134,6 +142,10 @@ EXPORTS = {   # name -> (restype, argtypes); tests check every symbol include/mr
     'mrphy_fused_partial_elems': (ctypes.c_size_t, [ctypes.POINTER(FusedArgs)]),
     'mrphy_blochsim_fused_fwd': (ctypes.c_int, [ctypes.POINTER(FusedArgs), c_vp]),
     'mrphy_blochsim_fused_bwd': (ctypes.c_int, [ctypes.POINTER(FusedArgs), ctypes.c_int, c_vp]),
+    'mrphy_fused_readout_elems': (ctypes.c_size_t, [ctypes.POINTER(FusedArgs), ctypes.POINTER(ReadoutArgs)]),
+    'mrphy_blochsim_fused_readout_fwd': (ctypes.c_int, [ctypes.POINTER(FusedArgs), ctypes.POINTER(ReadoutArgs), c_vp]),
+    'mrphy_blochsim_fused_readout_bwd': (ctypes.c_int, [ctypes.POINTER(FusedArgs), ctypes.POINTER(ReadoutArgs), ctypes.c_int,
+                                                        c_vp]),
     'mrphy_beff_ckpt_elems': (ctypes.c_size_t, [ctypes.POINTER(BeffArgs)]),
     'mrphy_blochsim_beff_fwd': (ctypes.c_int, [ctypes.POINTER(BeffArgs), c_vp]),
     'mrphy_blochsim_beff_bwd': (ctypes.c_int, [ctypes.POINTER(BeffArgs), c_vp]),
@@ -175,7 +187,7 @@ def lib():
                     raise RuntimeError(f'mrphy (B200): ABI version mismatch: library {L.mrphy_abi_version()} '
                                        f'!= binding {ABI_VERSION}; rebuild with mrphy.py_b200/build.py')
                 mirrors = (Param, FusedArgs, BeffArgs, RfGr2BeffArgs, Beff2abArgs, Beff2uphiArgs, FreePrecArgs, ReparamArgs,
-                           MaskArgs, ClampArgs)
+                           MaskArgs, ClampArgs, ReadoutArgs)
                 for which, cls in enumerate(mirrors):
                     if L.mrphy_sizeof_args(which) != ctypes.sizeof(cls):
                         raise RuntimeError(f'mrphy (B200): layout of {cls.__name__} ({ctypes.sizeof(cls)} B) differs from '

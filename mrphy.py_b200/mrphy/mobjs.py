@@ -391,6 +391,9 @@ class SpinArray(_Obj):
         doRelax: bool = True,
         doUpdate: bool = False,
         record: Optional[int] = None,
+        readout: Optional[int] = None,
+        rxMap: OptT = None,
+        rxMap_: OptT = None,
     ):
         r"""Simulate ``pulse`` on these spins and return the magnetisation.
 
@@ -410,12 +413,28 @@ class SpinArray(_Obj):
         steps -- ``M`` of the pulse cut to its first (r+1)·s samples.  Compact ``Mt`` is a non-contiguous view.
         ``doUpdate`` stores ``M`` only.  Gradients flow through both.  Refused (ValueError) beyond 16 transmit coils
         with a ``b1Map``: the explicit-``Beff`` route does not record.
+
+        ``readout = s`` (an integer, 1 <= s <= nT) returns ``(M, S)``: the receive signal of the same states, summed over the
+        spins inside the fused kernels (no ``Mt`` is formed), ``S[n,0,r] + i·S[n,1,r] = Σ_i (cx + i·cy)[n,i] (Mx + i·My)[n,i]``
+        after (r+1)·s steps, with the receive map ``rxMap`` ⊻ ``rxMap_`` `(N,*Nd ⊻ nM,xy,(nRx))` (at most 16 receive coils;
+        none: c = 1).  No conjugation and no scale factor.  ``S`` is `(N,2,nR)`, `(N,2,nR,nRx)` with a coil dimension on the
+        map.  ``doUpdate`` stores ``M``; ``doEmbed`` applies to ``M``.  Gradients of losses on ``S`` (and ``M``) reach
+        everything ``M``'s do and the receive map.  Refused (ValueError) together with ``record``, beyond 16 receive coils,
+        and beyond 16 transmit coils with a ``b1Map`` (the explicit-``Beff`` route has no readout).
         """
         assert (loc_ is None) != (loc is None)
         loc_ = loc_ if loc is None else self.extract(loc)
         Δf_ = _one_of(Δf, Δf_, self.extract)
         b1Map_ = _one_of(b1Map, b1Map_, self.extract)
         T1_, T2_ = (self.T1_, self.T2_) if doRelax else (None, None)
+        if readout is not None:
+            rxMap_ = _one_of(rxMap, rxMap_, self.extract)
+            p = pulse.to(device=self.device, dtype=self.dtype)
+            M_, S = _ops.fused_applypulse(self.M_, p.rf, p.gr, loc_, Δf_=Δf_, b1Map_=b1Map_, T1_=T1_, T2_=T2_, γ_=self.γ_,
+                                          dt=p.dt, record=record, readout=readout, rxMap_=rxMap_)
+            if doUpdate:
+                self.M_ = M_
+            return (self.embed(M_) if doEmbed else M_), S
         if record is not None:
             p = pulse.to(device=self.device, dtype=self.dtype)
             M_, Mt_ = _ops.fused_applypulse(self.M_, p.rf, p.gr, loc_, Δf_=Δf_, b1Map_=b1Map_, T1_=T1_, T2_=T2_,
@@ -474,7 +493,8 @@ class SpinArray(_Obj):
         ``doUpdate=True`` (mobjs.py:394-450, 555-592), but the magnetisation stays a compact device tensor from the first
         kernel to the last -- no embed / extract / attribute coercion per stage, no host synchronisation -- and the result is
         differentiable w.r.t. every pulse's ``rf`` / ``gr``, ``M_`` and the spin inputs as in :meth:`applypulse`.  The chain is CUDA-graph capturable as a whole
-        (``mrphy.graphs.capture``): one replay per sequence.  Arguments and flags as in :meth:`applypulse`.
+        (``mrphy.graphs.capture``): one replay per sequence.  Arguments and flags as in :meth:`applypulse`, except
+        ``record`` and ``readout``, which only :meth:`applypulse` takes.
         """
         assert (loc_ is None) != (loc is None)
         loc_ = loc_ if loc is None else self.extract(loc)
@@ -629,11 +649,16 @@ class SpinCube(SpinArray):
         doRelax: bool = True,
         doUpdate: bool = False,
         record: Optional[int] = None,
+        readout: Optional[int] = None,
+        rxMap: OptT = None,
+        rxMap_: OptT = None,
     ):
-        r"""As :meth:`SpinArray.applypulse` with the cube's ``loc_`` and ``Δf_``; only ``b1Map`` ⊻ ``b1Map_`` is given."""
+        r"""As :meth:`SpinArray.applypulse` with the cube's ``loc_`` and ``Δf_``; only ``b1Map`` ⊻ ``b1Map_`` (and for
+        ``readout``, ``rxMap`` ⊻ ``rxMap_``) is given."""
         b1Map_ = _one_of(b1Map, b1Map_, self.extract)
+        rxMap_ = _one_of(rxMap, rxMap_, self.extract)
         return self.spinarray.applypulse(pulse, loc_=self.loc_, Δf_=self.Δf_, b1Map_=b1Map_, doEmbed=doEmbed,
-                                         doRelax=doRelax, doUpdate=doUpdate, record=record)
+                                         doRelax=doRelax, doUpdate=doUpdate, record=record, readout=readout, rxMap_=rxMap_)
 
     def applysequence(self, events, *, b1Map: OptT = None, b1Map_: OptT = None, doEmbed: bool = False, doRelax: bool = True,
                       doUpdate: bool = False) -> Tensor:

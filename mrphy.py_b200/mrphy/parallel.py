@@ -8,6 +8,10 @@ all-reduce(sum) of the flat ``[rf.grad ‖ gr.grad ‖ extras]`` buffer (N·nT·
 for nT=4000).  Geometry stays global: the shard is a ``SpinArray`` with explicit ``loc_`` sliced from the
 global cube -- do not rebuild a smaller ``SpinCube`` (``_update_loc_`` centres on ``n//2``).
 
+A readout (``applypulse(pulse, readout=s)``) on a shard is the sum over that rank's spins only: ``allreduce_signal`` sums
+it over ranks, and its backward hands every rank the gradient of the full signal unchanged, so ``allreduce_waveform_grads``
+then completes the waveform gradients as usual.
+
 Per-spin gradients (``loc_``, ``Δf_``, ``b1Map_``, ``γ_`` requiring grad) are local to a shard and need no collective.
 A ``Δf`` or ``γ`` that is ONE tensor broadcast over spins gets, on each rank, only the sum over that rank's spins; this
 module does not all-reduce it -- sum it over ranks yourself if you need the global gradient.
@@ -20,7 +24,7 @@ from torch import Tensor
 
 from mrphy import mobjs
 
-__all__ = ['shard_range', 'shard_spins', 'shard_batch', 'allreduce_waveform_grads', 'flat_wave_grads']
+__all__ = ['shard_range', 'shard_spins', 'shard_batch', 'allreduce_waveform_grads', 'flat_wave_grads', 'allreduce_signal']
 
 
 def shard_range(nM: int, rank: int, world: int) -> Tuple[int, int]:
@@ -126,3 +130,24 @@ def allreduce_waveform_grads(rf: Tensor, gr: Tensor, *extras: Tensor, group=None
         n = p.numel()
         p.copy_(flat[off:off + n].reshape(p.shape))
         off += n
+
+
+class _AllreduceSignal(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, S, group):
+        out = S.clone()
+        dist.all_reduce(out, op=dist.ReduceOp.SUM, group=group)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        # every rank forms the same loss on the full signal: dL/dS_local = dL/dS on each rank
+        return g, None
+
+
+def allreduce_signal(S: Tensor, group=None) -> Tensor:
+    """The full readout signal from each rank's partial sum (spins sharded with ``shard_spins``): a sum all-reduce forward,
+    the identity backward.  Returns ``S`` itself without an initialised process group or on one rank."""
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+        return S
+    return _AllreduceSignal.apply(S, group)

@@ -96,6 +96,8 @@ def blochsim(
         - ``T1``, ``T2``: `()` ⊻ `(N ⊻ 1, *Nd ⊻ 1,)` "Sec";  ``γ``: same, "Hz/Gauss";  ``dt``: `()` ⊻ `(N ⊻ 1,)` "Sec".
     Outputs:
         - ``Mo``: `(N, *Nd, xyz)`.
+    There is no ``readout`` here: the receive signal summed inside the kernels comes from the fused path
+    (``SpinArray.applypulse(pulse, readout=s)``).
     """
     assert (Mi.shape[:-1] == Beff.shape[:-2])        # sims.py:305
     Beff, ndim = Beff.to(Mi.device), Beff.ndim

@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define MRPHY_ABI_VERSION 7
+#define MRPHY_ABI_VERSION 8
 
 enum mrphy_dtype { MRPHY_F32 = 0, MRPHY_F64 = 1 };
 
@@ -102,6 +102,12 @@ typedef struct mrphy_fused_args {
   void* gsz;           /* per-spin gradients, bwd: out (N,nM) contiguous, or NULL                    */
   void* gb1;           /* per-spin gradients, bwd: out (N,nM,2,nC) contiguous, or NULL (needs b1)    */
   const struct mrphy_reparam_args* design;   /* design tail, bwd: the re-parametrisation, or NULL  */
+  int32_t nRx, _pad2;  /* readout: receive coils, 1..16                                              */
+  const void* rx; int64_t rx_sn, rx_sm; /* readout: (N,nM,2,nRx) receive map, inner (2,nRx) contiguous, or NULL (c = 1) */
+  void* S;             /* readout, fwd: out (N,2,nR,nRx) contiguous                                  */
+  const void* gS;      /* readout, bwd: in, dL/dS like S                                             */
+  void* grx;           /* readout, bwd: out dL/drx (N,nM,2,nRx) contiguous, or NULL                  */
+  void* S_work;        /* readout, fwd: scratch, mrphy_fused_readout_elems() elements of T           */
 } mrphy_fused_args;
 
 int mrphy_abi_version(void);
@@ -110,21 +116,30 @@ const char* mrphy_last_error(void);
 /* Device facts the host side needs for sizing (queried once per device, cached). */
 int mrphy_device_sm_count(int device);
 
-/* Workspace sizes, in ELEMENTS of T.  They depend only on dtype, N, nM, nT, nC, K, b1 != NULL. */
+/* Workspace sizes, in ELEMENTS of T.  They depend only on dtype, N, nM, nT, nC, K, b1 != NULL (the readout's S_work also
+ * on nR and nRx: 0 unless 1 <= nRx <= 16 and nR >= 1). */
 size_t mrphy_fused_ckpt_elems(const mrphy_fused_args* a);
 size_t mrphy_fused_wave_elems(const mrphy_fused_args* a);
 size_t mrphy_fused_partial_elems(const mrphy_fused_args* a);
+size_t mrphy_fused_readout_elems(const mrphy_fused_args* a);
 
-/* Forward: writes Mo and ckpt.  Launches: pack_waveform, blochsim_fused_fwd.
+/* Forward: writes Mo and ckpt.  Launches: pack_waveform, blochsim_fused_fwd.  Two options, off when their fields are zero:
  *
  * Record (a->every != 0): the magnetisation during the pulse.  The forward also writes the state after every `every` steps,
  *   Mt[n][r][xyz][i] = M of spin i after (r+1)*every steps, r = 0 .. nR-1, nR = nT / every   (lab frame, like Mo)
  * -- what the forward returns as Mo for the pulse cut to its first (r+1)*every samples.  Needs a->Mt.  Up to 16 transmit
- * coils, like every fused call.  No workspace beyond the existing ones.                                               */
+ * coils, like every fused call.  No workspace beyond the existing ones.
+ *
+ * Readout (any of a->nRx, a->rx, a->S, a->gS, a->grx, a->S_work set): the receive signal of the magnetisation every
+ * `a->every` steps, summed over the spins inside the forward kernel,
+ *   S[n][xy][r][k] (Sx + i Sy) = sum_i (cx + i cy)[n][i][k] * (Mx + i My)[n][i] after (r+1)*every steps,  r < nR = nT / every
+ * (lab frame, the state record would return; no conjugation, no scale).  rx == NULL: c = 1.  a->every / a->nR give the stride
+ * as for record.  Needs a->S and a->S_work; a readout_finalize launch follows.  S is bitwise reproducible: each CTA sums its
+ * tiles into its own slot of S_work, the finalize sums the slots in a fixed order.  Excludes record and the design tail. */
 int mrphy_blochsim_fused_fwd(const mrphy_fused_args* a, void* cuda_stream);
 /* Backward: reads Mo, ckpt, gMo; writes grf, ggr (and gMi).  Launches: pack_waveform (unless
  * `wave` still holds the packed waveform of the matching forward: pass wave_is_packed != 0),
- * blochsim_fused_bwd, grad_reduce_finalize.  Three options, each off when its fields are zero / NULL:
+ * blochsim_fused_bwd, grad_reduce_finalize.  Four options, each off when its fields are zero / NULL:
  *
  * Record (a->every != 0): the backward of a recording forward with the same every / nR.  It takes dL/dMt (a->gMt, in
  * the layout of Mt) on top of dL/dMo; a->gMo is required (zeros when the loss ignores Mo).
@@ -146,34 +161,13 @@ int mrphy_blochsim_fused_fwd(const mrphy_fused_args* a, void* cuda_stream);
  * nC = trailing coil dimension of rf; rf_kind 0..2 and gr_kind 0..2 as in mrphy_design_waveform (0: that waveform is
  * not re-parametrised); design->grf / ->ggr are ignored -- the tail reads a->grf / a->ggr, which are written as usual.
  * Same launches: the last CTA of the epilogue to finish for a batch entry evaluates that entry's adjoint and writes
- * design->grho, ->gtheta, ->gts.  Combines with neither record nor per-spin gradients (MRPHY_ERR_ARG).
+ * design->grho, ->gtheta, ->gts.  Combines with neither record, per-spin gradients nor readout (MRPHY_ERR_ARG).
  *
- * No option needs workspace beyond mrphy_fused_partial_elems().                                                      */
+ * Readout (the forward's fields): the backward of a readout forward.  It takes dL/dS (a->gS) on top of dL/dMo (zeros when
+ * the loss ignores M) and, with a->grx, writes dL/dcx = sum_r (gSx Mx + gSy My), dL/dcy = sum_r (gSy Mx - gSx My).  Combines
+ * with per-spin gradients.  MRPHY_ERR_ARG before any launch for: a->Mt / a->gMt or a->design set, nRx outside 1..16, a null
+ * S / S_work (fwd) or gS (bwd), every / nR inconsistent.  No workspace beyond mrphy_fused_partial_elems().            */
 int mrphy_blochsim_fused_bwd(const mrphy_fused_args* a, int wave_is_packed, void* cuda_stream);
-
-/* Readout: the receive signal of the magnetisation every `a->every` steps, summed over the spins inside the forward kernel,
- *   S[n][xy][r][k] (Sx + i Sy) = sum_i (cx + i cy)[n][i][k] * (Mx + i My)[n][i] after (r+1)*every steps,  r < nR = nT / every
- * (lab frame, the state record would return; no conjugation, no scale).  rx == NULL: c = 1.  a->every / a->nR give the stride
- * as for record; the readout excludes record (a->Mt, a->gMt) and the design tail.  S is bitwise reproducible: each CTA of the
- * forward sums its tiles into its own slot of `work`, and a finalize kernel sums the slots in a fixed order.             */
-typedef struct mrphy_readout_args {
-  int32_t nRx;                            /* receive coils, 1..16                                                  */
-  int32_t _pad;
-  const void* rx; int64_t rx_sn, rx_sm;   /* (N,nM,2,nRx) receive map, inner (2,nRx) contiguous, or NULL (c = 1)    */
-  void* S;                                /* fwd: out (N,2,nR,nRx) contiguous                                      */
-  const void* gS;                         /* bwd: in, dL/dS like S                                                 */
-  void* grx;                              /* bwd: out dL/drx (N,nM,2,nRx) contiguous, or NULL:
-                                             dL/dcx = sum_r (gSx Mx + gSy My),  dL/dcy = sum_r (gSy Mx - gSx My)         */
-  void* work;                             /* fwd: scratch, mrphy_fused_readout_elems() elements of T                */
-} mrphy_readout_args;
-size_t mrphy_fused_readout_elems(const mrphy_fused_args* a, const mrphy_readout_args* r);
-/* The fused pair with a readout; r == NULL is exactly mrphy_blochsim_fused_fwd / _bwd.  Forward launches: pack_waveform,
- * blochsim_fused_fwd, readout_finalize.  The backward takes dL/dS (r->gS) on top of dL/dMo (a->gMo, zeros when the loss
- * ignores M) and combines with per-spin gradients.  MRPHY_ERR_ARG before any launch for: a->Mt / a->gMt set, a->design set,
- * nRx outside 1..16, a null S / work (fwd) or gS (bwd), every / nR inconsistent.                                          */
-int mrphy_blochsim_fused_readout_fwd(const mrphy_fused_args* a, const mrphy_readout_args* r, void* cuda_stream);
-int mrphy_blochsim_fused_readout_bwd(const mrphy_fused_args* a, const mrphy_readout_args* r, int wave_is_packed,
-                                     void* cuda_stream);
 
 /* Arguments of the explicit-field path: the API-faithful replacement of sims.BlochSim
  * (sims.py:24-269) for callers that hand in a dense Beff (N,nM,nT,3), e.g. tests/test_sims.py:88
@@ -329,8 +323,8 @@ int mrphy_mask_copy(const mrphy_mask_args* a, void* cuda_stream);
 
 /* sizeof() of the argument structs as this library was compiled, for bindings to check their mirror of the layout:
  * which = 0 mrphy_param, 1 mrphy_fused_args, 2 mrphy_beff_args, 3 mrphy_rfgr2beff_args, 4 mrphy_beff2ab_args,
- * 5 mrphy_beff2uphi_args, 6 mrphy_freeprec_args, 7 mrphy_reparam_args, 8 mrphy_mask_args, 9 mrphy_clamp_args,
- * 10 mrphy_readout_args; 0 for any other value. */
+ * 5 mrphy_beff2uphi_args, 6 mrphy_freeprec_args, 7 mrphy_reparam_args, 8 mrphy_mask_args, 9 mrphy_clamp_args;
+ * 0 for any other value. */
 size_t mrphy_sizeof_args(int which);
 
 /* Number of kernel launches the last forward / backward call on this thread issued. */

@@ -467,7 +467,6 @@ extern "C" size_t mrphy_sizeof_args(int which) {
     case 7: return sizeof(mrphy_reparam_args);
     case 8: return sizeof(mrphy_mask_args);
     case 9: return sizeof(mrphy_clamp_args);
-    case 10: return sizeof(mrphy_readout_args);
   }
   return 0;
 }

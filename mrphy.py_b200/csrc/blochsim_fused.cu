@@ -6,8 +6,8 @@
 // Kernels in this file
 //   pack_waveform_kernel      rf (N,2,nT[,nC]), gr (N,3,nT) -> wave[N][chunk][W][TCP]  (W = 2*NC+3)
 //   fused_fwd_kernel<T,..>    one spin, or two spins packed in an f2 (FFMA2), per thread; checkpoint every K steps
-//                             REC: also the state every `every` steps (Mt, rec_store)
-//                             RD (POL & POL_RD): instead the receive signal of those states summed over the CTA's spins
+//                             REC (OPT_RECORD): also the state every `every` steps (Mt, rec_store)
+//                             RD (OPT_READOUT): instead the receive signal of those states summed over the CTA's spins
 //                             (ro_accum, ro_flush) into a per-CTA slot
 //   fused_bwd_kernel<T,..>    time-reversed state reconstruction + adjoint + spin reduction (only the gradient rows
 //                             asked for: ROWS); tiles owned through SM-aware virtual CTA ids (SCHED_*)
@@ -175,8 +175,9 @@ template <typename T> struct SgOut {
   T* gloc; T* gsz; T* gb1;
   bool any() const { return gloc || gsz || gb1; }
 };
-// readout of the RD kernels (mrphy_readout_args): the signal S[n][xy][r][k] = sum_i (cx + i cy)[n][i][k] (Mx + i My)[n][i] of
-// the state after (r+1)*every steps (lab frame).  The forward sums its tiles into its own slot of `part` [N][P][nR][2 nRx]
+// readout of the RD kernels (nRx, rx, S, gS, grx, S_work of mrphy_fused_args): the signal
+// S[n][xy][r][k] = sum_i (cx + i cy)[n][i][k] (Mx + i My)[n][i] of the state after (r+1)*every steps (lab frame).  The
+// forward sums its tiles into its own slot of `part` [N][P][nR][2 nRx]
 // (P = gridDim.x; x values, then y values; readout_finalize_kernel sums the slots in a fixed order); the backward adds the
 // adjoint of S to the adjoint state at the recorded steps (ro_adjoint) and, with grx, forms dL/drx per spin.
 template <typename T> struct RoOut {
@@ -196,10 +197,9 @@ template <typename T> struct RecOut {
   int every, nR;
   RoOut<T> ro;
 };
-// The readout kernels are the instantiations of fused_fwd_kernel, fused_fwd_tc_kernel and fused_bwd_kernel whose policy
-// parameter carries POL_RD (the policy itself is POL & ~POL_RD).  A flag on an existing parameter rather than a parameter of
-// its own keeps the names and the code of every kernel without readout as they are.
-constexpr int POL_RD = 16;
+// The option of fused_fwd_kernel, fused_fwd_tc_kernel and fused_bwd_kernel (template parameter OPT): none, record (REC) or
+// readout (RD); a call takes at most one of them.
+constexpr int OPT_NONE = 0, OPT_RECORD = 1, OPT_READOUT = 2;
 // Dynamic shared memory of the readout, behind what the kernel already uses (runtime-sized by nRx; V = Pack<T, PK>::type):
 //   forward   w V[2 nRx][BLKT]  |  tiles T[NW][32 columns][32 lanes]  |  ctab T[2][NW][32]
 //   backward  w V[2 nRx][BLKT]  |  acc V[2 nRx][BLKT] (dL/drx sums)   |  gs T[records per chunk][2 nRx] (dL/dS of the chunk)
@@ -484,10 +484,10 @@ __global__ void pack_waveform_kernel(const T* __restrict__ rf, int64_t rf_sn, in
 // ------------------------------------------------------------------------------------------
 // forward.  PK spins per thread (PK == 2: packed f2 arithmetic), BLKT threads per CTA.
 // REC: also the state after every `rec.every` steps (rec_store), tracked by a countdown (no per-step division).
-// RD (POL & POL_RD): instead the signal of the state after every `ro.every` steps, on the same countdown (ro_accum / ro_flush).
-template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, bool REC = false>
+// RD: instead the signal of the state after every `ro.every` steps, on the same countdown (ro_accum / ro_flush).
+template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, int OPT = OPT_NONE>
 __global__ void __launch_bounds__(BLKT, (PK == 2 ? (NC == 1 ? 14 : MRPHY_NC2_MINB) : 1)) fused_fwd_kernel(const KArgs<T> a, const RecOut<T> rec) {
-  constexpr bool RD = (POL & POL_RD) != 0;
+  constexpr bool REC = OPT == OPT_RECORD, RD = OPT == OPT_READOUT;
   const RoOut<T>& ro = rec.ro;
   typedef typename Pack<T, PK>::type V;
   constexpr int W = 2 * NC + 3;
@@ -553,7 +553,7 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? (NC == 1 ? 14 : MRPHY_NC2_MIN
 #pragma unroll
         for (int q = 0; q < NC; ++q) { rx[q] = V(s[q]); ry[q] = V(s[NC + q]); }
         field<V, NC>(k, rx, ry, V(s[2 * NC]), V(s[2 * NC + 1]), V(s[2 * NC + 2]), bx, by, bz);
-        step_fwd<V, POL & ~POL_RD, RELAX>(bx, by, bz, k.e1, k.e2, mx, my, mz);
+        step_fwd<V, POL, RELAX>(bx, by, bz, k.e1, k.e2, mx, my, mz);
         if constexpr (REC) {
           if (--rc == 0) {   // recorded states leave the spin frame (a copy: the state stays in it)
             V x = mx, y = my;
@@ -787,11 +787,10 @@ __device__ __forceinline__ void sg_fold(const KArgs<T>& a, const SgOut<T>& o, in
 // SG: also the per-spin gradients (sg_fold).  ROWS == 0 (SG only, a fixed pulse): no transposition tile, no partial sums.
 // REC: the loss also depends on the recorded states: dL/dMt[r] joins the adjoint before the adjoint of the step that
 // produced state r, so that everything downstream (F, the spin reduction, sg_fold, dL/dMi) sees the total dL/dm.
-// RD (POL & POL_RD): the adjoint of the readout joins instead, at the same steps (ro_adjoint), and with ro.grx the kernel
-// also forms dL/drx.
-template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, int ROWS = 3, bool SG = false, bool REC = false>
+// RD: the adjoint of the readout joins instead, at the same steps (ro_adjoint), and with ro.grx the kernel also forms dL/drx.
+template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, int ROWS = 3, bool SG = false, int OPT = OPT_NONE>
 __global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : (sizeof(T) == 8 && NC == 1 ? 4 : (sizeof(T) == 4 && NC > 1 ? MRPHY_MC_MINB : 1)))) fused_bwd_kernel(const KArgs<T> a, const int need_gmi, const SgOut<T> sgo, const RecOut<T> rec) {
-  constexpr bool RD = (POL & POL_RD) != 0;
+  constexpr bool REC = OPT == OPT_RECORD, RD = OPT == OPT_READOUT;
   const RoOut<T>& ro = rec.ro;
   typedef typename Pack<T, PK>::type V;
   using L = BwdSmem<T, NC, BLKT, PK>;
@@ -966,7 +965,7 @@ __global__ void __launch_bounds__(BLKT, (PK == 2 ? MRPHY_BWD_MINB * 64 / BLKT : 
 #pragma unroll
         for (int q = 0; q < NC; ++q) { rx[q] = V(s[q]); ry[q] = V(s[NC + q]); }
         field<V, NC>(k, rx, ry, V(s[2 * NC]), V(s[2 * NC + 1]), V(s[2 * NC + 2]), bx, by, bz);
-        step_bwd<V, POL & ~POL_RD, RELAX, NC>(k, bx, by, bz, mx, my, mz, hx, hy, hz, Fx, Fy, Fz);
+        step_bwd<V, POL, RELAX, NC>(k, bx, by, bz, mx, my, mz, hx, hy, hz, Fx, Fy, Fz);
         if constexpr (SG) {
           sacc[0] = fma_(V(s[2 * NC]), Fz, sacc[0]);
           sacc[1] = fma_(V(s[2 * NC + 1]), Fz, sacc[1]);
@@ -1266,9 +1265,9 @@ __device__ __forceinline__ void tc_issue(const float* sa, const float* wb, int r
 
 // REC, RD as in fused_fwd_kernel (this kernel has no spin frame: the state is in the lab frame throughout); the readout's
 // shared memory follows C::bytes.
-template <int POL, bool RELAX, int NC, int PK, bool REC = false>
+template <int POL, bool RELAX, int NC, int PK, int OPT = OPT_NONE>
 __global__ void __launch_bounds__(128, (NC <= 8 ? 4 : (PK == 1 ? 3 : 2))) fused_fwd_tc_kernel(const KArgs<float> a, const RecOut<float> rec) {
-  constexpr bool RD = (POL & POL_RD) != 0;
+  constexpr bool REC = OPT == OPT_RECORD, RD = OPT == OPT_READOUT;
   const RoOut<float>& ro = rec.ro;
   using L = TcLayout<NC>;
   using C = TcCfg<NC, PK>;
@@ -1361,7 +1360,7 @@ __global__ void __launch_bounds__(128, (NC <= 8 ? 4 : (PK == 1 ? 3 : 2))) fused_
           if (j0 + u < ns) {
             const V bz = fma_(glx, V(g[0][u]), fma_(gly, V(g[1][u]), fma_(glz, V(g[2][u]), gbz0)));
             const V bx = mkv(b[0][2 * u], b[PK - 1][2 * u], (V*)nullptr), by = mkv(b[0][2 * u + 1], b[PK - 1][2 * u + 1], (V*)nullptr);
-            step_fwd<V, POL & ~POL_RD, RELAX>(bx, by, bz, e1, e2, mx, my, mz);
+            step_fwd<V, POL, RELAX>(bx, by, bz, e1, e2, mx, my, mz);
             if constexpr (REC) {
               if (--rc == 0) {
                 rec_store<T, V, PK>(rec, nM, n, rr++, idx, ok, mx, my, mz);
@@ -1641,11 +1640,11 @@ extern "C" size_t mrphy_fused_partial_elems(const mrphy_fused_args* a) {
   return (size_t)a->N * p.Pmax * p.W * (size_t)a->nT + (size_t)(SCHED_CLAIM + p.Pmax) + (size_t)a->N;
 }
 
-extern "C" size_t mrphy_fused_readout_elems(const mrphy_fused_args* a, const mrphy_readout_args* r) {
+extern "C" size_t mrphy_fused_readout_elems(const mrphy_fused_args* a) {
   Plan p;
   if (make_plan(a, &p, true) != MRPHY_OK) return 0;
-  if (!r || r->nRx < 1 || r->nRx > 16 || a->nR < 1) return 0;
-  return (size_t)a->N * p.Pmax * (size_t)a->nR * 2 * r->nRx;
+  if (a->nRx < 1 || a->nRx > 16 || a->nR < 1) return 0;
+  return (size_t)a->N * p.Pmax * (size_t)a->nR * 2 * a->nRx;
 }
 
 namespace {
@@ -1719,15 +1718,12 @@ thread_local int g_last_fwd_P = 0;
 // records a staged chunk of K steps can produce (the backward's dL/dS staging)
 inline int ro_chunk_records(int K, int every) { return (K + every - 1) / every; }
 
-// OPT selects the option of the kernels: 0 none, 1 record (REC), 2 readout (RD, the *_ro_ kernels)
 template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, int OPT>
 int launch_fwd_s(KArgs<T> k, const Plan& p, cudaStream_t st, const RecOut<T>& rec) {
-  constexpr bool REC = OPT == 1;
-  const size_t smem = OPT == 2 ? ro_fwd_smem(rec.ro.nRx, BLKT, (int)sizeof(typename Pack<T, PK>::type), (int)sizeof(T)) : 0;
-  auto kern = [] {
-    if constexpr (OPT == 2) return fused_fwd_kernel<T, POL | POL_RD, RELAX, NC, PK, BLKT, false>;
-    else return fused_fwd_kernel<T, POL, RELAX, NC, PK, BLKT, REC>;
-  }();
+  constexpr bool REC = OPT == OPT_RECORD;
+  const size_t smem =
+      OPT == OPT_READOUT ? ro_fwd_smem(rec.ro.nRx, BLKT, (int)sizeof(typename Pack<T, PK>::type), (int)sizeof(T)) : 0;
+  auto kern = fused_fwd_kernel<T, POL, RELAX, NC, PK, BLKT, OPT>;
   if (smem) CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int occ = 0;
   CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, BLKT, smem));
@@ -1747,14 +1743,11 @@ int launch_fwd_s(KArgs<T> k, const Plan& p, cudaStream_t st, const RecOut<T>& re
 }
 template <typename T, int POL, bool RELAX, int NC, int PK, int BLKT, int ROWS, bool SG, int OPT>
 int launch_bwd_s(KArgs<T> k, const Plan& p, int need_gmi, cudaStream_t st, const SgOut<T>& sg, const RecOut<T>& rec) {
-  constexpr bool REC = OPT == 1;
+  constexpr bool REC = OPT == OPT_RECORD;
   const size_t smem = BwdSmem<T, NC, BLKT, PK>::bytes +
-                      (OPT == 2 ? ro_bwd_smem(rec.ro.nRx, BLKT, (int)sizeof(typename Pack<T, PK>::type), (int)sizeof(T),
-                                              ro_chunk_records(p.K, rec.ro.every)) : 0);
-  auto kern = [] {
-    if constexpr (OPT == 2) return fused_bwd_kernel<T, POL | POL_RD, RELAX, NC, PK, BLKT, ROWS, SG, false>;
-    else return fused_bwd_kernel<T, POL, RELAX, NC, PK, BLKT, ROWS, SG, REC>;
-  }();
+                      (OPT == OPT_READOUT ? ro_bwd_smem(rec.ro.nRx, BLKT, (int)sizeof(typename Pack<T, PK>::type), (int)sizeof(T),
+                                                        ro_chunk_records(p.K, rec.ro.every)) : 0);
+  auto kern = fused_bwd_kernel<T, POL, RELAX, NC, PK, BLKT, ROWS, SG, OPT>;
   CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   // static + dynamic may exceed 48 KB
   int occ = 0;
   CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, BLKT, smem));
@@ -1777,7 +1770,7 @@ int launch_bwd_s(KArgs<T> k, const Plan& p, int need_gmi, cudaStream_t st, const
   if (getenv("MRPHY_B200_DEBUG"))
     fprintf(stderr, "[mrphy_b200] fused_bwd<%s,NC=%d,PK=%d,BLK=%d,%s,ROWS=%d,SG=%d%s> grid=(%d,%d) tiles=%d occ=%d smem=%zu K=%d\n",
             sizeof(T) == 4 ? "f32" : "f64", NC, PK, BLKT, POL == TRIG_PRECISE ? "precise" : "fast", ROWS, (int)SG,
-            REC ? ",REC=1" : (OPT == 2 ? ",RD=1" : ""), k.P, k.N, q.tiles, occ, smem, p.K);
+            REC ? ",REC=1" : (OPT == OPT_READOUT ? ",RD=1" : ""), k.P, k.N, q.tiles, occ, smem, p.K);
   timing_begin(st);
   kern<<<grid, BLKT, smem, st>>>(k, need_gmi, sg, rec);
   timing_end(st);
@@ -1811,12 +1804,10 @@ int tc_occupancy(Kern kern, size_t dyn_smem, int tmem_cols) {
 template <int POL, bool RELAX, int NC, int PK, int OPT>
 int launch_fwd_tc_pk(KArgs<float> k, const Plan& p, cudaStream_t st, const RecOut<float>& rec) {
   using C = TcCfg<NC, PK>;
-  constexpr bool REC = OPT == 1;
-  const size_t smem = C::bytes + (OPT == 2 ? ro_fwd_smem(rec.ro.nRx, 128, (int)sizeof(typename Pack<float, PK>::type), 4) : 0);
-  auto kern = [] {
-    if constexpr (OPT == 2) return fused_fwd_tc_kernel<POL | POL_RD, RELAX, NC, PK, false>;
-    else return fused_fwd_tc_kernel<POL, RELAX, NC, PK, REC>;
-  }();
+  constexpr bool REC = OPT == OPT_RECORD;
+  const size_t smem =
+      C::bytes + (OPT == OPT_READOUT ? ro_fwd_smem(rec.ro.nRx, 128, (int)sizeof(typename Pack<float, PK>::type), 4) : 0);
+  auto kern = fused_fwd_tc_kernel<POL, RELAX, NC, PK, OPT>;
   CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   k.TCP = p.tc_TCP;
   k.chunk_elems = p.tc_chunk_elems;
@@ -1825,12 +1816,12 @@ int launch_fwd_tc_pk(KArgs<float> k, const Plan& p, cudaStream_t st, const RecOu
   k.P = (int)((int64_t)sm_count_cached() * occ / k.N);   // every resident slot (pick_ctas trades slots for even passes)
   if (k.P < 1) k.P = 1;
   if (k.P > tiles) k.P = tiles;
-  if (OPT == 2 && k.P > p.Pmax) k.P = p.Pmax;   // one readout slot per CTA: mrphy_fused_readout_elems sized Pmax of them
+  if (OPT == OPT_READOUT && k.P > p.Pmax) k.P = p.Pmax;   // one readout slot per CTA: mrphy_fused_readout_elems sized Pmax of them
   g_last_fwd_P = k.P;
   dim3 grid(k.P, k.N);
   if (getenv("MRPHY_B200_DEBUG"))
     fprintf(stderr, "[mrphy_b200] fused_fwd_tc<NC=%d,PK=%d%s> grid=(%d,%d) tiles=%d occ=%d smem=%zu K=%d\n", NC, PK,
-            REC ? ",REC=1" : (OPT == 2 ? ",RD=1" : ""), k.P, k.N, tiles, occ, smem, p.K);
+            REC ? ",REC=1" : (OPT == OPT_READOUT ? ",RD=1" : ""), k.P, k.N, tiles, occ, smem, p.K);
   timing_begin(st);
   kern<<<grid, 128, smem, st>>>(k, rec);
   timing_end(st);
@@ -1902,31 +1893,32 @@ int dispatch_nc(bool bwd, const KArgs<T>& k, const Plan& p, int need_gmi, cudaSt
 template <typename T, int POL>
 int dispatch_pol(bool bwd, const KArgs<T>& k, const Plan& p, bool relax, int opt, int need_gmi, cudaStream_t st,
                  const SgOut<T>& sg, const RecOut<T>& rec) {
-  if (opt == 2)
-    return relax ? dispatch_nc<T, POL, true, 2>(bwd, k, p, need_gmi, st, sg, rec)
-                 : dispatch_nc<T, POL, false, 2>(bwd, k, p, need_gmi, st, sg, rec);
-  if (opt == 1)
-    return relax ? dispatch_nc<T, POL, true, 1>(bwd, k, p, need_gmi, st, sg, rec)
-                 : dispatch_nc<T, POL, false, 1>(bwd, k, p, need_gmi, st, sg, rec);
-  return relax ? dispatch_nc<T, POL, true, 0>(bwd, k, p, need_gmi, st, sg, rec)
-               : dispatch_nc<T, POL, false, 0>(bwd, k, p, need_gmi, st, sg, rec);
+  if (opt == OPT_READOUT)
+    return relax ? dispatch_nc<T, POL, true, OPT_READOUT>(bwd, k, p, need_gmi, st, sg, rec)
+                 : dispatch_nc<T, POL, false, OPT_READOUT>(bwd, k, p, need_gmi, st, sg, rec);
+  if (opt == OPT_RECORD)
+    return relax ? dispatch_nc<T, POL, true, OPT_RECORD>(bwd, k, p, need_gmi, st, sg, rec)
+                 : dispatch_nc<T, POL, false, OPT_RECORD>(bwd, k, p, need_gmi, st, sg, rec);
+  return relax ? dispatch_nc<T, POL, true, OPT_NONE>(bwd, k, p, need_gmi, st, sg, rec)
+               : dispatch_nc<T, POL, false, OPT_NONE>(bwd, k, p, need_gmi, st, sg, rec);
 }
 
-// the record option is on when any of its fields is set (check_record then wants all of them consistent)
+// an option is on when any of its fields is set (check_record / check_readout then want all of them consistent); the
+// readout shares every / nR with the record
 bool recording(const mrphy_fused_args* a) { return a->every || a->nR || a->Mt || a->gMt; }
+bool reading_out(const mrphy_fused_args* a) { return a->nRx || a->rx || a->S || a->gS || a->grx || a->S_work; }
 
-// r: the readout, or null
 template <typename T>
-int dispatch(bool bwd, const mrphy_fused_args* a, const mrphy_readout_args* r, const Plan& p, cudaStream_t st, int* done) {
+int dispatch(bool bwd, const mrphy_fused_args* a, const Plan& p, cudaStream_t st, int* done) {
   KArgs<T> k = make_kargs<T>(a, p);
   k.done = done;
   const SgOut<T> sg{(T*)a->gloc, (T*)a->gsz, (T*)a->gb1};
-  const int opt = r ? 2 : recording(a) ? 1 : 0;
+  const int opt = reading_out(a) ? OPT_READOUT : recording(a) ? OPT_RECORD : OPT_NONE;
   RecOut<T> rec{};
-  if (opt == 1) rec = RecOut<T>{(T*)a->Mt, (const T*)a->gMt, a->every, a->nR, RoOut<T>{}};
-  if (opt == 2)
-    rec.ro = RoOut<T>{(const T*)r->rx, r->rx_sn, r->rx_sm, r->nRx, a->every, a->nR, RO_COLS / (2 * r->nRx), (T*)r->work,
-                      (const T*)r->gS, (T*)r->grx};
+  if (opt == OPT_RECORD) rec = RecOut<T>{(T*)a->Mt, (const T*)a->gMt, a->every, a->nR, RoOut<T>{}};
+  if (opt == OPT_READOUT)
+    rec.ro = RoOut<T>{(const T*)a->rx, a->rx_sn, a->rx_sm, a->nRx, a->every, a->nR, RO_COLS / (2 * a->nRx), (T*)a->S_work,
+                      (const T*)a->gS, (T*)a->grx};
   const bool relax = a->T1.ptr != nullptr;
   const int need_gmi = (a->flags & MRPHY_NEED_GMI) ? 1 : 0;
   // fp64 has one trigonometry (TRIG_FAST names it), so only fp32 instantiates both
@@ -1946,29 +1938,30 @@ int check_record(const mrphy_fused_args* a, bool bwd) {
 }
 
 // the readout: its stride (a->every, a->nR), coils and buffers; exclusive with record and the design tail
-int check_readout(const mrphy_fused_args* a, const mrphy_readout_args* r, bool bwd) {
+int check_readout(const mrphy_fused_args* a, bool bwd) {
   if (a->Mt || a->gMt) return fail(MRPHY_ERR_ARG, "readout: does not combine with record (Mt / gMt)%s");
   if (a->design) return fail(MRPHY_ERR_ARG, "readout: does not combine with the design tail%s");
   if (a->every < 1 || a->every > a->nT || a->nR != a->nT / a->every)
     return fail(MRPHY_ERR_ARG, "readout: need 1 <= every <= nT and nR == nT / every%s");
-  if (r->nRx < 1 || r->nRx > 16) return fail(MRPHY_ERR_ARG, "readout: need 1 <= nRx <= 16 receive coils%s");
-  if (bwd ? !r->gS : (!r->S || !r->work)) return fail(MRPHY_ERR_ARG, bwd ? "readout: gS is null%s" : "readout: S or work is null%s");
+  if (a->nRx < 1 || a->nRx > 16) return fail(MRPHY_ERR_ARG, "readout: need 1 <= nRx <= 16 receive coils%s");
+  if (bwd ? !a->gS : (!a->S || !a->S_work)) return fail(MRPHY_ERR_ARG, bwd ? "readout: gS is null%s" : "readout: S or work is null%s");
   return MRPHY_OK;
 }
 
 template <typename T>
-int run_fwd(const mrphy_fused_args* a, const mrphy_readout_args* r, cudaStream_t st) {
+int run_fwd(const mrphy_fused_args* a, cudaStream_t st) {
   Plan p;
   int rc = make_plan(a, &p, true);
   if (rc) return rc;
   if ((rc = check_common<T>(a, false))) return rc;
-  if (r && (rc = check_readout(a, r, false))) return rc;
-  if (!r && recording(a) && (rc = check_record(a, false))) return rc;
+  const bool ro = reading_out(a);
+  if (ro && (rc = check_readout(a, false))) return rc;
+  if (!ro && recording(a) && (rc = check_record(a, false))) return rc;
   if ((rc = launch_pack<T>(a, p, st, p.tc != 0))) return rc;
-  if ((rc = dispatch<T>(false, a, r, p, st, nullptr))) return rc;
-  if (!r) return MRPHY_OK;
-  dim3 grid((a->nR * 2 * r->nRx + 31) / 32, a->N), block(32, 8);
-  readout_finalize_kernel<T><<<grid, block, 0, st>>>((const T*)r->work, g_last_fwd_P, a->nR, r->nRx, (T*)r->S);
+  if ((rc = dispatch<T>(false, a, p, st, nullptr))) return rc;
+  if (!ro) return MRPHY_OK;
+  dim3 grid((a->nR * 2 * a->nRx + 31) / 32, a->N), block(32, 8);
+  readout_finalize_kernel<T><<<grid, block, 0, st>>>((const T*)a->S_work, g_last_fwd_P, a->nR, a->nRx, (T*)a->S);
   ++g_launches;
   CK(cudaGetLastError());
   return MRPHY_OK;
@@ -1993,14 +1986,15 @@ int check_design(const mrphy_fused_args* a, const mrphy_reparam_args* d) {
 }
 
 template <typename T>
-int run_bwd(const mrphy_fused_args* a, const mrphy_readout_args* r, int wave_is_packed, cudaStream_t st) {
+int run_bwd(const mrphy_fused_args* a, int wave_is_packed, cudaStream_t st) {
   Plan p;
   int rc = make_plan(a, &p, true);
   if (rc) return rc;
   if ((rc = check_common<T>(a, true))) return rc;
-  if (r && (rc = check_readout(a, r, true))) return rc;
+  const bool ro = reading_out(a);
+  if (ro && (rc = check_readout(a, true))) return rc;
   const mrphy_reparam_args* d = a->design;
-  const bool rec = !r && recording(a), sg = a->gloc || a->gsz || a->gb1;
+  const bool rec = !ro && recording(a), sg = a->gloc || a->gsz || a->gb1;
   if (d && (rec || sg)) return fail(MRPHY_ERR_ARG, "design: does not combine with record or per-spin gradients%s");
   if (d && (rc = check_design(a, d))) return rc;
   if (rec && (rc = check_record(a, true))) return rc;
@@ -2009,7 +2003,7 @@ int run_bwd(const mrphy_fused_args* a, const mrphy_readout_args* r, int wave_is_
   if ((!wave_is_packed || p.tc) && (rc = launch_pack<T>(a, p, st))) return rc;
   // finished-CTA counters of the design tail: behind the scheduling ints, zeroed by the backward kernel itself
   int* const done = d ? reinterpret_cast<int*>((T*)a->partials + (size_t)a->N * p.Pmax * p.W * (size_t)a->nT) + SCHED_CLAIM + p.Pmax : nullptr;
-  if ((rc = dispatch<T>(true, a, r, p, st, done))) return rc;
+  if ((rc = dispatch<T>(true, a, p, st, done))) return rc;
   if (sg && p.rows == 0) return MRPHY_OK;   // per-spin gradients only: nothing to finalize
   dim3 grid((a->nT + 31) / 32, p.W, a->N), block(32, 32);
   const int coil_dim = (a->flags & MRPHY_RF_COIL_DIM) ? 1 : 0;
@@ -2033,26 +2027,17 @@ int run_bwd(const mrphy_fused_args* a, const mrphy_readout_args* r, int wave_is_
 }  // namespace
 
 extern "C" int mrphy_blochsim_fused_fwd(const mrphy_fused_args* a, void* cuda_stream) {
-  return mrphy_blochsim_fused_readout_fwd(a, nullptr, cuda_stream);
+  g_launches = 0;
+  g_err[0] = 0;
+  if (!a) return fail(MRPHY_ERR_ARG, "null args%s");
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  return a->dtype == MRPHY_F64 ? run_fwd<double>(a, st) : run_fwd<float>(a, st);
 }
 
 extern "C" int mrphy_blochsim_fused_bwd(const mrphy_fused_args* a, int wave_is_packed, void* cuda_stream) {
-  return mrphy_blochsim_fused_readout_bwd(a, nullptr, wave_is_packed, cuda_stream);
-}
-
-extern "C" int mrphy_blochsim_fused_readout_fwd(const mrphy_fused_args* a, const mrphy_readout_args* r, void* cuda_stream) {
   g_launches = 0;
   g_err[0] = 0;
   if (!a) return fail(MRPHY_ERR_ARG, "null args%s");
   cudaStream_t st = (cudaStream_t)cuda_stream;
-  return a->dtype == MRPHY_F64 ? run_fwd<double>(a, r, st) : run_fwd<float>(a, r, st);
-}
-
-extern "C" int mrphy_blochsim_fused_readout_bwd(const mrphy_fused_args* a, const mrphy_readout_args* r, int wave_is_packed,
-                                                void* cuda_stream) {
-  g_launches = 0;
-  g_err[0] = 0;
-  if (!a) return fail(MRPHY_ERR_ARG, "null args%s");
-  cudaStream_t st = (cudaStream_t)cuda_stream;
-  return a->dtype == MRPHY_F64 ? run_bwd<double>(a, r, wave_is_packed, st) : run_bwd<float>(a, r, wave_is_packed, st);
+  return a->dtype == MRPHY_F64 ? run_bwd<double>(a, wave_is_packed, st) : run_bwd<float>(a, wave_is_packed, st);
 }

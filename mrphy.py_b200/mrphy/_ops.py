@@ -136,17 +136,22 @@ def _stream():
     return torch.cuda.current_stream().cuda_stream
 
 
-def _readout_args(rx: Optional[Tensor]) -> _cabi.ReadoutArgs:
-    """The receive map rx (N|1, nM, 2, nRx) with inner (2, nRx) contiguous, or None (c = 1, one receive coil)."""
-    r = _cabi.ReadoutArgs()
-    r.nRx = 1 if rx is None else rx.shape[3]
+def _fill_readout(a, nRx: int, rx: Optional[Tensor]):
+    """The readout fields: nRx receive coils, the map rx (N|1, nM, 2, nRx) with inner (2, nRx) contiguous, or None (c = 1)."""
+    a.nRx = nRx
     if rx is not None:
-        r.rx, r.rx_sn, r.rx_sm = rx.data_ptr(), _bstride(rx, 0), _bstride(rx, 1)
-    return r
+        assert rx.shape[3] == nRx, 'rx and nRx disagree on the receive coils'
+        a.rx, a.rx_sn, a.rx_sm = rx.data_ptr(), _bstride(rx, 0), _bstride(rx, 1)
 
 
-def _fused_fwd_call(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every, readout, rx):
-    """The fused forward; `readout` turns the recorded states into the signal (mrphy_blochsim_fused_readout_fwd)."""
+def _impl_blochsim_fused_fwd(Mi: Tensor, rf: Tensor, gr: Tensor, loc: Tensor, df: Optional[Tensor], b1: Optional[Tensor],
+                             T1: Optional[Tensor], T2: Optional[Tensor], gamma: Tensor, dt: Tensor, K: int, flags: int,
+                             every: int, nRx: int = 0, rx: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """-> (Mo (N,nM,3), out, ckpt, wave): final magnetisation, the option's output, K-step checkpoints, packed waveform.
+    - every > 0, nRx == 0: out = Mt (N, nR, 3, nM), nR = nT // every: the state after (r+1)*every steps, lab frame.
+    - nRx >= 1 (needs every > 0): out = S (N, 2, nR, nRx), the signal of those states summed over spins,
+      S[n, :, r, k] = sum_i rx[n, i, :, k] * (Mx + i My)[n, i] (complex product; rx None: 1, with nRx = 1).
+    - otherwise out is (0,)."""
     L = _cabi.lib()
     a = _cabi.FusedArgs()
     _fill_common(a, Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags)
@@ -157,40 +162,23 @@ def _fused_fwd_call(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every,
     a.Mo, a.ckpt, a.wave = Mo.data_ptr(), ckpt.data_ptr(), wave.data_ptr()
     if every:
         a.every, a.nR = every, a.nT // every
-    r = None
-    if readout:
-        r = _readout_args(rx)
-        out = torch.empty((a.N, 2, a.nR, r.nRx), **kw)
+    if nRx:
+        _fill_readout(a, nRx, rx)
+        out = torch.empty((a.N, 2, a.nR, nRx), **kw)
         with torch.cuda.device(Mi.device):        # the workspace is sized from THIS device's SM count
-            work = torch.empty(L.mrphy_fused_readout_elems(a, r), **kw)
-        r.S, r.work = out.data_ptr(), work.data_ptr()
+            work = torch.empty(L.mrphy_fused_readout_elems(a), **kw)
+        a.S, a.S_work = out.data_ptr(), work.data_ptr()
     else:
         out = torch.empty((a.N, a.nR, 3, a.nM) if every else (0,), **kw)
         if every:
             a.Mt = out.data_ptr()
     with torch.cuda.device(Mi.device):
-        _cabi.check(L.mrphy_blochsim_fused_readout_fwd(a, r, _stream()), 'blochsim_fused_fwd')
+        _cabi.check(L.mrphy_blochsim_fused_fwd(a, _stream()), 'blochsim_fused_fwd')
     _cabi.count_launches()
     return Mo, out, ckpt, wave
 
 
-def _impl_blochsim_fused_fwd(Mi: Tensor, rf: Tensor, gr: Tensor, loc: Tensor, df: Optional[Tensor], b1: Optional[Tensor],
-                       T1: Optional[Tensor], T2: Optional[Tensor], gamma: Tensor, dt: Tensor, K: int, flags: int,
-                       every: int) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
-    """-> (Mo (N,nM,3), Mt, ckpt, wave): final magnetisation, recorded states, K-step checkpoints, packed waveform.
-    every > 0 records Mt (N, nR, 3, nM), nR = nT // every: the state after (r+1)*every steps, lab frame; else Mt is (0,)."""
-    return _fused_fwd_call(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every, False, None)
-
-
-def _impl_blochsim_fused_readout_fwd(Mi: Tensor, rf: Tensor, gr: Tensor, loc: Tensor, df: Optional[Tensor],
-                                     b1: Optional[Tensor], T1: Optional[Tensor], T2: Optional[Tensor], gamma: Tensor, dt: Tensor,
-                                     K: int, flags: int, every: int, rx: Optional[Tensor]) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
-    """-> (Mo, S, ckpt, wave): as blochsim_fused_fwd with the signal S (N, 2, nR, nRx) in place of Mt,
-    S[n, :, r, k] = sum_i rx[n, i, :, k] * (Mx + i My)[n, i] after (r+1)*every steps (complex product; rx None: 1)."""
-    return _fused_fwd_call(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every, True, rx)
-
-
-def _fake_blochsim_fused_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every):
+def _fake_blochsim_fused_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every, nRx=0, rx=None):
     N, nM, nT = loc.shape[0], loc.shape[1], rf.shape[2]
     chunks = (nT + K - 1) // K
     nc = 1 if b1 is None else (rf.shape[3] if rf.ndim == 4 else 1)
@@ -200,19 +188,29 @@ def _fake_blochsim_fused_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flag
     chunk = WS * ((K + 3) // 4 * 4)
     if Mi.element_size() == 4 and NC >= 4 and K <= TC_K_MAX and os.environ.get('MRPHY_B200_TC', '1')[:1] != '0':
         chunk = max(chunk, ((K + 7) // 8 * 8) * (16 * (NC // 2) + 3))   # csrc: TcLayout (tensor-core operand tiles + gr rows)
-    return (Mi.new_empty((N, nM, 3)), Mi.new_empty((N, nT // every, 3, nM) if every else (0,)),
-            Mi.new_empty((max(N * (chunks - 1) * 3 * nM, 1),)), Mi.new_empty((N * chunks * chunk,)))
+    out = (N, 2, nT // every, nRx) if nRx else ((N, nT // every, 3, nM) if every else (0,))
+    return (Mi.new_empty((N, nM, 3)), Mi.new_empty(out), Mi.new_empty((max(N * (chunks - 1) * 3 * nM, 1),)),
+            Mi.new_empty((N * chunks * chunk,)))
 
 
-def _fake_blochsim_fused_readout_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every, rx):
-    Mo, _, ckpt, wave = _fake_blochsim_fused_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, 0)
-    return Mo, Mi.new_empty((loc.shape[0], 2, rf.shape[2] // every, 1 if rx is None else rx.shape[3])), ckpt, wave
-
-
-def _fused_bwd_call(gMo, gMt, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every, want_loc, want_sz,
-                    want_b1, rho, theta, rfmax, ts, smax, ddt, rf_kind, gr_kind, ro=None):
-    """The fused backward (mrphy_blochsim_fused_readout_bwd; ro = (gS, rx, want_rx) for a readout forward, else None)
-    -> (gMi, flat, gloc, gsz, gb1, grho, gtheta, gts, grx)."""
+def _impl_blochsim_fused_bwd(gMo: Tensor, gMt: Optional[Tensor], Mo: Tensor, ckpt: Tensor, wave: Tensor, rf: Tensor,
+                             gr: Tensor, loc: Tensor, df: Optional[Tensor], b1: Optional[Tensor], T1: Optional[Tensor],
+                             T2: Optional[Tensor], gamma: Tensor, dt: Tensor, K: int, flags: int, every: int, want_loc: bool,
+                             want_sz: bool, want_b1: bool, rho: Optional[Tensor], theta: Optional[Tensor],
+                             rfmax: Optional[Tensor], ts: Optional[Tensor], smax: Optional[Tensor], ddt: Optional[Tensor],
+                             rf_kind: int, gr_kind: int, nRx: int = 0, rx: Optional[Tensor] = None, want_rx: bool = False):
+    """-> (gMi (N,nM,3) or empty, flat, gloc, gsz, gb1, grho, gtheta, gts, grx); every output not asked for is (0,).
+    flat = [dL/drf like rf (absent with FLAG_SKIP_GRF) | dL/dgr (N,3,nT) (absent with FLAG_SKIP_GGR) | GRAD_TAIL spare
+    elements, zero]; `split_wave_grads` cuts the views.  Options:
+    - every > 0, nRx == 0: the backward of a recording forward; gMt = dL/dMt (N, nR, 3, nM) contiguous on top of dL/dMo.
+    - want_loc / want_sz / want_b1: the per-spin sums over time of dL/dBeff, formed inside the backward kernel without the
+      dense field: gloc (N,nM,3) = sum_t gr*gBz, gsz (N,nM) = sum_t gBz, gb1 (N,nM,2,nC) -- the outputs of
+      rfgr2beff_spin_grads.  want_b1 needs b1.
+    - rf_kind / gr_kind > 0: (dL/drho, dL/dtheta, dL/dts) of the re-parametrisation (rho, theta, rfmax) -> rf,
+      (ts, smax, ddt) -> gr, evaluated in the tail of the gradient epilogue: no launch of its own.  Combines with neither
+      of the others.
+    - nRx >= 1: the backward of a readout forward with the same every, nRx, rx; gMt = dL/dS (N, 2, nR, nRx) contiguous on
+      top of dL/dMo, and with want_rx grx = dL/drx (N, nM, 2, nRx).  Combines with the per-spin gradients."""
     L = _cabi.lib()
     a = _cabi.FusedArgs()
     _fill_common(a, None, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags)
@@ -236,11 +234,17 @@ def _fused_bwd_call(gMo, gMt, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma
     a.gMo, a.gMo_sn, a.gMo_sm = gMo.data_ptr(), _bstride(gMo, 0), _bstride(gMo, 1)
     a.gMi, a.grf, a.ggr, a.partials = (gMi.data_ptr() if need_gmi else None), (grf.data_ptr() if want_rf else None), \
         (ggr.data_ptr() if want_gr else None), partials.data_ptr()
-    gloc = gsz = gb1 = grho = gtheta = gts = flat[:0]
+    gloc = gsz = gb1 = grho = gtheta = gts = grx = flat[:0]
     if every:
         a.every, a.nR = every, a.nT // every
-        if gMt is not None:
-            a.gMt = gMt.data_ptr()
+    if nRx:
+        _fill_readout(a, nRx, rx)
+        a.gS = gMt.data_ptr()
+        if want_rx:
+            grx = torch.empty((a.N, a.nM, 2, nRx), **kw)
+            a.grx = grx.data_ptr()
+    elif every and gMt is not None:
+        a.gMt = gMt.data_ptr()
     if want_loc or want_sz or want_b1:
         e = lambda shape, on: torch.empty(shape if on else (0,), **kw)
         gloc, gsz, gb1 = e((a.N, a.nM, 3), want_loc), e((a.N, a.nM), want_sz), e((a.N, a.nM, 2, a.nC), want_b1)
@@ -256,66 +260,22 @@ def _fused_bwd_call(gMo, gMt, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma
             gts = torch.empty(ts.shape, **kw)
             d.gts = gts.data_ptr()
         a.design = ctypes.addressof(d)
-    r, grx = None, flat[:0]
-    if ro is not None:                        # (gS, rx, want_rx): the backward of a readout forward; gMt is None
-        gS, rx, want_rx = ro
-        r = _readout_args(rx)
-        r.gS = gS.data_ptr()
-        if want_rx:
-            grx = torch.empty((a.N, a.nM, 2, r.nRx), **kw)
-            r.grx = grx.data_ptr()
     with torch.cuda.device(Mo.device):
-        _cabi.check(L.mrphy_blochsim_fused_readout_bwd(a, r, 1, _stream()), 'blochsim_fused_bwd')
+        _cabi.check(L.mrphy_blochsim_fused_bwd(a, 1, _stream()), 'blochsim_fused_bwd')
     _cabi.count_launches()
     return gMi, flat, gloc, gsz, gb1, grho, gtheta, gts, grx
 
 
-def _impl_blochsim_fused_bwd(gMo: Tensor, gMt: Optional[Tensor], Mo: Tensor, ckpt: Tensor, wave: Tensor, rf: Tensor,
-                             gr: Tensor, loc: Tensor, df: Optional[Tensor], b1: Optional[Tensor], T1: Optional[Tensor],
-                             T2: Optional[Tensor], gamma: Tensor, dt: Tensor, K: int, flags: int, every: int, want_loc: bool,
-                             want_sz: bool, want_b1: bool, rho: Optional[Tensor], theta: Optional[Tensor],
-                             rfmax: Optional[Tensor], ts: Optional[Tensor], smax: Optional[Tensor], ddt: Optional[Tensor],
-                             rf_kind: int, gr_kind: int):
-    """-> (gMi (N,nM,3) or empty, flat, gloc, gsz, gb1, grho, gtheta, gts); every output not asked for is (0,).
-    flat = [dL/drf like rf (absent with FLAG_SKIP_GRF) | dL/dgr (N,3,nT) (absent with FLAG_SKIP_GGR) | GRAD_TAIL spare
-    elements, zero]; `split_wave_grads` cuts the views.  Options:
-    - every > 0: the backward of a recording forward; gMt = dL/dMt (N, nR, 3, nM) contiguous on top of dL/dMo.
-    - want_loc / want_sz / want_b1: the per-spin sums over time of dL/dBeff, formed inside the backward kernel without the
-      dense field: gloc (N,nM,3) = sum_t gr*gBz, gsz (N,nM) = sum_t gBz, gb1 (N,nM,2,nC) -- the outputs of
-      rfgr2beff_spin_grads.  want_b1 needs b1.
-    - rf_kind / gr_kind > 0: (dL/drho, dL/dtheta, dL/dts) of the re-parametrisation (rho, theta, rfmax) -> rf,
-      (ts, smax, ddt) -> gr, evaluated in the tail of the gradient epilogue: no launch of its own.  Combines with neither
-      of the others."""
-    return _fused_bwd_call(gMo, gMt, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every, want_loc, want_sz,
-                           want_b1, rho, theta, rfmax, ts, smax, ddt, rf_kind, gr_kind)[:8]
-
-
-def _impl_blochsim_fused_readout_bwd(gMo: Tensor, gS: Tensor, rx: Optional[Tensor], want_rx: bool, Mo: Tensor, ckpt: Tensor,
-                                     wave: Tensor, rf: Tensor, gr: Tensor, loc: Tensor, df: Optional[Tensor],
-                                     b1: Optional[Tensor], T1: Optional[Tensor], T2: Optional[Tensor], gamma: Tensor,
-                                     dt: Tensor, K: int, flags: int, every: int, want_loc: bool, want_sz: bool, want_b1: bool):
-    """The backward of a readout forward: gS = dL/dS (N, 2, nR, nRx) contiguous on top of dL/dMo -> (gMi, flat, gloc, gsz,
-    gb1, grx) as blochsim_fused_bwd, with grx = dL/drx (N, nM, 2, nRx) when want_rx, else (0,)."""
-    out = _fused_bwd_call(gMo, None, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every, want_loc,
-                          want_sz, want_b1, None, None, None, None, None, None, 0, 0, (gS, rx, want_rx))
-    return out[:5] + out[8:]
-
-
 def _fake_blochsim_fused_bwd(gMo, gMt, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every, want_loc,
-                             want_sz, want_b1, rho, theta, rfmax, ts, smax, ddt, rf_kind, gr_kind):
+                             want_sz, want_b1, rho, theta, rfmax, ts, smax, ddt, rf_kind, gr_kind, nRx=0, rx=None,
+                             want_rx=False):
     n = (0 if flags & _cabi.FLAG_SKIP_GRF else rf.numel()) + (0 if flags & _cabi.FLAG_SKIP_GGR else rf.shape[0] * 3 * rf.shape[2])
     N, nM, nC = loc.shape[0], loc.shape[1], (rf.shape[3] if rf.ndim == 4 else 1)
     e = lambda shape, on: Mo.new_empty(shape if on else (0,))
     return (e(Mo.shape, flags & _cabi.FLAG_NEED_GMI), Mo.new_empty((n + GRAD_TAIL,)), e((N, nM, 3), want_loc),
             e((N, nM), want_sz), e((N, nM, 2, nC), want_b1), e(rho.shape if rf_kind else (), rf_kind),
-            e(theta.shape if rf_kind else (), rf_kind), e(ts.shape if gr_kind else (), gr_kind))
-
-
-def _fake_blochsim_fused_readout_bwd(gMo, gS, rx, want_rx, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags,
-                                     every, want_loc, want_sz, want_b1):
-    out = _fake_blochsim_fused_bwd(gMo, None, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every,
-                                   want_loc, want_sz, want_b1, None, None, None, None, None, None, 0, 0)
-    return out[:5] + (Mo.new_empty((loc.shape[0], loc.shape[1], 2, 1 if rx is None else rx.shape[3]) if want_rx else (0,)),)
+            e(theta.shape if rf_kind else (), rf_kind), e(ts.shape if gr_kind else (), gr_kind),
+            e((N, nM, 2, nRx), nRx and want_rx))
 
 
 GRAD_TAIL = 4      # spare elements behind the waveform gradients (16-byte granule); [0] is where `parallel` puts the loss
@@ -330,31 +290,26 @@ def split_wave_grads(flat: Tensor, rf: Tensor, flags: int):
 
 
 def _fused_grads(ctx, want, gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, gMt=None, every=0,
-                 spin=(False, False, False), design=(None,) * 6 + (0, 0), readout=None):
+                 spin=(False, False, False), design=(None,) * 6 + (0, 0), readout=(0, None, False)):
     """The fused backward of a forward run with ctx.K, ctx.flags.  want = (dL/dMi, dL/drf, dL/dgr) wanted: the rows of the
-    spin reduction of the others are not even formed.  -> (gMi or None, grf, ggr, gloc, gsz, gb1, grho, gtheta, gts);
-    with readout = (rx, want_rx) gMt is dL/dS of a readout forward and the tail is (grx,) instead."""
+    spin reduction of the others are not even formed.  -> (gMi or None, grf, ggr, gloc, gsz, gb1, grho, gtheta, gts, grx);
+    with readout = (nRx, rx, want_rx), nRx >= 1, gMt is dL/dS of a readout forward."""
     if gMo is None:
         gMo = torch.zeros_like(Mo)
     if gMo.stride(-1) != 1 or gMo.dtype != Mo.dtype:
         gMo = gMo.to(Mo.dtype).contiguous()
     flags = ctx.flags | (_cabi.FLAG_NEED_GMI if want[0] else 0) | (0 if want[1] else _cabi.FLAG_SKIP_GRF) | \
         (0 if want[2] else _cabi.FLAG_SKIP_GGR)
-    if readout is not None:
-        gMi, flat, *rest = blochsim_fused_readout_bwd(gMo, gMt, *readout, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma,
-                                                      dt, ctx.K, flags, every, *spin)
-    else:
-        gMi, flat, *rest = blochsim_fused_bwd(gMo, gMt, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, ctx.K, flags,
-                                              every, *spin, *design)
+    gMi, flat, *rest = blochsim_fused_bwd(gMo, gMt, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, ctx.K, flags,
+                                          every, *spin, *design, *readout)
     return (gMi if want[0] else None, *split_wave_grads(flat, rf, flags), *rest)
 
 
 def _fused_setup(ctx, inputs, output):
-    """Both fused forwards: blochsim_fused_fwd, and blochsim_fused_readout_fwd with its receive map `rx` behind `every`."""
-    Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every, *ro = inputs
+    Mi, rf, gr, loc, df, b1, T1, T2, gamma, dt, K, flags, every, nRx, rx = inputs
     Mo, _Mt, ckpt, wave = output
-    ctx.K, ctx.flags, ctx.every, ctx.readout = K, flags, every, bool(ro)
-    opt = (df, b1, T1, T2, *ro)
+    ctx.K, ctx.flags, ctx.every, ctx.nRx = K, flags, every, nRx
+    opt = (df, b1, T1, T2, rx)
     ctx.has = [x is not None for x in opt]
     ctx.save_for_backward(Mo, ckpt, wave, rf, gr, loc, gamma, dt, *[x for x in opt if x is not None])
     if every:
@@ -380,13 +335,12 @@ def _fused_backward(ctx, gMo, gMt, _gckpt, _gwave):
     readout backward, with dL/dMo = 0 when the loss ignores M."""
     Mo, ckpt, wave, rf, gr, loc, gamma, dt, *opt = ctx.saved_tensors
     opt = list(opt)
-    df, b1, T1, T2, *ro = (opt.pop(0) if h else None for h in ctx.has)
-    need = ctx.needs_input_grad
+    df, b1, T1, T2, rx = (opt.pop(0) if h else None for h in ctx.has)
+    need = ctx.needs_input_grad           # (trailing inputs left at their defaults have no entry)
     # per-spin gradients (inputs loc, df, b1, gamma): γ reaches the loss only through Bz += df/γ, so without df it has none
     want_loc, want_b1 = bool(need[3]), bool(need[5] and b1 is not None)
     want_sz = df is not None and bool(need[4] or need[8])
-    rx = ro[0] if ro else None
-    want_rx = rx is not None and bool(need[13]) and gMt is not None
+    want_rx = rx is not None and bool(need[14]) and gMt is not None
     if not (any(need[0:3]) or want_loc or want_sz or want_b1 or want_rx):
         return (None,) * len(need)
     every = ctx.every if gMt is not None else 0
@@ -394,9 +348,10 @@ def _fused_backward(ctx, gMo, gMt, _gckpt, _gwave):
         # dL/dMt (dL/dS) in the kernel's layout (N, nR, 3, nM) ((N, 2, nR, nRx)) and dtype: a loss formed elementwise from the
         # view the caller got hands its gradient back in that layout already; anything else costs this one copy
         gMt = torch.empty(gMt.shape, dtype=Mo.dtype, device=Mo.device).copy_(gMt)
-    gMi, grf, ggr, gloc, gsz, gb1, *rest = _fused_grads(ctx, need[0:3], gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2,
-                                                        gamma, dt, gMt if every else None, every, (want_loc, want_sz, want_b1),
-                                                        readout=(rx, want_rx) if (ctx.readout and every) else None)
+    gMi, grf, ggr, gloc, gsz, gb1, *_, grx = _fused_grads(ctx, need[0:3], gMo, Mo, ckpt, wave, rf, gr, loc, df, b1, T1, T2,
+                                                          gamma, dt, gMt if every else None, every,
+                                                          (want_loc, want_sz, want_b1),
+                                                          readout=(ctx.nRx if every else 0, rx, want_rx))
     gdf = ggam = None
     if want_sz:     # ∂Δf = gsz/γ, ∂γ = -gsz·Δf/γ² (the chain rule of Bz += Δf/γ, beffective.py:142)
         gam2, df2 = _param_2d(gamma), _param_2d(df)
@@ -404,11 +359,8 @@ def _fused_backward(ctx, gMo, gMt, _gckpt, _gwave):
             gdf = _as_param_grad(gsz / gam2, df)
         if need[8]:
             ggam = _as_param_grad(-gsz * df2 / (gam2 * gam2), gamma)
-    grads = (gMi, grf, ggr, gloc if want_loc else None, gdf, gb1 if want_b1 else None, None, None, ggam, None, None, None,
-             None)
-    if not ctx.readout:
-        return grads
-    return grads + ((rest[0].sum_to_size(rx.shape) if want_rx else None),)
+    return (gMi, grf, ggr, gloc if want_loc else None, gdf, gb1 if want_b1 else None, None, None, ggam, None, None, None,
+            None, None, grx.sum_to_size(rx.shape) if want_rx else None)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -848,7 +800,7 @@ def _mask_backward(ctx, g):
 # registration: raw torch.library definitions (schema + CUDA impl + fake), which cost ~20 us per call instead of
 # the ~130 us of the `torch.library.custom_op` convenience wrapper -- it matters for test-scale problems
 _LIB = torch.library.Library('mrphy_b200', 'DEF')
-_SCHEMAS = {'blochsim_fused_fwd': '(Tensor Mi, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, int every) -> (Tensor, Tensor, Tensor, Tensor)', 'blochsim_fused_bwd': '(Tensor gMo, Tensor? gMt, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, int every, bool want_loc, bool want_sz, bool want_b1, Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? ddt, int rf_kind, int gr_kind) -> (Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor)', 'blochsim_fused_readout_fwd': '(Tensor Mi, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, int every, Tensor? rx) -> (Tensor, Tensor, Tensor, Tensor)', 'blochsim_fused_readout_bwd': '(Tensor gMo, Tensor gS, Tensor? rx, bool want_rx, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, int every, bool want_loc, bool want_sz, bool want_b1) -> (Tensor, Tensor, Tensor, Tensor, Tensor, Tensor)', 'blochsim_beff_fwd': '(Tensor Mi, Tensor Beff, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'blochsim_beff_bwd': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor Beff, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'rfgr2beff': '(Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor gamma) -> Tensor', 'rfgr2beff_bwd': '(Tensor gB, Tensor rf, Tensor gr, Tensor loc, Tensor? b1) -> (Tensor, Tensor)', 'rfgr2beff_spin_grads': '(Tensor gB, Tensor rf, Tensor gr, bool want_loc, bool want_b1) -> (Tensor, Tensor, Tensor)', 'beff2ab': '(Tensor beff, Tensor E1, Tensor E2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor, Tensor)', 'beff2ab_bwd': '(Tensor gA, Tensor gB, Tensor A, Tensor B, Tensor ckpt, Tensor beff, Tensor E1, Tensor E2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'beff2uphi': '(Tensor beff, Tensor g) -> (Tensor, Tensor)', 'beff2uphi_bwd': '(Tensor? gU, Tensor? gPhi, Tensor beff, Tensor g) -> (Tensor, Tensor)', 'freeprec': '(Tensor Mi, Tensor dur, Tensor? T1, Tensor? T2, Tensor? df, bool adjoint) -> Tensor', 'design_waveform': '(Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? dt, int rf_kind, int gr_kind) -> (Tensor, Tensor)', 'design_waveform_bwd': '(Tensor? grf, Tensor? ggr, Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? dt, int rf_kind, int gr_kind) -> (Tensor, Tensor, Tensor)', 'mask_copy': '(Tensor v, Tensor idx, Tensor inv, bool fill_zero) -> Tensor', 'clamp_waveform': '(Tensor x, Tensor lim, float eps, int kind) -> Tensor', 'clamp_waveform_bwd': '(Tensor g, Tensor x, Tensor lim, float eps, int kind) -> Tensor'}
+_SCHEMAS = {'blochsim_fused_fwd': '(Tensor Mi, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, int every, int nRx=0, Tensor? rx=None) -> (Tensor, Tensor, Tensor, Tensor)', 'blochsim_fused_bwd': '(Tensor gMo, Tensor? gMt, Tensor Mo, Tensor ckpt, Tensor wave, Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags, int every, bool want_loc, bool want_sz, bool want_b1, Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? ddt, int rf_kind, int gr_kind, int nRx=0, Tensor? rx=None, bool want_rx=False) -> (Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor)', 'blochsim_beff_fwd': '(Tensor Mi, Tensor Beff, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'blochsim_beff_bwd': '(Tensor gMo, Tensor Mo, Tensor ckpt, Tensor Beff, Tensor? T1, Tensor? T2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'rfgr2beff': '(Tensor rf, Tensor gr, Tensor loc, Tensor? df, Tensor? b1, Tensor gamma) -> Tensor', 'rfgr2beff_bwd': '(Tensor gB, Tensor rf, Tensor gr, Tensor loc, Tensor? b1) -> (Tensor, Tensor)', 'rfgr2beff_spin_grads': '(Tensor gB, Tensor rf, Tensor gr, bool want_loc, bool want_b1) -> (Tensor, Tensor, Tensor)', 'beff2ab': '(Tensor beff, Tensor E1, Tensor E2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor, Tensor)', 'beff2ab_bwd': '(Tensor gA, Tensor gB, Tensor A, Tensor B, Tensor ckpt, Tensor beff, Tensor E1, Tensor E2, Tensor gamma, Tensor dt, int K, int flags) -> (Tensor, Tensor)', 'beff2uphi': '(Tensor beff, Tensor g) -> (Tensor, Tensor)', 'beff2uphi_bwd': '(Tensor? gU, Tensor? gPhi, Tensor beff, Tensor g) -> (Tensor, Tensor)', 'freeprec': '(Tensor Mi, Tensor dur, Tensor? T1, Tensor? T2, Tensor? df, bool adjoint) -> Tensor', 'design_waveform': '(Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? dt, int rf_kind, int gr_kind) -> (Tensor, Tensor)', 'design_waveform_bwd': '(Tensor? grf, Tensor? ggr, Tensor? rho, Tensor? theta, Tensor? rfmax, Tensor? ts, Tensor? smax, Tensor? dt, int rf_kind, int gr_kind) -> (Tensor, Tensor, Tensor)', 'mask_copy': '(Tensor v, Tensor idx, Tensor inv, bool fill_zero) -> Tensor', 'clamp_waveform': '(Tensor x, Tensor lim, float eps, int kind) -> Tensor', 'clamp_waveform_bwd': '(Tensor g, Tensor x, Tensor lim, float eps, int kind) -> Tensor'}
 
 
 def _register(name, impl, fake):
@@ -860,10 +812,6 @@ def _register(name, impl, fake):
 
 blochsim_fused_fwd = _register('blochsim_fused_fwd', _impl_blochsim_fused_fwd, _fake_blochsim_fused_fwd)
 blochsim_fused_bwd = _register('blochsim_fused_bwd', _impl_blochsim_fused_bwd, _fake_blochsim_fused_bwd)
-blochsim_fused_readout_fwd = _register('blochsim_fused_readout_fwd', _impl_blochsim_fused_readout_fwd,
-                                       _fake_blochsim_fused_readout_fwd)
-blochsim_fused_readout_bwd = _register('blochsim_fused_readout_bwd', _impl_blochsim_fused_readout_bwd,
-                                       _fake_blochsim_fused_readout_bwd)
 blochsim_beff_fwd = _register('blochsim_beff_fwd', _impl_blochsim_beff_fwd, _fake_blochsim_beff_fwd)
 blochsim_beff_bwd = _register('blochsim_beff_bwd', _impl_blochsim_beff_bwd, _fake_blochsim_beff_bwd)
 rfgr2beff_cuda = _register('rfgr2beff', _impl_rfgr2beff, _fake_rfgr2beff)
@@ -880,8 +828,6 @@ mask_copy_cuda = _register('mask_copy', _impl_mask_copy, _fake_mask_copy)
 clamp_waveform_cuda = _register('clamp_waveform', _impl_clamp_waveform, lambda x, lim, eps, kind: x.new_empty(x.shape))
 clamp_waveform_bwd_cuda = _register('clamp_waveform_bwd', _impl_clamp_waveform_bwd, lambda g, x, lim, eps, kind: x.new_empty(x.shape))
 torch.library.register_autograd('mrphy_b200::blochsim_fused_fwd', _fused_backward, setup_context=_fused_setup, lib=_LIB)
-torch.library.register_autograd('mrphy_b200::blochsim_fused_readout_fwd', _fused_backward, setup_context=_fused_setup,
-                                lib=_LIB)
 torch.library.register_autograd('mrphy_b200::design_waveform', _design_backward, setup_context=_design_setup, lib=_LIB)
 torch.library.register_autograd('mrphy_b200::mask_copy', _mask_backward, setup_context=_mask_setup, lib=_LIB)
 torch.library.register_autograd('mrphy_b200::clamp_waveform', _clamp_backward, setup_context=_clamp_setup, lib=_LIB)
@@ -950,7 +896,7 @@ class _FusedDesignApply(torch.autograd.Function):
             return (None,) * 20
         design = (rho if rk else None, theta if rk else None, rfmax if rk else None, ts if gk else None,
                   smax if gk else None, ddt if gk else None, rk, gk)
-        gMi, grf, ggr, *_, grho, gtheta, gts = _fused_grads(ctx, (need[0], need[1] or rk, need[2] or gk), gMo, Mo, ckpt,
+        gMi, grf, ggr, *_, grho, gtheta, gts, _ = _fused_grads(ctx, (need[0], need[1] or rk, need[2] or gk), gMo, Mo, ckpt,
                                                             wave, rf, gr, loc, df, b1, T1, T2, gamma, dt, design=design)
         return (gMi, grf if need[1] else None, ggr if need[2] else None,
                 grho if (rk and need[3]) else None, gtheta if (rk and need[4]) else None, gts if gk else None) + (None,) * 14
@@ -1166,7 +1112,8 @@ def fused_applypulse(M_: Tensor, rf: Tensor, gr: Tensor, loc_: Tensor, *, Δf_: 
             assert rx.ndim == 4 and rx.shape[0] in (1, N) and rx.shape[1] in (1, nM) and rx.shape[2] == 2, \
                 f'rxMap_ of shape {tuple(rxMap_.shape)} is not (N|1, nM|1, 2[, nRx])'
             rx = _inner_contig(rx.expand(N, nM, 2, rx.shape[3]), 2)   # broadcasts stay stride 0: no copy
-        Mo, S, _, _ = blochsim_fused_readout_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gam, dtt, K, fl, readout, rx)
+        Mo, S, _, _ = blochsim_fused_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gam, dtt, K, fl, readout,
+                                         1 if rx is None else rx.shape[3], rx)
         return Mo, (S if coil_dim else S[..., 0])
     Mo, Mt, _, _ = blochsim_fused_fwd(Mi, rf, gr, loc, df, b1, T1, T2, gam, dtt, K, fl, record or 0)
     return Mo if record is None else (Mo, Mt.permute(0, 3, 1, 2))

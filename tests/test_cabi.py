@@ -35,13 +35,14 @@ def test_header_symbols_exported(cabi):
     assert set(names) == set(cabi.EXPORTS), 'python binding and header disagree'
 
 
-def test_abi_version_and_arg_struct_sizes(cabi):
+def test_abi_version_and_struct_sizes_match_mirrors(cabi):
     L = cabi.lib()
     assert L.mrphy_abi_version() == cabi.ABI_VERSION
     # struct sizes must match the C definition (all 8-byte aligned fields)
     assert ctypes.sizeof(cabi.Param) == 32
     assert ctypes.sizeof(cabi.FusedArgs) == 8 * 4 + 8 * 3 + 8 * 5 + 8 * 4 + 8 * 3 + 8 * 3 + 32 * 5 + 8 * 3 + 8 * 3 + 8 * 4 + \
-        4 * 2 + 8 * 2 + 8 * 3 + 8                    # options: record, per-spin gradients, design tail
+        4 * 2 + 8 * 2 + 8 * 3 + 8 + \
+        4 * 2 + 8 * 3 + 8 * 4                        # options: record, per-spin gradients, design tail, readout
     assert ctypes.sizeof(cabi.BeffArgs) == 6 * 4 + 8 * 3 + 8 * 4 + 32 * 4 + 8 * 2 + 8 * 3 + 8 * 2
     # ... and the C side agrees with every ctypes mirror (the loader checks the same and refuses a mismatch)
     for which, cls in enumerate((cabi.Param, cabi.FusedArgs, cabi.BeffArgs, cabi.RfGr2BeffArgs, cabi.Beff2abArgs,

@@ -344,7 +344,7 @@ def test_graph_capture_readout(dev):
 
 
 @pytest.mark.gpu
-def test_scale_memory(dev):
+def test_readout_scale_memory(dev):
     """128³ spins x 2000 steps, fp32, s = 1: peak memory at most the step without readout + S + the readout workspace +
     256 MB (the record route would need 2 x 50 GB).  The receive map is zero except on 256 seeded spins, so the full-size
     run's S -- every CTA summing many tiles into its slot -- is those spins' signal, checked against the oracle."""
@@ -376,10 +376,8 @@ def test_scale_memory(dev):
         del out
         rf.grad = gr.grad = None
     a = _cabi.FusedArgs()
-    a.dtype, a.N, a.nM, a.nT, a.nC, a.K, a.every, a.nR = _cabi.MRPHY_F32, 1, nM, nT, 1, 128, s, nT // s
-    r = _cabi.ReadoutArgs()
-    r.nRx = 1
-    work = _cabi.lib().mrphy_fused_readout_elems(a, r) * 4
+    a.dtype, a.N, a.nM, a.nT, a.nC, a.K, a.every, a.nR, a.nRx = _cabi.MRPHY_F32, 1, nM, nT, 1, 128, s, nT // s, 1
+    work = _cabi.lib().mrphy_fused_readout_elems(a) * 4
     assert peaks[1] <= peaks[0] + 2 * nT * 4 + work + 256 * 2 ** 20, (peaks, work)
     c = lambda x: x.detach()[:, sub].cpu().double()
     from oracle import bloch_oracle as orc
@@ -398,18 +396,23 @@ def test_scale_memory(dev):
 
 
 # ---------------------------------------------------------------------------------------------------------- host only
-def test_readout_args_mirror_matches_library():
+def test_readout_fields_mirror_matches_library():
+    """The readout fields close mrphy_fused_args, behind the design tail; no struct or entry point of their own."""
     from mrphy import _cabi
     L = _cabi.lib()
-    R = _cabi.ReadoutArgs
-    assert L.mrphy_sizeof_args(10) == ctypes.sizeof(R) == 4 * 2 + 8 * 3 + 8 * 4
-    assert L.mrphy_abi_version() == _cabi.ABI_VERSION == 7
-    assert {'mrphy_blochsim_fused_readout_fwd', 'mrphy_blochsim_fused_readout_bwd', 'mrphy_fused_readout_elems'} <= \
-        set(_cabi.EXPORTS)
+    F, P = _cabi.FusedArgs, ctypes.sizeof(ctypes.c_void_p)
+    assert L.mrphy_sizeof_args(1) == ctypes.sizeof(F) == F.S_work.offset + P
+    assert (F.nRx.offset, F.rx.offset) == (F.design.offset + P, F.design.offset + P + 8)
+    assert (F.rx_sn.offset, F.rx_sm.offset) == (F.rx.offset + P, F.rx.offset + P + 8)
+    assert (F.S.offset, F.gS.offset, F.grx.offset, F.S_work.offset) == tuple(F.rx_sm.offset + 8 + k * P for k in range(4))
+    assert L.mrphy_sizeof_args(10) == 0
+    assert L.mrphy_abi_version() == _cabi.ABI_VERSION == 8
+    assert {'mrphy_blochsim_fused_fwd', 'mrphy_blochsim_fused_bwd', 'mrphy_fused_readout_elems'} <= set(_cabi.EXPORTS)
+    assert not {f'mrphy_blochsim_fused_readout_{d}' for d in ('fwd', 'bwd')} & set(_cabi.EXPORTS)   # the former pair
 
 
 def _refusable_args():
-    """FusedArgs and ReadoutArgs whose checks all pass up to the readout's; the pointers are never dereferenced."""
+    """FusedArgs whose checks all pass up to the readout's; the pointers are never dereferenced."""
     from mrphy import _cabi
     a = _cabi.FusedArgs()
     a.dtype, a.N, a.nM, a.nT, a.nC, a.K = _cabi.MRPHY_F32, 1, 4, 10, 1, 8
@@ -417,17 +420,16 @@ def _refusable_args():
         setattr(a, p, 256)
     a.gamma.ptr = a.dt.ptr = 256
     a.every, a.nR = 3, 3
-    r = _cabi.ReadoutArgs()
-    r.nRx, r.S, r.gS, r.work = 2, 256, 256, 256
-    return a, r
+    a.nRx, a.S, a.gS, a.S_work = 2, 256, 256, 256
+    return a
 
 
 @pytest.mark.parametrize('bad', ['Mt', 'gMt', 'design', 'nRx0', 'nRx17', 'S', 'work', 'gS', 'every0', 'every11', 'nR'])
-def test_readout_entry_points_refuse(bad):
+def test_fused_entry_points_refuse_bad_readout(bad):
     """Every refusal is MRPHY_ERR_ARG with nothing launched."""
     from mrphy import _cabi
     L = _cabi.lib()
-    a, r = _refusable_args()
+    a = _refusable_args()
     bwd = bad in ('gMt', 'design', 'gS')
     d = _cabi.ReparamArgs()
     if bad in ('Mt', 'gMt'):
@@ -437,48 +439,48 @@ def test_readout_entry_points_refuse(bad):
         d.rho = d.theta = d.rfmax = d.grho = d.gtheta = 256
         a.design = ctypes.addressof(d)
     elif bad.startswith('nRx'):
-        r.nRx = int(bad[3:])
+        a.nRx = int(bad[3:])                 # nRx0: S, gS, S_work stay set, so the readout is on and refused
     elif bad in ('S', 'work', 'gS'):
-        setattr(r, bad, None)
+        setattr(a, 'S_work' if bad == 'work' else bad, None)
     elif bad.startswith('every'):
         a.every = int(bad[5:])
     else:
         a.nR = 2
     for b in ((False, True) if bad.startswith(('nRx', 'every', 'nR', 'Mt')) else (bwd,)):
-        rc = L.mrphy_blochsim_fused_readout_bwd(a, r, 1, None) if b else L.mrphy_blochsim_fused_readout_fwd(a, r, None)
+        rc = L.mrphy_blochsim_fused_bwd(a, 1, None) if b else L.mrphy_blochsim_fused_fwd(a, None)
         assert rc == -1, (bad, b, rc)
         assert L.mrphy_last_launch_count() == 0
         assert 'readout' in L.mrphy_last_error().decode()
 
 
-def test_readout_elems_sizing():
+def test_readout_elems_sizing_from_fused_args():
     from mrphy import _cabi
     L = _cabi.lib()
-    a, r = _refusable_args()
-    a.nM, a.nT, a.every, a.nR, r.nRx = 1000, 100, 7, 14, 3
+    a = _refusable_args()
+    a.nM, a.nT, a.every, a.nR, a.nRx = 1000, 100, 7, 14, 3
     # ceil(1000 / 128) = 8 CTAs per batch entry at most, one slot [nR][2 nRx] each
-    assert L.mrphy_fused_readout_elems(a, r) == 8 * 14 * 6
-    r.nRx = 17
-    assert L.mrphy_fused_readout_elems(a, r) == 0
+    assert L.mrphy_fused_readout_elems(a) == 8 * 14 * 6
+    a.nRx = 17
+    assert L.mrphy_fused_readout_elems(a) == 0
 
 
 @pytest.mark.parametrize('nRx', [0, 1, 8])
-def test_readout_fakes_allocate_implementation_shapes(nRx):
+def test_fused_fakes_allocate_readout_shapes(nRx):
     from mrphy import _cabi, _ops
     N, nM, nT, every, nC = 2, 37, 50, 7, 2
     e = lambda *s: torch.empty(s, device='meta')
     rf, b1 = e(N, 2, nT, nC), e(N, nM, 2, nC)
     rx = e(N, nM, 2, nRx) if nRx else None
     args = (e(N, nM, 3), rf, e(N, 3, nT), e(N, nM, 3), e(N, nM), b1, None, None, e(1, 1), e(1), 16, 0)
-    Mo, S, ckpt, wave = _ops._fake_blochsim_fused_readout_fwd(*args, every, rx)
+    Mo, S, ckpt, wave = _ops._fake_blochsim_fused_fwd(*args, every, max(nRx, 1), rx)
     ref = _ops._fake_blochsim_fused_fwd(*args, 0)
     assert Mo.shape == (N, nM, 3) and S.shape == (N, 2, nT // every, max(nRx, 1))
     assert ckpt.shape == ref[2].shape and wave.shape == ref[3].shape
     for want_rx in (False, True):
-        out = _ops._fake_blochsim_fused_readout_bwd(Mo, S, rx, want_rx, Mo, ckpt, wave, rf, e(N, 3, nT), e(N, nM, 3),
-                                                    e(N, nM), b1, None, None, e(1, 1), e(1), 16, _cabi.FLAG_NEED_GMI, every,
-                                                    True, True, True)
-        gMi, flat, gloc, gsz, gb1, grx = out
+        out = _ops._fake_blochsim_fused_bwd(Mo, S, Mo, ckpt, wave, rf, e(N, 3, nT), e(N, nM, 3), e(N, nM), b1, None, None,
+                                            e(1, 1), e(1), 16, _cabi.FLAG_NEED_GMI, every, True, True, True, *(None,) * 6, 0,
+                                            0, max(nRx, 1), rx, want_rx)
+        gMi, flat, gloc, gsz, gb1, *_, grx = out
         assert gMi.shape == (N, nM, 3) and flat.shape == (rf.numel() + N * 3 * nT + _ops.GRAD_TAIL,)
         assert gloc.shape == (N, nM, 3) and gsz.shape == (N, nM) and gb1.shape == (N, nM, 2, nC)
         assert grx.shape == ((N, nM, 2, max(nRx, 1)) if want_rx else (0,))

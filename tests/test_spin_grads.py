@@ -778,13 +778,13 @@ def test_spin_grads_shard_spins(dev, dtype):
 
 
 # ---- no GPU needed ----------------------------------------------------------------------------------------------------
-def test_spin_grad_fields_mirror_matches_library():
+def test_spin_grad_fields_keep_their_offsets():
     from mrphy import _cabi
     L = _cabi.lib()
     F, P = _cabi.FusedArgs, ctypes.sizeof(ctypes.c_void_p)
     assert L.mrphy_sizeof_args(1) == ctypes.sizeof(F)
     assert (F.gloc.offset, F.gsz.offset, F.gb1.offset) == (F.gMt.offset + P, F.gMt.offset + 2 * P, F.gMt.offset + 3 * P)
-    assert L.mrphy_abi_version() == _cabi.ABI_VERSION == 7
+    assert L.mrphy_abi_version() == _cabi.ABI_VERSION == 8
     assert 'mrphy_blochsim_fused_bwd' in _cabi.EXPORTS
 
 
